@@ -2,7 +2,7 @@
 """Benchmark of the densification hot path (BASELINE.json metric: depth pixels fused per second and
 HBM GB/s as a fraction of the roofline).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference] [--dump-outputs DIR]
 
 A step is one pass of the whole device pipeline (align -> [neighbour-depth exchange] -> back-project +
 consistency vote -> voxel fusion [-> voxel all-to-all]) over one synthetic scene.  Rank 0 prints ONE
@@ -46,10 +46,56 @@ WORKLOADS = {
 VOXEL = 0.01
 METRIC = "depth_pixels_fused_per_s"
 UNIT = "pixels/s"
+# --dump-outputs: rows of the fixed, seeded samples (split over the ranks); 56 MB of .npy files in all
+DUMP_PIXELS = 1 << 20
+DUMP_VOXELS = 1 << 19
 
 
 def env_int(name, default):
     return int(os.environ.get(name, default))
+
+
+def _sample(n: int, m: int, seed: int) -> np.ndarray:
+    """Sorted indices of a fixed, seeded sample of m of n rows (all rows when n <= m)."""
+    if n <= m:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).choice(n, m, replace=False))
+
+
+def dump_outputs(res, out_dir: str, rank: int, world: int) -> None:
+    """Write what one step returned to its caller as float32 / float64 .npy files, so that two builds run with the
+    same arguments can be compared output for output: the per-view alignment statistics and the fused counts whole,
+    the refined depth, world points and votes at a seeded sample of pixels, and the voxels at a seeded sample of the
+    fused ones.  Integer outputs are stored as float64 (exact); a 64-bit voxel key as its high and low 32 bits."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    sfx = "" if world == 1 else f".rank{rank}"
+
+    def save(name, a):
+        np.save(d / f"{name}{sfx}.npy", a)
+
+    def take(t, idx):
+        return t[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+
+    st = res.stats.cpu().numpy()  # [V,8] ddn_view_stats: status, correspondences, outliers, table rows, 3 floats, reserved
+    save("view_stats", np.concatenate([st[:, :4].astype(np.float64), st.view(np.float32)[:, 4:7].astype(np.float64)], 1))
+    idx = _sample(res.refined.numel(), DUMP_PIXELS // world, seed=1)
+    save("pixel_index", idx.astype(np.float64))
+    save("refined_depth", take(res.refined.reshape(-1), idx))
+    idx = _sample(res.votes.numel(), DUMP_PIXELS // world, seed=1)
+    save("xyz", take(res.xyz.reshape(-1, 3), idx))
+    save("votes", take(res.votes.reshape(-1), idx).astype(np.float32))
+    if res.counts is None or res.voxel_keys is None:
+        return
+    counts = res.counts.cpu().numpy()
+    save("counts", counts.astype(np.float64))
+    idx = _sample(int(counts[1]), DUMP_VOXELS // world, seed=2)
+    save("voxel_index", idx.astype(np.float64))
+    keys = take(res.voxel_keys, idx).view(np.uint64)
+    save("voxel_keys_hi_lo", np.stack([keys >> np.uint64(32), keys & np.uint64(0xFFFFFFFF)], 1).astype(np.float64))
+    save("voxel_xyz", take(res.voxel_xyz, idx))
+    save("voxel_rgb", take(res.voxel_rgb, idx).astype(np.float32))
+    save("voxel_count", take(res.voxel_count, idx).astype(np.float64))
 
 
 # ----------------------------------------------------------------------------------------------
@@ -208,8 +254,9 @@ class Ctx:
 
 def run_workload(ctx: Ctx, workload: str, scaling: str, steps: int, warmup: int, e2e: bool, sample_mode: str = "nearest",
                  pixel_layout: int = 0, clocks: bool = True, profile_kernels: bool = False, dedup_sparse: bool = False,
-                 overlap_align: bool = True) -> dict:
-    """Device-resident timing (+ optionally the end-to-end host path) of one workload on all ranks."""
+                 overlap_align: bool = True, dump_dir: str | None = None) -> dict:
+    """Device-resident timing (+ optionally the end-to-end host path) of one workload on all ranks; ``dump_dir``: write
+    the last timed step's outputs there (dump_outputs)."""
     from depthdensifier_b200 import _lib, ops
     from depthdensifier_b200.distributed import ShardedDensifier
     from depthdensifier_b200.engine import DensifyConfig
@@ -261,6 +308,8 @@ def run_workload(ctx: Ctx, workload: str, scaling: str, steps: int, warmup: int,
     launches = _lib.launch_count() - launches0
     clk = sampler.stop(t_wall0, t_wall1) if clocks else None
     res.check()
+    if dump_dir is not None:
+        dump_outputs(res, dump_dir, rank, world)
     ms_step = ctx.allreduce(ev0.elapsed_time(ev1) / steps, "max")
     stage_ms = {}
     for evs in stage_events:
@@ -339,7 +388,7 @@ def run_workload(ctx: Ctx, workload: str, scaling: str, steps: int, warmup: int,
                 sharded.collect_host(prev)
             ctx.barrier()
             t0 = time.perf_counter()
-            e_steps = max(3, min(steps, 6))
+            e_steps = steps
             if pipelined:
                 # the public two-call form for a stream of scenes: scene i+1 is submitted before scene i is collected, so
                 # its upload overlaps the kernels and the download of its predecessor; every step's inputs go up and
@@ -400,7 +449,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the extra strong-scaling block (cfg3)")
     ap.add_argument("--no-check", action="store_true", help="skip the multi-GPU equivalence check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.warmup < 3:
         args.warmup = max(args.warmup, 1) if args.workload == "small" else 3
     if args.impl == "reference":
@@ -451,7 +505,7 @@ def main():
     overlap = world > 1 and not args.no_overlap_align
     main_run = run_workload(ctx, args.workload, args.scaling, args.steps, args.warmup, e2e=not args.no_e2e,
                             sample_mode=args.sample_mode, pixel_layout=args.pixel_layout, dedup_sparse=args.dedup_sparse,
-                            overlap_align=overlap,
+                            overlap_align=overlap, dump_dir=args.dump_outputs,
                             profile_kernels=args.workload != "cfg2")
     K, H, W = main_run["K"], main_run["H"], main_run["W"]
     n_valid_local, k4_local_ms = main_run["n_valid_local"], main_run["k4_local_ms"]
@@ -491,7 +545,7 @@ def main():
     # ---- strong scaling block: cfg3 (200 views at 1920x1080, K=8) split over the ranks, at every N ----
     strong = None
     if not args.no_strong and args.workload == "cfg2" and args.scaling == "weak":
-        sr = run_workload(ctx, "cfg3", "strong", steps=max(5, min(args.steps, 10)), warmup=3, e2e=False, clocks=False,
+        sr = run_workload(ctx, "cfg3", "strong", steps=args.steps, warmup=3, e2e=False, clocks=False,
                           profile_kernels=True, overlap_align=overlap)
         strong = {"workload": "cfg3", "scaling": "strong", "ms_per_step": sr["ms_per_step"], "value": sr["value"], "unit": UNIT,
                   "steps": sr["steps"], "stages_ms": sr["stages_ms"], "stage4_kernels_ms": sr.get("stage4_kernels_ms"),

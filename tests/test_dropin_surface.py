@@ -1,109 +1,73 @@
-"""The drop-in surface: names, parameter lists and defaults of the reference's entry points are kept
-(compared against the reference's own modules where /root/reference exists), and the tyro CLI renders the same
-flags."""
+"""The drop-in surface: names, parameter lists and defaults of the reference's entry points are kept (compared
+against the reference's surface, recorded in tests/golden/ref_surface.json by oracle/make_golden.py), and the tyro
+CLI renders the same flags."""
 
-import dataclasses
-import inspect
+import json
 import subprocess
 import sys
 
 import pytest
 
-from oracle.run_reference import REFERENCE_ROOT, reference_available
-
-needs_ref = pytest.mark.skipif(not reference_available(), reason="/root/reference not present")
+from oracle.make_golden import _defaults, _params, batch_output_dir
 
 
-def _fields(dc):
-    return {f.name: (f.default if f.default is not dataclasses.MISSING else None) for f in dataclasses.fields(dc)}
+@pytest.fixture(scope="module")
+def ref(golden_dir):
+    return json.loads((golden_dir / "ref_surface.json").read_text())
 
 
-def _params(fn):
-    return [p for p in inspect.signature(fn).parameters if p != "self"]
-
-
-@needs_ref
-def test_depth_refiner_surface_matches_reference():
+def test_depth_refiner_surface_matches_reference(ref):
     from depthdensifier_b200 import DepthRefiner, RefinerConfig
-    from oracle.run_reference import import_reference_refiner
 
-    ref = import_reference_refiner()
-    assert _fields(RefinerConfig) == _fields(ref.RefinerConfig)
-    mine, theirs = _params(DepthRefiner.__init__), _params(ref.DepthRefiner.__init__)
+    assert _defaults(RefinerConfig) == ref["RefinerConfig"]
+    mine, theirs = _params(DepthRefiner.__init__), ref["DepthRefiner.__init__"]
     assert mine[: len(theirs)] == theirs  # extras (align_mode, subsample_seed, device) are keyword-only additions
-    assert _params(DepthRefiner.refine_depth)[:6] == _params(ref.DepthRefiner.refine_depth)[:6]
+    assert _params(DepthRefiner.refine_depth)[:6] == ref["DepthRefiner.refine_depth"]
 
 
-@needs_ref
-def test_script_config_tree_matches_reference():
+def test_script_config_tree_matches_reference(ref):
     from depthdensifier_b200 import pipeline as P
-    from oracle.run_reference import _import_reference_script
 
-    ref = _import_reference_script()
     for name in ("PathsConfig", "MoGeConfig", "ProcessingConfig", "FilteringConfig"):
-        mine, theirs = _fields(getattr(P, name)), _fields(getattr(ref, name))
+        mine, theirs = _defaults(getattr(P, name)), ref[name]
         assert {k: mine[k] for k in theirs} == theirs, name  # every reference field, same default
-    assert set(_fields(ref.ScriptConfig)) <= set(_fields(P.ScriptConfig))
-    assert _params(P.project_points) == _params(ref.project_points)
-    assert _params(P.unproject_points) == _params(ref.unproject_points)
-    assert _params(P.main)[0] == _params(ref.main)[0] == "config"
+    assert set(ref["ScriptConfig"]) <= set(_defaults(P.ScriptConfig))
+    assert _params(P.project_points) == ref["project_points"]
+    assert _params(P.unproject_points) == ref["unproject_points"]
+    assert _params(P.main)[:1] == ref["main"] == ["config"]
 
 
-@needs_ref
-def test_fast_pchip_surface_matches_reference():
+def test_fast_pchip_surface_matches_reference(ref):
     from depthdensifier_b200 import fast_pchip_refiner as mine
-    from oracle.run_reference import import_reference_pchip
 
-    ref = import_reference_pchip()
-    assert _fields(mine.FastPCHIPRefinerConfig) == _fields(ref.FastPCHIPRefinerConfig)
-    theirs = _params(ref.FastPCHIPRefiner.__init__)
+    assert _defaults(mine.FastPCHIPRefinerConfig) == ref["FastPCHIPRefinerConfig"]
+    theirs = ref["FastPCHIPRefiner.__init__"]
     assert _params(mine.FastPCHIPRefiner.__init__)[: len(theirs)] == theirs
-    assert _params(mine.FastPCHIPRefiner.refine_depth) == _params(ref.FastPCHIPRefiner.refine_depth)
-    assert _params(mine.refine_depth_from_colmap) == _params(ref.refine_depth_from_colmap)
+    assert _params(mine.FastPCHIPRefiner.refine_depth) == ref["FastPCHIPRefiner.refine_depth"]
+    assert _params(mine.refine_depth_from_colmap) == ref["refine_depth_from_colmap"]
 
 
-@needs_ref
-def test_gradient_mask_signature_matches_reference():
-    import importlib.util
+def test_gradient_mask_signature_matches_reference(ref):
+    import inspect
 
     from depthdensifier_b200.edge_masks import compute_depth_normal_gradient_mask
 
-    spec = importlib.util.spec_from_file_location("ddn_ref_init_sig", REFERENCE_ROOT / "src" / "depthdensifier" / "initilizer.py")
-    init = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(init)
-    a, b = inspect.signature(compute_depth_normal_gradient_mask), inspect.signature(init.compute_depth_normal_gradient_mask)
-    assert [(p.name, p.default) for p in a.parameters.values()] == [(p.name, p.default) for p in b.parameters.values()]
+    a = inspect.signature(compute_depth_normal_gradient_mask)
+    assert [[p.name, repr(p.default)] for p in a.parameters.values()] == ref["compute_depth_normal_gradient_mask"]
 
 
-@needs_ref
-def test_batch_config_matches_reference(tmp_path, monkeypatch):
+def test_batch_config_matches_reference(ref, tmp_path):
     """scripts/run_batch.py: same BatchConfig fields (root_dir and output_dir required, the ScriptConfig embedded as
     `config`), and each scan's model goes to <output_dir>/<scan>/sparse/0 (scripts/run_batch.py:63-65)."""
-    import importlib.util
-    import sys
-    from pathlib import Path
+    import dataclasses
 
     from depthdensifier_b200 import run_batch as mine
-    from oracle.run_reference import _import_reference_script
 
-    _import_reference_script()  # installs the stand-ins and makes `test` importable the way run_batch.py imports it
-    sys.modules["test"] = sys.modules["ddn_reference_script"]
-    spec = importlib.util.spec_from_file_location("ddn_ref_run_batch", REFERENCE_ROOT / "scripts" / "run_batch.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    theirs = [(f.name, f.default is dataclasses.MISSING and f.default_factory is dataclasses.MISSING) for f in dataclasses.fields(ref.BatchConfig)]
+    theirs = [tuple(f) for f in ref["BatchConfig"]]
     ours = [(f.name, f.default is dataclasses.MISSING and f.default_factory is dataclasses.MISSING) for f in dataclasses.fields(mine.BatchConfig)]
     assert ours[: len(theirs)] == theirs  # root_dir (required), output_dir (required), config; additions follow
-    # output layout: run both mains over a root with one complete scan, densification itself stubbed out
-    (tmp_path / "root" / "scan_a" / "sparse" / "0").mkdir(parents=True)
-    (tmp_path / "root" / "scan_a" / "images").mkdir()
-    (tmp_path / "root" / "incomplete").mkdir()
-    seen = {}
-    monkeypatch.setattr(ref, "densify_main", lambda cfg: seen.setdefault("ref", Path(cfg.paths.output_model_dir)))
-    monkeypatch.setattr(mine, "densify_main", lambda cfg: seen.setdefault("mine", Path(cfg.paths.output_model_dir)))
-    ref.main(ref.BatchConfig(root_dir=tmp_path / "root", output_dir=tmp_path / "out"))
-    mine.main(mine.BatchConfig(root_dir=tmp_path / "root", output_dir=tmp_path / "out"))
-    assert seen["mine"] == seen["ref"] == tmp_path / "out" / "scan_a" / "sparse" / "0"
+    # output layout: main over a root with one complete scan, densification itself stubbed out
+    assert batch_output_dir(mine, tmp_path) == ref["batch_output_model_dir"] == "scan_a/sparse/0"
 
 
 def test_package_exports():

@@ -1,17 +1,12 @@
-"""Pins the oracle (oracle/restatement.py) to the reference: bit-identical to the reference's own
-code where /root/reference exists, and to the committed golden vectors everywhere."""
-
-import contextlib
-import io
+"""Pins the oracle (oracle/restatement.py) to the reference: bit-identical to the reference's own outputs, stored
+as golden vectors by oracle/make_golden.py."""
 
 import numpy as np
-import pytest
 
 from depthdensifier_b200.hashperm import hash_perm
 from depthdensifier_b200.neighbours import all_views_table
-from depthdensifier_b200.synthetic import SceneConfig, make_scene
 from oracle import restatement as R
-from oracle.run_reference import reference_available, run_reference_main, run_reference_refiner
+from oracle.make_golden import REFINER_FALLBACKS
 
 
 def _densify_from_npz(g, **kw):
@@ -32,8 +27,7 @@ def test_golden_main_allviews(golden_dir):
     assert np.array_equal(out["votes"], g["ref_votes"].astype(np.int64))
     assert np.array_equal(out["keep"], g["ref_keep"])
     assert np.array_equal(out["counts_per_view"], g["ref_counts_per_view"])
-    assert np.array_equal(out["points"][out["keep"]], g["ref_kept_points"])
-    assert np.array_equal(out["colors"][out["keep"]], g["ref_kept_colors"])
+    # the reference's kept cloud is its points and colours at `keep` (make_golden.py checks that when it records the file)
     assert 0 < (~out["keep"]).sum() < len(out["keep"])  # the filter does real work on this scene
 
 
@@ -74,37 +68,26 @@ def test_golden_refiner_cases(golden_dir):
     assert int(g["too_few/0/removed"]) == -1  # early-return dict has no outliers_removed key
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
-def test_restatement_equals_unmodified_reference_main():
-    sc = make_scene(SceneConfig(n_views=5, width=112, height=80, n_sparse=600, seed=11))
-    with contextlib.redirect_stdout(io.StringIO()), contextlib.redirect_stderr(io.StringIO()):
-        ref = run_reference_main(sc, vote_threshold=3, depth_threshold=0.8, randperm=lambda n: hash_perm(n, 5))
-    out = R.densify(
-        sc.mono_depth.numpy(), sc.normal.numpy(), sc.mask.numpy(), sc.rgb.numpy(), sc.sparse_xyz.numpy(),
-        sc.sparse_offsets.numpy(), sc.cam_from_world.numpy(), sc.intrinsics.numpy(), all_views_table(5), 3,
-        depth_threshold=0.8, randperm=lambda n: hash_perm(n, 5),
-    )
-    assert np.array_equal(out["refined"], ref["refined"])
-    assert np.array_equal(out["points"], ref["points"])
-    assert np.array_equal(out["colors"], ref["colors"])
-    assert np.array_equal(out["votes"], ref["votes"])
-    assert np.array_equal(out["keep"], ref["keep"])
+def test_restatement_equals_unmodified_reference_main(golden_dir):
+    g = np.load(golden_dir / "ref_main_seed11.npz")
+    out = _densify_from_npz(g, randperm=lambda n: hash_perm(n, 5))
+    assert np.array_equal(out["refined"], g["ref_refined"])
+    assert np.array_equal(out["points"], g["ref_points"])
+    assert np.array_equal(out["colors"], g["ref_colors"])
+    assert np.array_equal(out["votes"], g["ref_votes"].astype(np.int64))
+    assert np.array_equal(out["keep"], g["ref_keep"])
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
-def test_restatement_equals_reference_refiner_stride_and_fallbacks():
-    sc = make_scene(SceneConfig(n_views=2, width=96, height=64, n_sparse=300, seed=5))
-    a = sc
-    for kw in (dict(), dict(skip_smoothing=True), dict(min_correspondences=10_000), dict(edge_margin=40)):
+def test_restatement_equals_reference_refiner_stride_and_fallbacks(golden_dir):
+    g = np.load(golden_dir / "ref_refiner_fallbacks.npz")
+    for name, kw in REFINER_FALLBACKS.items():
         for v in range(2):
-            lo, hi = int(a.sparse_offsets[v]), int(a.sparse_offsets[v + 1])
-            args = (a.mono_depth[v].numpy().copy(), a.sparse_xyz[lo:hi].numpy(), a.cam_from_world[v].numpy(),
-                    R.kmatrix(a.intrinsics[v].numpy()), a.mask[v].numpy())
-            ref = run_reference_refiner(*args, adaptive_correspondences=False, **kw)
-            cfg = R.AlignConfig(adaptive_correspondences=False, **kw)
-            mine = R.refine_view(*args, cfg)
-            assert np.array_equal(np.asarray(ref["refined_depth"]), np.asarray(mine["refined_depth"]))
-            assert {k: ref[k] for k in ref if k != "refined_depth"} == {k: mine[k] for k in mine if k != "refined_depth"}
+            lo, hi = int(g["sparse_offsets"][v]), int(g["sparse_offsets"][v + 1])
+            args = (g["mono_depth"][v].copy(), g["sparse_xyz"][lo:hi], g["cam_from_world"][v], R.kmatrix(g["intrinsics"][v]), g["mask"][v])
+            mine = R.refine_view(*args, R.AlignConfig(adaptive_correspondences=False, **kw))
+            ref = {k.rsplit("/", 1)[1]: g[k] for k in g.files if k.startswith(f"{name}/{v}/")}
+            assert np.array_equal(ref.pop("refined_depth"), np.asarray(mine["refined_depth"])), (name, v)
+            assert {k: val.item() for k, val in ref.items()} == {k: mine[k] for k in mine if k != "refined_depth"}, (name, v)
 
 
 def test_explicit_bilinear_matches_grid_sample():

@@ -1,13 +1,12 @@
 """The FastPCHIP restatement (oracle/restatement_pchip.py) against the reference's own outputs: the committed
 golden cases (tests/golden/ref_pchip_cases.npz, produced by oracle/make_golden.py from the unmodified
-reference) and, where /root/reference exists, the reference module itself."""
+reference module)."""
 
 import numpy as np
 import pytest
 
 from oracle import restatement_pchip as P
 from oracle.restatement import kmatrix
-from oracle.run_reference import reference_available
 
 CASES = {
     "default": dict(kw={}, mask=True, rgb=False, normal=True),
@@ -42,14 +41,10 @@ def test_restatement_matches_golden(golden_dir, name):
         assert float(g[f"{name}/0/scale"]) != 1.0
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present")
 def test_restatement_matches_reference_module(golden_dir):
-    from oracle.run_reference import run_reference_pchip
-
+    """The restatement's output as it is returned (no cast), against the reference module's output."""
     g = np.load(golden_dir / "ref_pchip_cases.npz")
     for name in ("default", "image_edges"):
         args, kw = case_args(g, name, 1)
-        ref = run_reference_pchip(args["depth_map"], args["normal_map"], args["points3D"], args["cam_from_world"], args["K"],
-                                  args["mask"], rgb_image=args["rgb_image"], **kw)
         mine = P.refine_depth(cfg=P.PchipConfig(**kw), **args)
-        assert np.array_equal(ref["refined_depth"], mine["refined_depth"]) and ref["scale"] == mine["scale"]
+        assert np.array_equal(g[f"{name}/1/refined"], mine["refined_depth"]) and float(g[f"{name}/1/scale"]) == mine["scale"]
