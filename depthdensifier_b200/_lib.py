@@ -83,6 +83,7 @@ class FuseSession(C.Structure):
 GRID_OK, GRID_EMPTY, GRID_TOO_LARGE, GRID_TOO_MANY_BITS = 0, 1, 2, 3
 MAX_PEERS = 16
 PAIR_TABLE_FLOATS = 24
+LAYOUT_COLS = 8  # DDN_LAYOUT_COLS
 RECORD_WORDS = 6  # DDN_RECORD_WORDS
 
 # every symbol include/ddn_b200.h declares: name -> (restype, argtypes)
@@ -108,6 +109,15 @@ SYMBOLS = {
          C.POINTER(FuseSession), _vp],
     ),
     "ddn_bbox_init": (C.c_int, [_vp, _vp]),
+    "ddn_align_views_ragged": (
+        C.c_int,
+        [C.POINTER(AlignConfig), _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp],
+    ),
+    "ddn_build_pair_tables_ragged": (C.c_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "ddn_backproject_filter_ragged": (
+        C.c_int,
+        [C.POINTER(FilterConfig), _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, C.POINTER(FuseSession), _vp],
+    ),
     "ddn_pchip_workspace_bytes": (C.c_int, [_i64, _i64, C.POINTER(_i64)]),
     "ddn_pchip_edge_mask": (
         C.c_int,

@@ -170,11 +170,13 @@ __device__ double block_sum(double v, double* s_red) {
 }
 
 // ---- K1+K2 ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kStatsThreads, 1)
-align_stats_kernel(ddn_align_config cfg, int H, int W, const float* __restrict__ depth,
-                   const double* __restrict__ poses, const double* __restrict__ kmat,
-                   const double* __restrict__ sparse_xyz, const int64_t* __restrict__ offsets,
-                   AlignWorkspace ws, ddn_view_stats* __restrict__ stats, int sort_in_smem, int pairs_in_smem) {
+// kRagged (ddn_align_views_ragged): the view's H, W and map offset come from the layout.
+template <bool kRagged>
+__device__ __forceinline__ void align_stats_body(const ddn_align_config& cfg, int H, int W, const float* __restrict__ depth,
+                                                 const double* __restrict__ poses, const double* __restrict__ kmat,
+                                                 const double* __restrict__ sparse_xyz, const int64_t* __restrict__ offsets,
+                                                 const AlignWorkspace& ws, ddn_view_stats* __restrict__ stats, int sort_in_smem,
+                                                 int pairs_in_smem, const int64_t* __restrict__ layout) {
   extern __shared__ __align__(16) unsigned long long s_sort[];
   __shared__ int s_warp[33];
   __shared__ double s_red[32];
@@ -182,6 +184,7 @@ align_stats_kernel(ddn_align_config cfg, int H, int W, const float* __restrict__
 
   const int v = blockIdx.x;
   const int tid = threadIdx.x;
+  if (kRagged) H = (int)layout[(size_t)v * DDN_LAYOUT_COLS], W = (int)layout[(size_t)v * DDN_LAYOUT_COLS + 1];
   const int64_t lo = offsets[v];
   const int n_sparse = (int)(offsets[v + 1] - lo);
   // The pair arrays of a view (sampled depth, COLMAP depth, ratio, table x / y) live in shared memory next to the
@@ -196,7 +199,7 @@ align_stats_kernel(ddn_align_config cfg, int H, int W, const float* __restrict__
   float* tx = pairs_in_smem ? s_pairs + 3 * ws.C : gtx;
   float* ty = pairs_in_smem ? s_pairs + 4 * ws.C : gty;
   unsigned long long* sortbuf = sort_in_smem ? s_sort : ws.sortbuf + (size_t)v * ws.Cp;
-  const float* __restrict__ dmap = depth + (size_t)v * H * W;
+  const float* __restrict__ dmap = kRagged ? depth + layout[(size_t)v * DDN_LAYOUT_COLS + 2] : depth + (size_t)v * H * W;
 
   ddn_view_stats st;
   st.status = DDN_VIEW_REFINED;
@@ -427,6 +430,22 @@ align_stats_kernel(ddn_align_config cfg, int H, int W, const float* __restrict__
   }
 }
 
+__global__ void __launch_bounds__(kStatsThreads, 1)
+align_stats_kernel(ddn_align_config cfg, int H, int W, const float* __restrict__ depth,
+                   const double* __restrict__ poses, const double* __restrict__ kmat,
+                   const double* __restrict__ sparse_xyz, const int64_t* __restrict__ offsets,
+                   AlignWorkspace ws, ddn_view_stats* __restrict__ stats, int sort_in_smem, int pairs_in_smem) {
+  align_stats_body<false>(cfg, H, W, depth, poses, kmat, sparse_xyz, offsets, ws, stats, sort_in_smem, pairs_in_smem, nullptr);
+}
+
+__global__ void __launch_bounds__(kStatsThreads, 1)
+align_stats_ragged_kernel(ddn_align_config cfg, const int64_t* __restrict__ layout, const float* __restrict__ depth,
+                          const double* __restrict__ poses, const double* __restrict__ kmat,
+                          const double* __restrict__ sparse_xyz, const int64_t* __restrict__ offsets,
+                          AlignWorkspace ws, ddn_view_stats* __restrict__ stats, int sort_in_smem, int pairs_in_smem) {
+  align_stats_body<true>(cfg, 0, 0, depth, poses, kmat, sparse_xyz, offsets, ws, stats, sort_in_smem, pairs_in_smem, layout);
+}
+
 // ---- K3 ---------------------------------------------------------------------------------------------
 // One CTA = a 128 x 32 pixel tile (+1 replicate halo) of one view.  Phase 1 remaps tile + halo into
 // shared memory (lookup table and its bucket index also in shared memory); phase 2 takes the 3x3 median
@@ -434,6 +453,7 @@ align_stats_kernel(ddn_align_config cfg, int H, int W, const float* __restrict__
 // three windows that contain them (median9 = med3(max of the minima, med3 of the middles, min of the
 // maxima)), 3 LDS and ~20 min/max per pixel instead of 9 LDS and 38.
 constexpr int kTileW = 126, kTileH = 32, kRemapThreads = 256;
+static_assert(kTileW == kRemapTileW && kTileH == kRemapTileH, "the ragged layout counts tiles of kRemapTileW x kRemapTileH");
 constexpr int kHaloW = kTileW + 2, kHaloH = kTileH + 2;
 constexpr int kLutSmemMax = 4096;  // knots kept in shared memory (32 KB); larger tables read global
 
@@ -527,12 +547,16 @@ __device__ __forceinline__ void tile_bbox_epilogue(int* __restrict__ bbox, const
 constexpr int kTmaBoxW = 132;                                // 128 halo columns + up to 3 columns of alignment slack, x4 B = 528 B
 constexpr int kTmaGuard = 160;                               // floats in front of the box (>= one row + 1; 640 B keeps 128-B alignment)
 constexpr int kTmaFloats = kTmaGuard + kHaloH * kTmaBoxW;    // 18,592 B
-template <bool kPacked, bool kBox, bool kTma>
+// kRagged (ddn_align_views_ragged, byte mask, no TMA; layout = the device layout, nullptr otherwise): blockIdx.x runs
+// over the tiles of all views; a CTA finds its view from the layout's tile prefix (tiles_y = the number of views) and
+// takes H, W, tiles_x and the map offset from there.
+template <bool kPacked, bool kBox, bool kTma, bool kRagged>
 __global__ void __launch_bounds__(kRemapThreads, DDN_K3_MINB)
 remap_median_kernel(ddn_align_config cfg, int H, int W, int tiles_x, int tiles_y, const float* __restrict__ depth,
                     const uint8_t* __restrict__ mask, const ddn_view_stats* __restrict__ stats, AlignWorkspace ws,
                     float* __restrict__ refined, int lut_cap, const float* __restrict__ src_table, int* __restrict__ bbox,
-                    const CUtensorMap* __restrict__ depth_map) {
+                    const CUtensorMap* __restrict__ depth_map, const int64_t* __restrict__ layout) {
+  static_assert(!kRagged || (!kPacked && !kTma), "the ragged remap reads a byte mask with plain loads");
   extern __shared__ __align__(16) float s_dyn[];  // LUT xs | ys | bucket index (when the table fits)
   __shared__ __align__(128) float s_buf[kTma ? kTmaFloats : kHaloH * kHaloW];
   __shared__ __align__(8) unsigned long long s_bar;  // mbarrier of the TMA load (kTma)
@@ -549,16 +573,19 @@ remap_median_kernel(ddn_align_config cfg, int H, int W, int tiles_x, int tiles_y
   if (threadIdx.x == 0) s_dmin = 0x7f800000, s_dmax = 0;
 
   const int tid = threadIdx.x;
-  const int tile = blockIdx.x;
-  const int v = blockIdx.y;
+  const int vr = kRagged ? layout_view_of(layout, tiles_y, 4, blockIdx.x) : 0;  // ragged: the view of this tile
+  const int64_t* __restrict__ L = layout + (size_t)vr * DDN_LAYOUT_COLS;
+  if (kRagged) H = (int)L[0], W = (int)L[1], tiles_x = (W + kTileW - 1) / kTileW;
+  const int tile = kRagged ? (int)(blockIdx.x - L[4]) : blockIdx.x;
+  const int v = kRagged ? vr : blockIdx.y;
   const int ty0 = (tile / tiles_x) * kTileH, tx0 = (tile % tiles_x) * kTileW;
   const size_t HW = (size_t)H * W;
-  const float* __restrict__ dmap = depth + (size_t)v * HW;
+  const float* __restrict__ dmap = kRagged ? depth + L[2] : depth + (size_t)v * HW;
   // mask: one byte per pixel, or (cfg.mask_packed) one BIT per pixel - bit (g & 7) of byte g >> 3 of the view's
   // ceil(H W / 8) bytes: an eighth of the upload for the host path
-  const uint8_t* __restrict__ mmap = mask ? mask + (size_t)v * (kPacked ? (HW + 7) / 8 : HW) : nullptr;
+  const uint8_t* __restrict__ mmap = mask ? (kRagged ? mask + L[2] : mask + (size_t)v * (kPacked ? (HW + 7) / 8 : HW)) : nullptr;
   auto mask_at = [&](size_t g) -> bool { return kPacked ? ((__ldg(mmap + (g >> 3)) >> (g & 7)) & 1) != 0 : __ldg(mmap + g) != 0; };
-  float* __restrict__ out = refined + (size_t)v * HW;
+  float* __restrict__ out = kRagged ? refined + L[2] : refined + (size_t)v * HW;
   const ddn_view_stats st = stats[v];
 
   if (st.status != DDN_VIEW_REFINED) {
@@ -788,19 +815,19 @@ int ddn_align_views(const ddn_align_config* cfg, int64_t n_views, int64_t height
 #define DDN_LAUNCH_REMAP(P, B)                                                                                              \
   do {                                                                                                                      \
     if (tma) {                                                                                                              \
-      DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<P, B, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+      DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<P, B, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                               (int)smem_lut),                                                               \
                          "cudaFuncSetAttribute(remap_median)"));                                                            \
-      remap_median_kernel<P, B, true><<<grid, kRemapThreads, smem_lut, st>>>(                                               \
+      remap_median_kernel<P, B, true, false><<<grid, kRemapThreads, smem_lut, st>>>(                                               \
           *cfg, (int)height, (int)width, tiles_x, tiles_y, depth, mask, stats, ws, refined, (int)lut, src_table,            \
-          reinterpret_cast<int*>(bbox), depth_map_dev);                                                                     \
+          reinterpret_cast<int*>(bbox), depth_map_dev, nullptr);                                                            \
     } else {                                                                                                                \
-      DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<P, B, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+      DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<P, B, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                               (int)smem_lut),                                                               \
                          "cudaFuncSetAttribute(remap_median)"));                                                            \
-      remap_median_kernel<P, B, false><<<grid, kRemapThreads, smem_lut, st>>>(                                              \
+      remap_median_kernel<P, B, false, false><<<grid, kRemapThreads, smem_lut, st>>>(                                              \
           *cfg, (int)height, (int)width, tiles_x, tiles_y, depth, mask, stats, ws, refined, (int)lut, src_table,            \
-          reinterpret_cast<int*>(bbox), depth_map_dev);                                                                     \
+          reinterpret_cast<int*>(bbox), depth_map_dev, nullptr);                                                            \
     }                                                                                                                       \
   } while (0)
   const bool packed = cfg->mask_packed != 0 && mask != nullptr, box = bbox != nullptr;
@@ -809,6 +836,60 @@ int ddn_align_views(const ddn_align_config* cfg, int64_t n_views, int64_t height
   else if (box) DDN_LAUNCH_REMAP(false, true);
   else DDN_LAUNCH_REMAP(false, false);
 #undef DDN_LAUNCH_REMAP
+  return after_launch("remap_median_kernel", st);
+}
+
+int ddn_align_views_ragged(const ddn_align_config* cfg, int64_t n_views, const int64_t* layout, const int64_t* layout_host,
+                           const float* depth, const uint8_t* mask, const double* cam_from_world, const double* kmat,
+                           const double* sparse_xyz, const int64_t* sparse_offsets, int64_t max_sparse_per_view, float* refined,
+                           ddn_view_stats* stats, void* workspace, int64_t workspace_bytes, const float* src_table, float* bbox,
+                           void* stream) {
+  using namespace ddn;
+  DDN_REQUIRE(cfg != nullptr, "null config");
+  if (cfg->mask_packed || cfg->use_tma) {
+    set_error("ddn_align_views_ragged: mask_packed and use_tma are options of the uniform ddn_align_views only");
+    return DDN_ERR_UNSUPPORTED;
+  }
+  DDN_REQUIRE((src_table == nullptr) == (bbox == nullptr), "src_table and bbox go together");
+  DDN_REQUIRE(layout != nullptr, "null layout");
+  DDN_TRY(check_layout(n_views, layout_host));
+  for (int64_t v = 0; v < n_views; ++v)
+    DDN_REQUIRE(layout_host[v * DDN_LAYOUT_COLS] > 1 && layout_host[v * DDN_LAYOUT_COLS + 1] > 1, "every view needs H, W >= 2");
+  DDN_REQUIRE(cfg->mode == 0 || cfg->mode == 1, "mode");
+  DDN_REQUIRE(cfg->max_pairs >= 1, "max_pairs");
+  DDN_REQUIRE(depth && cam_from_world && kmat && sparse_offsets && refined && stats && workspace, "null pointer");
+  const int64_t C = max_sparse_per_view > 0 ? max_sparse_per_view : 1;
+  DDN_REQUIRE(C < (1ll << 30), "max_sparse_per_view");
+  if (workspace_bytes < align_ws_bytes(n_views, C)) {
+    set_error("align workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)align_ws_bytes(n_views, C));
+    return DDN_ERR_WORKSPACE_TOO_SMALL;
+  }
+  AlignWorkspace ws = carve(workspace, n_views, C);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int in_smem = ws.Cp <= kSortSmemMax ? 1 : 0;
+  const int pairs_smem = (in_smem && (size_t)ws.Cp * 8 + (size_t)ws.C * 20 <= 200 * 1024) ? 1 : 0;
+  const size_t smem_sort = (in_smem ? (size_t)ws.Cp * 8 : 0) + (pairs_smem ? (size_t)ws.C * 20 : 0);
+  DDN_TRY(check_cuda(cudaFuncSetAttribute(align_stats_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sort),
+                     "cudaFuncSetAttribute(align_stats_ragged)"));
+  align_stats_ragged_kernel<<<(unsigned)n_views, kStatsThreads, smem_sort, st>>>(*cfg, layout, depth, cam_from_world, kmat, sparse_xyz,
+                                                                                sparse_offsets, ws, stats, in_smem, pairs_smem);
+  DDN_TRY(after_launch("align_stats_ragged_kernel", st));
+  int64_t lut = (cfg->adaptive_correspondences && cfg->max_pairs < C) ? cfg->max_pairs : C;
+  if (cfg->mode != 0 || lut > kLutSmemMax) lut = 0;
+  const size_t smem_lut = lut > 0 ? (size_t)lut * 8 + (size_t)kBuckets * 4 : 0;
+  const unsigned tiles = (unsigned)layout_host[n_views * DDN_LAYOUT_COLS + 4];
+#define DDN_LAUNCH_REMAP_RAGGED(B)                                                                                               \
+  do {                                                                                                                           \
+    DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<false, B, false, true>,                                      \
+                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lut),                         \
+                       "cudaFuncSetAttribute(remap_median)"));                                                                   \
+    remap_median_kernel<false, B, false, true><<<tiles, kRemapThreads, smem_lut, st>>>(                                          \
+        *cfg, 0, 0, 1, (int)n_views, depth, mask, stats, ws, refined, (int)lut, src_table, reinterpret_cast<int*>(bbox), nullptr, \
+        layout);                                                                                                                 \
+  } while (0)
+  if (bbox != nullptr) DDN_LAUNCH_REMAP_RAGGED(true);
+  else DDN_LAUNCH_REMAP_RAGGED(false);
+#undef DDN_LAUNCH_REMAP_RAGGED
   return after_launch("remap_median_kernel", st);
 }
 

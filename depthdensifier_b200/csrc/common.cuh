@@ -51,8 +51,51 @@ inline int after_launch(const char* name, cudaStream_t st) {
   } while (0)
 
 constexpr int kNumSMs = 148;  // B200
+// Work units of the ragged layout: the remap kernel's 126 x 32 pixel tile (align.cu) and the consistency kernel's
+// points per CTA (filter.cu, kFilterChunk).
+constexpr int kRemapTileW = 126, kRemapTileH = 32, kFilterChunkPoints = 1024;
 
 inline int64_t align_up(int64_t x, int64_t a) { return (x + a - 1) / a * a; }
+
+// Host-side validation of a ragged view layout (include/ddn_b200.h, DDN_LAYOUT_COLS) before anything is launched:
+// the offsets and work-unit prefixes must be the prefix sums of the sizes, so no layout can send a kernel outside its
+// buffers.
+inline int check_layout(int64_t n_views, const int64_t* L) {
+  DDN_REQUIRE(L != nullptr, "null layout_host");
+  DDN_REQUIRE(n_views >= 1 && n_views <= 65535, "a ragged layout holds 1 to 65535 views");
+  const int64_t* last = L + n_views * DDN_LAYOUT_COLS;
+  const int64_t s = last[0];
+  DDN_REQUIRE(s >= 1 && last[1] == n_views, "layout: the last row must hold the stride and the view count");
+  int64_t pix = 0, grid = 0, tiles = 0, chunks = 0;
+  for (int64_t v = 0; v < n_views; ++v) {
+    const int64_t* r = L + v * DDN_LAYOUT_COLS;
+    const int64_t h = r[0], w = r[1];
+    DDN_REQUIRE(h >= 1 && w >= 1 && h < (1 << 22) && w < (1 << 22) && h * w < (1ll << 31),
+                "layout: every side must be 1 .. 2^22 - 1 and every view below 2^31 pixels");
+    DDN_REQUIRE(r[2] == pix && r[3] == grid && r[4] == tiles && r[5] == chunks,
+                "layout: the offsets are not the prefix sums of the view sizes");
+    const int64_t hs = (h + s - 1) / s, ws = (w + s - 1) / s;
+    pix += h * w;
+    grid += hs * ws;
+    tiles += ((h + kRemapTileH - 1) / kRemapTileH) * ((w + kRemapTileW - 1) / kRemapTileW);
+    chunks += (hs * ws + kFilterChunkPoints - 1) / kFilterChunkPoints;
+  }
+  DDN_REQUIRE(last[2] == pix && last[3] == grid && last[4] == tiles && last[5] == chunks,
+              "layout: the totals are not the sums of the view sizes");
+  DDN_REQUIRE(pix < (1ll << 32), "the views must hold fewer than 2^32 pixels in all (32-bit gather offsets)");
+  return DDN_OK;
+}
+
+// View of a flat work unit (remap tile or consistency chunk): the last v with layout[v][col] <= unit.  CTA-uniform.
+__device__ __forceinline__ int layout_view_of(const int64_t* __restrict__ layout, int n_views, int col, int64_t unit) {
+  int lo = 0, hi = n_views - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(layout + (size_t)mid * DDN_LAYOUT_COLS + col) <= unit) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
 
 // Order-preserving float <-> int encoding for atomicMin/atomicMax on floats.
 __device__ __forceinline__ int float_to_ordered(float f) {

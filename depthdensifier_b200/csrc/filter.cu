@@ -32,6 +32,7 @@ constexpr int kFilterThreads = 256;
 #endif
 constexpr int kFilterPX = DDN_K4_PX;  // pixels per thread
 constexpr int kFilterChunk = kFilterThreads * kFilterPX;
+static_assert(kFilterChunk == kFilterChunkPoints, "the ragged layout counts chunks of kFilterChunkPoints points");
 
 // ------------------------------------------------------------------------------------------------
 // Table set-up (float64, one thread per (source view, neighbour))
@@ -44,11 +45,13 @@ constexpr int kFilterChunk = kFilterThreads * kFilterPX;
 //   reference-parity table K = V lists it); entry 0 carries n_hot and n_own in floats 22, 23 (int bits).  K4's hot loop therefore runs over n_hot entries without any validity test.
 // src_table[s][16]: rows of R_s^T Kinv_s with c_s appended (12 floats), cx_s, cy_s, fx_s, fy_s.
 // ------------------------------------------------------------------------------------------------
-__global__ void build_pair_tables_kernel(int n_total, int src_begin, int n_src, int k_nbr, unsigned hw, unsigned width,
-                                         const double* __restrict__ poses,
-                                         const double* __restrict__ intr,
-                                         const int32_t* __restrict__ nbr, float* __restrict__ pair_table,
-                                         float* __restrict__ src_table) {
+// kRagged (ddn_build_pair_tables_ragged): the views' sizes and offsets come from the layout, and floats 16-19 describe
+// the neighbour's map instead of its intrinsics (K4 never reads those).
+template <bool kRagged>
+__device__ __forceinline__ void build_pair_tables_body(int n_total, int src_begin, int n_src, int k_nbr, unsigned hw, unsigned width,
+                                                       const double* __restrict__ poses, const double* __restrict__ intr,
+                                                       const int32_t* __restrict__ nbr, float* __restrict__ pair_table,
+                                                       float* __restrict__ src_table, const int64_t* __restrict__ layout) {
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
   int n_pairs = n_src * k_nbr;
   if (idx >= n_pairs + n_src) return;
@@ -123,12 +126,38 @@ __global__ void build_pair_tables_kernel(int n_total, int src_begin, int n_src, 
   for (int i = 0; i < 3; ++i)  // c_t = -R_t^T t_t
     o[12 + i] = (float)(-(Rt[0][i] * tt[0] + Rt[1][i] * tt[1] + Rt[2][i] * tt[2]));
   o[15] = __int_as_float(t);
+  if (kRagged) {
+    const int64_t* Lt = layout + (size_t)t * DDN_LAYOUT_COLS;
+    const unsigned ht = (unsigned)Lt[0], wt = (unsigned)Lt[1];
+    o[16] = __uint_as_float(wt);
+    o[17] = __uint_as_float(ht);
+    o[18] = (float)wt;  // K4's bounds test compares the raw bits of u, v with these
+    o[19] = (float)ht;
+    o[20] = (t == s) ? 1.f : 0.f;
+    o[21] = __uint_as_float((unsigned)Lt[2] - 0x4B000000u * (wt + 1u));
+    return;
+  }
   o[16] = (float)intr[t * 4 + 0];
   o[17] = (float)intr[t * 4 + 1];
   o[18] = (float)intr[t * 4 + 2];
   o[19] = (float)intr[t * 4 + 3];
   o[20] = (t == s) ? 1.f : 0.f;
   o[21] = __uint_as_float((unsigned)t * hw - 0x4B000000u * (width + 1u));
+}
+
+__global__ void build_pair_tables_kernel(int n_total, int src_begin, int n_src, int k_nbr, unsigned hw, unsigned width,
+                                         const double* __restrict__ poses,
+                                         const double* __restrict__ intr,
+                                         const int32_t* __restrict__ nbr, float* __restrict__ pair_table,
+                                         float* __restrict__ src_table) {
+  build_pair_tables_body<false>(n_total, src_begin, n_src, k_nbr, hw, width, poses, intr, nbr, pair_table, src_table, nullptr);
+}
+
+__global__ void build_pair_tables_ragged_kernel(int n_views, int k_nbr, const double* __restrict__ poses,
+                                                const double* __restrict__ intr, const int32_t* __restrict__ nbr,
+                                                float* __restrict__ pair_table, float* __restrict__ src_table,
+                                                const int64_t* __restrict__ layout) {
+  build_pair_tables_body<true>(n_views, 0, n_views, k_nbr, 0u, 0u, poses, intr, nbr, pair_table, src_table, layout);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -270,8 +299,13 @@ __device__ __forceinline__ void bulk_store_wait_read() { asm volatile("cp.async.
 constexpr int kWarpPix = 32 * kFilterPX;
 static_assert(kFilterPX == 4, "the layouts below are written for 4 pixels per thread");
 
-template <bool kBilinear, bool kStride1, bool kTwoSided, int kLayout>
-__global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOCKS) backproject_filter_kernel(const FilterParams p) {
+// kRagged (ddn_backproject_filter_ragged; layout = the device layout, nullptr otherwise): one flat grid over the chunks
+// of all views in view order (the L2 argument above holds unchanged); a CTA finds its view in the layout, and every
+// neighbour's W, H and bounds-test bits come from its table entry (floats 16-19) next to the gather offset.
+// p.n_src is then the number of views, and p.H, p.W, p.Hs, p.Ws, p.src_begin, p.wbits and p.hbits are not read.
+template <bool kBilinear, bool kStride1, bool kTwoSided, int kLayout, bool kRagged>
+__global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOCKS)
+    backproject_filter_kernel(const FilterParams p, const int64_t* __restrict__ layout) {
   extern __shared__ __align__(16) float smem[];
   float* s_src = smem;                     // 16 floats
   float* s_pair = s_src + 16;              // K*24 floats
@@ -280,13 +314,17 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   __shared__ int s_marked;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int sl = blockIdx.y;
-  const int s = p.src_begin + sl;
-  const int Ps = p.Hs * p.Ws;  // source-grid pixels per view
-  const int chunk0 = blockIdx.x * kFilterChunk;
+  const int sl = kRagged ? layout_view_of(layout, p.n_src, 5, blockIdx.x) : (int)blockIdx.y;
+  const int s = kRagged ? sl : p.src_begin + sl;
+  const int64_t* __restrict__ L = layout + (size_t)sl * DDN_LAYOUT_COLS;  // ragged: the source view's layout row
+  // the source view's full and strided row length, read where the uniform kernel reads p.W / p.Ws
+  auto W_src = [&]() -> int { return kRagged ? (int)L[1] : p.W; };
+  auto Ws_src = [&]() -> int { return kRagged ? ((int)L[1] + p.stride - 1) / p.stride : p.Ws; };
+  const int Ps = kRagged ? ((int)L[0] + p.stride - 1) / p.stride * Ws_src() : p.Hs * p.Ws;  // source-grid pixels per view
+  const int chunk0 = kRagged ? (int)(blockIdx.x - L[5]) * kFilterChunk : blockIdx.x * kFilterChunk;
   const size_t HW = (size_t)p.H * p.W;
-  const float* __restrict__ depth_s = p.refined_all + (size_t)s * HW;
-  const float* __restrict__ normal_s = p.normal + (size_t)sl * HW * 3;
+  const float* __restrict__ depth_s = kRagged ? p.refined_all + L[2] : p.refined_all + (size_t)s * HW;
+  const float* __restrict__ normal_s = kRagged ? p.normal + (size_t)L[2] * 3 : p.normal + (size_t)sl * HW * 3;
 
   // tables -> shared memory, as float4 (entries are 96 bytes; the gather offset t*H*W - bias*(W+1) of every
   // entry was put into float 21 by build_pair_tables_kernel)
@@ -303,8 +341,8 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   const int wbase = chunk0 + warp * kWarpPix;
   const int q0 = wbase + (kLayout == 1 ? lane * kFilterPX : lane);
   constexpr int kStep = kLayout == 1 ? 1 : 32;
-  int ys_run = q0 / p.Ws;
-  int xs_run = q0 - ys_run * p.Ws;
+  int ys_run = q0 / Ws_src();
+  int xs_run = q0 - ys_run * Ws_src();
 
   // Per-pixel state kept in registers: depth d (NaN = no point), P = d*x, Q = d*y, vote count.
   float d[kFilterPX], P[kFilterPX], Q[kFilterPX];
@@ -318,10 +356,10 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
     for (int j = 0; j < kFilterPX; ++j) {
       px[j] = kStride1 ? xs_run : xs_run * p.stride;
       py[j] = kStride1 ? ys_run : ys_run * p.stride;
-      src_pix[j] = kStride1 ? (unsigned)(q0 + j * kStep) : (unsigned)py[j] * (unsigned)p.W + (unsigned)px[j];
+      src_pix[j] = kStride1 ? (unsigned)(q0 + j * kStep) : (unsigned)py[j] * (unsigned)W_src() + (unsigned)px[j];
       xs_run += kStep;
-      while (xs_run >= p.Ws) {
-        xs_run -= p.Ws;
+      while (xs_run >= Ws_src()) {
+        xs_run -= Ws_src();
         ++ys_run;
       }
     }
@@ -380,13 +418,14 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
         const float4* t4 = reinterpret_cast<const float4*>(s_pair + k * DDN_PAIR_TABLE_FLOATS);
         const float4 r0 = t4[0], r1 = t4[1], r2 = t4[2];
         const unsigned off_k = __float_as_uint(s_pair[k * DDN_PAIR_TABLE_FLOATS + 21]);
+        const float4 wh = kRagged ? t4[4] : make_float4(0.f, 0.f, 0.f, 0.f);  // ragged: the neighbour's W, H, (float)W, (float)H
         float Z[kFilterPX], D[kFilterPX];
         bool inb[kFilterPX];
         if (all_live) {
 #pragma unroll
           for (int j = 0; j < kFilterPX; ++j)
-            pair_gather<kBilinear, !kBilinear && !kTwoSided>(r0, r1, r2, P[j], Q[j], d[j], p.refined_all, off_k, (unsigned)p.W, p.H, wbits, hbits, Z[j], D[j],
-                                   inb[j]);
+            pair_gather<kBilinear, !kBilinear && !kTwoSided>(r0, r1, r2, P[j], Q[j], d[j], p.refined_all, off_k, kRagged ? __float_as_uint(wh.x) : (unsigned)p.W, kRagged ? __float_as_int(wh.y) : p.H,
+                                   kRagged ? __float_as_uint(wh.z) : wbits, kRagged ? __float_as_uint(wh.w) : hbits, Z[j], D[j], inb[j]);
 #pragma unroll
           for (int j = 0; j < kFilterPX; ++j) {
             if (!kBilinear && !kTwoSided) {
@@ -399,8 +438,8 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
 #pragma unroll
           for (int j = 0; j < kFilterPX; ++j) {
             if (live[j]) {
-              pair_gather<kBilinear, !kBilinear && !kTwoSided>(r0, r1, r2, P[j], Q[j], d[j], p.refined_all, off_k, (unsigned)p.W, p.H, wbits, hbits, Z[j],
-                                     D[j], inb[j]);
+              pair_gather<kBilinear, !kBilinear && !kTwoSided>(r0, r1, r2, P[j], Q[j], d[j], p.refined_all, off_k, kRagged ? __float_as_uint(wh.x) : (unsigned)p.W, kRagged ? __float_as_int(wh.y) : p.H,
+                                   kRagged ? __float_as_uint(wh.z) : wbits, kRagged ? __float_as_uint(wh.w) : hbits, Z[j], D[j], inb[j]);
               if (pair_test<kTwoSided>(Z[j], D[j], inb[j], thr, tau)) cm[j] |= bit;
             }
           }
@@ -440,9 +479,9 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
 #pragma unroll
       for (int j = 0; j < kFilterPX; ++j) {
         if (d[j] > 0.f) {
-          const int py = (int)(src_pix[j] / (unsigned)p.W), px = (int)(src_pix[j] - (unsigned)py * (unsigned)p.W);
+          const int py = (int)(src_pix[j] / (unsigned)W_src()), px = (int)(src_pix[j] - (unsigned)py * (unsigned)W_src());
           const int ux = max(px - 1, 0), vy = max(py - 1, 0);
-          const float D = __ldg(depth_s + (size_t)vy * p.W + ux);
+          const float D = __ldg(depth_s + (size_t)vy * W_src() + ux);
           const bool bad = kTwoSided ? (fabsf(d[j] - D) > tau * D) : (d[j] < __fmul_rn(thr, D));
           if (D > 0.f && bad) {
             float n0, n1, n2, wx, wy, wz;
@@ -471,7 +510,7 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
     keep[j] = valid && nvotes[j] < p.vote_threshold;
     vote_bytes |= (valid ? (unsigned)min(nvotes[j], 254) : 255u) << (8 * j);
   }
-  const size_t out0 = (size_t)sl * Ps;  // first pixel of the view in the outputs
+  const size_t out0 = kRagged ? (size_t)L[3] : (size_t)sl * Ps;  // first pixel of the view in the outputs
   if (kLayout == 1) {
     uint8_t* vo = p.votes + out0 + q0;
     if (q0 + kFilterPX <= Ps && ((reinterpret_cast<uintptr_t>(vo) & 3) == 0)) {
@@ -601,6 +640,79 @@ __global__ void bbox_init_kernel(int* bbox) {
   else if (threadIdx.x < 6) bbox[threadIdx.x] = float_to_ordered(-INFINITY);
 }
 
+// The FilterParams fields both entry points share (everything but the sizes and the source range).
+static int fill_filter_params(const ddn_filter_config* cfg, const float* refined_all, const float* normal,
+                              const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
+                              uint8_t* votes, float* bbox, const ddn_fuse_session* mark, int64_t k_nbr, FilterParams& p) {
+  p.refined_all = refined_all;
+  p.normal = normal;
+  p.pair_table = pair_table;
+  p.src_table = src_table;
+  p.xyz = xyz;
+  p.votes = votes;
+  p.bbox = reinterpret_cast<int*>(bbox);
+  p.mark.grid = nullptr, p.mark.units = nullptr, p.mark.dirty = nullptr, p.mark.counts = nullptr;
+  if (mark != nullptr) {
+    DDN_REQUIRE(mark->grid && mark->units && mark->counts, "mark session: null buffer");
+    p.mark.grid = reinterpret_cast<const GridDev*>(mark->grid);
+    p.mark.units = reinterpret_cast<uint32_t*>(mark->units);
+    p.mark.dirty = mark->dirty;
+    p.mark.counts = reinterpret_cast<unsigned long long*>(mark->counts);
+  }
+  p.stride = cfg->stride;
+  p.K = (int)k_nbr;
+  p.vote_threshold = vote_threshold < 255 ? vote_threshold : 255;
+  p.depth_threshold = cfg->depth_threshold;
+  p.grazing_cos = cfg->grazing_cos;
+  p.two_sided_tau = cfg->two_sided_tau;
+  p.normals_in_world = cfg->normals_in_world;
+  return DDN_OK;
+}
+
+// Launches the K4 instantiation cfg selects: the uniform kernel (layout == nullptr, grid = chunks x views) or the
+// ragged one (grid = all chunks of the layout).
+static int launch_filter(const ddn_filter_config* cfg, const FilterParams& p, dim3 grid, const int64_t* layout, cudaStream_t st) {
+  const int pl = cfg->pixel_layout;
+  const size_t smem = (size_t)(16 + p.K * DDN_PAIR_TABLE_FLOATS + (pl == 0 ? kFilterChunk * 3 : 0)) * sizeof(float);
+  const bool bil = cfg->sample_mode == 1;
+  const bool s1 = cfg->stride == 1;
+  const bool two = cfg->two_sided_tau > 0.f;
+  DDN_REQUIRE(two || cfg->depth_threshold > 0.f, "depth_threshold must be positive");
+#define DDN_LAUNCH_FILTER(B, S, T, L)                                                                        \
+  do {                                                                                                       \
+    if (layout != nullptr) {                                                                                 \
+      DDN_TRY(check_cuda(cudaFuncSetAttribute(backproject_filter_kernel<B, S, T, L, true>,                   \
+                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),       \
+                         "cudaFuncSetAttribute"));                                                           \
+      backproject_filter_kernel<B, S, T, L, true><<<grid, kFilterThreads, smem, st>>>(p, layout);            \
+    } else {                                                                                                 \
+      DDN_TRY(check_cuda(cudaFuncSetAttribute(backproject_filter_kernel<B, S, T, L, false>,                  \
+                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),       \
+                         "cudaFuncSetAttribute"));                                                           \
+      backproject_filter_kernel<B, S, T, L, false><<<grid, kFilterThreads, smem, st>>>(p, nullptr);          \
+    }                                                                                                        \
+  } while (0)
+#define DDN_LAUNCH_FILTER_L(B, S, T)       \
+  do {                                     \
+    if (pl == 1) DDN_LAUNCH_FILTER(B, S, T, 1); \
+    else DDN_LAUNCH_FILTER(B, S, T, 0);    \
+  } while (0)
+  if (two) {
+    if (bil && s1) DDN_LAUNCH_FILTER_L(true, true, true);
+    else if (bil) DDN_LAUNCH_FILTER_L(true, false, true);
+    else if (s1) DDN_LAUNCH_FILTER_L(false, true, true);
+    else DDN_LAUNCH_FILTER_L(false, false, true);
+  } else {
+    if (bil && s1) DDN_LAUNCH_FILTER_L(true, true, false);
+    else if (bil) DDN_LAUNCH_FILTER_L(true, false, false);
+    else if (s1) DDN_LAUNCH_FILTER_L(false, true, false);
+    else DDN_LAUNCH_FILTER_L(false, false, false);
+  }
+#undef DDN_LAUNCH_FILTER_L
+#undef DDN_LAUNCH_FILTER
+  return DDN_OK;
+}
+
 }  // namespace ddn
 
 extern "C" {
@@ -648,34 +760,13 @@ int ddn_backproject_filter(const ddn_filter_config* cfg, int64_t n_views_total, 
               "pair_table / src_table must be 16-byte aligned");
   if (n_src == 0) return DDN_OK;
   FilterParams p;
-  p.refined_all = refined_all;
-  p.normal = normal;
-  p.pair_table = pair_table;
-  p.src_table = src_table;
-  p.xyz = xyz;
-  p.votes = votes;
-  p.bbox = reinterpret_cast<int*>(bbox);
-  p.mark.grid = nullptr, p.mark.units = nullptr, p.mark.dirty = nullptr, p.mark.counts = nullptr;
-  if (mark != nullptr) {
-    DDN_REQUIRE(mark->grid && mark->units && mark->counts, "mark session: null buffer");
-    p.mark.grid = reinterpret_cast<const GridDev*>(mark->grid);
-    p.mark.units = reinterpret_cast<uint32_t*>(mark->units);
-    p.mark.dirty = mark->dirty;
-    p.mark.counts = reinterpret_cast<unsigned long long*>(mark->counts);
-  }
+  DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
   p.src_begin = (int)src_begin;
   p.n_src = (int)n_src;
   p.H = (int)height;
   p.W = (int)width;
-  p.stride = cfg->stride;
   p.Hs = (p.H + p.stride - 1) / p.stride;
   p.Ws = (p.W + p.stride - 1) / p.stride;
-  p.K = (int)k_nbr;
-  p.vote_threshold = vote_threshold < 255 ? vote_threshold : 255;
-  p.depth_threshold = cfg->depth_threshold;
-  p.grazing_cos = cfg->grazing_cos;
-  p.two_sided_tau = cfg->two_sided_tau;
-  p.normals_in_world = cfg->normals_in_world;
   {
     const float wf = (float)p.W, hf = (float)p.H;
     memcpy(&p.wbits, &wf, 4);
@@ -684,38 +775,46 @@ int ddn_backproject_filter(const ddn_filter_config* cfg, int64_t n_views_total, 
   const int Ps = p.Hs * p.Ws;
   dim3 grid((Ps + kFilterChunk - 1) / kFilterChunk, (unsigned)n_src);
   DDN_REQUIRE(n_src <= 65535, "too many source views per call");
-  const int layout = cfg->pixel_layout;
-  const size_t smem = (size_t)(16 + p.K * DDN_PAIR_TABLE_FLOATS + (layout == 0 ? kFilterChunk * 3 : 0)) * sizeof(float);
-  cudaStream_t st = (cudaStream_t)stream;
-  const bool bil = cfg->sample_mode == 1;
-  const bool s1 = cfg->stride == 1;
-  const bool two = cfg->two_sided_tau > 0.f;
-  DDN_REQUIRE(two || cfg->depth_threshold > 0.f, "depth_threshold must be positive");
-#define DDN_LAUNCH_FILTER(B, S, T, L)                                                                      \
-  do {                                                                                                     \
-    DDN_TRY(check_cuda(cudaFuncSetAttribute(backproject_filter_kernel<B, S, T, L>,                         \
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),       \
-                       "cudaFuncSetAttribute"));                                                           \
-    backproject_filter_kernel<B, S, T, L><<<grid, kFilterThreads, smem, st>>>(p);                          \
-  } while (0)
-#define DDN_LAUNCH_FILTER_L(B, S, T)       \
-  do {                                     \
-    if (layout == 1) DDN_LAUNCH_FILTER(B, S, T, 1); \
-    else DDN_LAUNCH_FILTER(B, S, T, 0);    \
-  } while (0)
-  if (two) {
-    if (bil && s1) DDN_LAUNCH_FILTER_L(true, true, true);
-    else if (bil) DDN_LAUNCH_FILTER_L(true, false, true);
-    else if (s1) DDN_LAUNCH_FILTER_L(false, true, true);
-    else DDN_LAUNCH_FILTER_L(false, false, true);
-  } else {
-    if (bil && s1) DDN_LAUNCH_FILTER_L(true, true, false);
-    else if (bil) DDN_LAUNCH_FILTER_L(true, false, false);
-    else if (s1) DDN_LAUNCH_FILTER_L(false, true, false);
-    else DDN_LAUNCH_FILTER_L(false, false, false);
-  }
-#undef DDN_LAUNCH_FILTER_L
-#undef DDN_LAUNCH_FILTER
+  DDN_TRY(launch_filter(cfg, p, grid, nullptr, (cudaStream_t)stream));
+  return after_launch("backproject_filter_kernel");
+}
+
+int ddn_build_pair_tables_ragged(int64_t n_views, int64_t k_nbr, const int64_t* layout, const int64_t* layout_host,
+                                 const double* cam_from_world, const double* intr, const int32_t* nbr, float* pair_table,
+                                 float* src_table, void* stream) {
+  using namespace ddn;
+  DDN_REQUIRE(k_nbr > 0, "view counts");
+  DDN_REQUIRE(layout != nullptr, "null layout");
+  DDN_TRY(check_layout(n_views, layout_host));
+  DDN_REQUIRE(cam_from_world && intr && nbr && pair_table && src_table, "null pointer");
+  const int total = (int)(n_views * k_nbr + n_views);
+  build_pair_tables_ragged_kernel<<<(total + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+      (int)n_views, (int)k_nbr, cam_from_world, intr, nbr, pair_table, src_table, layout);
+  return after_launch("build_pair_tables_ragged_kernel");
+}
+
+int ddn_backproject_filter_ragged(const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr, const int64_t* layout,
+                                  const int64_t* layout_host, const float* refined_all, const float* normal,
+                                  const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
+                                  uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
+  using namespace ddn;
+  DDN_REQUIRE(cfg != nullptr, "null config");
+  DDN_REQUIRE(k_nbr > 0 && k_nbr <= 1024, "view counts (at most 1024 neighbours per view)");
+  DDN_REQUIRE(layout != nullptr, "null layout");
+  DDN_TRY(check_layout(n_views, layout_host));
+  DDN_REQUIRE(cfg->stride >= 1 && cfg->stride == layout_host[n_views * DDN_LAYOUT_COLS], "cfg->stride must be the layout's stride");
+  DDN_REQUIRE(cfg->pixel_layout == 0 || cfg->pixel_layout == 1, "pixel_layout");
+  DDN_REQUIRE(refined_all && normal && pair_table && src_table && xyz && votes, "null pointer");
+  DDN_REQUIRE((reinterpret_cast<uintptr_t>(pair_table) & 15) == 0 && (reinterpret_cast<uintptr_t>(src_table) & 15) == 0,
+              "pair_table / src_table must be 16-byte aligned");
+  FilterParams p;
+  DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
+  p.src_begin = 0;
+  p.n_src = (int)n_views;
+  p.H = p.W = p.Hs = p.Ws = 0;  // per view, from the layout and the table entries
+  p.wbits = p.hbits = 0;
+  const int64_t chunks = layout_host[n_views * DDN_LAYOUT_COLS + 5];  // >= 1: every view has a pixel
+  DDN_TRY(launch_filter(cfg, p, dim3((unsigned)chunks), layout, (cudaStream_t)stream));
   return after_launch("backproject_filter_kernel");
 }
 

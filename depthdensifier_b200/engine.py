@@ -52,6 +52,14 @@ class DensifyResult:
     counts: torch.Tensor | None = None  # [2] i64: fused points, voxels
     session: object | None = None  # ops.FuseSession that produced the voxels (device-resident grid)
     bbox_valid: torch.Tensor | None = None  # [6] i32: box of every back-projected pixel (the alignment kernel's bound)
+    layout: ops.ViewLayout | None = None  # run_views: refined [P], xyz [G,3], votes [G] are flat over the views of this layout
+
+    def per_view(self, name: str) -> list:
+        """Per-view views of a flat output of run_views: ``refined`` -> [H_v, W_v], ``xyz`` -> [Hs_v, Ws_v, 3],
+        ``votes`` -> [Hs_v, Ws_v] (no copy)."""
+        if self.layout is None:
+            return list(getattr(self, name))
+        return self.layout.split(getattr(self, name), grid=name != "refined")
 
     def keep_mask(self) -> torch.Tensor:
         return (self.votes != 255) & (self.votes < clamp_vote_threshold(self.vote_threshold))
@@ -99,6 +107,16 @@ class DensifyEngine:
         return ops.align_views(depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets, max_sparse_per_view,
                                self.cfg.align, out=out, src_table=src_table, bbox=bbox)
 
+    def _fuse(self, res, sess, grid, xyz, rgb_s, votes, sparse_xyz, thr, row_len, sync):
+        if self.cfg.dedup_sparse and sparse_xyz.shape[0] > 0:
+            sess.unmark_points(sparse_xyz.float().contiguous())
+        k, x, c, n, counts = ops.fuse_finish(sess, xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), thr, row_len=row_len)
+        res.session, res.grid = sess, grid
+        res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts.clone()
+        if sync:
+            mv = res.check()
+            res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count = k[:mv], x[:mv], c[:mv], n[:mv]
+
     def session(self) -> ops.FuseSession:
         if getattr(self, "_session", None) is None or self._session.max_cells != self.cfg.max_grid_cells:
             self._session = ops.FuseSession(self.device, self.cfg.max_grid_cells)
@@ -142,13 +160,60 @@ class DensifyEngine:
         if fuse:
             s = cfg.filter.stride
             rgb_s = rgb if s == 1 else rgb[:, ::s, ::s].contiguous()
-            if cfg.dedup_sparse and sparse_xyz.shape[0] > 0:
-                sess.unmark_points(sparse_xyz.float().contiguous())
-            k, x, c, n, counts = ops.fuse_finish(sess, xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), thr, row_len=xyz.shape[2])
-            res.session, res.grid = sess, grid
-            res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts.clone()
-            if sync:
-                mv = res.check()
-                res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count = k[:mv], x[:mv], c[:mv], n[:mv]
+            self._fuse(res, sess, grid, xyz, rgb_s, votes, sparse_xyz, thr, xyz.shape[2], sync)
+        res.bbox_valid = box
+        return res
+
+    def run_views(self, depths, normals, masks, rgbs, cam_from_world, intr, sparse_xyz, sparse_offsets, nbr,
+                  max_sparse_per_view: int | None = None, grid=None, sync: bool = True,
+                  layout: ops.ViewLayout | None = None) -> DensifyResult:
+        """``run`` for views of different sizes.  ``depths``, ``normals``, ``masks``, ``rgbs``: lists of per-view CUDA
+        tensors ([H_v,W_v] f32, [H_v,W_v,3] f32, [H_v,W_v] bool, [H_v,W_v,3] u8), or, with ``layout``, the flat
+        concatenations ([P], [P,3], [P], [P,3]); the other inputs as in ``run``.  ``normals`` may be pinned host memory.
+
+        The same step as ``run`` - one launch per stage over all views, no host round trip - on the flat layout
+        (include/ddn_b200.h, DDN_LAYOUT_COLS).  The result's refined [P], xyz [G,3] and votes [G] are flat in view order
+        (``DensifyResult.per_view`` splits them); keep_mask() and the voxel outputs mean what they mean for ``run``."""
+        cfg = self.cfg
+        dev = cam_from_world.device
+        if layout is None:
+            layout = ops.ViewLayout.from_shapes([tuple(d.shape) for d in depths], cfg.filter.stride)
+            depth = layout.flatten(depths, torch.float32)
+            normal = layout.flatten(normals, torch.float32) if normals[0].is_cuda else \
+                layout.flatten(normals, torch.float32).pin_memory()
+            mask = layout.flatten(masks) if masks is not None else None
+            rgb_flat = layout.flatten(rgbs) if rgbs is not None else None
+        else:
+            depth, normal, mask, rgb_flat = depths, normals, masks, rgbs
+        V = layout.n_views
+        K = nbr.shape[1]
+        if max_sparse_per_view is None:
+            off = sparse_offsets.cpu().numpy()
+            max_sparse_per_view = int(np.max(np.diff(off))) if V > 0 else 1
+        thr = clamp_vote_threshold(cfg.vote_threshold if cfg.vote_threshold is not None else default_vote_threshold(K))
+        pair, src = ops.build_pair_tables_ragged(layout, cam_from_world, intr, nbr)
+        fuse = cfg.voxel is not None
+        box = ops.new_bbox(dev) if fuse and grid is None else None
+        kmat = torch.zeros((V, 3, 3), dtype=torch.float64, device=dev)
+        kmat[:, 0, 0], kmat[:, 1, 1], kmat[:, 0, 2], kmat[:, 1, 2], kmat[:, 2, 2] = intr[:, 0], intr[:, 1], intr[:, 2], intr[:, 3], 1.0
+        refined, stats = ops.align_views_ragged(layout, depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets,
+                                                max(max_sparse_per_view, 1), cfg.align, src_table=src if box is not None else None,
+                                                bbox=box)
+        sess = None
+        if fuse:
+            sess = self.session()
+            if grid is None:
+                sess.begin([box], cfg.voxel)
+            else:
+                sess.begin_grid(grid)
+        bbox = ops.new_bbox(dev)
+        xyz, votes = ops.backproject_filter_ragged(layout, refined, normal, pair, src, thr, cfg.filter, bbox=bbox, mark=sess)
+        res = DensifyResult(refined=refined, stats=stats, xyz=xyz, votes=votes, vote_threshold=thr, bbox=bbox, layout=layout)
+        if fuse:
+            if layout.stride == 1:
+                rgb_s = rgb_flat
+            else:
+                rgb_s = torch.cat([r.reshape(-1, 3) for r in layout.strided(layout.split(rgb_flat))], 0)
+            self._fuse(res, sess, grid, xyz, rgb_s, votes, sparse_xyz, thr, 0, sync)  # row_len 0: rows differ per view
         res.bbox_valid = box
         return res

@@ -238,6 +238,180 @@ def backproject_filter(refined_all, normal, nbr, pair_table, src_table, src_begi
     return xyz, votes
 
 
+# ----------------------------------------------------------------------------------------------
+# Ragged views: V depth maps of different sizes in one pass (include/ddn_b200.h, DDN_LAYOUT_COLS)
+# ----------------------------------------------------------------------------------------------
+REMAP_TILE_H, REMAP_TILE_W = 32, 126  # remap_median_kernel tile (align.cu)
+FILTER_CHUNK = 1024  # points per consistency-kernel CTA (filter.cu kFilterChunk)
+MAX_RAGGED_VIEWS = 65535
+
+
+class ViewLayout:
+    """Sizes and offsets of V views of different sizes concatenated into flat buffers: per-pixel buffers (depth, mask,
+    refined, normal, rgb) hold the views' row-major maps one after the other, strided-grid buffers (xyz, votes) their
+    ceil(H/stride) x ceil(W/stride) grids.  ``table`` is the int64 [V+1, 8] layout of the C ABI (row v: H, W, pixel
+    offset, grid offset, first remap tile, first consistency chunk; last row: stride, V and the four totals)."""
+
+    def __init__(self, shapes, stride: int = 1):
+        shapes = [(int(h), int(w)) for h, w in shapes]
+        stride = int(stride)
+        V = len(shapes)
+        if V < 1 or V > MAX_RAGGED_VIEWS:
+            raise ValueError(f"a ragged layout holds 1 to {MAX_RAGGED_VIEWS} views, got {V}")
+        if stride < 1:
+            raise ValueError("stride must be >= 1")
+        for h, w in shapes:
+            if h < 1 or w < 1:
+                raise ValueError(f"zero-sized view {h}x{w}")
+            if h >= 1 << 22 or w >= 1 << 22 or h * w >= 1 << 31:
+                raise ValueError(f"view {h}x{w} too large (sides < 2^22, fewer than 2^31 pixels)")
+        hw = np.array(shapes, dtype=np.int64).reshape(V, 2)
+        hs, ws = (hw[:, 0] + stride - 1) // stride, (hw[:, 1] + stride - 1) // stride
+        units = np.stack([hw[:, 0] * hw[:, 1], hs * ws,
+                          ((hw[:, 0] + REMAP_TILE_H - 1) // REMAP_TILE_H) * ((hw[:, 1] + REMAP_TILE_W - 1) // REMAP_TILE_W),
+                          (hs * ws + FILTER_CHUNK - 1) // FILTER_CHUNK], axis=1)
+        if units[:, 0].sum() >= 1 << 32:
+            raise ValueError(f"{int(units[:, 0].sum())} pixels in all: the ragged kernels address fewer than 2^32")
+        t = np.zeros((V + 1, _lib.LAYOUT_COLS), dtype=np.int64)
+        t[:V, 0:2] = hw
+        t[1:, 2:6] = np.cumsum(units, axis=0)
+        t[V, 0:2] = stride, V
+        self.shapes, self.stride, self.table = shapes, stride, t
+        self.grid_shapes = list(zip(hs.tolist(), ws.tolist()))
+        self._dev = {}
+
+    @classmethod
+    def from_shapes(cls, shapes, stride: int = 1) -> "ViewLayout":
+        return cls(shapes, stride)
+
+    @property
+    def n_views(self) -> int:
+        return len(self.shapes)
+
+    @property
+    def pix_off(self) -> np.ndarray:  # [V+1]
+        return self.table[:, 2].copy()
+
+    @property
+    def grid_off(self) -> np.ndarray:  # [V+1]
+        return self.table[:, 3].copy()
+
+    @property
+    def total_pixels(self) -> int:
+        return int(self.table[-1, 2])
+
+    @property
+    def total_grid(self) -> int:
+        return int(self.table[-1, 3])
+
+    @property
+    def uniform(self) -> bool:
+        return len(set(self.shapes)) == 1
+
+    def device(self, dev) -> torch.Tensor:
+        """The layout in device memory (one copy per device, kept)."""
+        dev = torch.device(dev)
+        if dev not in self._dev:
+            self._dev[dev] = torch.from_numpy(self.table).to(dev)
+        return self._dev[dev]
+
+    def host_ptr(self):
+        return self.table.ctypes.data_as(C.c_void_p)
+
+    def flatten(self, maps, dtype=None) -> torch.Tensor:
+        """Concatenation of per-view maps [H_v, W_v, ...] (tensors or arrays, one device) into one flat tensor."""
+        ts = [torch.as_tensor(m) for m in maps]
+        assert [tuple(t.shape[:2]) for t in ts] == self.shapes, "maps do not match the layout"
+        out = torch.cat([t.reshape((-1,) + tuple(t.shape[2:])) for t in ts], 0)
+        return out.to(dtype).contiguous() if dtype is not None else out.contiguous()
+
+    def split(self, flat: torch.Tensor, grid: bool = False) -> list:
+        """Per-view views [H_v, W_v, ...] (or the strided grids with ``grid``) of a flat tensor; no copy."""
+        off = self.table[:, 3 if grid else 2]
+        shapes = self.grid_shapes if grid else self.shapes
+        return [flat[int(off[v]):int(off[v + 1])].view((h, w) + tuple(flat.shape[1:])) for v, (h, w) in enumerate(shapes)]
+
+    def strided(self, maps) -> list:
+        """Each view's map [H_v, W_v, ...] on its strided grid (every stride-th row and column)."""
+        s = self.stride
+        return [m if s == 1 else m[::s, ::s] for m in maps]
+
+
+def align_views_ragged(layout: ViewLayout, depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets, max_sparse_per_view: int,
+                       opts: AlignOptions, out=None, src_table=None, bbox=None):
+    """Stage 1 for the views of ``layout``: depth flat [P] f32, mask flat [P] bool/u8 or None, refined flat [P].  Returns
+    (refined, stats [V,8]).  ``src_table`` [V,16] + ``bbox`` [6]: the bounding-box epilogue, as in align_views."""
+    lib = _lib.load()
+    dev = _require_cuda(depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets, out, src_table, bbox)
+    assert (src_table is None) == (bbox is None)
+    V, P = layout.n_views, layout.total_pixels
+    assert depth.dtype == torch.float32 and tuple(depth.shape) == (P,)
+    assert mask is None or (mask.dtype in (torch.bool, torch.uint8) and tuple(mask.shape) == (P,))
+    assert tuple(cam_from_world.shape) == (V, 3, 4) and tuple(kmat.shape) == (V, 3, 3)
+    assert sparse_xyz.dtype == torch.float64 and sparse_offsets.dtype == torch.int64
+    refined = out if out is not None else torch.empty_like(depth)
+    stats = torch.zeros((V, 8), dtype=torch.int32, device=dev)
+    nbytes = C.c_int64(0)
+    _lib.check(lib.ddn_align_workspace_bytes(V, max_sparse_per_view, C.byref(nbytes)))
+    ws = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+    cfg = opts.to_c()
+    with torch.cuda.device(dev):
+        _lib.check(
+            lib.ddn_align_views_ragged(
+                C.byref(cfg), V, _p(layout.device(dev)), layout.host_ptr(), _p(depth), _p(mask), _p(cam_from_world), _p(kmat),
+                _p(sparse_xyz), _p(sparse_offsets), int(max_sparse_per_view), _p(refined), _p(stats), _p(ws), nbytes.value,
+                _p(src_table), _p(bbox), _stream(),
+            )
+        )
+    return refined, stats
+
+
+def build_pair_tables_ragged(layout: ViewLayout, cam_from_world, intr, nbr):
+    """Pair / source tables for all views of ``layout`` (entries carry the neighbour's own size)."""
+    lib = _lib.load()
+    dev = _require_cuda(cam_from_world, intr, nbr)
+    V, K = layout.n_views, nbr.shape[1]
+    assert cam_from_world.dtype == torch.float64 and intr.dtype == torch.float64 and nbr.dtype == torch.int32
+    assert tuple(cam_from_world.shape) == (V, 3, 4) and tuple(intr.shape) == (V, 4) and nbr.shape[0] == V
+    pair = torch.empty((V, K, _lib.PAIR_TABLE_FLOATS), dtype=torch.float32, device=dev)
+    src = torch.empty((V, 16), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ddn_build_pair_tables_ragged(V, K, _p(layout.device(dev)), layout.host_ptr(), _p(cam_from_world), _p(intr),
+                                                    _p(nbr), _p(pair), _p(src), _stream()))
+    return pair, src
+
+
+def backproject_filter_ragged(layout: ViewLayout, refined_all, normal, pair_table, src_table, vote_threshold: int,
+                              opts: FilterOptions, bbox=None, xyz_out=None, votes_out=None, mark=None):
+    """Stages 2+3 for all views of ``layout``: refined_all flat [P] f32, normal flat [P,3] f32 (device, or pinned host).
+    Returns xyz [G,3] f32 and votes [G] u8 on the views' strided grids (G = layout.total_grid); ``opts.stride`` must be
+    the layout's stride."""
+    lib = _lib.load()
+    normal_on_host = not normal.is_cuda
+    if normal_on_host and not (normal.is_pinned() and normal.is_contiguous()):
+        raise DDNError("a host normal map must be pinned and contiguous")
+    dev = _require_cuda(refined_all, None if normal_on_host else normal, pair_table, src_table, bbox, xyz_out, votes_out)
+    V, P, G = layout.n_views, layout.total_pixels, layout.total_grid
+    K = pair_table.shape[1]
+    assert refined_all.dtype == torch.float32 and tuple(refined_all.shape) == (P,)
+    assert normal.dtype == torch.float32 and tuple(normal.shape) == (P, 3)
+    assert tuple(pair_table.shape) == (V, K, _lib.PAIR_TABLE_FLOATS) and tuple(src_table.shape) == (V, 16)
+    if int(opts.stride) != layout.stride:
+        raise ValueError(f"filter stride {opts.stride} but the layout was built for stride {layout.stride}")
+    xyz = xyz_out if xyz_out is not None else torch.empty((G, 3), dtype=torch.float32, device=dev)
+    votes = votes_out if votes_out is not None else torch.empty(G, dtype=torch.uint8, device=dev)
+    cfg = opts.to_c()
+    with torch.cuda.device(dev):
+        _lib.check(
+            lib.ddn_backproject_filter_ragged(
+                C.byref(cfg), V, K, _p(layout.device(dev)), layout.host_ptr(), _p(refined_all), _p(normal), _p(pair_table),
+                _p(src_table), int(vote_threshold), _p(xyz), _p(votes), _p(bbox), C.byref(mark.c) if mark is not None else None,
+                _stream(),
+            )
+        )
+    return xyz, votes
+
+
 def make_grid(bbox_min, bbox_max, voxel: float):
     """Voxel grid from a bounding box: origin = floor(min/voxel)*voxel in float32 (SURVEY.md N4) and the
     number of significant bits per axis."""

@@ -6,7 +6,8 @@ COLMAP model with the kept dense points appended to the sparse ones), but
 
 * the COLMAP model is read / written by ``colmap_io`` (the reference needs ``pycolmap``),
 * all views are processed at once on the device by the batched kernels (align -> back-project + vote
-  [-> voxel fusion]) instead of three Python loops,
+  [-> voxel fusion]) instead of three Python loops; views of different sizes (several cameras, portrait and
+  landscape shots) go through the ragged form of the same kernels, one flat pass over all views,
 * MoGe inference is out of scope (BASELINE.json north_star): monocular depth / normal / mask come from a
   ``DepthProvider``.  ``PrecomputedDepth`` reads ``<depth_dir>/<image stem>.npz`` with arrays ``depth``
   [H,W] f32, ``normal`` [H,W,3] f32, ``mask`` [H,W] bool; ``MoGeDepth`` wraps the reference's model call
@@ -247,9 +248,7 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
         intr.append(np.array(camera.params[:4], dtype=np.float64))
     if not views:
         raise ValueError("no registered image observes any sparse point")
-    shapes = {d.shape for d in depths}
-    if len(shapes) != 1:
-        raise ValueError(f"all depth maps must share one size for the batched kernels, got {sorted(shapes)}")
+    uniform = len({d.shape for d in depths}) == 1  # else: views of different sizes, the ragged form of the device pipeline
     V = len(views)
     if (config.filtering.num_neighbours is None or config.filtering.num_neighbours >= V) and V > 1024:
         raise ValueError(f"{V} views: testing every view against every view (the reference's behaviour, K = V) is limited to "
@@ -278,16 +277,27 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
                                       voxel=config.fusion.voxel_size, dedup_sparse=bool(config.fusion.dedup_sparse)), device=dev)
     offsets = np.concatenate([[0], np.cumsum([len(p) for p in sparse])]).astype(np.int64)
     to = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(dev)
-    rgb_dev = to(np.stack(rgbs), torch.uint8)
-    res = eng.run(to(np.stack(depths), torch.float32), to(np.stack(normals), torch.float32), to(np.stack(masks), torch.bool),
-                  rgb_dev, to(poses_np, torch.float64), to(np.stack(intr), torch.float64),
-                  to(np.concatenate(sparse), torch.float64), to(offsets, torch.int64), to(nbr, torch.int32))
+    s = filt.stride
+    if uniform:
+        rgb_dev = to(np.stack(rgbs), torch.uint8)
+        res = eng.run(to(np.stack(depths), torch.float32), to(np.stack(normals), torch.float32), to(np.stack(masks), torch.bool),
+                      rgb_dev, to(poses_np, torch.float64), to(np.stack(intr), torch.float64),
+                      to(np.concatenate(sparse), torch.float64), to(offsets, torch.int64), to(nbr, torch.int32))
+    else:
+        layout = ops.ViewLayout.from_shapes([d.shape for d in depths], s)
+        flat = lambda maps, dt: to(np.concatenate([np.asarray(m).reshape((-1,) + np.asarray(m).shape[2:]) for m in maps]), dt)
+        rgb_flat = flat(rgbs, torch.uint8)
+        res = eng.run_views(flat(depths, torch.float32), flat(normals, torch.float32), flat(masks, torch.bool), rgb_flat,
+                            to(poses_np, torch.float64), to(np.stack(intr), torch.float64), to(np.concatenate(sparse), torch.float64),
+                            to(offsets, torch.int64), to(nbr, torch.int32), layout=layout)
     n_candidates = res.num_points()
     if config.fusion.voxel_size is None:
         keep = res.keep_mask()
-        s = filt.stride
         pts_out = res.xyz[keep].double().cpu().numpy()
-        col_out = rgb_dev[:, ::s, ::s][keep].cpu().numpy()
+        if uniform:
+            col_out = rgb_dev[:, ::s, ::s][keep].cpu().numpy()
+        else:  # each view's strided RGB, concatenated in the order of xyz
+            col_out = torch.cat([r.reshape(-1, 3) for r in layout.strided(layout.split(rgb_flat))], 0)[keep].cpu().numpy()
     else:
         mv = int(res.counts[1].item()) if res.counts is not None else 0
         pts_out = res.voxel_xyz[:mv].double().cpu().numpy() if mv else np.zeros((0, 3))

@@ -15,7 +15,7 @@ MoGe inference is out of scope (BASELINE.json north_star): these maps stand in f
 from __future__ import annotations
 
 import math
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, replace
 
 import numpy as np
 import torch
@@ -190,4 +190,45 @@ def make_scene(cfg: SceneConfig, device: str | torch.device = "cpu", views: rang
         sparse_xyz=torch.cat(sparse, 0) if sparse else torch.zeros((0, 3), dtype=torch.float64, device=dev),
         sparse_offsets=torch.tensor(offsets, dtype=torch.int64, device=dev),
         scale=torch.from_numpy(scale_np).to(dev),
+    )
+
+
+@dataclass
+class MixedScene:
+    """A scene whose views have different sizes: per-view lists of maps, the other arrays as in ``Scene``."""
+
+    cfg: SceneConfig
+    sizes: list  # [(H_v, W_v)]
+    cam_from_world: torch.Tensor  # [V,3,4] f64
+    intrinsics: torch.Tensor  # [V,4] f64, each view's own (fx = fy = 0.8 W_v, cx = W_v/2, cy = H_v/2)
+    mono_depth: list  # V x [H_v,W_v] f32
+    normal: list  # V x [H_v,W_v,3] f32
+    mask: list  # V x [H_v,W_v] bool
+    rgb: list  # V x [H_v,W_v,3] u8
+    sparse_xyz: torch.Tensor  # [sum C_v, 3] f64
+    sparse_offsets: torch.Tensor  # [V+1] i64
+
+    @property
+    def n_views(self) -> int:
+        return len(self.sizes)
+
+
+def make_mixed_scene(cfg: SceneConfig, sizes, device: str | torch.device = "cpu") -> MixedScene:
+    """The ring of ``cfg`` (poses from ring_poses(cfg), V = len(sizes)) with view v rendered at sizes[v] = (H_v, W_v):
+    its maps and sparse points are those of make_scene(replace(cfg, width=W_v, height=H_v), views=[v]), so a view's
+    content depends only on (cfg, v, its size)."""
+    cfg = replace(cfg, n_views=len(sizes))
+    per = [make_scene(replace(cfg, width=int(w), height=int(h)), device, views=[v]) for v, (h, w) in enumerate(sizes)]
+    counts = [sc.sparse_xyz.shape[0] for sc in per]
+    return MixedScene(
+        cfg=cfg,
+        sizes=[(int(h), int(w)) for h, w in sizes],
+        cam_from_world=per[0].cam_from_world,
+        intrinsics=torch.stack([sc.intrinsics[v] for v, sc in enumerate(per)]),
+        mono_depth=[sc.mono_depth[0] for sc in per],
+        normal=[sc.normal[0] for sc in per],
+        mask=[sc.mask[0] for sc in per],
+        rgb=[sc.rgb[0] for sc in per],
+        sparse_xyz=torch.cat([sc.sparse_xyz for sc in per], 0),
+        sparse_offsets=torch.tensor(np.concatenate([[0], np.cumsum(counts)]), dtype=torch.int64, device=torch.device(device)),
     )

@@ -167,6 +167,56 @@ DDN_API int ddn_backproject_filter(const ddn_filter_config* cfg, int64_t n_views
 
 DDN_API int ddn_bbox_init(float* bbox, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Ragged views: stages 1-3 for V views of DIFFERENT sizes (H_v, W_v) in one pass each, as the reference's
+ * per-image loop allows (scripts/test.py:145-173 refines each image at its own size, :275-328 votes with every
+ * cached view at that view's size).  Per-pixel buffers (depth, mask, refined, normal) are the concatenation of
+ * the views' row-major maps; strided-grid buffers (xyz, votes) the concatenation of their
+ * Hs_v x Ws_v = ceil(H_v/stride) x ceil(W_v/stride) grids.  Sizes and offsets travel as a LAYOUT,
+ * int64 [V + 1, DDN_LAYOUT_COLS]:
+ *   row v < V:  H_v, W_v, pix_off[v], grid_off[v], tile_off[v], chunk_off[v], 0, 0
+ *   row V:      stride, V, total pixels, total grid points, total tiles, total chunks, 0, 0
+ * with pix_off[v] = sum_{u<v} H_u W_u, grid_off[v] = sum_{u<v} Hs_u Ws_u, tile_off[v] = sum_{u<v} ceil(H_u/32)
+ * ceil(W_u/126) (remap tiles) and chunk_off[v] = sum_{u<v} ceil(Hs_u Ws_u / 1024) (consistency CTAs): the kernels
+ * run one flat grid over all tiles / chunks and find their view from these prefixes.  Limits: 1 <= V <= 65535,
+ * every side below 2^22, fewer than 2^32 pixels in all.  Each ragged call takes the layout twice: `layout` in
+ * device memory for the kernels and `layout_host`, the same values on the host, which the call validates (the
+ * offsets must be the prefix sums of the sizes) and sizes its launches from, so it never reads the device back.
+ * The uniform entry points above are unchanged; uniform views through the ragged path give the same bits.
+ * ------------------------------------------------------------------------------------------ */
+#define DDN_LAYOUT_COLS 8
+
+/* ddn_align_views over a layout: depth, mask (one byte per pixel, or NULL) and refined are flat [total pixels];
+ * workspace from ddn_align_workspace_bytes(V, ...); stats [V]; src_table [V,16] (ddn_build_pair_tables_ragged) and
+ * bbox as in ddn_align_views (the box's tiles are the ragged tiles of each view).  Needs H_v, W_v >= 2.
+ * cfg->mask_packed and cfg->use_tma are byte-layout options of the uniform call: here they return
+ * DDN_ERR_UNSUPPORTED. */
+DDN_API int ddn_align_views_ragged(const ddn_align_config* cfg, int64_t n_views, const int64_t* layout,
+                           const int64_t* layout_host, const float* depth, const uint8_t* mask,
+                           const double* cam_from_world, const double* kmat, const double* sparse_xyz,
+                           const int64_t* sparse_offsets, int64_t max_sparse_per_view, float* refined,
+                           ddn_view_stats* stats, void* workspace, int64_t workspace_bytes, const float* src_table,
+                           float* bbox, void* stream);
+
+/* ddn_build_pair_tables for all V views of a layout (sources 0..V-1).  Entries as in the uniform tables except
+ * floats 16-19, which describe the NEIGHBOUR's map: W_t, H_t (int bits), (float)W_t, (float)H_t, and the gather
+ * offset (float 21) pix_off[t] - 0x4B000000 (W_t + 1) mod 2^32.  The sizes come from the same layout the
+ * consistency kernel reads, so a table cannot disagree with the maps it is used with. */
+DDN_API int ddn_build_pair_tables_ragged(int64_t n_views, int64_t k_nbr, const int64_t* layout,
+                                 const int64_t* layout_host, const double* cam_from_world, const double* intr,
+                                 const int32_t* nbr, float* pair_table, float* src_table, void* stream);
+
+/* ddn_backproject_filter for all V views of a layout: refined_all flat [total pixels] f32; normal flat
+ * [total pixels, 3] f32 (device or pinned host memory); pair_table / src_table from ddn_build_pair_tables_ragged;
+ * xyz [total grid points, 3] f32 and votes [total grid points] u8 on each view's strided grid.  cfg->stride must
+ * equal the layout's stride.  bbox, vote_threshold and mark as in ddn_backproject_filter; a fusion session then
+ * finishes with row_len = 0. */
+DDN_API int ddn_backproject_filter_ragged(const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
+                                  const int64_t* layout, const int64_t* layout_host, const float* refined_all,
+                                  const float* normal, const float* pair_table, const float* src_table,
+                                  int32_t vote_threshold, float* xyz, uint8_t* votes, float* bbox,
+                                  const struct ddn_fuse_session* mark, void* stream);
+
 /* Neighbouring per-pixel helpers (SURVEY.md 8(f) rank 4).
  * ddn_gradient_mask: compute_depth_normal_gradient_mask, src/depthdensifier/initilizer.py:236-328 - mask_out [H,W]
  *   u8 = 1 where the Sobel magnitude of the (zero-padded, separable) Gaussian-smoothed depth relative to that depth
