@@ -733,6 +733,56 @@ remap_median_kernel(ddn_align_config cfg, int H, int W, int tiles_x, int tiles_y
   if (kBox) tile_bbox_epilogue(bbox, src_table, v, tx0, ty0, W, H, t_dmin, t_dmax, &s_dmin, &s_dmax);
 }
 
+// What an alignment call derives from its config and sparse-point bound: the carved workspace, where K1+K2 sort and keep
+// their pairs (shared or global memory), and how much of K3's lookup table sits in shared memory (lut = 0: none).
+struct AlignPlan {
+  AlignWorkspace ws;
+  int in_smem, pairs_smem, lut;
+  size_t smem_sort, smem_lut;
+};
+
+// The checks and sizes both entry points share, after each has checked its shapes or layout.  With no views it checks
+// the config only and plans nothing.
+static int plan_align(const ddn_align_config* cfg, int64_t n_views, const float* depth, const double* cam_from_world,
+                      const double* kmat, const int64_t* sparse_offsets, const float* refined, const ddn_view_stats* stats,
+                      int64_t max_sparse_per_view, void* workspace, int64_t workspace_bytes, const float* src_table,
+                      const float* bbox, AlignPlan& p) {
+  DDN_REQUIRE(cfg != nullptr, "null config");
+  DDN_REQUIRE((src_table == nullptr) == (bbox == nullptr), "src_table and bbox go together");
+  DDN_REQUIRE(cfg->mode == 0 || cfg->mode == 1, "mode");
+  DDN_REQUIRE(cfg->max_pairs >= 1, "max_pairs");
+  if (n_views == 0) return DDN_OK;
+  DDN_REQUIRE(depth && cam_from_world && kmat && sparse_offsets && refined && stats && workspace, "null pointer");
+  const int64_t C = max_sparse_per_view > 0 ? max_sparse_per_view : 1;
+  DDN_REQUIRE(C < (1ll << 30), "max_sparse_per_view");
+  if (workspace_bytes < align_ws_bytes(n_views, C)) {
+    set_error("align workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)align_ws_bytes(n_views, C));
+    return DDN_ERR_WORKSPACE_TOO_SMALL;
+  }
+  p.ws = carve(workspace, n_views, C);
+  p.in_smem = p.ws.Cp <= kSortSmemMax ? 1 : 0;
+  p.pairs_smem = (p.in_smem && (size_t)p.ws.Cp * 8 + (size_t)p.ws.C * 20 <= 200 * 1024) ? 1 : 0;
+  p.smem_sort = (p.in_smem ? (size_t)p.ws.Cp * 8 : 0) + (p.pairs_smem ? (size_t)p.ws.C * 20 : 0);
+  // largest table any view can have: max_pairs when subsampling, else every surviving pair
+  int64_t lut = (cfg->adaptive_correspondences && cfg->max_pairs < C) ? cfg->max_pairs : C;
+  if (cfg->mode != 0 || lut > kLutSmemMax) lut = 0;  // affine mode has no table; huge tables stay in global
+  p.lut = (int)lut;
+  p.smem_lut = lut > 0 ? (size_t)lut * 8 + (size_t)kBuckets * 4 : 0;
+  return DDN_OK;
+}
+
+template <bool kPacked, bool kBox, bool kTma, bool kRagged>
+static int launch_remap(const ddn_align_config& cfg, const AlignPlan& p, dim3 grid, int H, int W, int tiles_x, int tiles_y,
+                        const float* depth, const uint8_t* mask, const ddn_view_stats* stats, float* refined,
+                        const float* src_table, float* bbox, const CUtensorMap* depth_map, const int64_t* layout, cudaStream_t st) {
+  DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<kPacked, kBox, kTma, kRagged>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)p.smem_lut),
+                     "cudaFuncSetAttribute(remap_median)"));
+  remap_median_kernel<kPacked, kBox, kTma, kRagged><<<grid, kRemapThreads, p.smem_lut, st>>>(
+      cfg, H, W, tiles_x, tiles_y, depth, mask, stats, p.ws, refined, p.lut, src_table, reinterpret_cast<int*>(bbox), depth_map, layout);
+  return after_launch("remap_median_kernel", st);
+}
+
 }  // namespace ddn
 
 extern "C" {
@@ -751,45 +801,29 @@ int ddn_align_views(const ddn_align_config* cfg, int64_t n_views, int64_t height
                     int64_t max_sparse_per_view, float* refined, ddn_view_stats* stats,
                     void* workspace, int64_t workspace_bytes, const float* src_table, float* bbox, void* stream) {
   using namespace ddn;
-  DDN_REQUIRE(cfg != nullptr, "null config");
-  DDN_REQUIRE((src_table == nullptr) == (bbox == nullptr), "src_table and bbox go together");
   DDN_REQUIRE(n_views >= 0 && height > 1 && width > 1, "shape");
   DDN_REQUIRE(height * width < (1ll << 31), "image too large");
-  DDN_REQUIRE(cfg->mode == 0 || cfg->mode == 1, "mode");
-  DDN_REQUIRE(cfg->max_pairs >= 1, "max_pairs");
-  if (n_views == 0) return DDN_OK;
   DDN_REQUIRE(n_views <= 65535, "too many views per call");
-  DDN_REQUIRE(depth && cam_from_world && kmat && sparse_offsets && refined && stats && workspace, "null pointer");
-  const int64_t C = max_sparse_per_view > 0 ? max_sparse_per_view : 1;
-  DDN_REQUIRE(C < (1ll << 30), "max_sparse_per_view");
-  if (cfg->use_tma) {  // tensor-copy form of the remap kernel: checked before anything is launched
+  AlignPlan p;
+  DDN_TRY(plan_align(cfg, n_views, depth, cam_from_world, kmat, sparse_offsets, refined, stats, max_sparse_per_view, workspace,
+                     workspace_bytes, src_table, bbox, p));
+  if (n_views == 0) return DDN_OK;
+  const bool tma = cfg->use_tma != 0;
+  if (tma) {  // tensor-copy form of the remap kernel: checked before anything is launched
     DDN_REQUIRE(width % 4 == 0 && ((uintptr_t)depth & 15) == 0, "use_tma needs W % 4 == 0 and a 16-byte aligned depth pointer");
     DDN_REQUIRE(width >= kTmaBoxW && height >= kHaloH, "use_tma needs an image of at least 132 x 34 pixels");
   }
-  if (workspace_bytes < align_ws_bytes(n_views, C)) {
-    set_error("align workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)align_ws_bytes(n_views, C));
-    return DDN_ERR_WORKSPACE_TOO_SMALL;
-  }
-  AlignWorkspace ws = carve(workspace, n_views, C);
   cudaStream_t st = (cudaStream_t)stream;
-  const int in_smem = ws.Cp <= kSortSmemMax ? 1 : 0;
-  const int pairs_smem = (in_smem && (size_t)ws.Cp * 8 + (size_t)ws.C * 20 <= 200 * 1024) ? 1 : 0;
-  const size_t smem_sort = (in_smem ? (size_t)ws.Cp * 8 : 0) + (pairs_smem ? (size_t)ws.C * 20 : 0);
-  DDN_TRY(check_cuda(cudaFuncSetAttribute(align_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sort),
+  DDN_TRY(check_cuda(cudaFuncSetAttribute(align_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_sort),
                      "cudaFuncSetAttribute(align_stats)"));
-  align_stats_kernel<<<(unsigned)n_views, kStatsThreads, smem_sort, st>>>(*cfg, (int)height, (int)width, depth,
-                                                                         cam_from_world, kmat, sparse_xyz,
-                                                                         sparse_offsets, ws, stats, in_smem, pairs_smem);
+  align_stats_kernel<<<(unsigned)n_views, kStatsThreads, p.smem_sort, st>>>(*cfg, (int)height, (int)width, depth,
+                                                                           cam_from_world, kmat, sparse_xyz,
+                                                                           sparse_offsets, p.ws, stats, p.in_smem, p.pairs_smem);
   DDN_TRY(after_launch("align_stats_kernel", st));
   const int tiles_x = (int)((width + kTileW - 1) / kTileW), tiles_y = (int)((height + kTileH - 1) / kTileH);
-  // largest table any view can have: max_pairs when subsampling, else every surviving pair
-  int64_t lut = (cfg->adaptive_correspondences && cfg->max_pairs < C) ? cfg->max_pairs : C;
-  if (cfg->mode != 0 || lut > kLutSmemMax) lut = 0;  // affine mode has no table; huge tables stay in global
-  const size_t smem_lut = lut > 0 ? (size_t)lut * 8 + (size_t)kBuckets * 4 : 0;
   dim3 grid((unsigned)(tiles_x * tiles_y), (unsigned)n_views);
   CUtensorMap depth_map;
   memset(&depth_map, 0, sizeof(depth_map));
-  const bool tma = cfg->use_tma != 0;
   if (tma) {
     typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -809,34 +843,15 @@ int ddn_align_views(const ddn_align_config* cfg, int64_t n_views, int64_t height
       set_error("cuTensorMapEncodeTiled failed: %d", (int)r);
       return DDN_ERR_CUDA;
     }
-    DDN_TRY(check_cuda(cudaMemcpyAsync(ws.tensor_map, &depth_map, sizeof(depth_map), cudaMemcpyHostToDevice, st), "tensor map upload"));
+    DDN_TRY(check_cuda(cudaMemcpyAsync(p.ws.tensor_map, &depth_map, sizeof(depth_map), cudaMemcpyHostToDevice, st), "tensor map upload"));
   }
-  const CUtensorMap* depth_map_dev = reinterpret_cast<const CUtensorMap*>(ws.tensor_map);
-#define DDN_LAUNCH_REMAP(P, B)                                                                                              \
-  do {                                                                                                                      \
-    if (tma) {                                                                                                              \
-      DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<P, B, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                              (int)smem_lut),                                                               \
-                         "cudaFuncSetAttribute(remap_median)"));                                                            \
-      remap_median_kernel<P, B, true, false><<<grid, kRemapThreads, smem_lut, st>>>(                                               \
-          *cfg, (int)height, (int)width, tiles_x, tiles_y, depth, mask, stats, ws, refined, (int)lut, src_table,            \
-          reinterpret_cast<int*>(bbox), depth_map_dev, nullptr);                                                            \
-    } else {                                                                                                                \
-      DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<P, B, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                              (int)smem_lut),                                                               \
-                         "cudaFuncSetAttribute(remap_median)"));                                                            \
-      remap_median_kernel<P, B, false, false><<<grid, kRemapThreads, smem_lut, st>>>(                                              \
-          *cfg, (int)height, (int)width, tiles_x, tiles_y, depth, mask, stats, ws, refined, (int)lut, src_table,            \
-          reinterpret_cast<int*>(bbox), depth_map_dev, nullptr);                                                            \
-    }                                                                                                                       \
-  } while (0)
-  const bool packed = cfg->mask_packed != 0 && mask != nullptr, box = bbox != nullptr;
-  if (packed && box) DDN_LAUNCH_REMAP(true, true);
-  else if (packed) DDN_LAUNCH_REMAP(true, false);
-  else if (box) DDN_LAUNCH_REMAP(false, true);
-  else DDN_LAUNCH_REMAP(false, false);
-#undef DDN_LAUNCH_REMAP
-  return after_launch("remap_median_kernel", st);
+  const bool packed = cfg->mask_packed != 0 && mask != nullptr, with_box = bbox != nullptr;
+  const auto launch = packed ? (with_box ? (tma ? &launch_remap<true, true, true, false> : &launch_remap<true, true, false, false>)
+                                         : (tma ? &launch_remap<true, false, true, false> : &launch_remap<true, false, false, false>))
+                             : (with_box ? (tma ? &launch_remap<false, true, true, false> : &launch_remap<false, true, false, false>)
+                                         : (tma ? &launch_remap<false, false, true, false> : &launch_remap<false, false, false, false>));
+  return launch(*cfg, p, grid, (int)height, (int)width, tiles_x, tiles_y, depth, mask, stats, refined, src_table, bbox,
+                reinterpret_cast<const CUtensorMap*>(p.ws.tensor_map), nullptr, st);
 }
 
 int ddn_align_views_ragged(const ddn_align_config* cfg, int64_t n_views, const int64_t* layout, const int64_t* layout_host,
@@ -845,52 +860,26 @@ int ddn_align_views_ragged(const ddn_align_config* cfg, int64_t n_views, const i
                            ddn_view_stats* stats, void* workspace, int64_t workspace_bytes, const float* src_table, float* bbox,
                            void* stream) {
   using namespace ddn;
-  DDN_REQUIRE(cfg != nullptr, "null config");
-  if (cfg->mask_packed || cfg->use_tma) {
-    set_error("ddn_align_views_ragged: mask_packed and use_tma are options of the uniform ddn_align_views only");
-    return DDN_ERR_UNSUPPORTED;
-  }
-  DDN_REQUIRE((src_table == nullptr) == (bbox == nullptr), "src_table and bbox go together");
   DDN_REQUIRE(layout != nullptr, "null layout");
   DDN_TRY(check_layout(n_views, layout_host));
   for (int64_t v = 0; v < n_views; ++v)
     DDN_REQUIRE(layout_host[v * DDN_LAYOUT_COLS] > 1 && layout_host[v * DDN_LAYOUT_COLS + 1] > 1, "every view needs H, W >= 2");
-  DDN_REQUIRE(cfg->mode == 0 || cfg->mode == 1, "mode");
-  DDN_REQUIRE(cfg->max_pairs >= 1, "max_pairs");
-  DDN_REQUIRE(depth && cam_from_world && kmat && sparse_offsets && refined && stats && workspace, "null pointer");
-  const int64_t C = max_sparse_per_view > 0 ? max_sparse_per_view : 1;
-  DDN_REQUIRE(C < (1ll << 30), "max_sparse_per_view");
-  if (workspace_bytes < align_ws_bytes(n_views, C)) {
-    set_error("align workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)align_ws_bytes(n_views, C));
-    return DDN_ERR_WORKSPACE_TOO_SMALL;
+  AlignPlan p;
+  DDN_TRY(plan_align(cfg, n_views, depth, cam_from_world, kmat, sparse_offsets, refined, stats, max_sparse_per_view, workspace,
+                     workspace_bytes, src_table, bbox, p));
+  if (cfg->mask_packed || cfg->use_tma) {
+    set_error("ddn_align_views_ragged: mask_packed and use_tma are options of the uniform ddn_align_views only");
+    return DDN_ERR_UNSUPPORTED;
   }
-  AlignWorkspace ws = carve(workspace, n_views, C);
   cudaStream_t st = (cudaStream_t)stream;
-  const int in_smem = ws.Cp <= kSortSmemMax ? 1 : 0;
-  const int pairs_smem = (in_smem && (size_t)ws.Cp * 8 + (size_t)ws.C * 20 <= 200 * 1024) ? 1 : 0;
-  const size_t smem_sort = (in_smem ? (size_t)ws.Cp * 8 : 0) + (pairs_smem ? (size_t)ws.C * 20 : 0);
-  DDN_TRY(check_cuda(cudaFuncSetAttribute(align_stats_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sort),
+  DDN_TRY(check_cuda(cudaFuncSetAttribute(align_stats_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_sort),
                      "cudaFuncSetAttribute(align_stats_ragged)"));
-  align_stats_ragged_kernel<<<(unsigned)n_views, kStatsThreads, smem_sort, st>>>(*cfg, layout, depth, cam_from_world, kmat, sparse_xyz,
-                                                                                sparse_offsets, ws, stats, in_smem, pairs_smem);
+  align_stats_ragged_kernel<<<(unsigned)n_views, kStatsThreads, p.smem_sort, st>>>(*cfg, layout, depth, cam_from_world, kmat, sparse_xyz,
+                                                                                  sparse_offsets, p.ws, stats, p.in_smem, p.pairs_smem);
   DDN_TRY(after_launch("align_stats_ragged_kernel", st));
-  int64_t lut = (cfg->adaptive_correspondences && cfg->max_pairs < C) ? cfg->max_pairs : C;
-  if (cfg->mode != 0 || lut > kLutSmemMax) lut = 0;
-  const size_t smem_lut = lut > 0 ? (size_t)lut * 8 + (size_t)kBuckets * 4 : 0;
   const unsigned tiles = (unsigned)layout_host[n_views * DDN_LAYOUT_COLS + 4];
-#define DDN_LAUNCH_REMAP_RAGGED(B)                                                                                               \
-  do {                                                                                                                           \
-    DDN_TRY(check_cuda(cudaFuncSetAttribute(remap_median_kernel<false, B, false, true>,                                      \
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lut),                         \
-                       "cudaFuncSetAttribute(remap_median)"));                                                                   \
-    remap_median_kernel<false, B, false, true><<<tiles, kRemapThreads, smem_lut, st>>>(                                          \
-        *cfg, 0, 0, 1, (int)n_views, depth, mask, stats, ws, refined, (int)lut, src_table, reinterpret_cast<int*>(bbox), nullptr, \
-        layout);                                                                                                                 \
-  } while (0)
-  if (bbox != nullptr) DDN_LAUNCH_REMAP_RAGGED(true);
-  else DDN_LAUNCH_REMAP_RAGGED(false);
-#undef DDN_LAUNCH_REMAP_RAGGED
-  return after_launch("remap_median_kernel", st);
+  const auto launch = bbox != nullptr ? &launch_remap<false, true, false, true> : &launch_remap<false, false, false, true>;
+  return launch(*cfg, p, dim3(tiles), 0, 0, 1, (int)n_views, depth, mask, stats, refined, src_table, bbox, nullptr, layout, st);
 }
 
 }  // extern "C"

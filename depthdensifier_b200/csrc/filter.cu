@@ -640,10 +640,17 @@ __global__ void bbox_init_kernel(int* bbox) {
   else if (threadIdx.x < 6) bbox[threadIdx.x] = float_to_ordered(-INFINITY);
 }
 
-// The FilterParams fields both entry points share (everything but the sizes and the source range).
+// The checks and FilterParams fields both entry points share (everything but the sizes and the source range).
 static int fill_filter_params(const ddn_filter_config* cfg, const float* refined_all, const float* normal,
                               const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
                               uint8_t* votes, float* bbox, const ddn_fuse_session* mark, int64_t k_nbr, FilterParams& p) {
+  DDN_REQUIRE(cfg != nullptr, "null config");
+  DDN_REQUIRE(k_nbr > 0 && k_nbr <= 1024, "view counts (at most 1024 neighbours per view)");
+  DDN_REQUIRE(cfg->stride >= 1, "stride");
+  DDN_REQUIRE(cfg->pixel_layout == 0 || cfg->pixel_layout == 1, "pixel_layout");
+  DDN_REQUIRE(refined_all && normal && pair_table && src_table && xyz && votes, "null pointer");
+  DDN_REQUIRE((reinterpret_cast<uintptr_t>(pair_table) & 15) == 0 && (reinterpret_cast<uintptr_t>(src_table) & 15) == 0,
+              "pair_table / src_table must be 16-byte aligned");
   p.refined_all = refined_all;
   p.normal = normal;
   p.pair_table = pair_table;
@@ -747,20 +754,14 @@ int ddn_backproject_filter(const ddn_filter_config* cfg, int64_t n_views_total, 
                            float* xyz, uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
   using namespace ddn;
   (void)nbr;
-  DDN_REQUIRE(cfg != nullptr, "null config");
-  DDN_REQUIRE(n_views_total > 0 && n_src >= 0 && k_nbr > 0 && k_nbr <= 1024, "view counts (at most 1024 neighbours per view)");
+  DDN_REQUIRE(n_views_total > 0 && n_src >= 0, "view counts");
   DDN_REQUIRE(src_begin >= 0 && src_begin + n_src <= n_views_total, "source range");
   DDN_REQUIRE(height > 0 && width > 0 && height * width < (1ll << 31), "image size");
   DDN_REQUIRE(n_views_total * height * width < (1ll << 32), "refined_all must hold fewer than 2^32 pixels (32-bit gather offsets)");
   DDN_REQUIRE(width < (1 << 22) && height < (1 << 22), "image side too large for the truncation trick");
-  DDN_REQUIRE(cfg->stride >= 1, "stride");
-  DDN_REQUIRE(cfg->pixel_layout == 0 || cfg->pixel_layout == 1, "pixel_layout");
-  DDN_REQUIRE(refined_all && normal && pair_table && src_table && xyz && votes, "null pointer");
-  DDN_REQUIRE((reinterpret_cast<uintptr_t>(pair_table) & 15) == 0 && (reinterpret_cast<uintptr_t>(src_table) & 15) == 0,
-              "pair_table / src_table must be 16-byte aligned");
-  if (n_src == 0) return DDN_OK;
   FilterParams p;
   DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
+  if (n_src == 0) return DDN_OK;
   p.src_begin = (int)src_begin;
   p.n_src = (int)n_src;
   p.H = (int)height;
@@ -798,17 +799,11 @@ int ddn_backproject_filter_ragged(const ddn_filter_config* cfg, int64_t n_views,
                                   const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
                                   uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
   using namespace ddn;
-  DDN_REQUIRE(cfg != nullptr, "null config");
-  DDN_REQUIRE(k_nbr > 0 && k_nbr <= 1024, "view counts (at most 1024 neighbours per view)");
-  DDN_REQUIRE(layout != nullptr, "null layout");
-  DDN_TRY(check_layout(n_views, layout_host));
-  DDN_REQUIRE(cfg->stride >= 1 && cfg->stride == layout_host[n_views * DDN_LAYOUT_COLS], "cfg->stride must be the layout's stride");
-  DDN_REQUIRE(cfg->pixel_layout == 0 || cfg->pixel_layout == 1, "pixel_layout");
-  DDN_REQUIRE(refined_all && normal && pair_table && src_table && xyz && votes, "null pointer");
-  DDN_REQUIRE((reinterpret_cast<uintptr_t>(pair_table) & 15) == 0 && (reinterpret_cast<uintptr_t>(src_table) & 15) == 0,
-              "pair_table / src_table must be 16-byte aligned");
   FilterParams p;
   DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
+  DDN_REQUIRE(layout != nullptr, "null layout");
+  DDN_TRY(check_layout(n_views, layout_host));
+  DDN_REQUIRE(cfg->stride == layout_host[n_views * DDN_LAYOUT_COLS], "cfg->stride must be the layout's stride");
   p.src_begin = 0;
   p.n_src = (int)n_views;
   p.H = p.W = p.Hs = p.Ws = 0;  // per view, from the layout and the table entries

@@ -34,8 +34,7 @@ import numpy as np
 import torch
 
 from . import ops
-from .engine import DensifyConfig, DensifyResult, clamp_vote_threshold
-from .neighbours import default_vote_threshold
+from .engine import DensifyConfig, DensifyResult, max_sparse_count
 
 
 def shard_bounds(n_views: int, world: int) -> list[tuple[int, int]]:
@@ -150,7 +149,7 @@ class ShardedDensifier:
         self.rank, self.world, self.group = rank, world, group
         self.V, self.lo, self.hi, self.H, self.W = n_views_total, lo, hi, height, width
         self.K = nbr.shape[1]
-        self.thr = clamp_vote_threshold(cfg.vote_threshold if cfg.vote_threshold is not None else default_vote_threshold(self.K))
+        self.thr = cfg.vote_threshold_for(self.K)
         bounds = shard_bounds(n_views_total, world) if world > 1 else [(lo, hi)]
         if world > 1 and bounds[rank] != (lo, hi):
             raise ValueError(f"rank {rank}: shard {(lo, hi)} does not match the contiguous layout {bounds[rank]}")
@@ -161,10 +160,7 @@ class ShardedDensifier:
         self.nbr_slots = torch.from_numpy(self.plan.nbr_slots).to(self.device).contiguous()
         self.n_local = hi - lo
         self.n_slots = len(self.plan.slots)
-        kmat = torch.zeros((self.n_local, 3, 3), dtype=torch.float64, device=self.device)
-        il = self.intr_slots[: self.n_local]
-        kmat[:, 0, 0], kmat[:, 1, 1], kmat[:, 0, 2], kmat[:, 1, 2], kmat[:, 2, 2] = il[:, 0], il[:, 1], il[:, 2], il[:, 3], 1.0
-        self.kmat = kmat
+        self.kmat = ops.intrinsics_matrix(self.intr_slots[: self.n_local])
         self._max_sparse = None
         self._host_out = None
         # NVLink peer reads for the two exchange steps (CUDA, world > 1); the collective path (all-to-all-v)
@@ -321,8 +317,7 @@ class ShardedDensifier:
             return out
 
         if self._max_sparse is None:
-            off = sparse_offsets.cpu().numpy()
-            self._max_sparse = max(int(np.max(np.diff(off))) if len(off) > 1 else 1, 1)
+            self._max_sparse = max_sparse_count(sparse_offsets)
         fuse = cfg.voxel is not None
 
         def stage1():
@@ -387,10 +382,7 @@ class ShardedDensifier:
         return res
 
     def _pair_tables(self):
-        if self.device_path:
-            return self.ops.build_pair_tables(self.poses_slots, self.intr_slots, self._nbr_full(), 0, self.n_local, self.H, self.W)
-        return self.ops.build_pair_tables(self.poses_slots, self.intr_slots, self._nbr_full(), 0, self.n_local, height=self.H,
-                                          width=self.W)
+        return self.ops.build_pair_tables(self.poses_slots, self.intr_slots, self._nbr_full(), 0, self.n_local, self.H, self.W)
 
     def _new_box(self) -> torch.Tensor:
         """Bounding box of this rank's back-projected pixels (filled by the alignment kernel); in peer-visible
@@ -688,8 +680,7 @@ class ShardedDensifier:
             copy.wait_event(st["free"])  # the call before the previous one is done with this set's staging buffers
         n = self.n_local
         if self._max_sparse is None:
-            off = sparse_offsets.numpy()
-            self._max_sparse = max(int(np.max(np.diff(off))) if len(off) > 1 else 1, 1)
+            self._max_sparse = max_sparse_count(sparse_offsets)
         h2d = 0
 
         def upload(dst, src):

@@ -29,11 +29,21 @@ class DensifyConfig:
     # run() is called - they are not ordered against work the caller queued on the current stream just before.
     overlap_align: bool = False
 
+    def vote_threshold_for(self, k: int) -> int:
+        """The threshold a step with ``k`` neighbours per view votes with (``vote_threshold`` or ceil(k/2), clamped)."""
+        return clamp_vote_threshold(self.vote_threshold if self.vote_threshold is not None else default_vote_threshold(k))
+
 
 def clamp_vote_threshold(thr: int) -> int:
     """Votes are stored as u8, saturated at 254, with 255 = "pixel has no point": a threshold of 255 or more keeps
     every point that exists (and never a pixel without one), 0 or less keeps none."""
     return max(0, min(int(thr), 255))
+
+
+def max_sparse_count(sparse_offsets) -> int:
+    """The most sparse points any view has (at least 1), from the offsets [V+1] (synchronises on a device tensor)."""
+    off = sparse_offsets.cpu().numpy()
+    return max(int(np.max(np.diff(off))) if len(off) > 1 else 1, 1)
 
 
 @dataclass
@@ -53,6 +63,8 @@ class DensifyResult:
     session: object | None = None  # ops.FuseSession that produced the voxels (device-resident grid)
     bbox_valid: torch.Tensor | None = None  # [6] i32: box of every back-projected pixel (the alignment kernel's bound)
     layout: ops.ViewLayout | None = None  # run_views: refined [P], xyz [G,3], votes [G] are flat over the views of this layout
+    rgb: torch.Tensor | None = None  # the step's colours: [V,H,W,3] u8, or flat [P,3] u8 over the views of ``layout``
+    stride: int = 1  # back-projection grid stride: xyz / votes hold every stride-th row and column
 
     def per_view(self, name: str) -> list:
         """Per-view views of a flat output of run_views: ``refined`` -> [H_v, W_v], ``xyz`` -> [Hs_v, Ws_v, 3],
@@ -63,6 +75,20 @@ class DensifyResult:
 
     def keep_mask(self) -> torch.Tensor:
         return (self.votes != 255) & (self.votes < clamp_vote_threshold(self.vote_threshold))
+
+    def grid_rgb(self) -> torch.Tensor:
+        """The colours on the back-projection grid, in the order of ``xyz``: [V,Hs,Ws,3], or flat [G,3] for run_views."""
+        s = self.stride
+        if s == 1:
+            return self.rgb
+        if self.layout is None:
+            return self.rgb[:, ::s, ::s].contiguous()
+        return torch.cat([r.reshape(-1, 3) for r in self.layout.strided(self.layout.split(self.rgb))], 0)
+
+    def kept_points(self) -> tuple[torch.Tensor, torch.Tensor]:
+        """xyz [M,3] f32 and rgb [M,3] u8 of the points the vote keeps, view by view in grid order."""
+        keep = self.keep_mask()
+        return self.xyz[keep], self.grid_rgb()[keep]
 
     def host_grid(self):
         """The voxel grid as a host struct (synchronises; raises when the device could not build one)."""
@@ -97,25 +123,8 @@ class DensifyEngine:
 
     def align(self, depth, mask, cam_from_world, intr, sparse_xyz, sparse_offsets, max_sparse_per_view, out=None,
               src_table=None, bbox=None):
-        V = depth.shape[0]
-        kmat = torch.zeros((V, 3, 3), dtype=torch.float64, device=depth.device)
-        kmat[:, 0, 0] = intr[:, 0]
-        kmat[:, 1, 1] = intr[:, 1]
-        kmat[:, 0, 2] = intr[:, 2]
-        kmat[:, 1, 2] = intr[:, 3]
-        kmat[:, 2, 2] = 1.0
-        return ops.align_views(depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets, max_sparse_per_view,
-                               self.cfg.align, out=out, src_table=src_table, bbox=bbox)
-
-    def _fuse(self, res, sess, grid, xyz, rgb_s, votes, sparse_xyz, thr, row_len, sync):
-        if self.cfg.dedup_sparse and sparse_xyz.shape[0] > 0:
-            sess.unmark_points(sparse_xyz.float().contiguous())
-        k, x, c, n, counts = ops.fuse_finish(sess, xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), thr, row_len=row_len)
-        res.session, res.grid = sess, grid
-        res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts.clone()
-        if sync:
-            mv = res.check()
-            res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count = k[:mv], x[:mv], c[:mv], n[:mv]
+        return ops.align_views(depth, mask, cam_from_world, ops.intrinsics_matrix(intr), sparse_xyz, sparse_offsets,
+                               max_sparse_per_view, self.cfg.align, out=out, src_table=src_table, bbox=bbox)
 
     def session(self) -> ops.FuseSession:
         if getattr(self, "_session", None) is None or self._session.max_cells != self.cfg.max_grid_cells:
@@ -133,36 +142,8 @@ class DensifyEngine:
         fusion passes read the grid from device memory.  ``sync`` (default): wait at the end, validate
         (``DensifyResult.check()``) and trim the voxel arrays to their count; without it the arrays keep their
         capacity and ``counts`` [2] on the device says how many entries are valid."""
-        cfg = self.cfg
-        V, H, W = depth.shape
-        K = nbr.shape[1]
-        if max_sparse_per_view is None:
-            off = sparse_offsets.cpu().numpy()
-            max_sparse_per_view = int(np.max(np.diff(off))) if V > 0 else 1
-        thr = clamp_vote_threshold(cfg.vote_threshold if cfg.vote_threshold is not None else default_vote_threshold(K))
-        pair, src = ops.build_pair_tables(cam_from_world, intr, nbr, 0, V, H, W)
-        fuse = cfg.voxel is not None
-        box = ops.new_bbox(depth.device) if fuse and grid is None else None
-        kmat = None
-        refined = torch.empty_like(depth)
-        refined, stats = self.align(depth, mask, cam_from_world, intr, sparse_xyz, sparse_offsets, max(max_sparse_per_view, 1),
-                                    out=refined, src_table=src if box is not None else None, bbox=box)
-        sess = None
-        if fuse:
-            sess = self.session()
-            if grid is None:
-                sess.begin([box], cfg.voxel)
-            else:
-                sess.begin_grid(grid)
-        bbox = ops.new_bbox(depth.device)
-        xyz, votes = ops.backproject_filter(refined, normal, nbr, pair, src, 0, thr, cfg.filter, bbox=bbox, mark=sess)
-        res = DensifyResult(refined=refined, stats=stats, xyz=xyz, votes=votes, vote_threshold=thr, bbox=bbox)
-        if fuse:
-            s = cfg.filter.stride
-            rgb_s = rgb if s == 1 else rgb[:, ::s, ::s].contiguous()
-            self._fuse(res, sess, grid, xyz, rgb_s, votes, sparse_xyz, thr, xyz.shape[2], sync)
-        res.bbox_valid = box
-        return res
+        return self._step(None, depth, normal, mask, rgb, cam_from_world, intr, sparse_xyz, sparse_offsets, nbr,
+                          max_sparse_per_view, grid, sync)
 
     def run_views(self, depths, normals, masks, rgbs, cam_from_world, intr, sparse_xyz, sparse_offsets, nbr,
                   max_sparse_per_view: int | None = None, grid=None, sync: bool = True,
@@ -174,31 +155,34 @@ class DensifyEngine:
         The same step as ``run`` - one launch per stage over all views, no host round trip - on the flat layout
         (include/ddn_b200.h, DDN_LAYOUT_COLS).  The result's refined [P], xyz [G,3] and votes [G] are flat in view order
         (``DensifyResult.per_view`` splits them); keep_mask() and the voxel outputs mean what they mean for ``run``."""
+        if layout is None:
+            layout = ops.ViewLayout.from_shapes([tuple(d.shape) for d in depths], self.cfg.filter.stride)
+            on_device = normals[0].is_cuda
+            depths, normals = layout.flatten(depths, torch.float32), layout.flatten(normals, torch.float32)
+            normals = normals if on_device else normals.pin_memory()
+            masks = layout.flatten(masks) if masks is not None else None
+            rgbs = layout.flatten(rgbs) if rgbs is not None else None
+        return self._step(layout, depths, normals, masks, rgbs, cam_from_world, intr, sparse_xyz, sparse_offsets, nbr,
+                          max_sparse_per_view, grid, sync)
+
+    def _step(self, layout, depth, normal, mask, rgb, cam_from_world, intr, sparse_xyz, sparse_offsets, nbr,
+              max_sparse_per_view, grid, sync) -> DensifyResult:
+        """align -> back-project + vote with mark -> fusion over [V,H,W] maps (``layout`` None, the uniform kernels) or
+        over the flat maps of ``layout`` (the ragged kernels)."""
         cfg = self.cfg
         dev = cam_from_world.device
-        if layout is None:
-            layout = ops.ViewLayout.from_shapes([tuple(d.shape) for d in depths], cfg.filter.stride)
-            depth = layout.flatten(depths, torch.float32)
-            normal = layout.flatten(normals, torch.float32) if normals[0].is_cuda else \
-                layout.flatten(normals, torch.float32).pin_memory()
-            mask = layout.flatten(masks) if masks is not None else None
-            rgb_flat = layout.flatten(rgbs) if rgbs is not None else None
-        else:
-            depth, normal, mask, rgb_flat = depths, normals, masks, rgbs
-        V = layout.n_views
-        K = nbr.shape[1]
+        thr = cfg.vote_threshold_for(nbr.shape[1])
         if max_sparse_per_view is None:
-            off = sparse_offsets.cpu().numpy()
-            max_sparse_per_view = int(np.max(np.diff(off))) if V > 0 else 1
-        thr = clamp_vote_threshold(cfg.vote_threshold if cfg.vote_threshold is not None else default_vote_threshold(K))
-        pair, src = ops.build_pair_tables_ragged(layout, cam_from_world, intr, nbr)
+            max_sparse_per_view = max_sparse_count(sparse_offsets)
+        pair, src = (ops.build_pair_tables(cam_from_world, intr, nbr, 0, *depth.shape) if layout is None
+                     else ops.build_pair_tables_ragged(layout, cam_from_world, intr, nbr))
         fuse = cfg.voxel is not None
         box = ops.new_bbox(dev) if fuse and grid is None else None
-        kmat = torch.zeros((V, 3, 3), dtype=torch.float64, device=dev)
-        kmat[:, 0, 0], kmat[:, 1, 1], kmat[:, 0, 2], kmat[:, 1, 2], kmat[:, 2, 2] = intr[:, 0], intr[:, 1], intr[:, 2], intr[:, 3], 1.0
-        refined, stats = ops.align_views_ragged(layout, depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets,
-                                                max(max_sparse_per_view, 1), cfg.align, src_table=src if box is not None else None,
-                                                bbox=box)
+        args = (depth, mask, cam_from_world, ops.intrinsics_matrix(intr), sparse_xyz, sparse_offsets, max(max_sparse_per_view, 1),
+                cfg.align)
+        box_args = dict(src_table=src if box is not None else None, bbox=box)
+        refined, stats = (ops.align_views(*args, **box_args) if layout is None
+                          else ops.align_views_ragged(layout, *args, **box_args))
         sess = None
         if fuse:
             sess = self.session()
@@ -207,13 +191,20 @@ class DensifyEngine:
             else:
                 sess.begin_grid(grid)
         bbox = ops.new_bbox(dev)
-        xyz, votes = ops.backproject_filter_ragged(layout, refined, normal, pair, src, thr, cfg.filter, bbox=bbox, mark=sess)
-        res = DensifyResult(refined=refined, stats=stats, xyz=xyz, votes=votes, vote_threshold=thr, bbox=bbox, layout=layout)
+        xyz, votes = (ops.backproject_filter(refined, normal, nbr, pair, src, 0, thr, cfg.filter, bbox=bbox, mark=sess)
+                      if layout is None else
+                      ops.backproject_filter_ragged(layout, refined, normal, pair, src, thr, cfg.filter, bbox=bbox, mark=sess))
+        res = DensifyResult(refined=refined, stats=stats, xyz=xyz, votes=votes, vote_threshold=thr, bbox=bbox, bbox_valid=box,
+                            layout=layout, rgb=rgb, stride=cfg.filter.stride)
         if fuse:
-            if layout.stride == 1:
-                rgb_s = rgb_flat
-            else:
-                rgb_s = torch.cat([r.reshape(-1, 3) for r in layout.strided(layout.split(rgb_flat))], 0)
-            self._fuse(res, sess, grid, xyz, rgb_s, votes, sparse_xyz, thr, 0, sync)  # row_len 0: rows differ per view
-        res.bbox_valid = box
+            rgb_s = res.grid_rgb()
+            if cfg.dedup_sparse and sparse_xyz.shape[0] > 0:
+                sess.unmark_points(sparse_xyz.float().contiguous())
+            row_len = xyz.shape[2] if layout is None else 0  # 0: the rows differ from view to view
+            k, x, c, n, counts = ops.fuse_finish(sess, xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), thr, row_len=row_len)
+            res.session, res.grid = sess, grid
+            res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts.clone()
+            if sync:
+                mv = res.check()
+                res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count = k[:mv], x[:mv], c[:mv], n[:mv]
         return res

@@ -41,6 +41,14 @@ def _require_cuda(*tensors) -> torch.device:
     return dev
 
 
+def _require_cuda_normal(normal, *tensors) -> torch.device:
+    """_require_cuda for the consistency kernel's inputs: ``normal`` may also be a pinned host tensor."""
+    normal_on_host = not normal.is_cuda
+    if normal_on_host and not (normal.is_pinned() and normal.is_contiguous()):
+        raise DDNError("a host normal map must be pinned and contiguous")
+    return _require_cuda(None if normal_on_host else normal, *tensors)
+
+
 def _p(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
@@ -108,6 +116,21 @@ class FilterOptions:
         )
 
 
+def intrinsics_matrix(intr) -> torch.Tensor:
+    """[V,3,3] f64 camera matrices from PINHOLE intrinsics [V,4] = (fx, fy, cx, cy)."""
+    kmat = torch.zeros((intr.shape[0], 3, 3), dtype=torch.float64, device=intr.device)
+    kmat[:, 0, 0], kmat[:, 1, 1], kmat[:, 0, 2], kmat[:, 1, 2], kmat[:, 2, 2] = intr[:, 0], intr[:, 1], intr[:, 2], intr[:, 3], 1.0
+    return kmat
+
+
+def _align_scratch(lib, n_views: int, max_sparse_per_view: int, dev):
+    """The zeroed stats [V,8] and the workspace (tensor, bytes) of one alignment call."""
+    stats = torch.zeros((n_views, 8), dtype=torch.int32, device=dev)
+    nbytes = C.c_int64(0)
+    _lib.check(lib.ddn_align_workspace_bytes(n_views, max_sparse_per_view, C.byref(nbytes)))
+    return stats, torch.empty(nbytes.value, dtype=torch.uint8, device=dev), nbytes.value
+
+
 def align_views(depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets, max_sparse_per_view: int,
                 opts: AlignOptions, out=None, src_table=None, bbox=None):
     """Stage 1 for V views.  Returns (refined [V,H,W] f32, stats [V,8] int32 raw ddn_view_stats).
@@ -126,16 +149,13 @@ def align_views(depth, mask, cam_from_world, kmat, sparse_xyz, sparse_offsets, m
         mask.dtype in (torch.bool, torch.uint8) and mask.shape == depth.shape)
     assert tuple(cam_from_world.shape) == (V, 3, 4) and tuple(kmat.shape) == (V, 3, 3)
     refined = out if out is not None else torch.empty_like(depth)
-    stats = torch.zeros((V, 8), dtype=torch.int32, device=dev)
-    nbytes = C.c_int64(0)
-    _lib.check(lib.ddn_align_workspace_bytes(V, max_sparse_per_view, C.byref(nbytes)))
-    ws = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+    stats, ws, nbytes = _align_scratch(lib, V, max_sparse_per_view, dev)
     cfg = opts.to_c(mask_packed=packed)
     with torch.cuda.device(dev):
         _lib.check(
             lib.ddn_align_views(
                 C.byref(cfg), V, H, W, _p(depth), _p(mask), _p(cam_from_world), _p(kmat), _p(sparse_xyz),
-                _p(sparse_offsets), int(max_sparse_per_view), _p(refined), _p(stats), _p(ws), nbytes.value, _p(src_table),
+                _p(sparse_offsets), int(max_sparse_per_view), _p(refined), _p(stats), _p(ws), nbytes, _p(src_table),
                 _p(bbox), _stream(),
             )
         )
@@ -212,10 +232,7 @@ def backproject_filter(refined_all, normal, nbr, pair_table, src_table, src_begi
     (unified addressing) and the 12 B/pixel normal map never moves to the device.  ``mark``: an open
     ``FuseSession``; the kernel then also sets the occupancy bits of the kept points (stage 4's mark pass)."""
     lib = _lib.load()
-    normal_on_host = not normal.is_cuda
-    if normal_on_host and not (normal.is_pinned() and normal.is_contiguous()):
-        raise DDNError("a host normal map must be pinned and contiguous")
-    dev = _require_cuda(refined_all, None if normal_on_host else normal, nbr, pair_table, src_table, bbox, xyz_out, votes_out)
+    dev = _require_cuda_normal(normal, refined_all, nbr, pair_table, src_table, bbox, xyz_out, votes_out)
     V, H, W = refined_all.shape
     n_src = normal.shape[0]
     K = nbr.shape[1]
@@ -350,16 +367,13 @@ def align_views_ragged(layout: ViewLayout, depth, mask, cam_from_world, kmat, sp
     assert tuple(cam_from_world.shape) == (V, 3, 4) and tuple(kmat.shape) == (V, 3, 3)
     assert sparse_xyz.dtype == torch.float64 and sparse_offsets.dtype == torch.int64
     refined = out if out is not None else torch.empty_like(depth)
-    stats = torch.zeros((V, 8), dtype=torch.int32, device=dev)
-    nbytes = C.c_int64(0)
-    _lib.check(lib.ddn_align_workspace_bytes(V, max_sparse_per_view, C.byref(nbytes)))
-    ws = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+    stats, ws, nbytes = _align_scratch(lib, V, max_sparse_per_view, dev)
     cfg = opts.to_c()
     with torch.cuda.device(dev):
         _lib.check(
             lib.ddn_align_views_ragged(
                 C.byref(cfg), V, _p(layout.device(dev)), layout.host_ptr(), _p(depth), _p(mask), _p(cam_from_world), _p(kmat),
-                _p(sparse_xyz), _p(sparse_offsets), int(max_sparse_per_view), _p(refined), _p(stats), _p(ws), nbytes.value,
+                _p(sparse_xyz), _p(sparse_offsets), int(max_sparse_per_view), _p(refined), _p(stats), _p(ws), nbytes,
                 _p(src_table), _p(bbox), _stream(),
             )
         )
@@ -387,10 +401,7 @@ def backproject_filter_ragged(layout: ViewLayout, refined_all, normal, pair_tabl
     Returns xyz [G,3] f32 and votes [G] u8 on the views' strided grids (G = layout.total_grid); ``opts.stride`` must be
     the layout's stride."""
     lib = _lib.load()
-    normal_on_host = not normal.is_cuda
-    if normal_on_host and not (normal.is_pinned() and normal.is_contiguous()):
-        raise DDNError("a host normal map must be pinned and contiguous")
-    dev = _require_cuda(refined_all, None if normal_on_host else normal, pair_table, src_table, bbox, xyz_out, votes_out)
+    dev = _require_cuda_normal(normal, refined_all, pair_table, src_table, bbox, xyz_out, votes_out)
     V, P, G = layout.n_views, layout.total_pixels, layout.total_grid
     K = pair_table.shape[1]
     assert refined_all.dtype == torch.float32 and tuple(refined_all.shape) == (P,)

@@ -248,7 +248,6 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
         intr.append(np.array(camera.params[:4], dtype=np.float64))
     if not views:
         raise ValueError("no registered image observes any sparse point")
-    uniform = len({d.shape for d in depths}) == 1  # else: views of different sizes, the ragged form of the device pipeline
     V = len(views)
     if (config.filtering.num_neighbours is None or config.filtering.num_neighbours >= V) and V > 1024:
         raise ValueError(f"{V} views: testing every view against every view (the reference's behaviour, K = V) is limited to "
@@ -277,27 +276,17 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
                                       voxel=config.fusion.voxel_size, dedup_sparse=bool(config.fusion.dedup_sparse)), device=dev)
     offsets = np.concatenate([[0], np.cumsum([len(p) for p in sparse])]).astype(np.int64)
     to = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(dev)
-    s = filt.stride
-    if uniform:
-        rgb_dev = to(np.stack(rgbs), torch.uint8)
-        res = eng.run(to(np.stack(depths), torch.float32), to(np.stack(normals), torch.float32), to(np.stack(masks), torch.bool),
-                      rgb_dev, to(poses_np, torch.float64), to(np.stack(intr), torch.float64),
-                      to(np.concatenate(sparse), torch.float64), to(offsets, torch.int64), to(nbr, torch.int32))
-    else:
-        layout = ops.ViewLayout.from_shapes([d.shape for d in depths], s)
-        flat = lambda maps, dt: to(np.concatenate([np.asarray(m).reshape((-1,) + np.asarray(m).shape[2:]) for m in maps]), dt)
-        rgb_flat = flat(rgbs, torch.uint8)
-        res = eng.run_views(flat(depths, torch.float32), flat(normals, torch.float32), flat(masks, torch.bool), rgb_flat,
-                            to(poses_np, torch.float64), to(np.stack(intr), torch.float64), to(np.concatenate(sparse), torch.float64),
-                            to(offsets, torch.int64), to(nbr, torch.int32), layout=layout)
+    maps = ((depths, torch.float32), (normals, torch.float32), (masks, torch.bool), (rgbs, torch.uint8))
+    if len({d.shape for d in depths}) == 1:
+        run, maps = eng.run, [to(np.stack(m), dt) for m, dt in maps]
+    else:  # views of different sizes: the ragged form of the device pipeline
+        run, maps = eng.run_views, [[to(x, dt) for x in m] for m, dt in maps]
+    res = run(*maps, to(poses_np, torch.float64), to(np.stack(intr), torch.float64), to(np.concatenate(sparse), torch.float64),
+              to(offsets, torch.int64), to(nbr, torch.int32))
     n_candidates = res.num_points()
     if config.fusion.voxel_size is None:
-        keep = res.keep_mask()
-        pts_out = res.xyz[keep].double().cpu().numpy()
-        if uniform:
-            col_out = rgb_dev[:, ::s, ::s][keep].cpu().numpy()
-        else:  # each view's strided RGB, concatenated in the order of xyz
-            col_out = torch.cat([r.reshape(-1, 3) for r in layout.strided(layout.split(rgb_flat))], 0)[keep].cpu().numpy()
+        pts, cols = res.kept_points()
+        pts_out, col_out = pts.double().cpu().numpy(), cols.cpu().numpy()
     else:
         mv = int(res.counts[1].item()) if res.counts is not None else 0
         pts_out = res.voxel_xyz[:mv].double().cpu().numpy() if mv else np.zeros((0, 3))
