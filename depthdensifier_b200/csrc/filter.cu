@@ -248,7 +248,8 @@ __device__ __forceinline__ bool pair_test(float Z, float D, bool inb, float thr,
 
 // Normal of one source pixel for the grazing gate (scripts/test.py:291), read on demand: only vote
 // candidates need it, and they are rare (floaters), so the 12 B/pixel normal map is not streamed.
-// normals_in_world rotates it by R_s^T (rows recovered from the source table).
+// normals_in_world rotates it by R_s^T (rows recovered from the source table) and divides by (|n| + 1e-8), as
+// oracle/restatement_masks.py:transform_normals states it; the default camera-frame normal is used as given.
 __device__ __forceinline__ void load_normal(const float* __restrict__ normal_view, size_t pixel, bool in_world,
                                             const float* __restrict__ s_src, float& n0, float& n1, float& n2) {
   const float* np_ = normal_view + pixel * 3;
@@ -264,7 +265,8 @@ __device__ __forceinline__ void load_normal(const float* __restrict__ normal_vie
       const float rc = s_src[i * 4 + 2] + s_src[i * 4 + 0] * cx + s_src[i * 4 + 1] * cy;
       w[i] = ra * n0 + rb * n1 + rc * n2;
     }
-    n0 = w[0], n1 = w[1], n2 = w[2];
+    const float inv = rcp_approx(sqrt_approx(fmaf(w[0], w[0], fmaf(w[1], w[1], w[2] * w[2]))) + 1e-8f);
+    n0 = w[0] * inv, n1 = w[1] * inv, n2 = w[2] * inv;
   }
 }
 
@@ -467,12 +469,16 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
     }
   }
 
-  if (n_own > 0) {
-    // Own view (only present in the reference-parity table K = V).  The reference normalises by (z + 1e-8)
-    // before applying K (scripts/test.py:71-75), so u = x * z/(z+1e-8) lands ~x*1e-8/z BELOW the integer x
-    // (far above float64 round-off) and the truncation at :308-309 looks up pixel (x-1, y-1) for
-    // x, y >= 1.  Reproduced in integer arithmetic; z is the pixel's own depth.  (x == 0 or y == 0 is a
-    // round-off tie in the reference.)
+  // Own view (only present in the reference-parity table K = V).  The reference normalises by (z + 1e-8)
+  // before applying K (scripts/test.py:71-75), so u = x * z/(z+1e-8) lands ~x*1e-8/z BELOW the integer x
+  // (far above float64 round-off) and the truncation at :308-309 looks up pixel (x-1, y-1) for
+  // x, y >= 1.  Reproduced in integer arithmetic; z is the pixel's own depth.  (x == 0 or y == 0 is a
+  // round-off tie in the reference.)
+  // Bilinear sampling never votes here: the sample at (u, v) puts a weight of about e = (x + y)*1e-8/z on the
+  // neighbouring taps and 1 - e on the pixel's own depth z, so z < thr*D needs a tap above (1/thr - 1)/e times z and
+  // |z - D| > tau*D one above tau/e times z (a zero tap makes D = 0: no vote).  At x + y < 2^13 and z = 1 that is
+  // more than 600 times the pixel's depth for tau = 0.05.  The loop is not compiled into the bilinear instantiations.
+  if (!kBilinear && n_own > 0) {
     for (int k = n_hot; k < n_hot + n_own; ++k) {
       const float4* t4 = reinterpret_cast<const float4*>(s_pair + k * DDN_PAIR_TABLE_FLOATS);
       const float4 cc = t4[3];
@@ -668,7 +674,10 @@ static int fill_filter_params(const ddn_filter_config* cfg, const float* refined
   }
   p.stride = cfg->stride;
   p.K = (int)k_nbr;
-  p.vote_threshold = vote_threshold < 255 ? vote_threshold : 255;
+  // The vote byte is min(votes, 254) and the callers' clamp makes any threshold >= 255 keep every valid point.  K4
+  // decides keep (and the occupancy mark) on the unsaturated count, so such a threshold must keep whatever the count:
+  // then keep == (byte < min(threshold, 255)) at every threshold, and fusion and keep_mask agree with the mark.
+  p.vote_threshold = vote_threshold < 255 ? vote_threshold : INT_MAX;
   p.depth_threshold = cfg->depth_threshold;
   p.grazing_cos = cfg->grazing_cos;
   p.two_sided_tau = cfg->two_sided_tau;

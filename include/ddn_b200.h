@@ -132,7 +132,8 @@ typedef struct {
   int32_t sample_mode;     /* 0 = nearest/truncate (reference, :308-309); 1 = bilinear 4-tap (new) */
   float two_sided_tau;     /* <= 0: one-sided z < thr*D (reference, :319-321); > 0: |z-D| > tau*D (new) */
   int32_t stride;          /* ProcessingConfig.downsample_density (scripts/test.py:37); 1 = densest */
-  int32_t normals_in_world; /* 0 = reference quirk (camera-frame normal vs world dir, :291); 1 = rotate by R_src^T */
+  int32_t normals_in_world; /* 0 = reference quirk (camera-frame normal vs world dir, :291, used as given);
+                               1 = rotate by R_src^T and divide by (|n| + 1e-8) (visualizer.py:346-376) */
   int32_t pixel_layout;    /* which 4 pixels a thread owns: 0 = 32 apart (default), 1 = adjacent (vector I/O); same results */
 } ddn_filter_config;
 
@@ -153,7 +154,8 @@ DDN_API int ddn_build_pair_tables(int64_t n_views_total, int64_t src_begin, int6
  * bbox [6] f32 (optional, may be NULL): running min xyz / max xyz over points with
  * votes < vote_threshold; must be initialised to +inf/-inf by ddn_bbox_init.
  * vote_threshold is clamped to 255: votes saturate at 254 and 255 marks "no point", so a threshold of 255
- * or more keeps every point that exists and never a pixel without one.
+ * or more keeps every point that exists and never a pixel without one, whatever its count (also 255 or
+ * more), so votes[i] < min(vote_threshold, 255) reproduces the kernel's keep and mark exactly.
  * mark (optional, may be NULL): a fusion session opened by ddn_fuse_begin*; the kernel then also sets the
  * occupancy bit of every kept point (the "mark" pass of stage 4 fused into the epilogue, where the point
  * is still in registers) and adds their number to the session's counts[0]. */

@@ -24,11 +24,13 @@ EPS_REL = 2e-5
 EPS_Z = 1e-5
 
 
-def pair_ties(points, normals, src_view, t, refined_t, pose_t, intr_t, depth_threshold=0.7, grazing=0.087):
-    """Returns (vote[N] bool, tie[N] bool) of all points against target view t (nearest mode)."""
+def pair_ties(points, normals, src_view, t, refined_t, pose_t, intr_t, depth_threshold=0.7, grazing=0.087,
+              two_sided_tau=None):
+    """Returns (vote[N] bool, tie[N] bool) of all points against target view t (nearest mode), one-sided
+    (z < float32(thr * D)) or two-sided (|z - D| > float32(tau) * D); the threshold band is EPS_REL * D in both."""
     h, w = refined_t.shape
     vote, det = R.votes_against_view(points, normals, refined_t, pose_t, intr_t, depth_threshold=depth_threshold,
-                                     grazing=grazing, return_detail=True)
+                                     grazing=grazing, two_sided_tau=two_sided_tau, return_detail=True)
     u, v, z, dot = det["u"], det["v"], det["z"], det["dot"]
     own = src_view == t
     tie = np.zeros(len(points), dtype=bool)
@@ -38,14 +40,22 @@ def pair_ties(points, normals, src_view, t, refined_t, pose_t, intr_t, depth_thr
     tie |= np.abs(dot - grazing) < EPS_DOT
     # decision with the looked-up depth D
     thr32 = np.float32(depth_threshold)
+    tau32 = None if two_sided_tau is None else np.float32(two_sided_tau)
+
+    def test(D):
+        """(decision, near-threshold flag) for looked-up depths D (float32; 0 where the lookup is invalid)."""
+        D64 = D.astype(np.float64)
+        if tau32 is None:
+            return (D > 0) & (z < (thr32 * D)), (D > 0) & (np.abs(z - thr32 * D64) < EPS_REL * D64)
+        q = np.abs(z - D64) - (tau32 * D).astype(np.float64)
+        return (D > 0) & (q > 0), (D > 0) & (np.abs(q) < EPS_REL * D64)
 
     def decide(ui, vi):
         ok = (ui >= 0) & (ui < w) & (vi >= 0) & (vi < h)
         D = np.zeros(len(points), dtype=np.float32)
         D[ok] = refined_t[vi[ok], ui[ok]]
-        dec = ok & (D > 0) & (z < (thr32 * D))
-        near_thr = ok & (D > 0) & (np.abs(z - thr32 * D.astype(np.float64)) < EPS_REL * D)
-        return dec, near_thr
+        dec, near_thr = test(D)
+        return ok & dec, ok & near_thr
 
     cand = det["inb"] & ~own
     ui = np.where(cand, u, 0).astype(int)
@@ -67,8 +77,7 @@ def pair_ties(points, normals, src_view, t, refined_t, pose_t, intr_t, depth_thr
     # pixel is (x-1, y-1) except in column/row 0 where float64 round-off decides (tie); otherwise
     # only the threshold band applies
     if own.any():
-        D = det["D"]
-        tie |= own & det["inb"] & (D > 0) & (np.abs(z - thr32 * D.astype(np.float64)) < EPS_REL * D)
+        tie |= own & det["inb"] & test(det["D"])[1]
         tie |= own & ((np.abs(u) < 0.5) | (np.abs(v) < 0.5))
     return vote, tie
 
@@ -88,8 +97,7 @@ def pair_ties_bilinear(points, normals, src_view, t, refined_t, pose_t, intr_t, 
                                      sample_mode="bilinear", two_sided_tau=two_sided_tau, return_detail=True)
     u, v, z, dot = det["u"], det["v"], det["z"], det["dot"]
     own = src_view == t
-    tie = own.copy()  # the own view is not part of a K-nearest table; never compared
-    tie |= (np.abs(u) < EPS_PX) | (np.abs(u - w) < EPS_PX) | (np.abs(v) < EPS_PX) | (np.abs(v - h) < EPS_PX)
+    tie = (np.abs(u) < EPS_PX) | (np.abs(u - w) < EPS_PX) | (np.abs(v) < EPS_PX) | (np.abs(v - h) < EPS_PX)
     tie |= np.abs(z) < EPS_Z
     tie |= np.abs(dot - grazing) < EPS_DOT
     cand = det["inb"] & ~own
@@ -127,6 +135,10 @@ def pair_ties_bilinear(points, normals, src_view, t, refined_t, pose_t, intr_t, 
         if sel.any():
             alt, near_alt = decide(x0 + du, y0 + dv)
             tie |= sel & ((alt != base) | near_alt)
+    # own view: it reprojects to u = x*d/(d+1e-8), a hair below the pixel itself, so the sample is the pixel's own
+    # depth up to a relative weight of x*1e-8/d on its neighbours and neither test can fire (K4 skips these pairs).
+    # A pair only differs from K4's "no vote" where the statement votes after all.
+    tie = np.where(own, vote, tie)
     return vote, tie
 
 
@@ -151,6 +163,15 @@ def votes_with_ties(points, normals, src_view, refined_all, poses, intr, nbr, ac
         votes[sel] += vt
         nties[sel] += tt
     return votes, nties
+
+
+def own_view_votes(points, normals, src_view, refined_all, poses, intr, **kw):
+    """Number of points the statement's own view votes against (pair_ties_bilinear counts each as a tie)."""
+    n = 0
+    for s in np.unique(src_view):
+        sel = np.where(src_view == s)[0]
+        n += int(R.votes_against_view(points[sel], normals[sel], refined_all[s], poses[s], intr[s], **kw).sum())
+    return n
 
 
 def assert_votes_match(gpu_votes, ref_votes, nties, max_tie_fraction=0.02):
