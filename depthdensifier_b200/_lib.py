@@ -80,7 +80,15 @@ class FuseSession(C.Structure):
                 ("tile_sums", C.c_void_p), ("tile_prefix", C.c_void_p), ("counts", C.c_void_p)]
 
 
-GRID_OK, GRID_EMPTY, GRID_TOO_LARGE, GRID_TOO_MANY_BITS = 0, 1, 2, 3
+class HashFuse(C.Structure):
+    """struct ddn_hash_fuse: host struct of device pointers (the hashed fusion path's buffers)."""
+
+    _fields_ = [("table", C.c_void_p), ("slots", C.c_void_p), ("sort", C.c_void_p), ("hist", C.c_void_p), ("state", C.c_void_p),
+                ("cap_slots", C.c_int64), ("cap_voxels", C.c_int64)]
+
+
+GRID_OK, GRID_EMPTY, GRID_TOO_LARGE, GRID_TOO_MANY_BITS, GRID_HASHED = 0, 1, 2, 3, 4
+HASH_STATE_BYTES = 64  # DDN_HASH_STATE_BYTES
 MAX_PEERS = 16
 PAIR_TABLE_FLOATS = 24
 LAYOUT_COLS = 8  # DDN_LAYOUT_COLS
@@ -161,6 +169,13 @@ SYMBOLS = {
     "ddn_fuse_merge_peers": (
         C.c_int,
         [C.POINTER(FuseSession), _i32, _i32, C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _i64, _vp, _i64,
+         _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
+    ),
+    "ddn_hash_fuse_sizes": (C.c_int, [_i64] + [C.POINTER(_i64)] * 5),
+    "ddn_hash_fuse_reset": (C.c_int, [C.POINTER(HashFuse), _vp]),
+    "ddn_fuse_finish_hashed": (
+        C.c_int,
+        [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i64,
          _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
     ),
 }

@@ -61,6 +61,7 @@ class DensifyResult:
     voxel_count: torch.Tensor | None = None
     counts: torch.Tensor | None = None  # [2] i64: fused points, voxels
     session: object | None = None  # ops.FuseSession that produced the voxels (device-resident grid)
+    hash: object | None = None  # ops.HashFuse of the step: fused the voxels when the grid was too large for the session
     bbox_valid: torch.Tensor | None = None  # [6] i32: box of every back-projected pixel (the alignment kernel's bound)
     layout: ops.ViewLayout | None = None  # run_views: refined [P], xyz [G,3], votes [G] are flat over the views of this layout
     rgb: torch.Tensor | None = None  # the step's colours: [V,H,W,3] u8, or flat [P,3] u8 over the views of ``layout``
@@ -104,7 +105,9 @@ class DensifyResult:
             st = self.session.grid_state()
             if st.status == 1:  # no valid point at all
                 return 0
-            self.host_grid()
+            self.host_grid()  # raises on a grid neither path could fuse
+            if self.hash is not None:
+                self.hash.check()
         mv = ops.checked_voxel_count(self.counts)
         if self.voxel_keys is not None and mv > self.voxel_keys.shape[0]:
             raise ops.DDNError(f"voxel fusion: {mv} voxels exceed the output capacity {self.voxel_keys.shape[0]}")
@@ -130,6 +133,13 @@ class DensifyEngine:
         if getattr(self, "_session", None) is None or self._session.max_cells != self.cfg.max_grid_cells:
             self._session = ops.FuseSession(self.device, self.cfg.max_grid_cells)
         return self._session
+
+    def hash_fuse(self, n_points: int) -> ops.HashFuse:
+        """The hashed fusion path's buffers, grown when a step has more points (+ dedup points) than they hold."""
+        if getattr(self, "_hash", None) is None or self._hash.cap_voxels < n_points:
+            self._hash = None  # free the old buffers first
+            self._hash = ops.HashFuse(self.device, n_points)
+        return self._hash
 
     def run(self, depth, normal, mask, rgb, cam_from_world, intr, sparse_xyz, sparse_offsets, nbr,
             max_sparse_per_view: int | None = None, grid=None, sync: bool = True) -> DensifyResult:
@@ -197,12 +207,17 @@ class DensifyEngine:
         res = DensifyResult(refined=refined, stats=stats, xyz=xyz, votes=votes, vote_threshold=thr, bbox=bbox, bbox_valid=box,
                             layout=layout, rgb=rgb, stride=cfg.filter.stride)
         if fuse:
-            rgb_s = res.grid_rgb()
-            if cfg.dedup_sparse and sparse_xyz.shape[0] > 0:
-                sess.unmark_points(sparse_xyz.float().contiguous())
+            points = (xyz.view(-1, 3), res.grid_rgb().view(-1, 3), votes.view(-1))
+            dedup = sparse_xyz.float().contiguous() if cfg.dedup_sparse and sparse_xyz.shape[0] > 0 else None
+            if dedup is not None:
+                sess.unmark_points(dedup)
             row_len = xyz.shape[2] if layout is None else 0  # 0: the rows differ from view to view
-            k, x, c, n, counts = ops.fuse_finish(sess, xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), thr, row_len=row_len)
-            res.session, res.grid = sess, grid
+            # Both finishes are enqueued on the same outputs; the device grid decides which one runs (the hashed path
+            # takes a grid too large for the session's bitmap, the dense one every other), so nothing is read back.
+            out = ops.fuse_finish(sess, *points, thr, row_len=row_len)[:4]
+            hf = self.hash_fuse(points[0].shape[0] + (0 if dedup is None else dedup.shape[0]))
+            k, x, c, n, counts = ops.fuse_finish_hashed(sess, hf, *points, thr, row_len=row_len, dedup_xyz=dedup, out=out)
+            res.session, res.grid, res.hash = sess, grid, hf
             res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts.clone()
             if sync:
                 mv = res.check()

@@ -452,7 +452,7 @@ def checked_voxel_count(counts: torch.Tensor) -> int:
 
 
 GRID_STATUS = {0: "ok", 1: "empty (no finite bounding box)", 2: "grid larger than the session's capacity",
-               3: "an axis needs more than 21 bits"}
+               3: "an axis needs more than 21 bits", 4: "fused through the hash table"}
 
 
 class FuseSession:
@@ -515,7 +515,10 @@ class FuseSession:
         """The device grid as the host struct the host-grid entry points and the tests take (synchronises);
         raises when the session could not build one."""
         st = self.grid_state()
-        if st.status != _lib.GRID_OK:
+        if st.status == _lib.GRID_TOO_MANY_BITS:
+            raise DDNError(f"fusion grid: {GRID_STATUS[st.status]} (dims {list(st.dims)}): the 3x21-bit voxel key cannot "
+                           "address the bounding box at this voxel size; use a larger voxel")
+        if st.status not in (_lib.GRID_OK, _lib.GRID_HASHED):
             raise DDNError(f"fusion grid: {GRID_STATUS.get(st.status, st.status)} (dims {list(st.dims)}, "
                            f"capacity {self.max_cells} cells); raise max_grid_cells or use a larger voxel")
         g = _lib.VoxelGrid()
@@ -555,6 +558,41 @@ class FuseSession:
             _lib.check(lib.ddn_fuse_unmark_points(C.byref(self.c), xyz.shape[0], _p(xyz), _stream()))
 
 
+class HashFuse:
+    """Buffers of the hashed fusion path (include/ddn_b200.h: struct ddn_hash_fuse) for steps of up to ``cap_voxels``
+    points + dedup points: a table of 2x the next power of two >= cap_voxels slots (12 bytes each, at least 64 slots),
+    the slot list and the sort buffers (28 bytes per point).  Allocated once and emptied; every step leaves the table empty again."""
+
+    def __init__(self, device, cap_voxels: int):
+        lib = _lib.load()
+        if not torch.cuda.is_available():
+            raise DDNError("no CUDA device available: depthdensifier_b200 has no CPU fallback")
+        self.device = torch.device(device)
+        self.cap_voxels = max(int(cap_voxels), 1)
+        sizes = [C.c_int64(0) for _ in range(5)]
+        _lib.check(lib.ddn_hash_fuse_sizes(self.cap_voxels, *[C.byref(x) for x in sizes]))
+        self.cap_slots, table_b, slots_b, sort_b, hist_b = (x.value for x in sizes)
+        new = lambda n: torch.empty(n, dtype=torch.uint8, device=self.device)
+        self.table, self.slots, self.sort, self.hist = new(table_b), new(slots_b), new(sort_b), new(hist_b)
+        self.state = torch.zeros(_lib.HASH_STATE_BYTES // 8, dtype=torch.int64, device=self.device)
+        self.c = _lib.HashFuse(self.table.data_ptr(), self.slots.data_ptr(), self.sort.data_ptr(), self.hist.data_ptr(),
+                               self.state.data_ptr(), self.cap_slots, self.cap_voxels)
+        with torch.cuda.device(self.device):
+            _lib.check(lib.ddn_hash_fuse_reset(C.byref(self.c), _stream()))
+
+    def nbytes(self) -> int:
+        return sum(t.numel() * t.element_size() for t in (self.table, self.slots, self.sort, self.hist, self.state))
+
+    def ran(self) -> bool:
+        """Whether the last step went through the hash table (synchronises)."""
+        return int(self.state[0]) == 1
+
+    def check(self) -> None:
+        """Raises if the last step overflowed the table (synchronises); with ddn_hash_fuse_sizes' sizing it cannot."""
+        if int(self.state[0]) == 1 and int(self.state[1]) != 0:
+            raise DDNError("hashed voxel fusion: table overflow, the step's voxels are incomplete")
+
+
 def new_voxel_outputs(cap_out: int, dev):
     return (torch.empty(cap_out, dtype=torch.int64, device=dev), torch.empty((cap_out, 3), dtype=torch.float32, device=dev),
             torch.empty((cap_out, 3), dtype=torch.uint8, device=dev), torch.empty(cap_out, dtype=torch.int32, device=dev))
@@ -573,6 +611,28 @@ def fuse_finish(sess: FuseSession, xyz, rgb, votes, vote_threshold: int, row_len
     with torch.cuda.device(dev):
         _lib.check(lib.ddn_fuse_finish(C.byref(sess.c), N, int(row_len), _p(xyz), _p(rgb), _p(votes), int(vote_threshold), _p(k), _p(x),
                                        _p(c), _p(n), cap, _p(acc), acc.numel(), _stream()))
+    return k, x, c, n, sess.counts
+
+
+def fuse_finish_hashed(sess: FuseSession, hf: HashFuse, xyz, rgb, votes, vote_threshold: int, row_len: int = 0,
+                       dedup_xyz=None, mode: int = 0, cap_out: int | None = None, out=None):
+    """Hashed fusion of the step's points (include/ddn_b200.h: ddn_fuse_finish_hashed).  ``mode`` 0: only when the
+    session's grid is too large for its bitmap (the dense finish returns at once then); 1: on any grid.  ``dedup_xyz``
+    [n,3] f32: N5, no voxel in the cells of these points.  Returns keys, xyz, rgb, count and the device counts [2], as
+    fuse_finish; pass the same ``out`` as the dense finish so that one set of outputs holds whichever path ran."""
+    lib = _lib.load()
+    dev = _require_cuda(xyz, rgb, votes, dedup_xyz)
+    N = xyz.shape[0]
+    assert xyz.dtype == torch.float32 and rgb.dtype == torch.uint8 and tuple(rgb.shape) == (N, 3)
+    assert dedup_xyz is None or (dedup_xyz.dtype == torch.float32 and dedup_xyz.dim() == 2 and dedup_xyz.shape[1] == 3)
+    cap = max(int(cap_out if cap_out is not None else N), 1)
+    k, x, c, n = out if out is not None else new_voxel_outputs(cap, dev)
+    acc = sess.accum(max(cap, N))  # a voxel's accumulator is indexed by the point that created it
+    n_dedup = 0 if dedup_xyz is None else dedup_xyz.shape[0]
+    with torch.cuda.device(dev):
+        _lib.check(lib.ddn_fuse_finish_hashed(C.byref(sess.c), C.byref(hf.c), int(mode), N, int(row_len), _p(xyz), _p(rgb), _p(votes),
+                                              int(vote_threshold), _p(dedup_xyz), n_dedup, _p(k), _p(x), _p(c), _p(n), cap, _p(acc),
+                                              acc.numel(), _stream()))
     return k, x, c, n, sess.counts
 
 

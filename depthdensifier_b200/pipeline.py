@@ -86,7 +86,9 @@ class FilteringConfig:
 
 @dataclass
 class FusionConfig:
-    """new: voxel-grid fusion of the kept points (the reference only concatenates)."""
+    """new: voxel-grid fusion of the kept points (the reference only concatenates).  Works for scenes of any extent:
+    when the box of the back-projected points is too large for the dense occupancy bitmap (unbounded outdoor scenes,
+    distant background, an outlier depth), the device fuses through a hash table sized by the points instead."""
 
     voxel_size: float | None = None
     dedup_sparse: bool = False

@@ -35,6 +35,9 @@ class SceneConfig:
     seed: int = 0
     ring_radius: float = 4.0
     ring_height: float = 2.0
+    dome_radius: float | None = None
+    """Distant background: rays that hit nothing within ``max_depth`` hit the inside of a sphere of this radius around
+    the origin (masked in, with analytic normals and colours).  None: no background (those pixels are masked out)."""
 
 
 @dataclass
@@ -83,8 +86,9 @@ def ring_poses(cfg: SceneConfig) -> np.ndarray:
     return np.concatenate([R, t[:, :, None]], axis=2)
 
 
-def _raycast(c: torch.Tensor, dw: torch.Tensor, max_depth: float):
-    """First hit of rays c + d*dw (d = z-depth since dw = R^T (x, y, 1)). Returns d, n_world, hit."""
+def _raycast(c: torch.Tensor, dw: torch.Tensor, max_depth: float, dome_radius: float | None = None):
+    """First hit of rays c + d*dw (d = z-depth since dw = R^T (x, y, 1)). Returns d, n_world, hit.  With
+    ``dome_radius``, rays without a hit within ``max_depth`` hit the inside of that sphere around the origin."""
     inf = torch.full(dw.shape[:-1], float("inf"), dtype=dw.dtype, device=dw.device)
     d_plane = torch.where(dw[..., 2] < 0, -c[2] / dw[..., 2].clamp(max=-1e-12), inf)
     best = d_plane
@@ -105,6 +109,14 @@ def _raycast(c: torch.Tensor, dw: torch.Tensor, max_depth: float):
         best = torch.where(ok, d, best)
         n = torch.where(ok.unsqueeze(-1), ns, n)
     hit = torch.isfinite(best) & (best < max_depth) & (best > 0)
+    if dome_radius is not None:  # the camera is inside the dome: the far root of |c + d dw| = R
+        b = (dw * c).sum(-1)
+        disc = b * b - a * ((c * c).sum() - dome_radius * dome_radius)
+        d_dome = (-b + torch.sqrt(disc.clamp(min=0))) / a
+        dome = ~hit & (disc > 0) & (d_dome > 0)
+        best = torch.where(dome, d_dome, best)
+        n = torch.where(dome.unsqueeze(-1), -(c + d_dome.unsqueeze(-1) * dw) / dome_radius, n)
+        hit = hit | dome
     return best, n, hit
 
 
@@ -149,7 +161,7 @@ def make_scene(cfg: SceneConfig, device: str | torch.device = "cpu", views: rang
         t = poses[v, :, 3]
         c = -(R.T @ t)
         dw = dir_cam @ R  # rows: R^T dir
-        d, n_w, hit = _raycast(c, dw, cfg.max_depth)
+        d, n_w, hit = _raycast(c, dw, cfg.max_depth, cfg.dome_radius)
         d = torch.where(hit, d, torch.zeros_like(d))
         n_c = n_w @ R.T
         p_w = c + d.unsqueeze(-1) * dw
@@ -173,7 +185,7 @@ def make_scene(cfg: SceneConfig, device: str | torch.device = "cpu", views: rang
         w_ = uv[:, 1] * (H - 1)
         dc = torch.stack([(u - cx) / fx, (w_ - cy) / fy, torch.ones_like(u)], dim=-1)
         dws = dc @ R
-        ds, _, hs = _raycast(c, dws, cfg.max_depth)
+        ds, _, hs = _raycast(c, dws, cfg.max_depth, cfg.dome_radius)
         pts = (c + ds.unsqueeze(-1) * dws)[hs][: cfg.n_sparse]
         sparse.append(pts)
         offsets.append(offsets[-1] + pts.shape[0])

@@ -330,7 +330,7 @@ DDN_API int ddn_voxel_merge(const ddn_voxel_grid* grid_host, int64_t n_records, 
  *   [-> ddn_fuse_merge_peers]
  * and never needs the host to look at a result in between.
  * ------------------------------------------------------------------------------------------ */
-enum { DDN_GRID_OK = 0, DDN_GRID_EMPTY = 1, DDN_GRID_TOO_LARGE = 2, DDN_GRID_TOO_MANY_BITS = 3 };
+enum { DDN_GRID_OK = 0, DDN_GRID_EMPTY = 1, DDN_GRID_TOO_LARGE = 2, DDN_GRID_TOO_MANY_BITS = 3, DDN_GRID_HASHED = 4 };
 
 typedef struct ddn_grid_state { /* 64 bytes of DEVICE memory, written by ddn_fuse_begin* */
   float voxel;
@@ -338,7 +338,8 @@ typedef struct ddn_grid_state { /* 64 bytes of DEVICE memory, written by ddn_fus
   int32_t bits[3];
   int32_t dims[3];
   int64_t n_units; /* occupancy units in use: ceil(cells / 96); 0 unless status == DDN_GRID_OK */
-  int32_t status;  /* DDN_GRID_*: EMPTY = no finite box, TOO_LARGE = more cells than cap_units * 96 */
+  int32_t status;  /* DDN_GRID_*: EMPTY = no finite box, TOO_LARGE = more cells than cap_units * 96, HASHED = a
+                      TOO_LARGE grid that ddn_fuse_finish_hashed fused (origin, bits and dims are valid) */
   int32_t reserved;
   int64_t cells;
 } ddn_grid_state;
@@ -408,6 +409,48 @@ DDN_API int ddn_fuse_merge_peers(const ddn_fuse_session* s, int32_t rank, int32_
                          const void* const* peer_tile_prefix_host, int64_t* plan, void* scratch, int64_t scratch_bytes,
                          const float* drop_xyz, int64_t n_drop, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
                          int32_t* out_count, int64_t cap_out, void* accum, int64_t accum_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Stage 4 for grids too large for the session's occupancy bitmap: the HASHED PATH (one GPU).  Memory is sized by
+ * the points of a step, not by the volume of its box.  An open-addressing table of canonical keys gives every
+ * occupied cell a dense voxel index while the points are accumulated (one pass); the voxel keys are then radix-sorted
+ * with a count read from device memory and finalised in key order.  Outputs are those of ddn_fuse_finish on the same
+ * grid, bit for bit.  A step enqueues ddn_fuse_finish and then ddn_fuse_finish_hashed(mode 0) on the same outputs:
+ * whichever path the device grid selects runs, the other returns at once, and nothing is read back.
+ * ------------------------------------------------------------------------------------------ */
+#define DDN_HASH_STATE_BYTES 64
+
+struct ddn_hash_fuse { /* HOST struct of DEVICE pointers, owned by the caller; sizes from ddn_hash_fuse_sizes */
+  void* table;           /* [cap_slots] u64 keys (all bits set = empty), then [cap_slots] u32 voxel indices */
+  uint32_t* slots;       /* [cap_voxels] the table slot of every voxel, at the index of the point that created it
+                            (and of every tombstone, from the top); all bits set = unused */
+  void* sort;            /* [2, cap_voxels] u64 compact keys, then (256-byte aligned) [2, cap_voxels] u32 indices */
+  uint32_t* hist;        /* radix histograms */
+  int64_t* state;        /* DDN_HASH_STATE_BYTES: [0] 1 = the path ran this step, [1] 1 = table overflow (the step's
+                            voxels are incomplete), [2] tombstones */
+  int64_t cap_slots;     /* table slots: 2 x the next power of two >= cap_voxels, at least 64 */
+  int64_t cap_voxels;    /* the most points (+ dedup points) one step may pass */
+};
+
+/* Buffer sizes (bytes) for steps of up to cap_voxels points + dedup points; the table then never gets more than half
+ * full, so it cannot overflow. */
+DDN_API int ddn_hash_fuse_sizes(int64_t cap_voxels, int64_t* cap_slots, int64_t* table_bytes, int64_t* slots_bytes,
+                        int64_t* sort_bytes, int64_t* hist_bytes);
+/* Once after allocation (and after any error): empties the table and the slot list and clears the state.  Every step
+ * leaves them empty again (it clears the entries it used). */
+DDN_API int ddn_hash_fuse_reset(const struct ddn_hash_fuse* hash, void* stream);
+/* Fusion of the points of a session step through the hash table.  mode 0: runs only when the session's grid is
+ * DDN_GRID_TOO_LARGE (which it rewrites to DDN_GRID_HASHED) or HASHED; mode 1: on any grid with valid dims (tests
+ * compare it with the dense path on one grid).  When it runs it resets counts and fills them itself: [0] = points
+ * that pass the vote and fall inside the grid (what K4's mark counts), [1] = voxels.  dedup_xyz [n_dedup,3] f32
+ * (optional): N5 as ddn_fuse_unmark_points - no voxel in the cells of these points, whose points still count in
+ * counts[0].  Needs n_points + n_dedup <= hash->cap_voxels.  accum: max(cap_out, n_points) * 40 bytes (a voxel's
+ * accumulator is indexed by the point that created it).  Other arguments and outputs as ddn_fuse_finish. */
+DDN_API int ddn_fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_hash_fuse* hash, int32_t mode, int64_t n_points,
+                           int64_t row_len, const float* xyz, const uint8_t* rgb, const uint8_t* votes,
+                           int32_t vote_threshold, const float* dedup_xyz, int64_t n_dedup, uint64_t* out_keys,
+                           float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t cap_out, void* accum,
+                           int64_t accum_bytes, void* stream);
 
 /* Stand-alone pieces of stage 4 (used by the multi-GPU path and by tests). */
 DDN_API int ddn_voxel_keys(const ddn_voxel_grid* grid_host, int64_t n_points, const float* xyz,
