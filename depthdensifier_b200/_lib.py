@@ -93,6 +93,7 @@ MAX_PEERS = 16
 PAIR_TABLE_FLOATS = 24
 LAYOUT_COLS = 8  # DDN_LAYOUT_COLS
 RECORD_WORDS = 6  # DDN_RECORD_WORDS
+HASH_SAMPLES = 4096  # DDN_HASH_SAMPLES
 
 # every symbol include/ddn_b200.h declares: name -> (restype, argtypes)
 _vp, _i64, _i32 = C.c_void_p, C.c_int64, C.c_int32
@@ -177,6 +178,16 @@ SYMBOLS = {
         C.c_int,
         [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i64,
          _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
+    ),
+    "ddn_fuse_finish_hashed_partial": (
+        C.c_int,
+        [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp],
+    ),
+    "ddn_fuse_merge_hashed_scratch_bytes": (C.c_int, [_i32, _i64, C.POINTER(_i64)]),
+    "ddn_fuse_merge_hashed_peers": (
+        C.c_int,
+        [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i32, C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _i64, _vp, _vp, _vp, _vp,
+         _i64, _vp],
     ),
 }
 

@@ -682,10 +682,6 @@ constexpr int kPlanWords = 4 + 3 * DDN_MAX_PEERS;
 static_assert(kPlanWords <= 64, "plan scratch is 64 words");
 static_assert(DDN_MAX_PEERS <= 31, "the plan kernel is one warp");
 
-struct PeerPtrs {
-  const void* p[DDN_MAX_PEERS];
-};
-
 // Step 0 of the merge: every rank's tile prefix (whole array, n_own + 1 entries) is copied into local memory in
 // ONE bulk pass over NVLink - local[q * stride + t] - with their sum over the ranks in row R.  Everything the plan
 // and the occupancy merge decide afterwards reads local memory: no chain of dependent remote round trips.
@@ -795,38 +791,7 @@ merge_pull_mark_kernel(FuseDev f, PeerPtrs peer_records, int rank, int R, const 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long n_warps = (long long)gridDim.x * 8;
   for (long long w0 = ((long long)blockIdx.x * 8 + warp) * 32; w0 < total; w0 += n_warps * 32) {
-    const long long i = w0 + lane;
-    const bool in = i < total;
-    int kq = 0;
-#pragma unroll
-    for (int k = 1; k < DDN_MAX_PEERS; ++k) kq += (k < R && i >= plan[4 + 2 * DDN_MAX_PEERS + k]) ? 1 : 0;
-    const long long j = plan[4 + kq] + (i - plan[4 + 2 * DDN_MAX_PEERS + kq]);
-    int q = rank + kq;
-    q -= q >= R ? R : 0;
-    const unsigned long long* base = reinterpret_cast<const unsigned long long*>(peer_records.p[q]);
-    // whole warp inside one rank's share (the usual case): three coalesced 512-byte loads and stores
-    const int kq0 = __shfl_sync(0xffffffffu, kq, 0);
-    const bool uniform = __all_sync(0xffffffffu, in && kq == kq0);
-    unsigned long long key = ~0ull;
-    if (uniform) {
-      const long long j0 = __shfl_sync(0xffffffffu, j, 0);
-      const ulonglong2* src = reinterpret_cast<const ulonglong2*>(base + j0 * kRecWords);
-      ulonglong2* dst = staging + w0 * 3;
-#pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        const ulonglong2 v = __ldcv(src + k * 32 + lane);
-        s_rec[warp][k * 32 + lane] = v;
-        dst[k * 32 + lane] = v;
-      }
-      __syncwarp();
-      key = s_rec[warp][lane * 3].x;
-      __syncwarp();
-    } else if (in) {
-      const ulonglong2* r = reinterpret_cast<const ulonglong2*>(base + j * kRecWords);
-      const ulonglong2 a = __ldcv(r), b = __ldcv(r + 1), c = __ldcv(r + 2);
-      staging[i * 3 + 0] = a, staging[i * 3 + 1] = b, staging[i * 3 + 2] = c;
-      key = a.x;
-    }
+    const unsigned long long key = pull_share_warp(peer_records, rank, R, plan, staging, w0, total, s_rec[warp], lane);
     uint64_t cell = cell_of_key(g, key);
     if (cell < cell_begin || cell >= cell_end) cell = kNoCell;
     uint64_t left = __shfl_up_sync(0xffffffffu, cell, 1);

@@ -142,6 +142,55 @@ struct FuseDev {
   unsigned long long* counts;       // [0] participating points, [1] voxels
 };
 
+// ---- multi-GPU exchange ------------------------------------------------------------------------------
+struct PeerPtrs {
+  const void* p[DDN_MAX_PEERS];
+};
+
+// One warp's step of the owner-side pull: records w0 .. w0 + 31 of this rank's share, which plan (the layout of
+// merge_plan_kernel, include/ddn_b200.h) lays out as the concatenation of its slices of every rank's sorted records
+// in rotated rank order, are copied from the peers' memory into staging[w0 ...] (DDN_RECORD_WORDS u64 each).  A warp
+// inside one rank's slice (the usual case) moves its 1536 bytes as three fully coalesced 512-byte requests (lane l
+// takes bytes 16 l of each) and re-distributes them through s_rec (this warp's 96 entries of shared memory).
+// Returns the key of record w0 + lane, ~0 past the end of the share (total).
+__device__ __forceinline__ unsigned long long pull_share_warp(const PeerPtrs& peer_records, int rank, int R, const long long* __restrict__ plan,
+                                                              ulonglong2* __restrict__ staging, long long w0, long long total,
+                                                              ulonglong2* s_rec, int lane) {
+  const long long i = w0 + lane;
+  const bool in = i < total;
+  int kq = 0;
+#pragma unroll
+  for (int k = 1; k < DDN_MAX_PEERS; ++k) kq += (k < R && i >= plan[4 + 2 * DDN_MAX_PEERS + k]) ? 1 : 0;
+  const long long j = plan[4 + kq] + (i - plan[4 + 2 * DDN_MAX_PEERS + kq]);
+  int q = rank + kq;
+  q -= q >= R ? R : 0;
+  const unsigned long long* base = reinterpret_cast<const unsigned long long*>(peer_records.p[q]);
+  // whole warp inside one rank's share (the usual case): three coalesced 512-byte loads and stores
+  const int kq0 = __shfl_sync(0xffffffffu, kq, 0);
+  const bool uniform = __all_sync(0xffffffffu, in && kq == kq0);
+  unsigned long long key = ~0ull;
+  if (uniform) {
+    const long long j0 = __shfl_sync(0xffffffffu, j, 0);
+    const ulonglong2* src = reinterpret_cast<const ulonglong2*>(base + j0 * DDN_RECORD_WORDS);
+    ulonglong2* dst = staging + w0 * 3;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      const ulonglong2 v = __ldcv(src + k * 32 + lane);
+      s_rec[k * 32 + lane] = v;
+      dst[k * 32 + lane] = v;
+    }
+    __syncwarp();
+    key = s_rec[lane * 3].x;
+    __syncwarp();
+  } else if (in) {
+    const ulonglong2* r = reinterpret_cast<const ulonglong2*>(base + j * DDN_RECORD_WORDS);
+    const ulonglong2 a = __ldcv(r), b = __ldcv(r + 1), c = __ldcv(r + 2);
+    staging[i * 3 + 0] = a, staging[i * 3 + 1] = b, staging[i * 3 + 2] = c;
+    key = a.x;
+  }
+  return key;
+}
+
 // ---- sort path (fuse_sort.cu) -------------------------------------------------------------------
 // records != nullptr: partial mode, output = records [.,DDN_RECORD_WORDS] (see include/ddn_b200.h)
 int sort_fuse_workspace_bytes(int64_t n_points, int64_t* bytes_out);

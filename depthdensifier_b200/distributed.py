@@ -224,11 +224,13 @@ class ShardedDensifier:
         ptrs = lambda name, shape, dt: [int(v.data_ptr()) for v in self.peer.buffer(name, shape, dt)[2]]
         self._peer_prefix = ptrs("fuse_tile_prefix", (self.session.tile_prefix.numel(),), torch.uint8)
         self._peer_records = ptrs("records", tuple(self.peer_records_shape), torch.int64)
+        self._peer_samples = ptrs("hash_samples", (ops._lib.HASH_SAMPLES + 1,), torch.int64)
         self._peer_bbox = [ptrs(f"bbox{par}", (64,), torch.int32) for par in (0, 1)]
         self._plan = torch.zeros(64, dtype=torch.int64, device=self.device)
         # a rank's share of the merged voxels: the cuts balance the global record count, up to one tile per rank
+        # (the hashed merge: its sampled splitters balance the global record count up to hashed_merge_capacity)
         n_max = self._local_max * self.Hs * self.Ws
-        self._cap_merge = n_max + 24576 * self.world + 1024
+        self._cap_merge = max(n_max + 24576 * self.world + 1024, ops.hashed_merge_capacity(n_max, self.world))
         self._merge_out = [ops.new_voxel_outputs(self._cap_merge, self.device), None]  # second set: pipelined host calls
         self.session.merge_scratch(self.world, self._cap_merge)
 
@@ -363,7 +365,7 @@ class ShardedDensifier:
         if self.device_path:
             drop = self._sparse_for_dedup(sparse_xyz) if cfg.dedup_sparse else None
             k, x, c, n, counts = mark("voxel_fuse", lambda: self._fuse_device(xyz, rgb_s, votes, mark, drop))
-            res.session, res.grid = self.session, grid
+            res.session, res.grid, res.hash = self.session, grid, self._hash
             res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts
             return res
         # collective path: the grid is made on the host from the (all-reduced) box of the kept points
@@ -485,24 +487,52 @@ class ShardedDensifier:
         dist.all_gather_into_tensor(allp, pad, group=self.group)
         return allp
 
+    def hash_fuse(self, n_points: int) -> ops.HashFuse:
+        """The hashed fusion path's buffers, grown when a step has more points (+ dedup points) than they hold; with peers
+        also large enough for the owner's share of the merge."""
+        need = max(int(n_points), self._cap_merge if self.peer is not None else 0)
+        if getattr(self, "_hash", None) is None or self._hash.cap_voxels < need:
+            self._hash = None  # free the old buffers first
+            self._hash = ops.HashFuse(self.device, need)
+        return self._hash
+
     def _fuse_device(self, xyz, rgb, votes, mark=None, drop=None, out_slot: int = 0):
         """Stage 4 on the device path.  One rank: rank + accumulate + finalise.  R ranks: partial records into
         peer-visible memory, one barrier, then the owner-side merge that reads the peers' units and records over
-        NVLink.  Returns persistent output buffers (valid until the next step) and a snapshot of the counts."""
+        NVLink.  Both the dense and the hashed form of each half are enqueued on the same outputs; the device grid
+        decides which one runs (the hashed path takes a grid too large for the session's bitmap), so nothing is read
+        back.  Returns persistent output buffers (valid until the next step) and a snapshot of the counts."""
         if mark is None:
             mark = lambda name, fn: fn()
         sess = self.session
         flat = (xyz.view(-1, 3), rgb.view(-1, 3), votes.view(-1))
+        if drop is not None and drop.shape[0] == 0:
+            drop = None
+        hf = self.hash_fuse(flat[0].shape[0] + (0 if drop is None else drop.shape[0]))
         if self.peer is None:
-            if drop is not None and drop.shape[0] > 0:
+            if drop is not None:
                 sess.unmark_points(drop)
-            k, x, c, n, counts = self.ops.fuse_finish(sess, *flat, self.thr, row_len=xyz.shape[2])
+            out = self.ops.fuse_finish(sess, *flat, self.thr, row_len=xyz.shape[2])[:4]
+            k, x, c, n, counts = self.ops.fuse_finish_hashed(sess, hf, *flat, self.thr, row_len=xyz.shape[2], dedup_xyz=drop, out=out)
             return k, x, c, n, counts.clone()
         rec, hdl, _ = self.peer.buffer("records", tuple(self.peer_records_shape), torch.int64)
-        mark("fuse_partials", lambda: self.ops.fuse_finish_partial(sess, *flat, self.thr, rec, row_len=xyz.shape[2]))
-        hdl.barrier()  # every rank's units, tile prefix and records are complete
-        k, x, c, n, counts = mark("fuse_merge", lambda: self.ops.fuse_merge_peers(
-            sess, self.rank, self.world, self._peer_records, self._peer_prefix, self._plan, self._cap_merge, out=self._merge_outputs(out_slot), drop_xyz=drop))
+        samples = self.peer.buffer("hash_samples", (ops._lib.HASH_SAMPLES + 1,), torch.int64)[0]
+
+        def partials():
+            self.ops.fuse_finish_partial(sess, *flat, self.thr, rec, row_len=xyz.shape[2])
+            # N5 on the hashed path: every rank tombstones the cells of all ranks' sparse points, so their points are
+            # never sent
+            self.ops.fuse_finish_hashed_partial(sess, hf, *flat, self.thr, rec, samples, row_len=xyz.shape[2], dedup_xyz=drop)
+
+        def merge():
+            out = self.ops.fuse_merge_peers(sess, self.rank, self.world, self._peer_records, self._peer_prefix, self._plan, self._cap_merge,
+                                            out=self._merge_outputs(out_slot), drop_xyz=drop)[:4]
+            return self.ops.fuse_merge_hashed_peers(sess, hf, self.rank, self.world, self._peer_records, self._peer_samples, self._plan,
+                                                    self._cap_merge, out=out)
+
+        mark("fuse_partials", partials)
+        hdl.barrier()  # every rank's units, tile prefix, records and samples are complete
+        k, x, c, n, counts = mark("fuse_merge", merge)
         return k, x, c, n, counts.clone()
 
     def _nbr_full(self) -> torch.Tensor:
@@ -736,6 +766,7 @@ class ShardedDensifier:
             k, x, c, m, counts = self._fuse_device(xyz, rgb_s, votes, drop=drop, out_slot=hs["next"] ^ 1)
             st["small"][:2].copy_(counts, non_blocking=True)
             st["small"][2:10].copy_(self.session.grid.view(torch.int64), non_blocking=True)
+            st["small"][10:12].copy_(self._hash.state[:2], non_blocking=True)
             ticket["fused"] = (k, x, c, m)
         elif fuse:
             # collective fallback (host-side grid and plan: it waits for the device on its way)
@@ -775,7 +806,8 @@ class ShardedDensifier:
             out["d2h_bytes"] += 64
             if gs.status == ops._lib.GRID_EMPTY:
                 return out
-            if gs.status != ops._lib.GRID_OK:
+            ops.check_hash_state(small[10:12].tolist())
+            if gs.status not in (ops._lib.GRID_OK, ops._lib.GRID_HASHED):
                 raise ops.DDNError(f"fusion grid: {ops.GRID_STATUS.get(gs.status, gs.status)} (dims {list(gs.dims)}); raise "
                                    "max_grid_cells or use a larger voxel")
             grid = ops._lib.VoxelGrid()

@@ -589,8 +589,33 @@ class HashFuse:
 
     def check(self) -> None:
         """Raises if the last step overflowed the table (synchronises); with ddn_hash_fuse_sizes' sizing it cannot."""
-        if int(self.state[0]) == 1 and int(self.state[1]) != 0:
-            raise DDNError("hashed voxel fusion: table overflow, the step's voxels are incomplete")
+        check_hash_state(self.state[:2].tolist())
+
+    def merge_scratch(self, world: int, cap_out: int) -> torch.Tensor:
+        """Scratch of fuse_merge_hashed_peers for ``world`` ranks and ``cap_out`` records (allocated once)."""
+        if getattr(self, "_merge_scratch", None) is None or self._merge_scratch[0] != (world, cap_out):
+            nbytes = C.c_int64(0)
+            _lib.check(_lib.load().ddn_fuse_merge_hashed_scratch_bytes(int(world), int(cap_out), C.byref(nbytes)))
+            self._merge_scratch = None
+            self._merge_scratch = ((world, cap_out), torch.empty(nbytes.value, dtype=torch.uint8, device=self.device))
+        return self._merge_scratch[1]
+
+
+def check_hash_state(state) -> None:
+    """Raises on a host copy of the hash state words [ran, overflow] that report an incomplete step."""
+    if int(state[0]) == 1 and int(state[1]) != 0:
+        raise DDNError("hashed voxel fusion: table overflow, the step's voxels are incomplete")
+
+
+def hashed_merge_capacity(n_max: int, world: int) -> int:
+    """Records an owner of the hashed multi-GPU merge can receive when no rank has more than ``n_max`` points: at most
+    n_max + ceil(2 world n_max / S) + 2 world (S = DDN_HASH_SAMPLES, DESIGN.md §6)."""
+    return int(n_max) + -(-2 * int(world) * int(n_max) // _lib.HASH_SAMPLES) + 2 * int(world)
+
+
+def new_hash_samples(dev) -> torch.Tensor:
+    """Sample array of fuse_finish_hashed_partial: [DDN_HASH_SAMPLES + 1] i64."""
+    return torch.empty(_lib.HASH_SAMPLES + 1, dtype=torch.int64, device=dev)
 
 
 def new_voxel_outputs(cap_out: int, dev):
@@ -633,6 +658,45 @@ def fuse_finish_hashed(sess: FuseSession, hf: HashFuse, xyz, rgb, votes, vote_th
         _lib.check(lib.ddn_fuse_finish_hashed(C.byref(sess.c), C.byref(hf.c), int(mode), N, int(row_len), _p(xyz), _p(rgb), _p(votes),
                                               int(vote_threshold), _p(dedup_xyz), n_dedup, _p(k), _p(x), _p(c), _p(n), cap, _p(acc),
                                               acc.numel(), _stream()))
+    return k, x, c, n, sess.counts
+
+
+def fuse_finish_hashed_partial(sess: FuseSession, hf: HashFuse, xyz, rgb, votes, vote_threshold: int, records, samples, row_len: int = 0,
+                               dedup_xyz=None, mode: int = 0):
+    """Hashed fusion of this rank's points into sorted partial ``records`` [cap, 6] i64 and ``samples``
+    [DDN_HASH_SAMPLES + 1] i64 (include/ddn_b200.h: ddn_fuse_finish_hashed_partial); ``mode`` and ``dedup_xyz`` as
+    fuse_finish_hashed.  Returns the session's device counts [2] = (points of this rank, records)."""
+    lib = _lib.load()
+    dev = _require_cuda(xyz, rgb, votes, records, samples, dedup_xyz)
+    N = xyz.shape[0]
+    assert xyz.dtype == torch.float32 and rgb.dtype == torch.uint8 and tuple(rgb.shape) == (N, 3)
+    assert records.dtype == torch.int64 and records.shape[1] == _lib.RECORD_WORDS and records.is_contiguous()
+    assert samples.dtype == torch.int64 and samples.numel() >= _lib.HASH_SAMPLES + 1
+    assert dedup_xyz is None or (dedup_xyz.dtype == torch.float32 and dedup_xyz.dim() == 2 and dedup_xyz.shape[1] == 3)
+    acc = sess.accum(max(N, 1))
+    n_dedup = 0 if dedup_xyz is None else dedup_xyz.shape[0]
+    with torch.cuda.device(dev):
+        _lib.check(lib.ddn_fuse_finish_hashed_partial(C.byref(sess.c), C.byref(hf.c), int(mode), N, int(row_len), _p(xyz), _p(rgb), _p(votes),
+                                                      int(vote_threshold), _p(dedup_xyz), n_dedup, _p(records), records.shape[0],
+                                                      _p(samples), _p(acc), acc.numel(), _stream()))
+    return sess.counts
+
+
+def fuse_merge_hashed_peers(sess: FuseSession, hf: HashFuse, rank: int, world: int, peer_records, peer_samples, plan, cap_out: int,
+                            out=None):
+    """Owner-side merge of the hashed partials over peer memory (include/ddn_b200.h: ddn_fuse_merge_hashed_peers); runs
+    when this rank's fuse_finish_hashed_partial ran.  ``peer_*``: per rank, the device address of that rank's records /
+    samples as mapped into this process.  ``cap_out`` (<= hf.cap_voxels): hashed_merge_capacity of the largest rank.
+    Returns keys, xyz, rgb, count and the device counts, as fuse_merge_peers."""
+    lib = _lib.load()
+    dev = sess.device
+    k, x, c, n = out if out is not None else new_voxel_outputs(cap_out, dev)
+    scratch = hf.merge_scratch(world, cap_out)
+    arr = lambda ptrs: (C.c_void_p * world)(*[int(v) for v in ptrs])
+    with torch.cuda.device(dev):
+        _lib.check(lib.ddn_fuse_merge_hashed_peers(C.byref(sess.c), C.byref(hf.c), int(rank), int(world), arr(peer_records),
+                                                   arr(peer_samples), _p(plan), _p(scratch), scratch.numel(), _p(k), _p(x), _p(c), _p(n),
+                                                   int(cap_out), _stream()))
     return k, x, c, n, sess.counts
 
 

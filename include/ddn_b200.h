@@ -452,6 +452,46 @@ DDN_API int ddn_fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_h
                            float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t cap_out, void* accum,
                            int64_t accum_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * The HASHED PATH on several GPUs (one process per GPU, peer memory as for ddn_fuse_merge_peers).  A step enqueues
+ *   ddn_fuse_finish_partial, ddn_fuse_finish_hashed_partial(mode 0) -> barrier -> ddn_fuse_merge_peers,
+ *   ddn_fuse_merge_hashed_peers
+ * on the same outputs; whichever path the device grid selects runs, the other returns at once.  The rank-ordered
+ * concatenation of the owners' outputs equals ddn_fuse_finish_hashed on one GPU over all points, bit for bit.
+ * ------------------------------------------------------------------------------------------ */
+#define DDN_HASH_SAMPLES 4096
+/* Hashed fusion of this rank's points into sorted partial RECORDS (DDN_RECORD_WORDS u64 each, keys ascending, as
+ * ddn_voxel_partials) and SAMPLES [DDN_HASH_SAMPLES + 1] u64: the keys of records floor(i M / DDN_HASH_SAMPLES) for
+ * i < DDN_HASH_SAMPLES, then the record count M.  Both in peer-visible memory; other ranks read them in their merge
+ * (after the caller's barrier) until this rank's next step.  mode, dedup_xyz (N5: applied on every rank, pass ALL
+ * ranks' sparse points) and the other point arguments as ddn_fuse_finish_hashed.  counts[0] = the rank's points that
+ * pass the vote and fall inside the grid (their sum over the ranks is the one-GPU count), counts[1] = M.  Needs
+ * n_points + n_dedup <= hash->cap_voxels; records: cap_records >= n_points, 16-byte aligned; accum: n_points * 40
+ * bytes, 16-byte aligned. */
+DDN_API int ddn_fuse_finish_hashed_partial(const ddn_fuse_session* s, const struct ddn_hash_fuse* hash, int32_t mode, int64_t n_points,
+                                   int64_t row_len, const float* xyz, const uint8_t* rgb, const uint8_t* votes,
+                                   int32_t vote_threshold, const float* dedup_xyz, int64_t n_dedup, uint64_t* records,
+                                   int64_t cap_records, uint64_t* samples, void* accum, int64_t accum_bytes, void* stream);
+/* Size of ddn_fuse_merge_hashed_peers' scratch for n_ranks ranks and an output capacity of cap_out voxels. */
+DDN_API int ddn_fuse_merge_hashed_scratch_bytes(int32_t n_ranks, int64_t cap_out, int64_t* bytes_out);
+/* Owner-side merge of the hashed partials over PEER MEMORY; runs when this rank's ddn_fuse_finish_hashed_partial ran
+ * (same hash buffers), returns at once otherwise.  peer_*_host: HOST arrays of n_ranks device pointers - every rank's
+ * records and samples as mapped into this process.  Every rank derives the same n_ranks - 1 splitter keys from all
+ * samples (copied into local memory in one bulk pass): an owner's share of T records in all is at most
+ * T / n_ranks + 2 (T / DDN_HASH_SAMPLES + n_ranks) records, so cap_out >= n_max + ceil(2 n_ranks n_max /
+ * DDN_HASH_SAMPLES) + 2 n_ranks, n_max = the most points of any rank, cannot overflow (a status word reports it
+ * anyway: ddn_hash_fuse.state[1]).  This rank pulls its share of every rank's records once - coalesced 512-byte
+ * requests, peers in rotated order - adds the copies of every key through its hash table and finalises.  Needs
+ * cap_out <= hash->cap_voxels.  plan: device scratch [64] i64 in ddn_fuse_merge_peers' layout, with [0], [1] = the
+ * owned key range [begin, end) (end -1: unbounded), [2] = records received, [3] = records of all ranks.  scratch:
+ * ddn_fuse_merge_hashed_scratch_bytes, 16-byte aligned.  counts[0] keeps the rank's own points (-1 when a merged
+ * voxel holds 2^24 or more points), counts[1] = the voxels of this rank's range.  Outputs as ddn_fuse_finish; the
+ * rank-ordered concatenation of the outputs is globally key-sorted. */
+DDN_API int ddn_fuse_merge_hashed_peers(const ddn_fuse_session* s, const struct ddn_hash_fuse* hash, int32_t rank, int32_t n_ranks,
+                                const void* const* peer_records_host, const void* const* peer_samples_host, int64_t* plan,
+                                void* scratch, int64_t scratch_bytes, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
+                                int32_t* out_count, int64_t cap_out, void* stream);
+
 /* Stand-alone pieces of stage 4 (used by the multi-GPU path and by tests). */
 DDN_API int ddn_voxel_keys(const ddn_voxel_grid* grid_host, int64_t n_points, const float* xyz,
                    uint64_t* keys, void* stream);

@@ -5,7 +5,7 @@
 Kernels are matched by name.  A `kRagged = false` instantiation (trailing `kRagged` template argument and `const int64_t*
 layout` parameter: K3, K4) whose name the base build lacks is compared with the base kernel of its pre-ragged name, so a
 base from before the ragged layout can be checked too; kernels only the new build has are listed as NEW."""
-import re, subprocess, sys
+import os, re, subprocess, sys
 def funcs(obj):
     out = subprocess.run(["/usr/local/cuda/bin/cuobjdump", "-sass", obj], capture_output=True, text=True, check=True).stdout
     d, cur = {}, None
@@ -20,8 +20,9 @@ def norm(name):  # new uniform instantiation -> the pre-ragged name
     return re.sub(r", false>\(", ">(", name).replace(", long const*)", ")")
 base, new = sys.argv[1], sys.argv[2]
 tot = same = 0
-for src in ["align.cu.o", "filter.cu.o", "fuse.cu.o", "fuse_sort.cu.o", "api.cu.o", "geometry.cu.o", "pchip.cu.o", "masks.cu.o"]:
-    a, b = funcs(f"{base}/{src}"), funcs(f"{new}/{src}")
+for src in ["align.cu.o", "filter.cu.o", "fuse.cu.o", "fuse_sort.cu.o", "fuse_hash.cu.o", "fuse_hash_peers.cu.o", "api.cu.o", "geometry.cu.o",
+            "pchip.cu.o", "masks.cu.o"]:
+    a, b = (funcs(f"{d}/{src}") if os.path.exists(f"{d}/{src}") else {} for d in (base, new))
     pre_ragged = {norm(k): k for k in b if k not in a and k.endswith(", long const*)") and ", false>(" in k}
     matched = set()
     for name, ins in a.items():
