@@ -12,7 +12,7 @@ from pathlib import Path
 PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 LIB_PATH = PKG_DIR / "libddn_b200.so"
-SOURCES = ["api.cu", "align.cu", "filter.cu", "fuse.cu", "fuse_sort.cu", "fuse_hash.cu", "fuse_hash_peers.cu", "geometry.cu", "pchip.cu", "masks.cu"]
+SOURCES = ["api.cu", "align.cu", "filter.cu", "fuse.cu", "fuse_hash.cu", "fuse_hash_peers.cu", "geometry.cu", "pchip.cu", "masks.cu"]
 NVCC_FLAGS = [
     "-std=c++17",
     "-O3",

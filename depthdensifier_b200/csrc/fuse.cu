@@ -23,10 +23,10 @@
 // bounding boxes on the device, every grid-sized pass is a persistent kernel that reads the actual
 // extent, so a whole step - and the multi-GPU exchange + merge over peer memory at the end of this
 // file - runs without the host looking at any intermediate result.
-// Grids with more than 2^35 cells take the sort path in fuse_sort.cu (host-grid entry points only).
+// The host-grid entry points fuse grids of more than 2^35 cells with the hashed path (fuse_hash.cu).
 #include <algorithm>
 
-#include "fuse_common.cuh"
+#include "fuse_hash.cuh"
 
 namespace ddn {
 
@@ -962,23 +962,28 @@ struct DenseLayout {
   size_t grid, units, tile_sums, accum, total;
 };
 
+// consecutive 256-byte aligned pieces of a workspace
+struct WorkspaceOffsets {
+  size_t off = 0;
+  size_t take(size_t bytes) {
+    const size_t o = off;
+    off += (size_t)align_up((int64_t)bytes, 256);
+    return o;
+  }
+};
+
 static void dense_layout(const GridDev& g, int64_t n, DenseLayout* L) {  // sized for the non-partial form
   L->cells = grid_cells(g);
   L->n_units = (L->cells + kUnitBits - 1) / kUnitBits;
   L->tiles = (L->n_units + kTileUnits - 1) / kTileUnits;
   L->own_tiles = (L->n_units + kOwnUnits - 1) / kOwnUnits;
   const uint64_t max_vox = (uint64_t)n < L->cells ? (uint64_t)n : L->cells;
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    size_t o = off;
-    off += (size_t)align_up((int64_t)bytes, 256);
-    return o;
-  };
-  L->grid = take(sizeof(GridDev));
-  L->units = take((size_t)L->n_units * 16);
-  L->tile_sums = take((size_t)(L->own_tiles + 2) * 4);
-  L->accum = take((size_t)max_vox * kAccWords * 8 + 16);
-  L->total = off + 256;
+  WorkspaceOffsets o;
+  L->grid = o.take(sizeof(GridDev));
+  L->units = o.take((size_t)L->n_units * 16);
+  L->tile_sums = o.take((size_t)(L->own_tiles + 2) * 4);
+  L->accum = o.take((size_t)max_vox * kAccWords * 8 + 16);
+  L->total = o.off + 256;
 }
 
 static int carve_session(const GridDev& g, int64_t n, void* workspace, int64_t workspace_bytes, ddn_fuse_session* s,
@@ -1007,6 +1012,62 @@ static int begin_with_grid(const ddn_fuse_session* s, const GridDev& g, cudaStre
   return launch_clear(s, st);
 }
 
+// Grids of more than 2^35 cells: the hashed path on a session and hash buffers carved out of the caller's workspace.
+// One layout serves ddn_voxel_fuse, ddn_voxel_partials and ddn_voxel_merge on n points (or records), so
+// ddn_fuse_workspace_bytes is the most any of them needs.
+struct HashedWork {
+  ddn_fuse_session s;  // grid and counts only
+  ddn_hash_fuse hf;
+  uint64_t* samples;   // [DDN_HASH_SAMPLES + 1]
+  int64_t* plan;       // [64]
+  void* scratch;       // the accumulator of fuse and partials, the merge's staging
+  int64_t scratch_bytes;
+};
+
+// Bytes of the layout for n > 0 points; with a (256-byte aligned) base also the pointers into it.
+static int hashed_layout(int64_t n, char* base, HashedWork* w, int64_t* total) {
+  int64_t cap_slots, table_bytes, slots_bytes, sort_bytes, hist_bytes, merge_bytes;
+  DDN_TRY(ddn_hash_fuse_sizes(n, &cap_slots, &table_bytes, &slots_bytes, &sort_bytes, &hist_bytes));
+  DDN_TRY(ddn_fuse_merge_hashed_scratch_bytes(1, n, &merge_bytes));
+  const int64_t scratch_bytes = std::max<int64_t>(n * kAccWords * 8 + 16, merge_bytes);
+  WorkspaceOffsets o;
+  const size_t grid = o.take(sizeof(GridDev)), table = o.take(table_bytes), slots = o.take(slots_bytes),
+               sort = o.take(sort_bytes), hist = o.take(hist_bytes), state = o.take(DDN_HASH_STATE_BYTES),
+               samples = o.take((DDN_HASH_SAMPLES + 1) * 8), plan = o.take(64 * 8), scratch = o.take(scratch_bytes);
+  *total = (int64_t)o.off + 256;
+  if (base == nullptr) return DDN_OK;
+  w->s = ddn_fuse_session{};
+  w->s.grid = reinterpret_cast<ddn_grid_state*>(base + grid);
+  w->hf.table = base + table;
+  w->hf.slots = reinterpret_cast<uint32_t*>(base + slots);
+  w->hf.sort = base + sort;
+  w->hf.hist = reinterpret_cast<uint32_t*>(base + hist);
+  w->hf.state = reinterpret_cast<int64_t*>(base + state);
+  w->hf.cap_slots = cap_slots;
+  w->hf.cap_voxels = n;
+  w->samples = reinterpret_cast<uint64_t*>(base + samples);
+  w->plan = reinterpret_cast<int64_t*>(base + plan);
+  w->scratch = base + scratch;
+  w->scratch_bytes = scratch_bytes;
+  return DDN_OK;
+}
+
+// Checks the workspace before anything is enqueued, then stores the grid with cap_units = 0, i.e. as
+// DDN_GRID_TOO_LARGE (the status on which the hashed path's mode 0 runs), and empties the hash buffers.
+static int carve_hashed(const GridDev& g, int64_t n, void* workspace, int64_t workspace_bytes, int64_t* counts_out, HashedWork* w,
+                        cudaStream_t st) {
+  int64_t total = 0;
+  DDN_TRY(hashed_layout(n, reinterpret_cast<char*>(align_up((int64_t)(uintptr_t)workspace, 256)), w, &total));
+  if (total > workspace_bytes) {
+    set_error("fuse workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)total);
+    return DDN_ERR_WORKSPACE_TOO_SMALL;
+  }
+  w->s.counts = counts_out;
+  grid_store_kernel<<<1, 32, 0, st>>>(g, 0, reinterpret_cast<GridDev*>(w->s.grid), reinterpret_cast<unsigned long long*>(counts_out));
+  DDN_TRY(after_launch("grid_store_kernel"));
+  return ddn_hash_fuse_reset(&w->hf, st);
+}
+
 }  // namespace ddn
 
 extern "C" {
@@ -1026,7 +1087,8 @@ int ddn_fuse_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, 
       return DDN_OK;
     }
   }
-  return sort_fuse_workspace_bytes(n, bytes_out);
+  HashedWork w;
+  return hashed_layout(n, nullptr, &w, bytes_out);
 }
 
 int ddn_voxel_fuse(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
@@ -1043,9 +1105,12 @@ int ddn_voxel_fuse(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t ro
   vote_threshold = std::min(vote_threshold, 255);
   if (n_points == 0) return check_cuda(cudaMemsetAsync(counts_out, 0, 16, st), "memset counts");
   DDN_REQUIRE(xyz && rgb && out_keys && out_xyz && out_rgb && out_count && workspace, "null pointer");
-  if (!use_dense(g))
-    return sort_fuse_points(g, n_points, xyz, rgb, votes, vote_threshold, out_keys, out_xyz, out_rgb, out_count, counts_out,
-                            workspace, workspace_bytes, st, nullptr);
+  if (!use_dense(g)) {
+    HashedWork w;
+    DDN_TRY(carve_hashed(g, n_points, workspace, workspace_bytes, counts_out, &w, st));
+    return ddn_fuse_finish_hashed(&w.s, &w.hf, 0, n_points, row_len, xyz, rgb, votes, vote_threshold, nullptr, 0, out_keys, out_xyz,
+                                  out_rgb, out_count, n_points, w.scratch, w.scratch_bytes, st);
+  }
   ddn_fuse_session s;
   unsigned long long* accum;
   DenseLayout L;
@@ -1094,9 +1159,12 @@ int ddn_voxel_partials(const ddn_voxel_grid* grid_host, int64_t n_points, int64_
   }
   DDN_REQUIRE(xyz && rgb && records && workspace, "null pointer");
   DDN_REQUIRE((uintptr_t)records % 16 == 0, "records must be 16-byte aligned");
-  if (!use_dense(g))
-    return sort_fuse_points(g, n_points, xyz, rgb, votes, vote_threshold, nullptr, nullptr, nullptr, nullptr, counts_out, workspace,
-                            workspace_bytes, st, (unsigned long long*)records);
+  if (!use_dense(g)) {  // records sorted by compact key, which orders as the canonical key
+    HashedWork w;
+    DDN_TRY(carve_hashed(g, n_points, workspace, workspace_bytes, counts_out, &w, st));
+    return ddn_fuse_finish_hashed_partial(&w.s, &w.hf, 0, n_points, row_len, xyz, rgb, votes, vote_threshold, nullptr, 0, records,
+                                          n_points, w.samples, w.scratch, w.scratch_bytes, st);
+  }
   ddn_fuse_session s;
   unsigned long long* accum;
   DenseLayout L;
@@ -1120,9 +1188,25 @@ int ddn_voxel_merge(const ddn_voxel_grid* grid_host, int64_t n_records, const ui
   cudaStream_t st = (cudaStream_t)stream;
   if (n_records == 0) return check_cuda(cudaMemsetAsync(counts_out, 0, 16, st), "memset counts");
   DDN_REQUIRE(records && out_keys && out_xyz && out_rgb && out_count && workspace, "null pointer");
-  if (!use_dense(g))
-    return sort_merge_records(g, n_records, (const unsigned long long*)records, out_keys, out_xyz, out_rgb, out_count, counts_out,
-                              workspace, workspace_bytes, st);
+  if (!use_dense(g)) {
+    // The records, in any order, merged as the only rank's: with no splitters the cut is [0, n_records) whatever the
+    // sample keys, as long as they stay below ~0.  hash_begin on an empty step arms the path first (and zeroes
+    // counts); counts[0] then reports the records, or -1 when the merge finds a voxel of 2^24 or more points.
+    HashedWork w;
+    DDN_TRY(carve_hashed(g, n_records, workspace, workspace_bytes, counts_out, &w, st));
+    HashDev h;
+    DDN_TRY(hash_dev(&w.hf, &h));
+    DDN_TRY(hash_launch_points(reinterpret_cast<GridDev*>(w.s.grid), h, reinterpret_cast<unsigned long long*>(counts_out), 0, 0, 0,
+                               nullptr, nullptr, nullptr, 0, nullptr, 0, nullptr, st));
+    const int64_t m = n_records;
+    DDN_TRY(check_cuda(cudaMemsetAsync(w.samples, 0, DDN_HASH_SAMPLES * 8, st), "memset samples"));
+    DDN_TRY(check_cuda(cudaMemcpyAsync(w.samples + DDN_HASH_SAMPLES, &m, 8, cudaMemcpyHostToDevice, st), "copy record count"));
+    DDN_TRY(check_cuda(cudaMemcpyAsync(counts_out, &m, 8, cudaMemcpyHostToDevice, st), "copy record count"));
+    const void* rec = records;
+    const void* smp = w.samples;
+    return ddn_fuse_merge_hashed_peers(&w.s, &w.hf, 0, 1, &rec, &smp, w.plan, w.scratch, w.scratch_bytes, out_keys, out_xyz, out_rgb,
+                                       out_count, n_records, st);
+  }
   ddn_fuse_session s;
   unsigned long long* accum;
   DenseLayout L;

@@ -1,7 +1,7 @@
 // Shared definitions of stage 4 (voxel-grid fusion): grid description, IEEE-exact voxel coordinates,
 // the occupancy-unit layout, fixed-point offsets and the finalisation of one voxel.  Used by the
-// dense-rank path (fuse.cu), by K4's fused occupancy marking (filter.cu) and by the sort path kept for
-// grids too large for a dense occupancy bitmap (fuse_sort.cu).
+// dense-rank path (fuse.cu), by K4's fused occupancy marking (filter.cu) and by the hashed path for grids
+// too large for a dense occupancy bitmap (fuse_hash.cu, fuse_hash_peers.cu).
 #pragma once
 
 #include "common.cuh"
@@ -13,7 +13,7 @@ namespace ddn {
 // the host and pass it by value to a one-thread kernel that stores it.
 struct GridDev {
   float voxel, ox, oy, oz;
-  int bx, by, bz;     // significant bits per axis (sort path key packing)
+  int bx, by, bz;     // significant bits per axis (the hashed path's compact key packing)
   int nx, ny, nz;     // cells per axis; a point outside [0, n) on any axis does not participate
   long long n_units;  // ceil(cells / 96); 0 when status != DDN_GRID_OK
   int status, reserved;
@@ -190,15 +190,5 @@ __device__ __forceinline__ unsigned long long pull_share_warp(const PeerPtrs& pe
   }
   return key;
 }
-
-// ---- sort path (fuse_sort.cu) -------------------------------------------------------------------
-// records != nullptr: partial mode, output = records [.,DDN_RECORD_WORDS] (see include/ddn_b200.h)
-int sort_fuse_workspace_bytes(int64_t n_points, int64_t* bytes_out);
-int sort_fuse_points(const GridDev& g, int64_t n, const float* xyz, const uint8_t* rgb, const uint8_t* votes, int thr,
-                     uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t* counts_out,
-                     void* workspace, int64_t workspace_bytes, cudaStream_t st, unsigned long long* records);
-int sort_merge_records(const GridDev& g, int64_t n, const unsigned long long* records, uint64_t* out_keys, float* out_xyz,
-                       uint8_t* out_rgb, int32_t* out_count, int64_t* counts_out, void* workspace, int64_t workspace_bytes,
-                       cudaStream_t st);
 
 }  // namespace ddn

@@ -549,13 +549,8 @@ class ShardedDensifier:
             mark = lambda name, fn: fn()
         n_tiles, _ = self.ops.fuse_tile_info(grid)
         tile_prefix = torch.empty(n_tiles + 1, dtype=torch.int32, device=self.device) if n_tiles > 0 else None
-        rec_out = None
-        if self.peer is not None and tile_prefix is not None:
-            rec_out, hdl, _ = self.peer.buffer("records", self.peer_records_shape, torch.int64)
-            hdl.barrier()  # peers finished pulling last step's records
         rec, counts = mark("fuse_partials", lambda: self.ops.voxel_fuse_partial(
-            xyz.view(-1, 3), rgb.view(-1, 3), votes.view(-1), self.thr, grid, row_len=xyz.shape[2], tile_prefix=tile_prefix,
-            out=rec_out))
+            xyz.view(-1, 3), rgb.view(-1, 3), votes.view(-1), self.thr, grid, row_len=xyz.shape[2], tile_prefix=tile_prefix))
         return mark("fuse_exchange_merge", lambda: self._exchange_and_merge(rec, counts, grid, mark, tile_prefix))
 
     def _plan_by_tiles(self, tile_prefix):
@@ -578,12 +573,11 @@ class ShardedDensifier:
         at = allp[:, bnd]  # [R, R + 1] record index of every rank at every boundary
         send = at[r, 1:] - at[r, :-1]
         recv = at[:, r + 1] - at[:, r]
-        host = torch.cat([send, recv, bnd[r:r + 2], at[r, -1:], at[:, r]]).cpu().tolist()  # the one readback
-        self._peer_offsets = host[2 * R + 3:]  # where my share starts in every rank's records
+        host = torch.cat([send, recv, bnd[r:r + 2], at[r, -1:]]).cpu().tolist()  # the one readback
         return host[:R], host[R:2 * R], (host[2 * R], host[2 * R + 1]), host[2 * R + 2]
 
     def _plan_by_samples(self, rec, mv):
-        """Sort-path fallback (grids too large for tiles): R-1 sampled splitter keys."""
+        """Grids too large for tiles: R-1 sampled splitter keys."""
         import torch.distributed as dist
 
         R = self.world
@@ -620,17 +614,6 @@ class ShardedDensifier:
         def exchange():
             # the sorted records of one destination are one contiguous slice: no pack kernel
             out = torch.empty((n_recv, W), dtype=rec.dtype, device=self.device)
-            if self.peer is not None and tile_prefix is not None:
-                # pull my share out of every rank's record buffer over NVLink (copy engines, peer reads)
-                _, hdl, views = self.peer.buffer("records", tuple(self.peer_records_shape), torch.int64)
-                hdl.barrier()  # everybody's records are complete
-                o = 0
-                for k in range(self.world):
-                    q = (self.rank + k) % self.world  # start with the local share, then stagger the peers
-                    o_q = sum(rc[:q])
-                    if rc[q]:
-                        out[o_q:o_q + rc[q]].copy_(views[q][self._peer_offsets[q]:self._peer_offsets[q] + rc[q]], non_blocking=True)
-                return out
             dist.all_to_all_single(out.view(-1), rec.reshape(-1), output_split_sizes=[c * W for c in rc],
                                    input_split_sizes=[c * W for c in sc], group=self.group)
             return out

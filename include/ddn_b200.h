@@ -278,8 +278,9 @@ typedef struct {
 
 /* Scratch for ddn_voxel_fuse / ddn_voxel_partials / ddn_voxel_merge on `grid_host` with up to
  * n_points points (or records).  Grids of up to 2^35 cells use a dense occupancy bitmap
- * (cells/8 bytes + 40 B per possible voxel); larger grids (or grid_host == NULL: worst case of the
- * sort path) use a radix sort. */
+ * (cells/8 bytes + 40 B per possible voxel); larger grids (and grid_host == NULL) use the hashed path
+ * (ddn_fuse_finish_hashed and its partial and merge forms) on hash buffers carved out of the workspace:
+ * 100-124 B per point or record, the most any of the three calls needs. */
 DDN_API int ddn_fuse_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t* bytes_out);
 
 /* xyz [N,3] f32, rgb [N,3] u8, votes [N] u8 (point i participates iff votes[i] < vote_threshold;

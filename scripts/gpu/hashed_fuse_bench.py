@@ -6,8 +6,9 @@ stride 1), one B200:
             counts are first asserted bit-identical to `dense`
   dome      a cfg-2-sized scene with distant background (dome_radius 200 m): its box is far beyond 2^35 cells, so only
             the hashed path can fuse it (step time, voxels, grid cells)
-  sort      ops.voxel_fuse (the host-grid entry point's CUB sort path) over the kept points of the cfg 2 step on a grid
-            of more than 2^35 cells, the existing alternative for such grids
+  host_grid the host-grid entry points on a grid of more than 2^35 cells, which also fuse through the hashed kernels:
+            ops.voxel_fuse over the first 10^4 and 10^6 kept points of the cfg 2 step and over all of them, and
+            ops.voxel_fuse_partial on two halves of all kept points followed by ops.voxel_merge_partials
 
 dense and hashed are timed alternately in the same run (`--rounds` pairs).  Step times: CUDA events around `steps`
 back-to-back steps after `warmup`; per-stage times: a separate pass with events between align, K4 + fused mark, the
@@ -126,16 +127,24 @@ def main() -> None:
     dev_ms = lambda e: getattr(e, "device_time_total", getattr(e, "cuda_time_total", 0.0)) / 1000.0 / 2
     out["hashed"]["kernels_ms_per_step"] = {e.key.split("(")[0]: dev_ms(e) for e in prof.key_averages() if "hash_" in e.key}
 
-    # sort path: the same kept points on a host grid of more than 2^35 cells
+    # host-grid entry points: the same kept points on a host grid of more than 2^35 cells
     lo = kept_xyz.min(0).values.cpu().numpy()
     grid = ops.make_grid(lo, lo + 400.0, VOXEL)
     cells = int(np.prod([grid.dims[i] for i in range(3)], dtype=np.float64))
     assert cells > 2**35
-    sort = lambda: ops.voxel_fuse(kept_xyz, kept_rgb, None, 1, grid, trim=False)
-    k_sort = ops.voxel_fuse(kept_xyz, kept_rgb, None, 1, grid)
-    out["sort"] = {"ms_per_call": timed(sort, args.steps, args.warmup), "grid_cells": cells, "points": int(kept_xyz.shape[0]),
-                   "voxels": int(k_sort[0].shape[0])}
-    del k_sort, kept_xyz, kept_rgb, sc, inputs
+    n_all = int(kept_xyz.shape[0])
+    out["host_grid"] = {"grid_cells": cells}
+    for n in (10**4, 10**6, n_all):
+        fuse = lambda: ops.voxel_fuse(kept_xyz[:n], kept_rgb[:n], None, 1, grid, trim=False)
+        out["host_grid"][f"voxel_fuse_{n}"] = {"ms_per_call": timed(fuse, args.steps, args.warmup), "voxels": int(fuse()[4][1])}
+
+    def partials_merge():
+        parts = [ops.voxel_fuse_partial(kept_xyz[a:b], kept_rgb[a:b], None, 1, grid) for a, b in ((0, n_all // 2), (n_all // 2, n_all))]
+        return ops.voxel_merge_partials(torch.cat([r[: int(c[1])] for r, c in parts]), grid)
+
+    out["host_grid"][f"partials_merge_{n_all}"] = {"ms_per_call": timed(partials_merge, args.steps, args.warmup),
+                                                   "voxels": int(partials_merge()[4][1])}
+    del kept_xyz, kept_rgb, sc, inputs
     engines["dense"] = None
     torch.cuda.empty_cache()
 

@@ -4,7 +4,8 @@
 
 Kernels are matched by name.  A `kRagged = false` instantiation (trailing `kRagged` template argument and `const int64_t*
 layout` parameter: K3, K4) whose name the base build lacks is compared with the base kernel of its pre-ragged name, so a
-base from before the ragged layout can be checked too; kernels only the new build has are listed as NEW."""
+base from before the ragged layout can be checked too; kernels only the new build has are listed as NEW, and base kernels
+the new build no longer has (a deleted source or kernel) as GONE.  Every *.cu.o of either directory is read.  The exit status checks the kernels both builds have."""
 import os, re, subprocess, sys
 def funcs(obj):
     out = subprocess.run(["/usr/local/cuda/bin/cuobjdump", "-sass", obj], capture_output=True, text=True, check=True).stdout
@@ -19,19 +20,20 @@ def funcs(obj):
 def norm(name):  # new uniform instantiation -> the pre-ragged name
     return re.sub(r", false>\(", ">(", name).replace(", long const*)", ")")
 base, new = sys.argv[1], sys.argv[2]
-tot = same = 0
-for src in ["align.cu.o", "filter.cu.o", "fuse.cu.o", "fuse_sort.cu.o", "fuse_hash.cu.o", "fuse_hash_peers.cu.o", "api.cu.o", "geometry.cu.o",
-            "pchip.cu.o", "masks.cu.o"]:
+tot = same = gone = 0
+for src in sorted({f for d in (base, new) for f in os.listdir(d) if f.endswith(".cu.o")}):
     a, b = (funcs(f"{d}/{src}") if os.path.exists(f"{d}/{src}") else {} for d in (base, new))
     pre_ragged = {norm(k): k for k in b if k not in a and k.endswith(", long const*)") and ", false>(" in k}
     matched = set()
     for name, ins in a.items():
-        tot += 1
         twin = name if name in b else pre_ragged.get(name)
+        if twin is None:
+            print("GONE", src, name, len(ins)); gone += 1; continue
+        tot += 1
         matched.add(twin)
         if b.get(twin) == ins: same += 1
         else: print("DIFF", src, name, len(ins), len(b.get(twin, [])))
     for name in b:
         if name not in matched: print("NEW ", src, name, len(b[name]))
-print(f"{same}/{tot} base kernels instruction-identical")
+print(f"{same}/{tot} base kernels instruction-identical, {gone} gone")
 sys.exit(0 if same == tot else 1)

@@ -27,7 +27,8 @@ def canonical_keys(xyz32, voxel, origin):
 
 
 def partial_sums_numpy(xyz32, rgb, voxel, origin):
-    """Per-voxel integer sums exactly as segment_mean_kernel<.., true> computes them."""
+    """Per-voxel integer sums exactly as the partial-record kernels (accumulate_points_kernel, hash_insert_kernel)
+    compute them: keys ascending, the records' words 1..5 before packing."""
     if len(xyz32) == 0:
         z = np.zeros
         return z(0, np.int64), z((0, 3), np.int64), z((0, 3), np.int64), z(0, np.int32)

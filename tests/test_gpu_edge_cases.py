@@ -21,9 +21,20 @@ def _cuda(x):
 
 
 def test_fuse_empty_and_fully_rejected(lib_built):
+    """Empty input, all points rejected, points outside the grid, empty partials and an empty merge."""
+    _check_empty_and_rejected(large=False)
+
+
+def test_fuse_empty_and_fully_rejected_over_2e35_cells(lib_built):
+    """The same on a grid of more than 2^35 cells (hashed path)."""
+    _check_empty_and_rejected(large=True)
+
+
+def _check_empty_and_rejected(large: bool):
     from depthdensifier_b200 import ops
 
-    grid = ops.make_grid([0, 0, 0], [1, 1, 1], 0.1)
+    grid = ops.make_grid([0, 0, 0], [100, 100, 100], 0.01) if large else ops.make_grid([0, 0, 0], [1, 1, 1], 0.1)
+    assert (ops.fuse_tile_info(grid)[0] == 0) == large
     e = ops.voxel_fuse(torch.zeros((0, 3), device="cuda"), torch.zeros((0, 3), dtype=torch.uint8, device="cuda"), None, 1, grid)
     assert e[4].cpu().tolist() == [0, 0] and all(len(t) == 0 for t in e[:4])
     xyz = _cuda(np.random.default_rng(0).uniform(0, 1, (1000, 3)).astype(np.float32))
@@ -32,7 +43,7 @@ def test_fuse_empty_and_fully_rejected(lib_built):
     k, x, c, n, counts = ops.voxel_fuse(xyz, rgb, votes, 3, grid)
     assert counts.cpu().tolist() == [0, 0] and len(k) == 0
     # points outside the grid do not participate either
-    far = xyz + 100.0
+    far = xyz + 1000.0
     k, x, c, n, counts = ops.voxel_fuse(far, rgb, None, 1, grid)
     assert counts.cpu().tolist() == [0, 0]
     rec, cnt = ops.voxel_fuse_partial(xyz, rgb, votes, 3, grid)
@@ -43,12 +54,15 @@ def test_fuse_empty_and_fully_rejected(lib_built):
 
 @settings(max_examples=25, deadline=None, derandomize=True, suppress_health_check=[HealthCheck.function_scoped_fixture])
 @given(n=st.integers(1, 3000), voxel=st.sampled_from([0.5, 0.1, 0.03]), seed=st.integers(0, 10_000),
-       row_len=st.sampled_from([0, 8, 13, 64]), clustered=st.booleans())
-def test_fuse_random_vs_numpy(lib_built, n, voxel, seed, row_len, clustered):
+       row_len=st.sampled_from([0, 8, 13, 64]), clustered=st.booleans(), far=st.booleans())
+def test_fuse_random_vs_numpy(lib_built, n, voxel, seed, row_len, clustered, far):
+    """far: a quarter of the points (at least one) 4 km away, so the grid has more than 2^35 cells (hashed path)."""
     from depthdensifier_b200 import ops
 
     rng = np.random.default_rng(seed)
     xyz = (rng.normal(0, 0.02 if clustered else 1.0, (n, 3)) + rng.uniform(-3, 3, 3)).astype(np.float32)
+    if far:
+        xyz[: max(1, n // 4)] += np.float32(4000.0)
     rgb = rng.integers(0, 256, (n, 3)).astype(np.uint8)
     origin = R.voxel_origin(xyz, voxel)
     k_ref, m_ref, c_ref, n_ref = R.voxel_fuse(xyz, rgb, voxel, origin)
@@ -58,6 +72,23 @@ def test_fuse_random_vs_numpy(lib_built, n, voxel, seed, row_len, clustered):
     assert np.array_equal(k.cpu().numpy().view(np.uint64), k_ref) and np.array_equal(cnt.cpu().numpy(), n_ref)
     assert np.array_equal(c.cpu().numpy(), c_ref)
     assert np.abs(m.cpu().numpy() - m_ref).max() <= 1e-5 * max(1.0, np.abs(m_ref).max())
+
+
+@pytest.mark.parametrize("large", [False, True], ids=["dense", "over_2e35_cells"])
+def test_fuse_flags_a_voxel_of_2e24_points(lib_built, large):
+    """A voxel that collects 2^24 points (32-bit colour sums) sets counts[0] = -1 on every grid, and trim raises."""
+    from depthdensifier_b200 import ops
+    from depthdensifier_b200._lib import DDNError
+
+    grid = ops.make_grid([0, 0, 0], [100, 100, 100], 0.01) if large else ops.make_grid([0, 0, 0], [1, 1, 1], 0.1)
+    assert (ops.fuse_tile_info(grid)[0] == 0) == large
+    n = 1 << 24
+    xyz = torch.full((n, 3), 0.555, dtype=torch.float32, device="cuda")
+    rgb = torch.full((n, 3), 255, dtype=torch.uint8, device="cuda")
+    counts = ops.voxel_fuse(xyz, rgb, None, 1, grid, trim=False)[4]
+    assert counts.cpu().tolist() == [-1, 1]
+    with pytest.raises(DDNError, match="2\\^24"):
+        ops.voxel_fuse(xyz, rgb, None, 1, grid, trim=True)
 
 
 def test_filter_padded_and_duplicate_neighbours(lib_built):

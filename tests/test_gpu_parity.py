@@ -212,11 +212,12 @@ def test_depth_refiner_dropin(lib_built, golden_dir):
 
 
 @pytest.mark.parametrize("n,voxel,spread,row_len", [(20000, 0.05, 1.0, 0), (200000, 0.01, 3.0, 37), (1, 0.01, 1.0, 8),
-                                                    (5000, 0.001, 40.0, 0), (70001, 0.2, 2.0, 512), (33333, 0.02, 0.3, 33333)])
+                                                    (5000, 0.001, 40.0, 0), (70001, 0.2, 2.0, 512), (33333, 0.02, 0.3, 33333),
+                                                    (200000, 0.001, 40.0, 37)])
 def test_voxel_fuse_vs_oracle(lib_built, n, voxel, spread, row_len):
-    """N4: keys and counts bit-exact, positions within 1e-5 relative, colours exact.  The 0.001 / 40 case
-    has a grid of more than 2^35 cells and takes the sort path, the others the dense-rank path; row_len
-    (the image-width locality hint) must not change the result."""
+    """N4: keys and counts bit-exact, positions within 1e-5 relative, colours exact.  The 0.001 / 40 cases
+    have a grid of more than 2^35 cells and take the hashed path (200 000 points: several sort CTAs and the tiled
+    insert), the others the dense-rank path; row_len (the image-width locality hint) must not change the result."""
     from depthdensifier_b200 import ops
 
     rng = np.random.default_rng(n)
@@ -286,13 +287,25 @@ def test_pipeline_end_to_end_vs_oracle(lib_built):
 
 def test_voxel_partials_and_merge_bit_exact(lib_built):
     """Multi-GPU form of N4: partial sums and their merge are integer arithmetic -> bit-exact against the
-    numpy statement in tests/cpu_backend.py, and merge(partials of two halves) == fuse(all)."""
+    numpy statement in tests/cpu_backend.py, and merge(partials of two halves) == fuse(all), also when the
+    records arrive in random order."""
+    _check_partials_and_merge(far=False)
+
+
+def test_voxel_partials_and_merge_bit_exact_over_2e35_cells(lib_built):
+    """The same on a grid of more than 2^35 cells (a second cluster 400 m away): the hashed path, no ownership tiles."""
+    _check_partials_and_merge(far=True)
+
+
+def _check_partials_and_merge(far: bool):
     from cpu_backend import finalize_numpy, merge_numpy, pack_records, partial_sums_numpy, unpack_records
     from depthdensifier_b200 import ops
 
     rng = np.random.default_rng(5)
     n = 150000
     xyz = rng.normal(0, 0.7, (n, 3)).astype(np.float32)
+    if far:
+        xyz[rng.random(n) < 0.2] += np.float32(400.0)
     rgb = rng.integers(0, 256, (n, 3)).astype(np.uint8)
     voxel = 0.02
     grid = ops.make_grid(xyz.min(0), xyz.max(0), voxel)
@@ -309,20 +322,29 @@ def test_voxel_partials_and_merge_bit_exact(lib_built):
     parts = [ops.voxel_fuse_partial(_cuda(xyz[a:b]), _cuda(rgb[a:b]), None, 1, grid) for a, b in ((0, h), (h, n))]
     cat = torch.cat([p[0][: int(p[1][1])] for p in parts]).contiguous()
     k, x, c, m, mc = ops.voxel_merge_partials(cat, grid, trim=True)
-    # ownership tiles: the prefix of records per tile, and merges restricted to tile ranges
+    assert mc.cpu().tolist() == [cat.shape[0], len(uk)]
+    perm = torch.from_numpy(rng.permutation(cat.shape[0])).cuda()
+    shuffled = ops.voxel_merge_partials(cat[perm].contiguous(), grid, trim=True)
+    for i in range(5):
+        assert np.array_equal(shuffled[i].cpu().numpy(), (k, x, c, m, mc)[i].cpu().numpy())
+    # ownership tiles (none on a grid beyond 2^35 cells): the prefix of records per tile, and merges restricted to
+    # tile ranges
     from cpu_backend import OracleBackend
 
     n_tiles, cells_per_tile = ops.fuse_tile_info(grid)
-    assert (n_tiles, cells_per_tile) == OracleBackend().fuse_tile_info(grid)
-    tp = torch.full((n_tiles + 1,), -7, dtype=torch.int32, device="cuda")
-    rec2, _ = ops.voxel_fuse_partial(_cuda(xyz), _cuda(rgb), None, 1, grid, tile_prefix=tp)
-    tiles_of = OracleBackend()._tile_of_keys(uk, grid)
-    assert np.array_equal(tp.cpu().numpy(), np.searchsorted(tiles_of, np.arange(n_tiles + 1)))
-    cut = int(np.searchsorted(np.cumsum(np.bincount(tiles_of, minlength=n_tiles)), len(uk) // 2))
-    halves = [ops.voxel_merge_partials(cat, grid, trim=True, tile_range=r) for r in ((0, cut), (cut, n_tiles))]
-    assert len(halves[0][0]) > 0 and len(halves[1][0]) > 0
-    for i in range(4):
-        assert np.array_equal(torch.cat([halves[0][i], halves[1][i]]).cpu().numpy(), (k, x, c, m)[i].cpu().numpy())
+    if far:
+        assert n_tiles == 0
+    else:
+        assert (n_tiles, cells_per_tile) == OracleBackend().fuse_tile_info(grid)
+        tp = torch.full((n_tiles + 1,), -7, dtype=torch.int32, device="cuda")
+        rec2, _ = ops.voxel_fuse_partial(_cuda(xyz), _cuda(rgb), None, 1, grid, tile_prefix=tp)
+        tiles_of = OracleBackend()._tile_of_keys(uk, grid)
+        assert np.array_equal(tp.cpu().numpy(), np.searchsorted(tiles_of, np.arange(n_tiles + 1)))
+        cut = int(np.searchsorted(np.cumsum(np.bincount(tiles_of, minlength=n_tiles)), len(uk) // 2))
+        halves = [ops.voxel_merge_partials(cat, grid, trim=True, tile_range=r) for r in ((0, cut), (cut, n_tiles))]
+        assert len(halves[0][0]) > 0 and len(halves[1][0]) > 0
+        for i in range(4):
+            assert np.array_equal(torch.cat([halves[0][i], halves[1][i]]).cpu().numpy(), (k, x, c, m)[i].cpu().numpy())
     full = ops.voxel_fuse(_cuda(xyz), _cuda(rgb), None, 1, grid)
     assert np.array_equal(k.cpu().numpy(), full[0].cpu().numpy()) and np.array_equal(m.cpu().numpy(), full[3].cpu().numpy())
     assert np.array_equal(x.cpu().numpy(), full[1].cpu().numpy()) and np.array_equal(c.cpu().numpy(), full[2].cpu().numpy())

@@ -54,6 +54,36 @@ def test_hash_fuse_sizes_and_argument_checks(lib_built):
     assert b"invalid argument" in lib.ddn_last_error_string()
 
 
+@pytest.mark.parametrize("large", [False, True], ids=["dense", "over_2e35_cells"])
+def test_host_grid_workspace_is_checked_before_any_launch(lib_built, large):
+    """ddn_fuse_workspace_bytes sizes ddn_voxel_fuse, ddn_voxel_partials and ddn_voxel_merge on a dense grid and on one of
+    more than 2^35 cells (the hashed path, also the size for grid NULL); 16 bytes less makes each of them return
+    DDN_ERR_WORKSPACE_TOO_SMALL without launching anything (the dummy device pointers are never touched)."""
+    from depthdensifier_b200 import _lib
+
+    lib = _lib.load()
+    g = _lib.VoxelGrid()
+    g.voxel = 0.01
+    for i, d in enumerate([4000, 4000, 4000] if large else [100, 80, 60]):
+        g.bits[i] = int(d - 1).bit_length()
+        g.dims[i] = d
+    assert (int(g.dims[0]) * g.dims[1] * g.dims[2] > 2**35) == large
+    n = 100_000
+    nbytes = ctypes.c_int64(0)
+    assert lib.ddn_fuse_workspace_bytes(ctypes.byref(g), n, ctypes.byref(nbytes)) == 0
+    if large:
+        assert 100 * n <= nbytes.value <= 124 * n + (1 << 17)
+        null_bytes = ctypes.c_int64(0)
+        assert lib.ddn_fuse_workspace_bytes(None, n, ctypes.byref(null_bytes)) == 0 and null_bytes.value == nbytes.value
+    ws, short = ctypes.c_void_p(1 << 20), nbytes.value - 16
+    p = ctypes.c_void_p(1 << 12)  # any 256-byte aligned address
+    too_small = -3  # DDN_ERR_WORKSPACE_TOO_SMALL
+    assert lib.ddn_voxel_fuse(ctypes.byref(g), n, 0, p, p, None, 1, p, p, p, p, p, ws, short, None) == too_small
+    assert lib.ddn_voxel_partials(ctypes.byref(g), n, 0, p, p, None, 1, p, None, p, ws, short, None) == too_small
+    assert lib.ddn_voxel_merge(ctypes.byref(g), n, p, 0, 0, p, p, p, p, p, ws, short, None) == too_small
+    assert b"workspace too small" in lib.ddn_last_error_string()
+
+
 def test_default_scene_is_unchanged(golden_dir):
     """dome_radius=None (the default) leaves every scene as it was: the seed-11 scene of the golden reference run."""
     g = np.load(golden_dir / "ref_main_seed11.npz")
