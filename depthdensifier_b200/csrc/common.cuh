@@ -106,6 +106,44 @@ __device__ __forceinline__ float ordered_to_float(int i) {
   return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff);
 }
 
+// Packed FP32 pairs: sm_100's FFMA2 / FMUL2 / FADD2 do two float32 operations per issue slot.  Each lane is exactly
+// the IEEE operation of the scalar form (fma.rn, mul.rn, sub.rn, add.rz, no flush to zero), so evaluating two values
+// as a pair gives the same bits as evaluating them one by one.  A pair is one 64-bit register pair, first value in
+// the low half.
+typedef unsigned long long f32x2;
+__device__ __forceinline__ f32x2 pack2(float lo, float hi) {
+  f32x2 r;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+  return r;
+}
+__device__ __forceinline__ f32x2 splat2(float x) { return pack2(x, x); }
+__device__ __forceinline__ void unpack2(f32x2 p, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(p)); }
+__device__ __forceinline__ float lane2(f32x2 p, int e) {
+  float lo, hi;
+  unpack2(p, lo, hi);
+  return e ? hi : lo;
+}
+__device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) {
+  f32x2 r;
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
+  return r;
+}
+__device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) {
+  f32x2 r;
+  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+__device__ __forceinline__ f32x2 sub2(f32x2 a, f32x2 b) {
+  f32x2 r;
+  asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+__device__ __forceinline__ f32x2 add_rz2(f32x2 a, f32x2 b) {
+  f32x2 r;
+  asm("add.rz.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+
 // World position of a pixel from P = d*x, Q = d*y, d and the view's 16-float src_table row (rows of
 // R_s^T Kinv_s with the camera centre appended; scripts/test.py:79-90 then :233).  K4 (filter.cu) and the
 // bounding-box epilogue of K3 (align.cu) both call this, so the box encloses K4's points bit for bit.
@@ -114,6 +152,13 @@ __device__ __forceinline__ void backproject_pqd(const float* __restrict__ s, flo
   X = fmaf(s[0], P, fmaf(s[1], Q, fmaf(s[2], d, s[3])));
   Y = fmaf(s[4], P, fmaf(s[5], Q, fmaf(s[6], d, s[7])));
   Z = fmaf(s[8], P, fmaf(s[9], Q, fmaf(s[10], d, s[11])));
+}
+// The same for a pair of pixels, bit for bit per lane.
+__device__ __forceinline__ void backproject_pqd2(const float* __restrict__ s, f32x2 P, f32x2 Q, f32x2 d, f32x2& X, f32x2& Y,
+                                                 f32x2& Z) {
+  X = fma2(splat2(s[0]), P, fma2(splat2(s[1]), Q, fma2(splat2(s[2]), d, splat2(s[3]))));
+  Y = fma2(splat2(s[4]), P, fma2(splat2(s[5]), Q, fma2(splat2(s[6]), d, splat2(s[7]))));
+  Z = fma2(splat2(s[8]), P, fma2(splat2(s[9]), Q, fma2(splat2(s[10]), d, splat2(s[11]))));
 }
 
 }  // namespace ddn

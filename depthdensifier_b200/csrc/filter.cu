@@ -189,27 +189,23 @@ __device__ __forceinline__ float sqrt_approx(float x) {
   asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
   return r;
 }
-// trunc(u) for 0 <= u < 2^22, biased by 0x4B000000, on the FMA pipe (no F2I).
-__device__ __forceinline__ int trunc_biased(float u) { return __float_as_int(__fadd_rz(u, 8388608.0f)); }
+// The bits of u + 2^23 rounded toward zero are trunc(u) biased by kTruncBias, for 0 <= u < 2^22: the truncation
+// runs on the FMA pipe (no F2I).
 constexpr int kTruncBias = 0x4B000000;
 
-// One (pixel, neighbour) evaluation, in two steps so that the gathers of a thread's four pixels are all in
-// flight before the first one is consumed.  pair_gather: project, bounds test, issue the depth lookup.
+// The (pixel, neighbour) evaluations of a pixel pair, in two steps so that the gathers of a thread's four pixels
+// are all in flight before the first one is consumed.  pair_gather: project, bounds test, issue the depth lookups.
 // pair_test: the candidate flag ("would vote if the grazing gate passes").
+// The projection and the truncation run on both pixels at once (FFMA2, FMUL2, FADD2.RZ), with the scalar order of
+// operations in each lane: U = fma(r.x, P, fma(r.y, Q, fma(r.z, d, r.w))), u = U * (1/Z), trunc(u) = u + 2^23 (RZ).
+// A pixel without a point (NaN depth) computes along with its partner and fails the bounds test.
 template <bool kBilinear, bool kFoldMask>
-__device__ __forceinline__ void pair_gather(const float4& r0, const float4& r1, const float4& r2, float P, float Q, float d,
-                                            const float* __restrict__ depth_all, unsigned off_k, unsigned W, int H,
-                                            unsigned wbits, unsigned hbits, float& Z, float& D, bool& inb) {
-  const float U = fmaf(r0.x, P, fmaf(r0.y, Q, fmaf(r0.z, d, r0.w)));
-  const float V = fmaf(r1.x, P, fmaf(r1.y, Q, fmaf(r1.z, d, r1.w)));
-  Z = fmaf(r2.x, P, fmaf(r2.y, Q, fmaf(r2.z, d, r2.w)));
-  const float inv = rcp_approx(Z);
-  const float u = U * inv;
-  const float v = V * inv;
+__device__ __forceinline__ void pixel_gather(float u, float v, unsigned ub, unsigned vb, const float* __restrict__ depth_all,
+                                             unsigned off_k, unsigned W, int H, unsigned wbits, unsigned hbits, float& Z,
+                                             float& D, bool& inb) {
   // 0 <= u < W and 0 <= v < H on the raw bits (negative floats and NaN compare as huge unsigned);
   // invalid pixels carry NaN depth, so Z > 0 rejects them too.
   inb = (__float_as_uint(u) < wbits) & (__float_as_uint(v) < hbits) & (Z > 0.f);
-  const unsigned ub = (unsigned)trunc_biased(u), vb = (unsigned)trunc_biased(v);
   if (kFoldMask && !inb) Z = INFINITY;  // folds the bounds mask into the one-sided test: inf < thr*D is false
   if (!kBilinear) {
     // 32-bit element offset from the start of refined_all; off_k = t*H*W - bias*(W+1) removes the 2^23
@@ -232,18 +228,50 @@ __device__ __forceinline__ void pair_gather(const float4& r0, const float4& r1, 
   }
 }
 
+__device__ __forceinline__ f32x2 row_dot2(const float4& r, f32x2 P, f32x2 Q, f32x2 d) {
+  return fma2(splat2(r.x), P, fma2(splat2(r.y), Q, fma2(splat2(r.z), d, splat2(r.w))));
+}
+
+template <bool kBilinear, bool kFoldMask>
+__device__ __forceinline__ void pair_gather(const float4& r0, const float4& r1, const float4& r2, f32x2 P, f32x2 Q, f32x2 d,
+                                            const float* __restrict__ depth_all, unsigned off_k, unsigned W, int H,
+                                            unsigned wbits, unsigned hbits, float* Z, float* D, bool* inb) {
+  const f32x2 U = row_dot2(r0, P, Q, d), V = row_dot2(r1, P, Q, d);
+  unpack2(row_dot2(r2, P, Q, d), Z[0], Z[1]);
+  const f32x2 inv = pack2(rcp_approx(Z[0]), rcp_approx(Z[1]));
+  const f32x2 u = mul2(U, inv), v = mul2(V, inv);
+  const f32x2 bias = splat2(8388608.0f);
+  const f32x2 ub = add_rz2(u, bias), vb = add_rz2(v, bias);  // trunc(u), trunc(v) + kTruncBias per lane
+#pragma unroll
+  for (int e = 0; e < 2; ++e)
+    pixel_gather<kBilinear, kFoldMask>(lane2(u, e), lane2(v, e), __float_as_uint(lane2(ub, e)), __float_as_uint(lane2(vb, e)),
+                                       depth_all, off_k, W, H, wbits, hbits, Z[e], D[e], inb[e]);
+}
+
 // cm |= bit when a < b, as one compare and one predicated OR (the compiler would otherwise build the bit with
 // two selects)
 __device__ __forceinline__ void or_bit_if_less(unsigned& cm, float a, float b, unsigned bit) {
   asm("{\n\t.reg .pred p;\n\tsetp.lt.f32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(cm) : "f"(a), "f"(b), "r"(bit));
 }
 
-template <bool kTwoSided>
-__device__ __forceinline__ bool pair_test(float Z, float D, bool inb, float thr, float tau) {
-  if (kTwoSided) return inb & (D > 0.f) & (fabsf(Z - D) > tau * D);
+// Candidate bits of a pixel pair.  kFoldMask: Z is +inf for out-of-bounds lanes, so the bounds mask is already in Z.
+template <bool kTwoSided, bool kFoldMask>
+__device__ __forceinline__ void pair_test(const float* Z, const float* D, const bool* inb, float thr, float tau, unsigned bit,
+                                          unsigned* cm) {
+  if (kTwoSided) {
+#pragma unroll
+    for (int e = 0; e < 2; ++e)
+      if (inb[e] & (D[e] > 0.f) & (fabsf(Z[e] - D[e]) > tau * D[e])) cm[e] |= bit;
+    return;
+  }
   // one-sided floater test z < float32(thr * D) (scripts/test.py:319-321, NEP-50 product in float32).
   // The lookup-valid gate D > 0 (:315) is implied: inb has Z > 0 and thr > 0, so Z < thr*D needs D > 0.
-  return inb & (Z < __fmul_rn(thr, D));
+  const f32x2 thrD = mul2(splat2(thr), pack2(D[0], D[1]));
+#pragma unroll
+  for (int e = 0; e < 2; ++e) {
+    if (kFoldMask) or_bit_if_less(cm[e], Z[e], lane2(thrD, e), bit);
+    else if (inb[e] & (Z[e] < lane2(thrD, e))) cm[e] |= bit;
+  }
 }
 
 // Normal of one source pixel for the grazing gate (scripts/test.py:291), read on demand: only vote
@@ -346,8 +374,10 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   int ys_run = q0 / Ws_src();
   int xs_run = q0 - ys_run * Ws_src();
 
-  // Per-pixel state kept in registers: depth d (NaN = no point), P = d*x, Q = d*y, vote count.
-  float d[kFilterPX], P[kFilterPX], Q[kFilterPX];
+  // Per-pixel state kept in registers: depth d (NaN = no point), P = d*x, Q = d*y, vote count.  d, P and Q are held
+  // as pairs of pixels (0, 1) and (2, 3) for the packed projection; d(j) reads one pixel's depth.
+  constexpr int kPairs = kFilterPX / 2;
+  f32x2 d2[kPairs], P2[kPairs], Q2[kPairs];
   int nvotes[kFilterPX];
   unsigned src_pix[kFilterPX];  // element index of the pixel in its own full-resolution map
   const float qnan = __int_as_float(0x7fc00000);
@@ -373,24 +403,25 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
       for (int j = 0; j < kFilterPX; ++j) dd[j] = (q0 + j * kStep) < Ps ? __ldg(depth_s + src_pix[j]) : 0.f;
     }
 #pragma unroll
-    for (int j = 0; j < kFilterPX; ++j) {
-      const bool valid = dd[j] > 0.f;
-      d[j] = valid ? dd[j] : qnan;
-      asm volatile("" : "+f"(d[j]));  // keep the NaN-tagged depth in a register (no per-neighbour recompute)
-      P[j] = d[j] * (float)px[j];
-      Q[j] = d[j] * (float)py[j];
-      nvotes[j] = 0;
+    for (int h = 0; h < kPairs; ++h) {
+      d2[h] = pack2(dd[2 * h] > 0.f ? dd[2 * h] : qnan, dd[2 * h + 1] > 0.f ? dd[2 * h + 1] : qnan);
+      asm volatile("" : "+l"(d2[h]));  // keep the NaN-tagged depths in registers (no per-neighbour recompute)
+      P2[h] = mul2(d2[h], pack2((float)px[2 * h], (float)px[2 * h + 1]));
+      Q2[h] = mul2(d2[h], pack2((float)py[2 * h], (float)py[2 * h + 1]));
     }
+#pragma unroll
+    for (int j = 0; j < kFilterPX; ++j) nvotes[j] = 0;
   }
+  auto d = [&](int j) { return lane2(d2[j >> 1], j & 1); };
   __syncthreads();  // tables visible
-  // warp-uniform flags: pixel group j of this warp has at least one point (sky / masked regions are
-  // contiguous, so whole groups drop out of the pair loop)
-  bool live[kFilterPX];
+  // warp-uniform flags: pixel pair h of this warp has at least one point (sky / masked regions are
+  // contiguous, so whole pairs drop out of the neighbour loop)
+  bool live[kPairs];
   bool any_live = false;
 #pragma unroll
-  for (int j = 0; j < kFilterPX; ++j) {
-    live[j] = __any_sync(0xffffffffu, d[j] > 0.f);
-    any_live |= live[j];
+  for (int h = 0; h < kPairs; ++h) {
+    live[h] = __any_sync(0xffffffffu, d(2 * h) > 0.f || d(2 * h + 1) > 0.f);
+    any_live |= live[h];
   }
 
   const unsigned wbits = p.wbits, hbits = p.hbits;
@@ -400,7 +431,9 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
 
   // world position of pixel j (scripts/test.py:79-90 then :233), fp32 with float64-precomputed rows;
   // the same expression ddn_align_views' bounding-box epilogue evaluates (backproject_px)
-  auto world_of = [&](int j, float& X, float& Y, float& Z) { backproject_pqd(s_src, P[j], Q[j], d[j], X, Y, Z); };
+  auto world_of = [&](int j, float& X, float& Y, float& Z) {
+    backproject_pqd(s_src, lane2(P2[j >> 1], j & 1), lane2(Q2[j >> 1], j & 1), d(j), X, Y, Z);
+  };
 
   // Hot loop: branch-free candidate test for every (pixel, neighbour); the four gathers of a thread
   // issue back to back.  Candidates ("would vote if the grazing gate passes") are only recorded as a
@@ -409,7 +442,7 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   if (any_live) {
     bool all_live = true;
 #pragma unroll
-    for (int j = 0; j < kFilterPX; ++j) all_live &= live[j];
+    for (int h = 0; h < kPairs; ++h) all_live &= live[h];
     for (int k0 = 0; k0 < n_hot; k0 += 32) {
       const int k1 = min(k0 + 32, n_hot);
       unsigned cm[kFilterPX];
@@ -423,26 +456,24 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
         const float4 wh = kRagged ? t4[4] : make_float4(0.f, 0.f, 0.f, 0.f);  // ragged: the neighbour's W, H, (float)W, (float)H
         float Z[kFilterPX], D[kFilterPX];
         bool inb[kFilterPX];
+        constexpr bool kFold = !kBilinear && !kTwoSided;
+        auto gather = [&](int h) {
+          pair_gather<kBilinear, kFold>(r0, r1, r2, P2[h], Q2[h], d2[h], p.refined_all, off_k, kRagged ? __float_as_uint(wh.x) : (unsigned)p.W,
+                                        kRagged ? __float_as_int(wh.y) : p.H, kRagged ? __float_as_uint(wh.z) : wbits,
+                                        kRagged ? __float_as_uint(wh.w) : hbits, Z + 2 * h, D + 2 * h, inb + 2 * h);
+        };
+        auto test = [&](int h) { pair_test<kTwoSided, kFold>(Z + 2 * h, D + 2 * h, inb + 2 * h, thr, tau, bit, cm + 2 * h); };
         if (all_live) {
 #pragma unroll
-          for (int j = 0; j < kFilterPX; ++j)
-            pair_gather<kBilinear, !kBilinear && !kTwoSided>(r0, r1, r2, P[j], Q[j], d[j], p.refined_all, off_k, kRagged ? __float_as_uint(wh.x) : (unsigned)p.W, kRagged ? __float_as_int(wh.y) : p.H,
-                                   kRagged ? __float_as_uint(wh.z) : wbits, kRagged ? __float_as_uint(wh.w) : hbits, Z[j], D[j], inb[j]);
+          for (int h = 0; h < kPairs; ++h) gather(h);
 #pragma unroll
-          for (int j = 0; j < kFilterPX; ++j) {
-            if (!kBilinear && !kTwoSided) {
-              or_bit_if_less(cm[j], Z[j], __fmul_rn(thr, D[j]), bit);  // Z is +inf for out-of-bounds lanes
-              continue;
-            }
-            if (pair_test<kTwoSided>(Z[j], D[j], inb[j], thr, tau)) cm[j] |= bit;
-          }
+          for (int h = 0; h < kPairs; ++h) test(h);
         } else {
 #pragma unroll
-          for (int j = 0; j < kFilterPX; ++j) {
-            if (live[j]) {
-              pair_gather<kBilinear, !kBilinear && !kTwoSided>(r0, r1, r2, P[j], Q[j], d[j], p.refined_all, off_k, kRagged ? __float_as_uint(wh.x) : (unsigned)p.W, kRagged ? __float_as_int(wh.y) : p.H,
-                                   kRagged ? __float_as_uint(wh.z) : wbits, kRagged ? __float_as_uint(wh.w) : hbits, Z[j], D[j], inb[j]);
-              if (pair_test<kTwoSided>(Z[j], D[j], inb[j], thr, tau)) cm[j] |= bit;
+          for (int h = 0; h < kPairs; ++h) {
+            if (live[h]) {
+              gather(h);
+              test(h);
             }
           }
         }
@@ -484,11 +515,11 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
       const float4 cc = t4[3];
 #pragma unroll
       for (int j = 0; j < kFilterPX; ++j) {
-        if (d[j] > 0.f) {
+        if (d(j) > 0.f) {
           const int py = (int)(src_pix[j] / (unsigned)W_src()), px = (int)(src_pix[j] - (unsigned)py * (unsigned)W_src());
           const int ux = max(px - 1, 0), vy = max(py - 1, 0);
           const float D = __ldg(depth_s + (size_t)vy * W_src() + ux);
-          const bool bad = kTwoSided ? (fabsf(d[j] - D) > tau * D) : (d[j] < __fmul_rn(thr, D));
+          const bool bad = kTwoSided ? (fabsf(d(j) - D) > tau * D) : (d(j) < __fmul_rn(thr, D));
           if (D > 0.f && bad) {
             float n0, n1, n2, wx, wy, wz;
             load_normal(normal_s, src_pix[j], in_world, s_src, n0, n1, n2);
@@ -509,9 +540,16 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   bool keep[kFilterPX];
   unsigned vote_bytes = 0;
 #pragma unroll
+  for (int h = 0; h < kPairs; ++h) {
+    f32x2 X2, Y2, Z2;
+    backproject_pqd2(s_src, P2[h], Q2[h], d2[h], X2, Y2, Z2);
+    unpack2(X2, X[2 * h], X[2 * h + 1]);
+    unpack2(Y2, Y[2 * h], Y[2 * h + 1]);
+    unpack2(Z2, Zw[2 * h], Zw[2 * h + 1]);
+  }
+#pragma unroll
   for (int j = 0; j < kFilterPX; ++j) {
-    const bool valid = d[j] > 0.f;
-    world_of(j, X[j], Y[j], Zw[j]);
+    const bool valid = d(j) > 0.f;
     if (!valid) X[j] = 0.f, Y[j] = 0.f, Zw[j] = 0.f;
     keep[j] = valid && nvotes[j] < p.vote_threshold;
     vote_bytes |= (valid ? (unsigned)min(nvotes[j], 254) : 255u) << (8 * j);
@@ -608,13 +646,26 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
       uint64_t cell[kFilterPX];
       int mine = 0;
 #pragma unroll
-      for (int j = 0; j < kFilterPX; ++j) {
-        cell[j] = kNoCell;
-        if (keep[j]) {
-          uint32_t kx, ky, kz;
-          cell[j] = cell_of_point(g, rv, X[j], Y[j], Zw[j], kx, ky, kz);
+      for (int h = 0; h < kPairs; ++h) {
+        // cell_of_point of both pixels, with voxel_coord's subtract and multiply done as pairs
+        f32x2 a[3], t[3];
+        a[0] = sub2(pack2(X[2 * h], X[2 * h + 1]), splat2(g.ox));
+        a[1] = sub2(pack2(Y[2 * h], Y[2 * h + 1]), splat2(g.oy));
+        a[2] = sub2(pack2(Zw[2 * h], Zw[2 * h + 1]), splat2(g.oz));
+#pragma unroll
+        for (int i = 0; i < 3; ++i) t[i] = mul2(a[i], splat2(rv));
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int j = 2 * h + e;
+          cell[j] = kNoCell;
+          if (keep[j]) {
+            uint32_t kx, ky, kz;
+            cell[j] = cell_of_coords(g, voxel_floor(lane2(a[0], e), lane2(t[0], e), g.voxel),
+                                     voxel_floor(lane2(a[1], e), lane2(t[1], e), g.voxel),
+                                     voxel_floor(lane2(a[2], e), lane2(t[2], e), g.voxel), kx, ky, kz);
+          }
+          mine += cell[j] != kNoCell ? 1 : 0;
         }
-        mine += cell[j] != kNoCell ? 1 : 0;
       }
 #pragma unroll
       for (int j = 0; j < kFilterPX; ++j) {

@@ -48,14 +48,17 @@ inline int grid_from_host(const ddn_voxel_grid* h, GridDev* g) {
 // SURVEY.md N4: x/v and x*(1/v) round differently).  The quotient is first estimated with one multiply
 // by the rounded reciprocal; the two can only floor differently when the estimate sits within a few
 // ulp of an integer, and only then is the IEEE division issued.
-__device__ __forceinline__ float voxel_coord(float p, float o, float voxel, float rvoxel) {
-  const float a = __fsub_rn(p, o);
-  const float t = __fmul_rn(a, rvoxel);
+// voxel_floor takes a = p - o and the estimate t = a * rvoxel already computed (K4 does both in pairs).
+__device__ __forceinline__ float voxel_floor(float a, float t, float voxel) {
   const float k = floorf(t);
   const float r = t - k;
   const float eps = fmaxf(fabsf(t), 1.f) * 1e-6f;
   if (r < eps || r > 1.f - eps || !(fabsf(t) < 4194304.f)) return floorf(__fdiv_rn(a, voxel));
   return k;
+}
+__device__ __forceinline__ float voxel_coord(float p, float o, float voxel, float rvoxel) {
+  const float a = __fsub_rn(p, o);
+  return voxel_floor(a, __fmul_rn(a, rvoxel), voxel);
 }
 
 constexpr int kFixShift = 20;  // offsets are stored in units of voxel * 2^-20
@@ -100,17 +103,20 @@ constexpr int kOwnUnits = kScanThreads;
 constexpr int kOwnPerScanTile = kTileUnits / kOwnUnits;
 constexpr uint64_t kNoCell = ~0ull;
 
-__device__ __forceinline__ uint64_t cell_of_point(const GridDev& g, float rv, float x, float y, float z, uint32_t& kx,
-                                                  uint32_t& ky, uint32_t& kz) {
-  const float fx = voxel_coord(x, g.ox, g.voxel, rv);
-  const float fy = voxel_coord(y, g.oy, g.voxel, rv);
-  const float fz = voxel_coord(z, g.oz, g.voxel, rv);
+// Cell of the voxel coordinates (fx, fy, fz), kNoCell outside the grid.
+__device__ __forceinline__ uint64_t cell_of_coords(const GridDev& g, float fx, float fy, float fz, uint32_t& kx, uint32_t& ky,
+                                                   uint32_t& kz) {
   const bool inside = fx >= 0.f && fy >= 0.f && fz >= 0.f && fx < (float)g.nx && fy < (float)g.ny && fz < (float)g.nz;
   if (!inside) return kNoCell;
   kx = (uint32_t)fx;
   ky = (uint32_t)fy;
   kz = (uint32_t)fz;
   return (uint64_t)kx + (uint64_t)g.nx * ((uint64_t)ky + (uint64_t)g.ny * (uint64_t)kz);
+}
+__device__ __forceinline__ uint64_t cell_of_point(const GridDev& g, float rv, float x, float y, float z, uint32_t& kx,
+                                                  uint32_t& ky, uint32_t& kz) {
+  return cell_of_coords(g, voxel_coord(x, g.ox, g.voxel, rv), voxel_coord(y, g.oy, g.voxel, rv), voxel_coord(z, g.oz, g.voxel, rv),
+                        kx, ky, kz);
 }
 
 // Sets the occupancy bit of `cell`.  `dirty` (optional): one byte per scan tile, set when a tile receives a
