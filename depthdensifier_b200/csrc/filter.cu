@@ -643,29 +643,45 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
     const GridDev g = *p.mark.grid;
     if (g.n_units != 0) {
       const float rv = 1.0f / g.voxel;
+      // cell_of_point of every kept pixel, with voxel_coord's quotient evaluated as pairs.  While the estimate of every
+      // kept pixel is in voxel_quotient_in_domain (finite, 2^-126 <= |q| < 2^22) the floor converts straight to an
+      // integer and the inside test is one unsigned compare per axis.
+      int kx[kFilterPX], ky[kFilterPX], kz[kFilterPX];
+      bool all_exact = true;
+#pragma unroll
+      for (int h = 0; h < kPairs; ++h) {
+        const bool u0 = keep[2 * h], u1 = keep[2 * h + 1];
+        f32x2 q[3];
+        q[0] = voxel_quotient2(pack2(X[2 * h], X[2 * h + 1]), g.ox, g.voxel, rv, u0, u1, all_exact);
+        q[1] = voxel_quotient2(pack2(Y[2 * h], Y[2 * h + 1]), g.oy, g.voxel, rv, u0, u1, all_exact);
+        q[2] = voxel_quotient2(pack2(Zw[2 * h], Zw[2 * h + 1]), g.oz, g.voxel, rv, u0, u1, all_exact);
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          kx[2 * h + e] = __float2int_rd(lane2(q[0], e));
+          ky[2 * h + e] = __float2int_rd(lane2(q[1], e));
+          kz[2 * h + e] = __float2int_rd(lane2(q[2], e));
+        }
+      }
+      if (!all_exact) {  // a kept point beyond 2^22 voxels of the origin on some axis, or not finite: outside is -1
+        auto coord = [&](float p, float o, int n) {
+          const float f = voxel_coord(p, o, g.voxel, rv);
+          return f >= 0.f && f < (float)n ? (int)f : -1;
+        };
+#pragma unroll
+        for (int j = 0; j < kFilterPX; ++j) {
+          kx[j] = coord(X[j], g.ox, g.nx);
+          ky[j] = coord(Y[j], g.oy, g.ny);
+          kz[j] = coord(Zw[j], g.oz, g.nz);
+        }
+      }
       uint64_t cell[kFilterPX];
       int mine = 0;
 #pragma unroll
-      for (int h = 0; h < kPairs; ++h) {
-        // cell_of_point of both pixels, with voxel_coord's subtract and multiply done as pairs
-        f32x2 a[3], t[3];
-        a[0] = sub2(pack2(X[2 * h], X[2 * h + 1]), splat2(g.ox));
-        a[1] = sub2(pack2(Y[2 * h], Y[2 * h + 1]), splat2(g.oy));
-        a[2] = sub2(pack2(Zw[2 * h], Zw[2 * h + 1]), splat2(g.oz));
-#pragma unroll
-        for (int i = 0; i < 3; ++i) t[i] = mul2(a[i], splat2(rv));
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-          const int j = 2 * h + e;
-          cell[j] = kNoCell;
-          if (keep[j]) {
-            uint32_t kx, ky, kz;
-            cell[j] = cell_of_coords(g, voxel_floor(lane2(a[0], e), lane2(t[0], e), g.voxel),
-                                     voxel_floor(lane2(a[1], e), lane2(t[1], e), g.voxel),
-                                     voxel_floor(lane2(a[2], e), lane2(t[2], e), g.voxel), kx, ky, kz);
-          }
-          mine += cell[j] != kNoCell ? 1 : 0;
-        }
+      for (int j = 0; j < kFilterPX; ++j) {
+        const bool inside = keep[j] & ((unsigned)kx[j] < (unsigned)g.nx) & ((unsigned)ky[j] < (unsigned)g.ny) & ((unsigned)kz[j] < (unsigned)g.nz);
+        const uint64_t c = cell_of_index(g, kx[j], ky[j], kz[j]);  // computed for every pixel: a select, no branch
+        cell[j] = inside ? c : kNoCell;
+        mine += inside ? 1 : 0;
       }
 #pragma unroll
       for (int j = 0; j < kFilterPX; ++j) {

@@ -450,7 +450,7 @@ __device__ __forceinline__ uint32_t slot_of_cell(uint64_t cell, const uint4* __r
 // accumulate: one point per lane, aggregated ACROSS THE WARP before touching memory.  With a row length
 // (points are pixels of [rows, row_len] images) a warp covers a 16 x 2 pixel tile, otherwise 32
 // consecutive points.  Lanes whose points fall into the same cell are found with MATCH.ANY; every lane
-// walks its peer mask with shuffles (32-bit partial sums: at most 32 points of |offset| <= 2^19), and
+// walks its peer mask with shuffles (32-bit partial sums: at most 32 points of |offset| <= 2^19 + 1), and
 // the lowest lane of each group looks the slot up and issues the five 64-bit REDs.  The L2 atomic units
 // are the bound of this pass, so points per RED group is what matters: ~2 at cfg 2.
 // (-DDDN_ACC_REDUX sums each group with REDUX over its own peer mask instead of the shuffle walk: the
@@ -566,6 +566,11 @@ accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len,
     int sx = 0, sy = 0, sz = 0;
     uint32_t srg = 0, sb = 0;
 #ifndef DDN_ACC_REDUX
+    // Three shuffles per step of the walk instead of five: a word per axis holds the offset (|offset| <= 2^19 + 1, far
+    // inside 24 signed bits) above one colour byte.  s* sums the offsets (arithmetic shift), t* the whole words modulo
+    // 2^32, so a colour sum is t - (s << 8), exact because it is at most 32 * 255 < 2^13.
+    const uint32_t wx = ((uint32_t)ox << 8) | (rg >> 16), wy = ((uint32_t)oy << 8) | (rg & 0xffffu), wz = ((uint32_t)oz << 8) | bb;
+    uint32_t tx = 0, ty = 0, tz = 0;
     const int iters = __reduce_max_sync(0xffffffffu, __popc(peers));
     uint32_t rest = peers;
 #pragma unroll 1
@@ -573,11 +578,15 @@ accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len,
       const bool has = rest != 0;
       const int src = has ? __ffs(rest) - 1 : lane;
       rest &= rest - 1;
-      const int ax = __shfl_sync(0xffffffffu, ox, src), ay = __shfl_sync(0xffffffffu, oy, src);
-      const int az = __shfl_sync(0xffffffffu, oz, src);
-      const uint32_t arg = __shfl_sync(0xffffffffu, rg, src), ab = __shfl_sync(0xffffffffu, bb, src);
-      if (has) sx += ax, sy += ay, sz += az, srg += arg, sb += ab;
+      const uint32_t ax = __shfl_sync(0xffffffffu, wx, src), ay = __shfl_sync(0xffffffffu, wy, src);
+      const uint32_t az = __shfl_sync(0xffffffffu, wz, src);
+      if (has) {
+        sx += (int)ax >> 8, sy += (int)ay >> 8, sz += (int)az >> 8;
+        tx += ax, ty += ay, tz += az;
+      }
     }
+    srg = ((tx - ((uint32_t)sx << 8)) << 16) | (ty - ((uint32_t)sy << 8));
+    sb = tz - ((uint32_t)sz << 8);
 #else
     if (valid) {  // every lane of a group passes the same mask: REDUX over the group only
       sx = __reduce_add_sync(peers, ox);
@@ -660,9 +669,10 @@ __global__ void canonical_key_kernel(GridDev g, int64_t n, const float* __restri
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float x = xyz[i * 3 + 0], y = xyz[i * 3 + 1], z = xyz[i * 3 + 2];
-  const int64_t kx = (int64_t)floorf(__fdiv_rn(__fsub_rn(x, g.ox), g.voxel));
-  const int64_t ky = (int64_t)floorf(__fdiv_rn(__fsub_rn(y, g.oy), g.voxel));
-  const int64_t kz = (int64_t)floorf(__fdiv_rn(__fsub_rn(z, g.oz), g.voxel));
+  const float rv = 1.0f / g.voxel;
+  const int64_t kx = (int64_t)voxel_coord(x, g.ox, g.voxel, rv);
+  const int64_t ky = (int64_t)voxel_coord(y, g.oy, g.voxel, rv);
+  const int64_t kz = (int64_t)voxel_coord(z, g.oz, g.voxel, rv);
   const bool ok = kx >= 0 && ky >= 0 && kz >= 0 && kx < (1 << 21) && ky < (1 << 21) && kz < (1 << 21);
   keys[i] = ok ? ((uint64_t)kx | ((uint64_t)ky << 21) | ((uint64_t)kz << 42)) : ~0ull;
 }

@@ -5,6 +5,7 @@
 #pragma once
 
 #include "common.cuh"
+#include "voxel_quotient.cuh"
 
 namespace ddn {
 
@@ -44,21 +45,23 @@ inline int grid_from_host(const ddn_voxel_grid* h, GridDev* g) {
   return DDN_OK;
 }
 
-// k = floor((p - o) / voxel) with IEEE float32 sub and div (bit-exact with the numpy definition,
-// SURVEY.md N4: x/v and x*(1/v) round differently).  The quotient is first estimated with one multiply
-// by the rounded reciprocal; the two can only floor differently when the estimate sits within a few
-// ulp of an integer, and only then is the IEEE division issued.
-// voxel_floor takes a = p - o and the estimate t = a * rvoxel already computed (K4 does both in pairs).
-__device__ __forceinline__ float voxel_floor(float a, float t, float voxel) {
-  const float k = floorf(t);
-  const float r = t - k;
-  const float eps = fmaxf(fabsf(t), 1.f) * 1e-6f;
-  if (r < eps || r > 1.f - eps || !(fabsf(t) < 4194304.f)) return floorf(__fdiv_rn(a, voxel));
-  return k;
-}
+// k = floor((p - o) / voxel) with IEEE float32 sub and div (bit-exact with the numpy definition), through the
+// division-free quotient of voxel_quotient.cuh.
 __device__ __forceinline__ float voxel_coord(float p, float o, float voxel, float rvoxel) {
-  const float a = __fsub_rn(p, o);
-  return voxel_floor(a, __fmul_rn(a, rvoxel), voxel);
+  return voxel_floor(__fsub_rn(p, o), voxel, rvoxel);
+}
+// voxel_coord's quotient for a pair of values (K4's fused mark), before the floor: each lane of the result is
+// fl((p - o) / voxel) where voxel_quotient_in_domain holds or the lane's `use` flag is clear.  `all_exact` is cleared
+// where neither holds; the caller then takes voxel_coord for those values.
+__device__ __forceinline__ f32x2 voxel_quotient2(f32x2 p, float o, float voxel, float rvoxel, bool use0, bool use1,
+                                                 bool& all_exact) {
+  const f32x2 a = sub2(p, splat2(o));
+  const f32x2 rv2 = splat2(rvoxel);
+  const f32x2 q = mul2(a, rv2);
+  float q0, q1;
+  unpack2(q, q0, q1);
+  all_exact &= (voxel_quotient_in_domain(q0) | !use0) & (voxel_quotient_in_domain(q1) | !use1);
+  return fma2(fma2(q, splat2(-voxel), a), rv2, q);
 }
 
 constexpr int kFixShift = 20;  // offsets are stored in units of voxel * 2^-20
@@ -103,6 +106,10 @@ constexpr int kOwnUnits = kScanThreads;
 constexpr int kOwnPerScanTile = kTileUnits / kOwnUnits;
 constexpr uint64_t kNoCell = ~0ull;
 
+// Cell of the integer voxel coordinates (kx, ky, kz) inside the grid.
+__device__ __forceinline__ uint64_t cell_of_index(const GridDev& g, uint32_t kx, uint32_t ky, uint32_t kz) {
+  return (uint64_t)kx + (uint64_t)g.nx * ((uint64_t)ky + (uint64_t)g.ny * (uint64_t)kz);
+}
 // Cell of the voxel coordinates (fx, fy, fz), kNoCell outside the grid.
 __device__ __forceinline__ uint64_t cell_of_coords(const GridDev& g, float fx, float fy, float fz, uint32_t& kx, uint32_t& ky,
                                                    uint32_t& kz) {
@@ -111,7 +118,7 @@ __device__ __forceinline__ uint64_t cell_of_coords(const GridDev& g, float fx, f
   kx = (uint32_t)fx;
   ky = (uint32_t)fy;
   kz = (uint32_t)fz;
-  return (uint64_t)kx + (uint64_t)g.nx * ((uint64_t)ky + (uint64_t)g.ny * (uint64_t)kz);
+  return cell_of_index(g, kx, ky, kz);
 }
 __device__ __forceinline__ uint64_t cell_of_point(const GridDev& g, float rv, float x, float y, float z, uint32_t& kx,
                                                   uint32_t& ky, uint32_t& kz) {
