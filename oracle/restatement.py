@@ -105,10 +105,12 @@ def iqr_inliers(z_colmap: torch.Tensor, z_depth: torch.Tensor, outlier_threshold
 
 def pwl_lookup(d: torch.Tensor, x: torch.Tensor, y: torch.Tensor) -> torch.Tensor:
     """A5 - depth_refiner.py:141-178 ('PCHIP' in name only): piecewise-linear through the pairs
-    sorted by x, constant extrapolation, floor at 1e-3."""
+    sorted by x, constant extrapolation, floor at 1e-3.  Knots of equal x keep their pair order (a stable sort, as
+    align_stats_kernel sorts): the reference's torch.sort leaves that order to the sort implementation, and a query
+    just above a repeated x takes the y of whichever repeat sorts last."""
     if d.numel() < 4:  # depth_refiner.py:143-145 (tests the number of *query pixels*)
         return d * torch.median(y / (d + 1e-6))
-    order = torch.argsort(x)
+    order = torch.argsort(x, stable=True)
     xs = x[order]
     ys = y[order]
     if xs.numel() < 2:

@@ -90,6 +90,29 @@ def test_restatement_equals_reference_refiner_stride_and_fallbacks(golden_dir):
             assert {k: val.item() for k, val in ref.items()} == {k: mine[k] for k in mine if k != "refined_depth"}, (name, v)
 
 
+def test_pwl_lookup_keeps_pair_order_of_repeated_knots():
+    """Knots of equal x and different y, in shuffled pair order: a query at a repeated x takes the y of the repeat that
+    comes first in pair order, a query just above it interpolates from the repeat that comes last (align_stats_kernel
+    sorts by (x, pair index)).  Either answer changes when the two repeats trade places."""
+    import torch
+
+    rng = np.random.default_rng(3)
+    reps = np.sort(rng.choice(np.arange(1, 99), 20, replace=False))
+    x = np.concatenate([np.arange(100), reps]).astype(np.float32)
+    order = rng.permutation(len(x))
+    x = x[order]
+    y = (rng.permutation(len(x)) * 2 + 1).astype(np.float32)  # distinct odd integers: every value below is exact
+    queries, expected = [], []
+    for r in reps:
+        first, last = np.flatnonzero(x == r)  # pair order
+        nxt = int(np.flatnonzero(x == r + 1)[0])  # searchsorted_left lands on the first knot of x = r + 1
+        queries += [r, r + 0.5]
+        expected += [y[first], y[last] + 0.5 * (y[nxt] - y[last])]
+        assert y[first] != y[last]
+    got = R.pwl_lookup(torch.tensor(queries, dtype=torch.float32), torch.from_numpy(x), torch.from_numpy(y))
+    assert np.array_equal(got.numpy(), np.array(expected, np.float32))
+
+
 def test_explicit_bilinear_matches_grid_sample():
     import torch
     import torch.nn.functional as F
