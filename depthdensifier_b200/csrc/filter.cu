@@ -26,6 +26,9 @@ namespace ddn {
 #ifndef DDN_K4_MINBLOCKS
 #define DDN_K4_MINBLOCKS 5
 #endif
+#ifndef DDN_K4_SUPPORT_MINBLOCKS
+#define DDN_K4_SUPPORT_MINBLOCKS 4
+#endif
 constexpr int kFilterThreads = 256;
 #ifndef DDN_K4_PX
 #define DDN_K4_PX 4
@@ -179,6 +182,16 @@ struct FilterParams {
   unsigned wbits, hbits;  // bit patterns of (float)W, (float)H for the bounds test on raw bits
 };
 
+// The arguments only ddn_backproject_filter_support* take: K4's optional third parameter, so that the parameters of the
+// plain instantiations keep their layout (and the kernels their code).
+struct SupportParams {
+  uint8_t* support;  // same grid as votes
+  int min_support;
+  float support_tau;
+};
+__device__ __forceinline__ SupportParams support_params() { return SupportParams{nullptr, 0, 0.f}; }
+__device__ __forceinline__ SupportParams support_params(const SupportParams& s) { return s; }
+
 __device__ __forceinline__ float rcp_approx(float x) {
   float r;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
@@ -274,6 +287,24 @@ __device__ __forceinline__ void pair_test(const float* Z, const float* D, const 
   }
 }
 
+// Support bits of a pixel pair: neighbour entry `bit` sees the surface of the pixel within the relative depth error
+// tau, |Z - D| <= tau*D.  No grazing gate.  kFoldMask: out-of-bounds lanes carry Z = +inf and pixels without a point
+// NaN, so both fail the comparison without the bounds mask; D > 0 is implied, since in-bounds lanes have Z > 0.
+template <bool kFoldMask>
+__device__ __forceinline__ void pair_support(const float* Z, const float* D, const bool* inb, float tau, unsigned bit,
+                                             unsigned* sm) {
+  const f32x2 D2 = pack2(D[0], D[1]);
+  const f32x2 dz = sub2(pack2(Z[0], Z[1]), D2), tD = mul2(splat2(tau), D2);
+#pragma unroll
+  for (int e = 0; e < 2; ++e) {
+    if (kFoldMask) {
+      if (fabsf(lane2(dz, e)) <= lane2(tD, e)) sm[e] |= bit;
+    } else if (inb[e] & (fabsf(lane2(dz, e)) <= lane2(tD, e))) {
+      sm[e] |= bit;
+    }
+  }
+}
+
 // Normal of one source pixel for the grazing gate (scripts/test.py:291), read on demand: only vote
 // candidates need it, and they are rare (floaters), so the 12 B/pixel normal map is not streamed.
 // normals_in_world rotates it by R_s^T (rows recovered from the source table) and divides by (|n| + 1e-8), as
@@ -333,9 +364,15 @@ static_assert(kFilterPX == 4, "the layouts below are written for 4 pixels per th
 // of all views in view order (the L2 argument above holds unchanged); a CTA finds its view in the layout, and every
 // neighbour's W, H and bounds-test bits come from its table entry (floats 16-19) next to the gather offset.
 // p.n_src is then the number of views, and p.H, p.W, p.Hs, p.Ws, p.src_begin, p.wbits and p.hbits are not read.
-template <bool kBilinear, bool kStride1, bool kTwoSided, int kLayout, bool kRagged>
-__global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOCKS)
-    backproject_filter_kernel(const FilterParams p, const int64_t* __restrict__ layout) {
+// kSupport (ddn_backproject_filter_support*; Support = SupportParams, the plain kernels have no third parameter): also
+// count, per pixel, the neighbour entries that support the point (pair_support), write the count to sp.support and apply
+// the keep rule and vote encoding of include/ddn_b200.h.  The support forms take 56 to 64 registers with nearest
+// sampling: at 5 CTAs per SM (48 registers) they would spill inside the neighbour loop, at 4 they do not.
+template <bool kBilinear, bool kStride1, bool kTwoSided, int kLayout, bool kRagged, class... Support>
+__global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : (sizeof...(Support) ? DDN_K4_SUPPORT_MINBLOCKS : DDN_K4_MINBLOCKS))
+    backproject_filter_kernel(const FilterParams p, const int64_t* __restrict__ layout, Support... support) {
+  constexpr bool kSupport = sizeof...(Support) != 0;
+  const SupportParams sp = support_params(support...);
   extern __shared__ __align__(16) float smem[];
   float* s_src = smem;                     // 16 floats
   float* s_pair = s_src + 16;              // K*24 floats
@@ -378,7 +415,7 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   // as pairs of pixels (0, 1) and (2, 3) for the packed projection; d(j) reads one pixel's depth.
   constexpr int kPairs = kFilterPX / 2;
   f32x2 d2[kPairs], P2[kPairs], Q2[kPairs];
-  int nvotes[kFilterPX];
+  int nvotes[kFilterPX];  // kSupport: the count of supporting neighbour entries in bits 16-31 (both counts <= 1024)
   unsigned src_pix[kFilterPX];  // element index of the pixel in its own full-resolution map
   const float qnan = __int_as_float(0x7fc00000);
   {
@@ -426,6 +463,7 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
 
   const unsigned wbits = p.wbits, hbits = p.hbits;
   const float thr = p.depth_threshold, gcos = p.grazing_cos, tau = p.two_sided_tau;
+  const float stau = kSupport ? sp.support_tau : 0.f;
   const bool in_world = p.normals_in_world != 0;
   const int n_hot = __float_as_int(s_pair[22]), n_own = __float_as_int(s_pair[23]);
 
@@ -445,9 +483,9 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
     for (int h = 0; h < kPairs; ++h) all_live &= live[h];
     for (int k0 = 0; k0 < n_hot; k0 += 32) {
       const int k1 = min(k0 + 32, n_hot);
-      unsigned cm[kFilterPX];
+      unsigned cm[kFilterPX], sm[kFilterPX];  // candidate and support bits of the block
 #pragma unroll
-      for (int j = 0; j < kFilterPX; ++j) cm[j] = 0u;
+      for (int j = 0; j < kFilterPX; ++j) cm[j] = 0u, sm[j] = 0u;
       unsigned bit = 1u;
       for (int k = k0; k < k1; ++k, bit <<= 1) {
         const float4* t4 = reinterpret_cast<const float4*>(s_pair + k * DDN_PAIR_TABLE_FLOATS);
@@ -462,7 +500,10 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
                                         kRagged ? __float_as_int(wh.y) : p.H, kRagged ? __float_as_uint(wh.z) : wbits,
                                         kRagged ? __float_as_uint(wh.w) : hbits, Z + 2 * h, D + 2 * h, inb + 2 * h);
         };
-        auto test = [&](int h) { pair_test<kTwoSided, kFold>(Z + 2 * h, D + 2 * h, inb + 2 * h, thr, tau, bit, cm + 2 * h); };
+        auto test = [&](int h) {
+          pair_test<kTwoSided, kFold>(Z + 2 * h, D + 2 * h, inb + 2 * h, thr, tau, bit, cm + 2 * h);
+          if (kSupport) pair_support<kFold>(Z + 2 * h, D + 2 * h, inb + 2 * h, stau, bit, sm + 2 * h);
+        };
         if (all_live) {
 #pragma unroll
           for (int h = 0; h < kPairs; ++h) gather(h);
@@ -477,6 +518,10 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
             }
           }
         }
+      }
+      if (kSupport) {
+#pragma unroll
+        for (int j = 0; j < kFilterPX; ++j) nvotes[j] += __popc(sm[j]) << 16;
       }
       // dot(n, -(Xw - c_t)/|Xw - c_t|) > cos  <=>  dot(n, c_t - Xw) > cos * |c_t - Xw|
 #pragma unroll
@@ -538,7 +583,10 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   bool bulk_pending = false;  // lane 0: a bulk copy out of this warp's staging slice is in flight
   float X[kFilterPX], Y[kFilterPX], Zw[kFilterPX];
   bool keep[kFilterPX];
-  unsigned vote_bytes = 0;
+  unsigned vote_bytes = 0, support_bytes = 0;
+  // kSupport: a valid point the neighbours do not support stores 254, which no fusion threshold min(thr, 254) passes;
+  // a supported one stores its count saturated at 254, or at 253 when every count passes (threshold >= 255)
+  const int vote_cap = (kSupport && p.vote_threshold == INT_MAX) ? 253 : 254;
 #pragma unroll
   for (int h = 0; h < kPairs; ++h) {
     f32x2 X2, Y2, Z2;
@@ -551,18 +599,31 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   for (int j = 0; j < kFilterPX; ++j) {
     const bool valid = d(j) > 0.f;
     if (!valid) X[j] = 0.f, Y[j] = 0.f, Zw[j] = 0.f;
-    keep[j] = valid && nvotes[j] < p.vote_threshold;
-    vote_bytes |= (valid ? (unsigned)min(nvotes[j], 254) : 255u) << (8 * j);
+    if (kSupport) {
+      const int nv = nvotes[j] & 0xffff, ns = nvotes[j] >> 16;
+      const bool supported = ns >= sp.min_support;
+      keep[j] = valid && nv < p.vote_threshold && supported;
+      vote_bytes |= (valid ? (supported ? (unsigned)min(nv, vote_cap) : 254u) : 255u) << (8 * j);
+      support_bytes |= (valid ? (unsigned)min(ns, 254) : 255u) << (8 * j);
+    } else {
+      keep[j] = valid && nvotes[j] < p.vote_threshold;
+      vote_bytes |= (valid ? (unsigned)min(nvotes[j], 254) : 255u) << (8 * j);
+    }
   }
   const size_t out0 = kRagged ? (size_t)L[3] : (size_t)sl * Ps;  // first pixel of the view in the outputs
   if (kLayout == 1) {
     uint8_t* vo = p.votes + out0 + q0;
-    if (q0 + kFilterPX <= Ps && ((reinterpret_cast<uintptr_t>(vo) & 3) == 0)) {
+    if (q0 + kFilterPX <= Ps && ((reinterpret_cast<uintptr_t>(vo) & 3) == 0) &&
+        (!kSupport || (reinterpret_cast<uintptr_t>(sp.support + out0 + q0) & 3) == 0)) {
       *reinterpret_cast<unsigned*>(vo) = vote_bytes;
+      if (kSupport) *reinterpret_cast<unsigned*>(sp.support + out0 + q0) = support_bytes;
     } else {
 #pragma unroll
       for (int j = 0; j < kFilterPX; ++j)
-        if (q0 + j < Ps) vo[j] = (uint8_t)(vote_bytes >> (8 * j));
+        if (q0 + j < Ps) {
+          vo[j] = (uint8_t)(vote_bytes >> (8 * j));
+          if (kSupport) sp.support[out0 + q0 + j] = (uint8_t)(support_bytes >> (8 * j));
+        }
     }
     float* xo = p.xyz + (out0 + q0) * 3;
     if (q0 + kFilterPX <= Ps && ((reinterpret_cast<uintptr_t>(xo) & 15) == 0)) {
@@ -582,7 +643,10 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : DDN_K4_MINBLOC
   } else {
 #pragma unroll
     for (int j = 0; j < kFilterPX; ++j)
-      if (q0 + j * 32 < Ps) p.votes[out0 + q0 + j * 32] = (uint8_t)(vote_bytes >> (8 * j));
+      if (q0 + j * 32 < Ps) {
+        p.votes[out0 + q0 + j * 32] = (uint8_t)(vote_bytes >> (8 * j));
+        if (kSupport) sp.support[out0 + q0 + j * 32] = (uint8_t)(support_bytes >> (8 * j));
+      }
     // xyz through the warp's staging slice: stride-3 STS (conflict free), float4 out (16 B per lane, coalesced)
     float* sw = s_stage + warp * (kWarpPix * 3);
 #pragma unroll
@@ -752,28 +816,36 @@ static int fill_filter_params(const ddn_filter_config* cfg, const float* refined
   return DDN_OK;
 }
 
+// One K4 instantiation, plain (sp == nullptr) or with the support count.
+template <bool kBilinear, bool kStride1, bool kTwoSided, int kLayout, bool kRagged>
+static int launch_k4(const FilterParams& p, const SupportParams* sp, dim3 grid, const int64_t* layout, size_t smem,
+                     cudaStream_t st) {
+  if (sp == nullptr) {
+    auto* k = backproject_filter_kernel<kBilinear, kStride1, kTwoSided, kLayout, kRagged>;
+    DDN_TRY(check_cuda(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute"));
+    k<<<grid, kFilterThreads, smem, st>>>(p, layout);
+  } else {
+    auto* k = backproject_filter_kernel<kBilinear, kStride1, kTwoSided, kLayout, kRagged, SupportParams>;
+    DDN_TRY(check_cuda(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute"));
+    k<<<grid, kFilterThreads, smem, st>>>(p, layout, *sp);
+  }
+  return DDN_OK;
+}
+
 // Launches the K4 instantiation cfg selects: the uniform kernel (layout == nullptr, grid = chunks x views) or the
-// ragged one (grid = all chunks of the layout).
-static int launch_filter(const ddn_filter_config* cfg, const FilterParams& p, dim3 grid, const int64_t* layout, cudaStream_t st) {
+// ragged one (grid = all chunks of the layout); sp != nullptr: the support form.
+static int launch_filter(const ddn_filter_config* cfg, const FilterParams& p, const SupportParams* sp, dim3 grid,
+                         const int64_t* layout, cudaStream_t st) {
   const int pl = cfg->pixel_layout;
   const size_t smem = (size_t)(16 + p.K * DDN_PAIR_TABLE_FLOATS + (pl == 0 ? kFilterChunk * 3 : 0)) * sizeof(float);
   const bool bil = cfg->sample_mode == 1;
   const bool s1 = cfg->stride == 1;
   const bool two = cfg->two_sided_tau > 0.f;
   DDN_REQUIRE(two || cfg->depth_threshold > 0.f, "depth_threshold must be positive");
-#define DDN_LAUNCH_FILTER(B, S, T, L)                                                                        \
-  do {                                                                                                       \
-    if (layout != nullptr) {                                                                                 \
-      DDN_TRY(check_cuda(cudaFuncSetAttribute(backproject_filter_kernel<B, S, T, L, true>,                   \
-                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),       \
-                         "cudaFuncSetAttribute"));                                                           \
-      backproject_filter_kernel<B, S, T, L, true><<<grid, kFilterThreads, smem, st>>>(p, layout);            \
-    } else {                                                                                                 \
-      DDN_TRY(check_cuda(cudaFuncSetAttribute(backproject_filter_kernel<B, S, T, L, false>,                  \
-                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),       \
-                         "cudaFuncSetAttribute"));                                                           \
-      backproject_filter_kernel<B, S, T, L, false><<<grid, kFilterThreads, smem, st>>>(p, nullptr);          \
-    }                                                                                                        \
+#define DDN_LAUNCH_FILTER(B, S, T, L)                                                      \
+  do {                                                                                     \
+    if (layout != nullptr) DDN_TRY((launch_k4<B, S, T, L, true>(p, sp, grid, layout, smem, st))); \
+    else DDN_TRY((launch_k4<B, S, T, L, false>(p, sp, grid, nullptr, smem, st)));          \
   } while (0)
 #define DDN_LAUNCH_FILTER_L(B, S, T)       \
   do {                                     \
@@ -794,6 +866,68 @@ static int launch_filter(const ddn_filter_config* cfg, const FilterParams& p, di
 #undef DDN_LAUNCH_FILTER_L
 #undef DDN_LAUNCH_FILTER
   return DDN_OK;
+}
+
+static int check_support(const SupportParams* sp) {
+  if (sp == nullptr) return DDN_OK;
+  DDN_REQUIRE(sp->min_support >= 0 && sp->min_support <= 1024, "min_support must be in [0, 1024]");
+  DDN_REQUIRE(sp->support_tau > 0.f && isfinite(sp->support_tau), "support_tau must be positive and finite");
+  DDN_REQUIRE(sp->support != nullptr, "null support");
+  return DDN_OK;
+}
+
+// The two uniform entry points (sup: nullptr for ddn_backproject_filter).
+static int filter_uniform(const SupportParams* sup, const ddn_filter_config* cfg, int64_t n_views_total, int64_t src_begin,
+                          int64_t n_src, int64_t height, int64_t width, int64_t k_nbr, const float* refined_all,
+                          const float* normal, const int32_t* nbr, const float* pair_table, const float* src_table,
+                          int32_t vote_threshold, float* xyz, uint8_t* votes, float* bbox, const ddn_fuse_session* mark,
+                          void* stream) {
+  (void)nbr;
+  DDN_REQUIRE(n_views_total > 0 && n_src >= 0, "view counts");
+  DDN_REQUIRE(src_begin >= 0 && src_begin + n_src <= n_views_total, "source range");
+  DDN_REQUIRE(height > 0 && width > 0 && height * width < (1ll << 31), "image size");
+  DDN_REQUIRE(n_views_total * height * width < (1ll << 32), "refined_all must hold fewer than 2^32 pixels (32-bit gather offsets)");
+  DDN_REQUIRE(width < (1 << 22) && height < (1 << 22), "image side too large for the truncation trick");
+  FilterParams p;
+  DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
+  DDN_TRY(check_support(sup));
+  if (n_src == 0) return DDN_OK;
+  p.src_begin = (int)src_begin;
+  p.n_src = (int)n_src;
+  p.H = (int)height;
+  p.W = (int)width;
+  p.Hs = (p.H + p.stride - 1) / p.stride;
+  p.Ws = (p.W + p.stride - 1) / p.stride;
+  {
+    const float wf = (float)p.W, hf = (float)p.H;
+    memcpy(&p.wbits, &wf, 4);
+    memcpy(&p.hbits, &hf, 4);
+  }
+  const int Ps = p.Hs * p.Ws;
+  dim3 grid((Ps + kFilterChunk - 1) / kFilterChunk, (unsigned)n_src);
+  DDN_REQUIRE(n_src <= 65535, "too many source views per call");
+  DDN_TRY(launch_filter(cfg, p, sup, grid, nullptr, (cudaStream_t)stream));
+  return after_launch("backproject_filter_kernel");
+}
+
+// The two ragged entry points (sup: nullptr for ddn_backproject_filter_ragged).
+static int filter_ragged(const SupportParams* sup, const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
+                         const int64_t* layout, const int64_t* layout_host, const float* refined_all, const float* normal,
+                         const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
+                         uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
+  FilterParams p;
+  DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
+  DDN_TRY(check_support(sup));
+  DDN_REQUIRE(layout != nullptr, "null layout");
+  DDN_TRY(check_layout(n_views, layout_host));
+  DDN_REQUIRE(cfg->stride == layout_host[n_views * DDN_LAYOUT_COLS], "cfg->stride must be the layout's stride");
+  p.src_begin = 0;
+  p.n_src = (int)n_views;
+  p.H = p.W = p.Hs = p.Ws = 0;  // per view, from the layout and the table entries
+  p.wbits = p.hbits = 0;
+  const int64_t chunks = layout_host[n_views * DDN_LAYOUT_COLS + 5];  // >= 1: every view has a pixel
+  DDN_TRY(launch_filter(cfg, p, sup, dim3((unsigned)chunks), layout, (cudaStream_t)stream));
+  return after_launch("backproject_filter_kernel");
 }
 
 }  // namespace ddn
@@ -828,32 +962,19 @@ int ddn_backproject_filter(const ddn_filter_config* cfg, int64_t n_views_total, 
                            const float* refined_all, const float* normal, const int32_t* nbr,
                            const float* pair_table, const float* src_table, int32_t vote_threshold,
                            float* xyz, uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
-  using namespace ddn;
-  (void)nbr;
-  DDN_REQUIRE(n_views_total > 0 && n_src >= 0, "view counts");
-  DDN_REQUIRE(src_begin >= 0 && src_begin + n_src <= n_views_total, "source range");
-  DDN_REQUIRE(height > 0 && width > 0 && height * width < (1ll << 31), "image size");
-  DDN_REQUIRE(n_views_total * height * width < (1ll << 32), "refined_all must hold fewer than 2^32 pixels (32-bit gather offsets)");
-  DDN_REQUIRE(width < (1 << 22) && height < (1 << 22), "image side too large for the truncation trick");
-  FilterParams p;
-  DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
-  if (n_src == 0) return DDN_OK;
-  p.src_begin = (int)src_begin;
-  p.n_src = (int)n_src;
-  p.H = (int)height;
-  p.W = (int)width;
-  p.Hs = (p.H + p.stride - 1) / p.stride;
-  p.Ws = (p.W + p.stride - 1) / p.stride;
-  {
-    const float wf = (float)p.W, hf = (float)p.H;
-    memcpy(&p.wbits, &wf, 4);
-    memcpy(&p.hbits, &hf, 4);
-  }
-  const int Ps = p.Hs * p.Ws;
-  dim3 grid((Ps + kFilterChunk - 1) / kFilterChunk, (unsigned)n_src);
-  DDN_REQUIRE(n_src <= 65535, "too many source views per call");
-  DDN_TRY(launch_filter(cfg, p, grid, nullptr, (cudaStream_t)stream));
-  return after_launch("backproject_filter_kernel");
+  return ddn::filter_uniform(nullptr, cfg, n_views_total, src_begin, n_src, height, width, k_nbr, refined_all, normal, nbr,
+                             pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, stream);
+}
+
+int ddn_backproject_filter_support(const ddn_filter_config* cfg, int64_t n_views_total, int64_t src_begin, int64_t n_src,
+                                   int64_t height, int64_t width, int64_t k_nbr, const float* refined_all,
+                                   const float* normal, const int32_t* nbr, const float* pair_table,
+                                   const float* src_table, int32_t vote_threshold, int32_t min_support, float support_tau,
+                                   float* xyz, uint8_t* votes, uint8_t* support, float* bbox,
+                                   const ddn_fuse_session* mark, void* stream) {
+  const ddn::SupportParams sup{support, min_support, support_tau};
+  return ddn::filter_uniform(&sup, cfg, n_views_total, src_begin, n_src, height, width, k_nbr, refined_all, normal, nbr,
+                             pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, stream);
 }
 
 int ddn_build_pair_tables_ragged(int64_t n_views, int64_t k_nbr, const int64_t* layout, const int64_t* layout_host,
@@ -874,19 +995,19 @@ int ddn_backproject_filter_ragged(const ddn_filter_config* cfg, int64_t n_views,
                                   const int64_t* layout_host, const float* refined_all, const float* normal,
                                   const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
                                   uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
-  using namespace ddn;
-  FilterParams p;
-  DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
-  DDN_REQUIRE(layout != nullptr, "null layout");
-  DDN_TRY(check_layout(n_views, layout_host));
-  DDN_REQUIRE(cfg->stride == layout_host[n_views * DDN_LAYOUT_COLS], "cfg->stride must be the layout's stride");
-  p.src_begin = 0;
-  p.n_src = (int)n_views;
-  p.H = p.W = p.Hs = p.Ws = 0;  // per view, from the layout and the table entries
-  p.wbits = p.hbits = 0;
-  const int64_t chunks = layout_host[n_views * DDN_LAYOUT_COLS + 5];  // >= 1: every view has a pixel
-  DDN_TRY(launch_filter(cfg, p, dim3((unsigned)chunks), layout, (cudaStream_t)stream));
-  return after_launch("backproject_filter_kernel");
+  return ddn::filter_ragged(nullptr, cfg, n_views, k_nbr, layout, layout_host, refined_all, normal, pair_table, src_table,
+                            vote_threshold, xyz, votes, bbox, mark, stream);
+}
+
+int ddn_backproject_filter_support_ragged(const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
+                                          const int64_t* layout, const int64_t* layout_host, const float* refined_all,
+                                          const float* normal, const float* pair_table, const float* src_table,
+                                          int32_t vote_threshold, int32_t min_support, float support_tau, float* xyz,
+                                          uint8_t* votes, uint8_t* support, float* bbox, const ddn_fuse_session* mark,
+                                          void* stream) {
+  const ddn::SupportParams sup{support, min_support, support_tau};
+  return ddn::filter_ragged(&sup, cfg, n_views, k_nbr, layout, layout_host, refined_all, normal, pair_table, src_table,
+                            vote_threshold, xyz, votes, bbox, mark, stream);
 }
 
 }  // extern "C"

@@ -150,6 +150,7 @@ class ShardedDensifier:
         self.V, self.lo, self.hi, self.H, self.W = n_views_total, lo, hi, height, width
         self.K = nbr.shape[1]
         self.thr = cfg.vote_threshold_for(self.K)
+        self.fthr = ops.fusion_threshold(self.thr, cfg.min_support is not None)  # what fusion tests the vote bytes with
         bounds = shard_bounds(n_views_total, world) if world > 1 else [(lo, hi)]
         if world > 1 and bounds[rank] != (lo, hi):
             raise ValueError(f"rank {rank}: shard {(lo, hi)} does not match the contiguous layout {bounds[rank]}")
@@ -355,9 +356,9 @@ class ShardedDensifier:
                     t.record_stream(main)
         else:
             refined_slots, pair, src, box, stats = stage1()
-        xyz, votes, bbox = self._halo_and_filter(refined_slots, normal, mark, pair, src, box=box, grid=grid)
+        xyz, votes, bbox, support = self._halo_and_filter(refined_slots, normal, mark, pair, src, box=box, grid=grid)
         res = ShardResult(refined=refined_slots[: self.n_local], stats=stats, xyz=xyz, votes=votes, vote_threshold=self.thr,
-                          bbox=bbox, events=ev)
+                          bbox=bbox, events=ev, support=support, min_support=cfg.min_support)
         if not fuse:
             return res
         s = cfg.filter.stride
@@ -377,7 +378,7 @@ class ShardedDensifier:
             grid = self.ops.make_grid(bb[:3], bb[3:], cfg.voxel)
         if self.world == 1:
             k, x, c, n, counts = mark("voxel_fuse", lambda: self.ops.voxel_fuse(
-                xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), self.thr, grid, trim=False, row_len=xyz.shape[2]))
+                xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), self.fthr, grid, trim=False, row_len=xyz.shape[2]))
         else:
             k, x, c, n, counts = mark("voxel_fuse", lambda: self._fuse_sharded(xyz, rgb_s, votes, grid, mark))
         res.grid, res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = grid, k, x, c, n, counts
@@ -440,6 +441,7 @@ class ShardedDensifier:
         bbox = self.ops.new_bbox(self.device) if not self.device_path or sess is None else None
         xyz = torch.empty((self.n_local, self.Hs, self.Ws, 3), dtype=torch.float32, device=self.device)
         votes = torch.empty((self.n_local, self.Hs, self.Ws), dtype=torch.uint8, device=self.device)
+        support = None if cfg.min_support is None else torch.empty_like(votes)
         if wait_normal is not None:
             wait_normal()
         extra = {"mark": sess} if self.device_path else {}
@@ -448,9 +450,10 @@ class ShardedDensifier:
             if c1 <= c0:
                 return
             whole = c0 == 0 and c1 == self.n_local
+            sup = {} if support is None else {"support": cfg.support(), "support_out": support[c0:c1]}
             self.ops.backproject_filter(refined_slots, normal if whole else normal[c0:c1], self.nbr_slots,
                                         pair if whole else pair[c0:c1], src if whole else src[c0:c1], c0, self.thr, cfg.filter,
-                                        bbox=bbox, xyz_out=xyz[c0:c1], votes_out=votes[c0:c1], **extra)
+                                        bbox=bbox, xyz_out=xyz[c0:c1], votes_out=votes[c0:c1], **extra, **sup)
 
         if join_halo is not None:
             i0, i1 = self._interior_range()
@@ -462,7 +465,7 @@ class ShardedDensifier:
             if self.device_path and cfg.overlap_align and self.peer is None:
                 self._ev_stage1_may_start = torch.cuda.Event()
                 self._ev_stage1_may_start.record(torch.cuda.current_stream(self.device))
-        return xyz, votes, bbox
+        return xyz, votes, bbox, support
 
     def _merge_outputs(self, slot: int):
         if self._merge_out[slot] is None:
@@ -512,17 +515,17 @@ class ShardedDensifier:
         if self.peer is None:
             if drop is not None:
                 sess.unmark_points(drop)
-            out = self.ops.fuse_finish(sess, *flat, self.thr, row_len=xyz.shape[2])[:4]
-            k, x, c, n, counts = self.ops.fuse_finish_hashed(sess, hf, *flat, self.thr, row_len=xyz.shape[2], dedup_xyz=drop, out=out)
+            out = self.ops.fuse_finish(sess, *flat, self.fthr, row_len=xyz.shape[2])[:4]
+            k, x, c, n, counts = self.ops.fuse_finish_hashed(sess, hf, *flat, self.fthr, row_len=xyz.shape[2], dedup_xyz=drop, out=out)
             return k, x, c, n, counts.clone()
         rec, hdl, _ = self.peer.buffer("records", tuple(self.peer_records_shape), torch.int64)
         samples = self.peer.buffer("hash_samples", (ops._lib.HASH_SAMPLES + 1,), torch.int64)[0]
 
         def partials():
-            self.ops.fuse_finish_partial(sess, *flat, self.thr, rec, row_len=xyz.shape[2])
+            self.ops.fuse_finish_partial(sess, *flat, self.fthr, rec, row_len=xyz.shape[2])
             # N5 on the hashed path: every rank tombstones the cells of all ranks' sparse points, so their points are
             # never sent
-            self.ops.fuse_finish_hashed_partial(sess, hf, *flat, self.thr, rec, samples, row_len=xyz.shape[2], dedup_xyz=drop)
+            self.ops.fuse_finish_hashed_partial(sess, hf, *flat, self.fthr, rec, samples, row_len=xyz.shape[2], dedup_xyz=drop)
 
         def merge():
             out = self.ops.fuse_merge_peers(sess, self.rank, self.world, self._peer_records, self._peer_prefix, self._plan, self._cap_merge,
@@ -550,7 +553,7 @@ class ShardedDensifier:
         n_tiles, _ = self.ops.fuse_tile_info(grid)
         tile_prefix = torch.empty(n_tiles + 1, dtype=torch.int32, device=self.device) if n_tiles > 0 else None
         rec, counts = mark("fuse_partials", lambda: self.ops.voxel_fuse_partial(
-            xyz.view(-1, 3), rgb.view(-1, 3), votes.view(-1), self.thr, grid, row_len=xyz.shape[2], tile_prefix=tile_prefix))
+            xyz.view(-1, 3), rgb.view(-1, 3), votes.view(-1), self.fthr, grid, row_len=xyz.shape[2], tile_prefix=tile_prefix))
         return mark("fuse_exchange_merge", lambda: self._exchange_and_merge(rec, counts, grid, mark, tile_prefix))
 
     def _plan_by_tiles(self, tile_prefix):
@@ -737,8 +740,8 @@ class ShardedDensifier:
             upload(st["rgb"], rgb)
             ev_rgb = torch.cuda.Event()
             ev_rgb.record(copy)
-        xyz, votes, bbox = self._halo_and_filter(refined_slots, normal_arg, lambda name, fn: fn(), pair, src,
-                                                 wait_normal=lambda: comp.wait_event(ev_n), box=box)
+        xyz, votes, bbox, _ = self._halo_and_filter(refined_slots, normal_arg, lambda name, fn: fn(), pair, src,
+                                                    wait_normal=lambda: comp.wait_event(ev_n), box=box)
         ticket = {"slot": st, "h2d_bytes": h2d, "stats": torch.cat(stats) if stats else None, "fused": None, "host_grid": None}
         s = cfg.filter.stride
         if fuse and self.device_path:
@@ -759,7 +762,7 @@ class ShardedDensifier:
                 comp.wait_event(ev_rgb)
                 rgb_s = st["rgb"] if s == 1 else st["rgb"][:, ::s, ::s].contiguous()
                 if self.world == 1:
-                    k, x, c, m, counts = self.ops.voxel_fuse(xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), self.thr, grid,
+                    k, x, c, m, counts = self.ops.voxel_fuse(xyz.view(-1, 3), rgb_s.view(-1, 3), votes.view(-1), self.fthr, grid,
                                                              trim=False, row_len=xyz.shape[2])
                 else:
                     k, x, c, m, counts = self._fuse_sharded(xyz, rgb_s, votes, grid)

@@ -28,6 +28,15 @@ class DensifyConfig:
     # fusing / merging (its NVLink-bound exchange leaves the SMs idle).  The caller's inputs must then be complete when
     # run() is called - they are not ordered against work the caller queued on the current stream just before.
     overlap_align: bool = False
+    # Multi-view support (parity unpinned): keep a point only when at least min_support neighbour views see its surface
+    # within the relative depth error support_tau, |z - D| <= support_tau * D.  None: off (reference behaviour);
+    # 0: count support (DensifyResult.support) without dropping anything.
+    min_support: int | None = None
+    support_tau: float = 0.01
+
+    def support(self) -> tuple[int, float] | None:
+        """The ``support`` argument of ops.backproject_filter: (min_support, support_tau), or None when off."""
+        return None if self.min_support is None else (int(self.min_support), float(self.support_tau))
 
     def vote_threshold_for(self, k: int) -> int:
         """The threshold a step with ``k`` neighbours per view votes with (``vote_threshold`` or ceil(k/2), clamped)."""
@@ -66,16 +75,22 @@ class DensifyResult:
     layout: ops.ViewLayout | None = None  # run_views: refined [P], xyz [G,3], votes [G] are flat over the views of this layout
     rgb: torch.Tensor | None = None  # the step's colours: [V,H,W,3] u8, or flat [P,3] u8 over the views of ``layout``
     stride: int = 1  # back-projection grid stride: xyz / votes hold every stride-th row and column
+    support: torch.Tensor | None = None  # like votes: supporting neighbours, min(count, 254), 255 = no point (None: off)
+    min_support: int | None = None  # the step's DensifyConfig.min_support
+
+    def fusion_threshold(self) -> int:
+        """The threshold the vote bytes are tested with (by keep_mask and the fusion passes)."""
+        return ops.fusion_threshold(clamp_vote_threshold(self.vote_threshold), self.min_support is not None)
 
     def per_view(self, name: str) -> list:
         """Per-view views of a flat output of run_views: ``refined`` -> [H_v, W_v], ``xyz`` -> [Hs_v, Ws_v, 3],
-        ``votes`` -> [Hs_v, Ws_v] (no copy)."""
+        ``votes``, ``support`` -> [Hs_v, Ws_v] (no copy)."""
         if self.layout is None:
             return list(getattr(self, name))
         return self.layout.split(getattr(self, name), grid=name != "refined")
 
     def keep_mask(self) -> torch.Tensor:
-        return (self.votes != 255) & (self.votes < clamp_vote_threshold(self.vote_threshold))
+        return (self.votes != 255) & (self.votes < self.fusion_threshold())
 
     def grid_rgb(self) -> torch.Tensor:
         """The colours on the back-projection grid, in the order of ``xyz``: [V,Hs,Ws,3], or flat [G,3] for run_views."""
@@ -201,11 +216,15 @@ class DensifyEngine:
             else:
                 sess.begin_grid(grid)
         bbox = ops.new_bbox(dev)
-        xyz, votes = (ops.backproject_filter(refined, normal, nbr, pair, src, 0, thr, cfg.filter, bbox=bbox, mark=sess)
-                      if layout is None else
-                      ops.backproject_filter_ragged(layout, refined, normal, pair, src, thr, cfg.filter, bbox=bbox, mark=sess))
+        extra = {} if cfg.min_support is None else {"support": cfg.support()}
+        out = (ops.backproject_filter(refined, normal, nbr, pair, src, 0, thr, cfg.filter, bbox=bbox, mark=sess, **extra)
+               if layout is None else
+               ops.backproject_filter_ragged(layout, refined, normal, pair, src, thr, cfg.filter, bbox=bbox, mark=sess, **extra))
+        xyz, votes = out[:2]
         res = DensifyResult(refined=refined, stats=stats, xyz=xyz, votes=votes, vote_threshold=thr, bbox=bbox, bbox_valid=box,
-                            layout=layout, rgb=rgb, stride=cfg.filter.stride)
+                            layout=layout, rgb=rgb, stride=cfg.filter.stride, support=out[2] if extra else None,
+                            min_support=cfg.min_support)
+        thr = res.fusion_threshold()
         if fuse:
             points = (xyz.view(-1, 3), res.grid_rgb().view(-1, 3), votes.view(-1))
             dedup = sparse_xyz.float().contiguous() if cfg.dedup_sparse and sparse_xyz.shape[0] > 0 else None

@@ -225,12 +225,32 @@ def decode_bbox(bbox: torch.Tensor) -> np.ndarray:
     return i.view(np.float32)
 
 
+def _support_args(support) -> tuple[int, float]:
+    m, tau = support
+    if not (0 <= int(m) <= 1024) or not (math.isfinite(float(tau)) and float(tau) > 0):
+        raise ValueError(f"support = (min_support in [0, 1024], tau > 0 finite), got {support}")
+    return int(m), float(tau)
+
+
+def fusion_threshold(vote_threshold: int, support: bool) -> int:
+    """The threshold fusion and keep masks test the vote bytes of a filter call with: ``vote_threshold``, or
+    min(vote_threshold, 254) when the call counted support (the vote byte then carries the keep decision; see
+    ddn_backproject_filter_support in include/ddn_b200.h)."""
+    return min(int(vote_threshold), 254) if support else int(vote_threshold)
+
+
 def backproject_filter(refined_all, normal, nbr, pair_table, src_table, src_begin: int, vote_threshold: int,
-                       opts: FilterOptions, bbox=None, xyz_out=None, votes_out=None, mark=None):
+                       opts: FilterOptions, bbox=None, xyz_out=None, votes_out=None, mark=None, support=None,
+                       support_out=None):
     """Stages 2+3 for the source views src_begin..src_begin+n_src (n_src = normal.shape[0]).  ``normal`` may
     be a PINNED HOST tensor: the kernel then reads the normals of its vote candidates in place over PCIe
     (unified addressing) and the 12 B/pixel normal map never moves to the device.  ``mark``: an open
-    ``FuseSession``; the kernel then also sets the occupancy bits of the kept points (stage 4's mark pass)."""
+    ``FuseSession``; the kernel then also sets the occupancy bits of the kept points (stage 4's mark pass).
+
+    ``support`` = (min_support, tau): also count the neighbours that see each point within the relative depth error
+    tau and keep only points with at least min_support of them (ddn_backproject_filter_support).  Returns
+    (xyz, votes, support) then, support [n_src,Hs,Ws] u8 (or ``support_out``); test the votes with
+    ``fusion_threshold(vote_threshold, True)``."""
     lib = _lib.load()
     dev = _require_cuda_normal(normal, refined_all, nbr, pair_table, src_table, bbox, xyz_out, votes_out)
     V, H, W = refined_all.shape
@@ -244,6 +264,19 @@ def backproject_filter(refined_all, normal, nbr, pair_table, src_table, src_begi
     xyz = xyz_out if xyz_out is not None else torch.empty((n_src, Hs, Ws, 3), dtype=torch.float32, device=dev)
     votes = votes_out if votes_out is not None else torch.empty((n_src, Hs, Ws), dtype=torch.uint8, device=dev)
     cfg = opts.to_c()
+    if support is not None:
+        m, tau = _support_args(support)
+        sup = support_out if support_out is not None else torch.empty((n_src, Hs, Ws), dtype=torch.uint8, device=dev)
+        assert sup.dtype == torch.uint8 and sup.is_contiguous() and tuple(sup.shape) == tuple(votes.shape)
+        with torch.cuda.device(dev):
+            _lib.check(
+                lib.ddn_backproject_filter_support(
+                    C.byref(cfg), V, src_begin, n_src, H, W, K, _p(refined_all), _p(normal), _p(nbr), _p(pair_table),
+                    _p(src_table), int(vote_threshold), m, tau, _p(xyz), _p(votes), _p(sup), _p(bbox),
+                    C.byref(mark.c) if mark is not None else None, _stream(),
+                )
+            )
+        return xyz, votes, sup
     with torch.cuda.device(dev):
         _lib.check(
             lib.ddn_backproject_filter(
@@ -396,10 +429,11 @@ def build_pair_tables_ragged(layout: ViewLayout, cam_from_world, intr, nbr):
 
 
 def backproject_filter_ragged(layout: ViewLayout, refined_all, normal, pair_table, src_table, vote_threshold: int,
-                              opts: FilterOptions, bbox=None, xyz_out=None, votes_out=None, mark=None):
+                              opts: FilterOptions, bbox=None, xyz_out=None, votes_out=None, mark=None, support=None,
+                              support_out=None):
     """Stages 2+3 for all views of ``layout``: refined_all flat [P] f32, normal flat [P,3] f32 (device, or pinned host).
     Returns xyz [G,3] f32 and votes [G] u8 on the views' strided grids (G = layout.total_grid); ``opts.stride`` must be
-    the layout's stride."""
+    the layout's stride.  ``support``, ``support_out``: as in ``backproject_filter`` (then also returns support [G] u8)."""
     lib = _lib.load()
     dev = _require_cuda_normal(normal, refined_all, pair_table, src_table, bbox, xyz_out, votes_out)
     V, P, G = layout.n_views, layout.total_pixels, layout.total_grid
@@ -412,6 +446,19 @@ def backproject_filter_ragged(layout: ViewLayout, refined_all, normal, pair_tabl
     xyz = xyz_out if xyz_out is not None else torch.empty((G, 3), dtype=torch.float32, device=dev)
     votes = votes_out if votes_out is not None else torch.empty(G, dtype=torch.uint8, device=dev)
     cfg = opts.to_c()
+    if support is not None:
+        m, tau = _support_args(support)
+        sup = support_out if support_out is not None else torch.empty(G, dtype=torch.uint8, device=dev)
+        assert sup.dtype == torch.uint8 and sup.is_contiguous() and tuple(sup.shape) == tuple(votes.shape)
+        with torch.cuda.device(dev):
+            _lib.check(
+                lib.ddn_backproject_filter_support_ragged(
+                    C.byref(cfg), V, K, _p(layout.device(dev)), layout.host_ptr(), _p(refined_all), _p(normal),
+                    _p(pair_table), _p(src_table), int(vote_threshold), m, tau, _p(xyz), _p(votes), _p(sup), _p(bbox),
+                    C.byref(mark.c) if mark is not None else None, _stream(),
+                )
+            )
+        return xyz, votes, sup
     with torch.cuda.device(dev):
         _lib.check(
             lib.ddn_backproject_filter_ragged(

@@ -82,6 +82,11 @@ class FilteringConfig:
     """new, with num_neighbours: 'covisibility' (views sharing the most sparse points) or 'nearest' (camera centres)."""
     sample_mode: str = "nearest"
     """new: 'nearest' (reference) or 'bilinear'."""
+    min_support: int | None = None
+    """new: also keep a point only when at least this many neighbour views see its surface within support_tau (relative
+    depth error); None = no such test (reference), 0 = count only."""
+    support_tau: float = 0.01
+    """new, with min_support: the relative depth error |z - D| <= support_tau * D within which a view supports a point."""
 
 
 @dataclass
@@ -274,8 +279,11 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
                              adaptive_correspondences=rc.adaptive_correspondences, zero_unmasked_passthrough=True)
     filt = ops.FilterOptions(depth_threshold=config.filtering.depth_threshold, sample_mode=config.filtering.sample_mode,
                              stride=max(int(config.processing.downsample_density), 1))
+    ms = config.filtering.min_support
     eng = DensifyEngine(DensifyConfig(align=align, filter=filt, vote_threshold=int(config.filtering.vote_threshold),
-                                      voxel=config.fusion.voxel_size, dedup_sparse=bool(config.fusion.dedup_sparse)), device=dev)
+                                      voxel=config.fusion.voxel_size, dedup_sparse=bool(config.fusion.dedup_sparse),
+                                      min_support=None if ms is None else int(ms),
+                                      support_tau=float(config.filtering.support_tau)), device=dev)
     offsets = np.concatenate([[0], np.cumsum([len(p) for p in sparse])]).astype(np.int64)
     to = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(dev)
     maps = ((depths, torch.float32), (normals, torch.float32), (masks, torch.bool), (rgbs, torch.uint8))
@@ -311,7 +319,7 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
     if return_candidates:
         valid = res.votes != 255
         out.candidates = res.xyz[valid].double().cpu().numpy()
-        out.keep = (res.votes[valid] < res.vote_threshold).cpu().numpy()
+        out.keep = (res.votes[valid] < res.fusion_threshold()).cpu().numpy()
     return out
 
 

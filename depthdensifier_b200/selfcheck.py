@@ -17,11 +17,12 @@ from .synthetic import SceneConfig, make_scene
 
 def multi_gpu_check(dev, rank: int, world: int, n_views: int = 24, width: int = 320, height: int = 240, k: int = 4,
                     voxel: float = 0.02, steps: int = 2, verbose: bool = False, dedup: bool = False, dome_radius: float | None = None,
-                    max_grid_cells: int | None = None) -> dict:
+                    max_grid_cells: int | None = None, min_support: int | None = None) -> dict:
     """Every rank calls this.  Rank 0 returns {"passed": bool, "path": "peer" | "collective", ...}; the other
     ranks the same dict with their local view of ``path``.  ``dome_radius``: the scene gets a distant background
     (SceneConfig.dome_radius), ``max_grid_cells``: the sessions' bitmap capacity - either can send the step through the
-    hashed fusion path (``report["grid"]`` says which path fused)."""
+    hashed fusion path (``report["grid"]`` says which path fused).  ``min_support``: DensifyConfig.min_support of both
+    pipelines (the support counts are then compared too)."""
     V, W, H = n_views, width, height
     sc = make_scene(SceneConfig(n_views=V, width=W, height=H, n_sparse=1500, seed=4, dome_radius=dome_radius))  # host, identical on all ranks
     nbr = nearest_views_table(sc.cam_from_world.numpy(), k)
@@ -35,10 +36,11 @@ def multi_gpu_check(dev, rank: int, world: int, n_views: int = 24, width: int = 
         mv = res.check()
         return {"keys": res.voxel_keys[:mv].cpu().numpy(), "xyz": res.voxel_xyz[:mv].cpu().numpy(),
                 "rgb": res.voxel_rgb[:mv].cpu().numpy(), "count": res.voxel_count[:mv].cpu().numpy(),
-                "votes": res.votes.cpu().numpy(), "refined": res.refined.cpu().numpy(), "n": int(res.counts[0])}
+                "votes": res.votes.cpu().numpy(), "refined": res.refined.cpu().numpy(), "n": int(res.counts[0]),
+                "support": None if res.support is None else res.support.cpu().numpy()}
 
     def config(**kw):
-        cfg = DensifyConfig(voxel=voxel, dedup_sparse=dedup, **kw)
+        cfg = DensifyConfig(voxel=voxel, dedup_sparse=dedup, min_support=min_support, **kw)
         if max_grid_cells is not None:
             cfg.max_grid_cells = max_grid_cells
         return cfg
@@ -53,6 +55,8 @@ def multi_gpu_check(dev, rank: int, world: int, n_views: int = 24, width: int = 
     gathered = [None] * world
     dist.gather_object(mine, gathered if rank == 0 else None, dst=0)
     report = {"passed": True, "path": path, "ranks": world, "views": V, "size": [W, H], "steps": steps, "dedup_sparse": dedup, "different": []}
+    if min_support is not None:
+        report["min_support"] = min_support
     if dome_radius is not None or max_grid_cells is not None:
         status = results[-1].session.grid_state().status if results[-1].session is not None else None
         report.update(dome_radius=dome_radius, max_grid_cells=max_grid_cells, grid={0: "dense", 4: "hashed"}.get(status, status))
@@ -60,7 +64,7 @@ def multi_gpu_check(dev, rank: int, world: int, n_views: int = 24, width: int = 
     if rank == 0:
         sd1 = ShardedDensifier(config(), dev, 0, 1, V, 0, V, sc.cam_from_world, sc.intrinsics, nbr, H, W)
         one = collect(sd1.run(*inputs(0, V, lambda t: t.to(dev).contiguous())))
-        for name in ("refined", "votes", "keys", "count", "rgb", "xyz"):
+        for name in ("refined", "votes", "keys", "count", "rgb", "xyz") + (() if min_support is None else ("support",)):
             cat = np.concatenate([g[name] for g in gathered])
             if not np.array_equal(cat, one[name]):
                 report["different"].append(name)

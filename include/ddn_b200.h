@@ -167,6 +167,29 @@ DDN_API int ddn_backproject_filter(const ddn_filter_config* cfg, int64_t n_views
                            float* xyz, uint8_t* votes, float* bbox, const struct ddn_fuse_session* mark,
                            void* stream);
 
+/* ddn_backproject_filter with a multi-view support count (new; parity unpinned, DESIGN.md §2).  Neighbour entry t of
+ * the table SUPPORTS the point of a pixel when the point projects into t's map in bounds, the sampled depth D
+ * (cfg->sample_mode, as for the vote) is > 0, and |z - D| <= support_tau * D, with z the point's depth in view t.  No
+ * grazing gate; entries of the source view itself never count.  support [n_src,Hs,Ws] u8 (same grid as votes):
+ * min(count, 254), 255 = no point.  A point is kept iff it exists, its vote count is below vote_threshold (as in
+ * ddn_backproject_filter) and count >= min_support.  min_support in [0, 1024]; support_tau > 0 and finite.
+ *
+ * The keep decision is carried in the vote byte, so every fusion call (ddn_fuse_*, ddn_voxel_*) and a host-side
+ * keep mask reproduce K4's keep, its bounding box and its occupancy mark (counts[0]) when they are given the
+ * threshold min(vote_threshold, 254).  For a point:
+ *   votes = 254                  when count < min_support;
+ *   votes = min(nvotes, 254)     otherwise, when vote_threshold <= 254;
+ *   votes = min(nvotes, 253)     otherwise, when vote_threshold >= 255 (every supported point is kept);
+ *   votes = 255                  when the pixel has no point.
+ * Then keep == (votes < min(vote_threshold, 254)) at every vote_threshold and min_support.  With min_support = 0 and
+ * vote_threshold <= 254, votes, xyz, bbox and the mark are those of ddn_backproject_filter, byte for byte. */
+DDN_API int ddn_backproject_filter_support(const ddn_filter_config* cfg, int64_t n_views_total, int64_t src_begin,
+                                   int64_t n_src, int64_t height, int64_t width, int64_t k_nbr,
+                                   const float* refined_all, const float* normal, const int32_t* nbr,
+                                   const float* pair_table, const float* src_table, int32_t vote_threshold,
+                                   int32_t min_support, float support_tau, float* xyz, uint8_t* votes,
+                                   uint8_t* support, float* bbox, const struct ddn_fuse_session* mark, void* stream);
+
 DDN_API int ddn_bbox_init(float* bbox, void* stream);
 
 /* ------------------------------------------------------------------------------------------
@@ -218,6 +241,15 @@ DDN_API int ddn_backproject_filter_ragged(const ddn_filter_config* cfg, int64_t 
                                   const float* normal, const float* pair_table, const float* src_table,
                                   int32_t vote_threshold, float* xyz, uint8_t* votes, float* bbox,
                                   const struct ddn_fuse_session* mark, void* stream);
+
+/* ddn_backproject_filter_ragged with the support count, keep rule and vote encoding of
+ * ddn_backproject_filter_support; support [total grid points] u8 on the same grids as votes. */
+DDN_API int ddn_backproject_filter_support_ragged(const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
+                                          const int64_t* layout, const int64_t* layout_host,
+                                          const float* refined_all, const float* normal, const float* pair_table,
+                                          const float* src_table, int32_t vote_threshold, int32_t min_support,
+                                          float support_tau, float* xyz, uint8_t* votes, uint8_t* support,
+                                          float* bbox, const struct ddn_fuse_session* mark, void* stream);
 
 /* Neighbouring per-pixel helpers (SURVEY.md 8(f) rank 4).
  * ddn_gradient_mask: compute_depth_normal_gradient_mask, src/depthdensifier/initilizer.py:236-328 - mask_out [H,W]

@@ -3,7 +3,9 @@
 reproduce the 1-rank pipeline bit for bit (depthdensifier_b200/selfcheck.py).  Rank 0 prints one JSON line.
 
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 \
-      scripts/check_multi_gpu.py
+      scripts/check_multi_gpu.py [--min-support M]
+
+--min-support M: run both checks with the multi-view support filter (DensifyConfig.min_support = M) as well.
 """
 
 import json
@@ -26,7 +28,13 @@ def main():
     dev = torch.device("cuda", local)
     os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
     dist.init_process_group("nccl", device_id=dev)
-    reports = [multi_gpu_check(dev, rank, world), multi_gpu_check(dev, rank, world, n_views=29, width=203, height=131, k=3, voxel=0.03, dedup=True)]
+    ms = [None]
+    if "--min-support" in sys.argv:
+        ms.append(int(sys.argv[sys.argv.index("--min-support") + 1]))
+    reports = []
+    for m in ms:
+        reports += [multi_gpu_check(dev, rank, world, min_support=m),
+                    multi_gpu_check(dev, rank, world, n_views=29, width=203, height=131, k=3, voxel=0.03, dedup=True, min_support=m)]
     if rank == 0:
         print(json.dumps({"multi_gpu_check": reports}))
     dist.barrier()
