@@ -122,6 +122,11 @@ SYMBOLS = {
         [C.POINTER(FilterConfig), _i64, _i64, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _i32, C.c_float, _vp, _vp,
          _vp, _vp, C.POINTER(FuseSession), _vp],
     ),
+    "ddn_backproject_filter_support_reproj": (
+        C.c_int,
+        [C.POINTER(FilterConfig), _i64, _i64, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _i32, C.c_float,
+         C.c_float, _vp, _vp, _vp, _vp, C.POINTER(FuseSession), _vp],
+    ),
     "ddn_bbox_init": (C.c_int, [_vp, _vp]),
     "ddn_align_views_ragged": (
         C.c_int,
@@ -136,6 +141,11 @@ SYMBOLS = {
         C.c_int,
         [C.POINTER(FilterConfig), _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, C.c_float, _vp, _vp, _vp, _vp,
          C.POINTER(FuseSession), _vp],
+    ),
+    "ddn_backproject_filter_support_reproj_ragged": (
+        C.c_int,
+        [C.POINTER(FilterConfig), _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, C.c_float, C.c_float, _vp, _vp, _vp,
+         _vp, C.POINTER(FuseSession), _vp],
     ),
     "ddn_pchip_workspace_bytes": (C.c_int, [_i64, _i64, C.POINTER(_i64)]),
     "ddn_pchip_edge_mask": (

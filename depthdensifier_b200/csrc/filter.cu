@@ -189,8 +189,27 @@ struct SupportParams {
   int min_support;
   float support_tau;
 };
+// The trailing parameter of the reprojection forms (ddn_backproject_filter_support_reproj*): the support arguments and
+// rho^2, the square of the round-trip pixel bound (+inf when rho^2 overflows float32: the bound then passes every
+// finite error).
+struct ReprojParams {
+  SupportParams support;
+  float reproj_px2;
+};
 __device__ __forceinline__ SupportParams support_params() { return SupportParams{nullptr, 0, 0.f}; }
 __device__ __forceinline__ SupportParams support_params(const SupportParams& s) { return s; }
+__device__ __forceinline__ SupportParams support_params(const ReprojParams& r) { return r.support; }
+__device__ __forceinline__ float reproj_px2() { return 0.f; }
+__device__ __forceinline__ float reproj_px2(const SupportParams&) { return 0.f; }
+__device__ __forceinline__ float reproj_px2(const ReprojParams& r) { return r.reproj_px2; }
+template <class... S>
+struct IsReproj {
+  static constexpr bool value = false;
+};
+template <>
+struct IsReproj<ReprojParams> {
+  static constexpr bool value = true;
+};
 
 __device__ __forceinline__ float rcp_approx(float x) {
   float r;
@@ -248,10 +267,10 @@ __device__ __forceinline__ f32x2 row_dot2(const float4& r, f32x2 P, f32x2 Q, f32
 template <bool kBilinear, bool kFoldMask>
 __device__ __forceinline__ void pair_gather(const float4& r0, const float4& r1, const float4& r2, f32x2 P, f32x2 Q, f32x2 d,
                                             const float* __restrict__ depth_all, unsigned off_k, unsigned W, int H,
-                                            unsigned wbits, unsigned hbits, float* Z, float* D, bool* inb) {
+                                            unsigned wbits, unsigned hbits, float* Z, float* D, bool* inb, f32x2& inv) {
   const f32x2 U = row_dot2(r0, P, Q, d), V = row_dot2(r1, P, Q, d);
   unpack2(row_dot2(r2, P, Q, d), Z[0], Z[1]);
-  const f32x2 inv = pack2(rcp_approx(Z[0]), rcp_approx(Z[1]));
+  inv = pack2(rcp_approx(Z[0]), rcp_approx(Z[1]));  // 1/Z, before the out-of-bounds lanes' Z becomes +inf
   const f32x2 u = mul2(U, inv), v = mul2(V, inv);
   const f32x2 bias = splat2(8388608.0f);
   const f32x2 ub = add_rz2(u, bias), vb = add_rz2(v, bias);  // trunc(u), trunc(v) + kTruncBias per lane
@@ -290,19 +309,62 @@ __device__ __forceinline__ void pair_test(const float* Z, const float* D, const 
 // Support bits of a pixel pair: neighbour entry `bit` sees the surface of the pixel within the relative depth error
 // tau, |Z - D| <= tau*D.  No grazing gate.  kFoldMask: out-of-bounds lanes carry Z = +inf and pixels without a point
 // NaN, so both fail the comparison without the bounds mask; D > 0 is implied, since in-bounds lanes have Z > 0.
-template <bool kFoldMask>
+// kReproj (the reprojection forms): the entry must also pass the forward-backward reprojection test of
+// include/ddn_b200.h in its closed form, from t's epipole in s, ep = (e_x, e_y, e_z, -e_z):
+//   w = (Z - D)/Z,  z' = d + w (e_z - d),  A = d e_x - P e_z,  B = d e_y - Q e_z,
+//   z' > 0  and  w^2 (A^2 + B^2) <= rho^2 (d z')^2.
+// inv = 1/Z of pair_gather.  Lanes that fail the depth test (out of bounds: Z = +inf; no point: NaN) fail the
+// conjunction whatever this evaluates to.
+template <bool kFoldMask, bool kReproj = false>
 __device__ __forceinline__ void pair_support(const float* Z, const float* D, const bool* inb, float tau, unsigned bit,
-                                             unsigned* sm) {
+                                             unsigned* sm, f32x2 inv = 0ull, f32x2 d = 0ull, f32x2 P = 0ull, f32x2 Q = 0ull,
+                                             float4 ep = float4{}, float rho2 = 0.f) {
   const f32x2 D2 = pack2(D[0], D[1]);
   const f32x2 dz = sub2(pack2(Z[0], Z[1]), D2), tD = mul2(splat2(tau), D2);
+  if (kReproj) {
+    const f32x2 w = mul2(dz, inv);
+    const f32x2 A = fma2(P, splat2(ep.w), mul2(d, splat2(ep.x)));
+    const f32x2 B = fma2(Q, splat2(ep.w), mul2(d, splat2(ep.y)));
+    const f32x2 zp = fma2(w, sub2(splat2(ep.z), d), d);
+    const f32x2 lhs = mul2(mul2(w, w), fma2(A, A, mul2(B, B)));
+    const f32x2 dzp = mul2(d, zp);
+    const f32x2 rhs = mul2(mul2(splat2(rho2), dzp), dzp);
 #pragma unroll
-  for (int e = 0; e < 2; ++e) {
-    if (kFoldMask) {
-      if (fabsf(lane2(dz, e)) <= lane2(tD, e)) sm[e] |= bit;
-    } else if (inb[e] & (fabsf(lane2(dz, e)) <= lane2(tD, e))) {
-      sm[e] |= bit;
+    for (int e = 0; e < 2; ++e) {
+      const bool ok = (lane2(zp, e) > 0.f) & (lane2(lhs, e) <= lane2(rhs, e)) & (fabsf(lane2(dz, e)) <= lane2(tD, e));
+      if (kFoldMask ? ok : (ok & inb[e])) sm[e] |= bit;
+    }
+  } else {
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      if (kFoldMask) {
+        if (fabsf(lane2(dz, e)) <= lane2(tD, e)) sm[e] |= bit;
+      } else if (inb[e] & (fabsf(lane2(dz, e)) <= lane2(tD, e))) {
+        sm[e] |= bit;
+      }
     }
   }
+}
+
+// t's epipole in s, e = K_s (R_s c_t + t_s) = K_s R_s (c_t - c_s), as (e_x, e_y, e_z, -e_z): from the source table
+// (rows of R_s^T K_s^-1 with c_s, then cx, cy, fx, fy; the rows of R_s^T recovered as load_normal does) and c_t, floats
+// 12-14 of t's pair-table entry.  Each rounding written out (no contraction), so tests/reproj_oracle.py replays it
+// bit for bit on the host.
+__device__ __forceinline__ float4 epipole(const float* __restrict__ src, const float* __restrict__ ct) {
+  const float fx = __ldg(src + 14), fy = __ldg(src + 15), cx = __ldg(src + 12), cy = __ldg(src + 13);
+  float a0 = 0.f, a1 = 0.f, a2 = 0.f;  // R_s (c_t - c_s) = sum_i (row i of R_s^T) * (c_t - c_s)_i
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const float m0 = __ldg(src + i * 4 + 0), m1 = __ldg(src + i * 4 + 1), m2 = __ldg(src + i * 4 + 2);
+    const float ra = __fmul_rn(m0, fx), rb = __fmul_rn(m1, fy);
+    const float rc = __fadd_rn(__fadd_rn(m2, __fmul_rn(m0, cx)), __fmul_rn(m1, cy));
+    const float c = __fsub_rn(__ldg(ct + i), __ldg(src + i * 4 + 3));
+    a0 = __fadd_rn(a0, __fmul_rn(ra, c));
+    a1 = __fadd_rn(a1, __fmul_rn(rb, c));
+    a2 = __fadd_rn(a2, __fmul_rn(rc, c));
+  }
+  const float ex = __fadd_rn(__fmul_rn(fx, a0), __fmul_rn(cx, a2)), ey = __fadd_rn(__fmul_rn(fy, a1), __fmul_rn(cy, a2));
+  return make_float4(ex, ey, a2, -a2);
 }
 
 // Normal of one source pixel for the grazing gate (scripts/test.py:291), read on demand: only vote
@@ -368,15 +430,21 @@ static_assert(kFilterPX == 4, "the layouts below are written for 4 pixels per th
 // count, per pixel, the neighbour entries that support the point (pair_support), write the count to sp.support and apply
 // the keep rule and vote encoding of include/ddn_b200.h.  The support forms take 56 to 64 registers with nearest
 // sampling: at 5 CTAs per SM (48 registers) they would spill inside the neighbour loop, at 4 they do not.
+// kReproj (ddn_backproject_filter_support_reproj*; Support = ReprojParams): the support test also requires the
+// forward-backward reprojection test (pair_support); the epipoles of the hot entries are computed once per CTA into
+// shared memory (16 B per entry, after the pair table).  With the support forms' bounds these take 64 registers with
+// nearest sampling and 80 with bilinear, and their few spills lie outside the per-neighbour loop.
 template <bool kBilinear, bool kStride1, bool kTwoSided, int kLayout, bool kRagged, class... Support>
 __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : (sizeof...(Support) ? DDN_K4_SUPPORT_MINBLOCKS : DDN_K4_MINBLOCKS))
     backproject_filter_kernel(const FilterParams p, const int64_t* __restrict__ layout, Support... support) {
   constexpr bool kSupport = sizeof...(Support) != 0;
+  constexpr bool kReproj = IsReproj<Support...>::value;
   const SupportParams sp = support_params(support...);
   extern __shared__ __align__(16) float smem[];
   float* s_src = smem;                     // 16 floats
   float* s_pair = s_src + 16;              // K*24 floats
-  float* s_stage = s_pair + p.K * DDN_PAIR_TABLE_FLOATS;  // layout 0: 8 warps x 128 px x 3 floats
+  float4* s_epi = reinterpret_cast<float4*>(s_pair + p.K * DDN_PAIR_TABLE_FLOATS);  // kReproj: K float4
+  float* s_stage = s_pair + p.K * (DDN_PAIR_TABLE_FLOATS + (kReproj ? 4 : 0));      // layout 0: 8 warps x 128 px x 3 floats
   __shared__ int s_bbox[6];
   __shared__ int s_marked;
 
@@ -402,6 +470,11 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : (sizeof...(Sup
     if (tid < 4) reinterpret_cast<float4*>(s_src)[tid] = __ldg(reinterpret_cast<const float4*>(p.src_table + (size_t)sl * 16) + tid);
     if (tid < 6) s_bbox[tid] = tid < 3 ? 0x7fffffff : (int)0x80000000;
     if (tid == 6) s_marked = 0;
+    if (kReproj) {  // read from the global tables, so that the barrier below covers them too
+      const float* g = p.pair_table + (size_t)sl * p.K * DDN_PAIR_TABLE_FLOATS;
+      const int nh = __float_as_int(__ldg(g + 22));
+      for (int k = tid; k < nh; k += kFilterThreads) s_epi[k] = epipole(p.src_table + (size_t)sl * 16, g + k * DDN_PAIR_TABLE_FLOATS + 12);
+    }
   }
 
   // first pixel of the thread on the source grid: q0 = y0 * Ws + x0 (one integer division per thread)
@@ -464,6 +537,7 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : (sizeof...(Sup
   const unsigned wbits = p.wbits, hbits = p.hbits;
   const float thr = p.depth_threshold, gcos = p.grazing_cos, tau = p.two_sided_tau;
   const float stau = kSupport ? sp.support_tau : 0.f;
+  const float rho2 = reproj_px2(support...);
   const bool in_world = p.normals_in_world != 0;
   const int n_hot = __float_as_int(s_pair[22]), n_own = __float_as_int(s_pair[23]);
 
@@ -494,15 +568,19 @@ __global__ void __launch_bounds__(kFilterThreads, kBilinear ? 3 : (sizeof...(Sup
         const float4 wh = kRagged ? t4[4] : make_float4(0.f, 0.f, 0.f, 0.f);  // ragged: the neighbour's W, H, (float)W, (float)H
         float Z[kFilterPX], D[kFilterPX];
         bool inb[kFilterPX];
+        f32x2 inv[kPairs];
         constexpr bool kFold = !kBilinear && !kTwoSided;
         auto gather = [&](int h) {
           pair_gather<kBilinear, kFold>(r0, r1, r2, P2[h], Q2[h], d2[h], p.refined_all, off_k, kRagged ? __float_as_uint(wh.x) : (unsigned)p.W,
                                         kRagged ? __float_as_int(wh.y) : p.H, kRagged ? __float_as_uint(wh.z) : wbits,
-                                        kRagged ? __float_as_uint(wh.w) : hbits, Z + 2 * h, D + 2 * h, inb + 2 * h);
+                                        kRagged ? __float_as_uint(wh.w) : hbits, Z + 2 * h, D + 2 * h, inb + 2 * h, inv[h]);
         };
         auto test = [&](int h) {
           pair_test<kTwoSided, kFold>(Z + 2 * h, D + 2 * h, inb + 2 * h, thr, tau, bit, cm + 2 * h);
-          if (kSupport) pair_support<kFold>(Z + 2 * h, D + 2 * h, inb + 2 * h, stau, bit, sm + 2 * h);
+          if (kReproj)
+            pair_support<kFold, true>(Z + 2 * h, D + 2 * h, inb + 2 * h, stau, bit, sm + 2 * h, inv[h], d2[h], P2[h], Q2[h], s_epi[k], rho2);
+          else if (kSupport)
+            pair_support<kFold>(Z + 2 * h, D + 2 * h, inb + 2 * h, stau, bit, sm + 2 * h);
         };
         if (all_live) {
 #pragma unroll
@@ -816,11 +894,16 @@ static int fill_filter_params(const ddn_filter_config* cfg, const float* refined
   return DDN_OK;
 }
 
-// One K4 instantiation, plain (sp == nullptr) or with the support count.
+// One K4 instantiation: plain (sp == nullptr), with the support count, or with the support count and the reprojection
+// test (rp != nullptr).
 template <bool kBilinear, bool kStride1, bool kTwoSided, int kLayout, bool kRagged>
-static int launch_k4(const FilterParams& p, const SupportParams* sp, dim3 grid, const int64_t* layout, size_t smem,
-                     cudaStream_t st) {
-  if (sp == nullptr) {
+static int launch_k4(const FilterParams& p, const SupportParams* sp, const ReprojParams* rp, dim3 grid, const int64_t* layout,
+                     size_t smem, cudaStream_t st) {
+  if (rp != nullptr) {
+    auto* k = backproject_filter_kernel<kBilinear, kStride1, kTwoSided, kLayout, kRagged, ReprojParams>;
+    DDN_TRY(check_cuda(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute"));
+    k<<<grid, kFilterThreads, smem, st>>>(p, layout, *rp);
+  } else if (sp == nullptr) {
     auto* k = backproject_filter_kernel<kBilinear, kStride1, kTwoSided, kLayout, kRagged>;
     DDN_TRY(check_cuda(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute"));
     k<<<grid, kFilterThreads, smem, st>>>(p, layout);
@@ -833,19 +916,20 @@ static int launch_k4(const FilterParams& p, const SupportParams* sp, dim3 grid, 
 }
 
 // Launches the K4 instantiation cfg selects: the uniform kernel (layout == nullptr, grid = chunks x views) or the
-// ragged one (grid = all chunks of the layout); sp != nullptr: the support form.
-static int launch_filter(const ddn_filter_config* cfg, const FilterParams& p, const SupportParams* sp, dim3 grid,
-                         const int64_t* layout, cudaStream_t st) {
+// ragged one (grid = all chunks of the layout); sp != nullptr: the support form; rp != nullptr: the reprojection form.
+static int launch_filter(const ddn_filter_config* cfg, const FilterParams& p, const SupportParams* sp, const ReprojParams* rp,
+                         dim3 grid, const int64_t* layout, cudaStream_t st) {
   const int pl = cfg->pixel_layout;
-  const size_t smem = (size_t)(16 + p.K * DDN_PAIR_TABLE_FLOATS + (pl == 0 ? kFilterChunk * 3 : 0)) * sizeof(float);
+  const size_t smem = (size_t)(16 + p.K * (DDN_PAIR_TABLE_FLOATS + (rp != nullptr ? 4 : 0)) + (pl == 0 ? kFilterChunk * 3 : 0)) *
+                      sizeof(float);
   const bool bil = cfg->sample_mode == 1;
   const bool s1 = cfg->stride == 1;
   const bool two = cfg->two_sided_tau > 0.f;
   DDN_REQUIRE(two || cfg->depth_threshold > 0.f, "depth_threshold must be positive");
 #define DDN_LAUNCH_FILTER(B, S, T, L)                                                      \
   do {                                                                                     \
-    if (layout != nullptr) DDN_TRY((launch_k4<B, S, T, L, true>(p, sp, grid, layout, smem, st))); \
-    else DDN_TRY((launch_k4<B, S, T, L, false>(p, sp, grid, nullptr, smem, st)));          \
+    if (layout != nullptr) DDN_TRY((launch_k4<B, S, T, L, true>(p, sp, rp, grid, layout, smem, st))); \
+    else DDN_TRY((launch_k4<B, S, T, L, false>(p, sp, rp, grid, nullptr, smem, st)));      \
   } while (0)
 #define DDN_LAUNCH_FILTER_L(B, S, T)       \
   do {                                     \
@@ -876,8 +960,18 @@ static int check_support(const SupportParams* sp) {
   return DDN_OK;
 }
 
-// The two uniform entry points (sup: nullptr for ddn_backproject_filter).
-static int filter_uniform(const SupportParams* sup, const ddn_filter_config* cfg, int64_t n_views_total, int64_t src_begin,
+// The reprojection form's argument (reproj_px > 0, checked by its entry points: the form is on; 0: off) -> rp, or
+// nullptr when off.
+static int reproj_params(const SupportParams* sp, float reproj_px, ReprojParams& r, const ReprojParams*& rp) {
+  rp = nullptr;
+  if (reproj_px == 0.f) return DDN_OK;
+  r = ReprojParams{*sp, reproj_px * reproj_px};
+  rp = &r;
+  return DDN_OK;
+}
+
+// The three uniform entry points (sup: nullptr for ddn_backproject_filter; reproj_px: 0 but for the reprojection form).
+static int filter_uniform(const SupportParams* sup, float reproj_px, const ddn_filter_config* cfg, int64_t n_views_total, int64_t src_begin,
                           int64_t n_src, int64_t height, int64_t width, int64_t k_nbr, const float* refined_all,
                           const float* normal, const int32_t* nbr, const float* pair_table, const float* src_table,
                           int32_t vote_threshold, float* xyz, uint8_t* votes, float* bbox, const ddn_fuse_session* mark,
@@ -891,6 +985,9 @@ static int filter_uniform(const SupportParams* sup, const ddn_filter_config* cfg
   FilterParams p;
   DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
   DDN_TRY(check_support(sup));
+  ReprojParams rpv;
+  const ReprojParams* rp;
+  DDN_TRY(reproj_params(sup, reproj_px, rpv, rp));
   if (n_src == 0) return DDN_OK;
   p.src_begin = (int)src_begin;
   p.n_src = (int)n_src;
@@ -906,18 +1003,21 @@ static int filter_uniform(const SupportParams* sup, const ddn_filter_config* cfg
   const int Ps = p.Hs * p.Ws;
   dim3 grid((Ps + kFilterChunk - 1) / kFilterChunk, (unsigned)n_src);
   DDN_REQUIRE(n_src <= 65535, "too many source views per call");
-  DDN_TRY(launch_filter(cfg, p, sup, grid, nullptr, (cudaStream_t)stream));
+  DDN_TRY(launch_filter(cfg, p, sup, rp, grid, nullptr, (cudaStream_t)stream));
   return after_launch("backproject_filter_kernel");
 }
 
-// The two ragged entry points (sup: nullptr for ddn_backproject_filter_ragged).
-static int filter_ragged(const SupportParams* sup, const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
+// The three ragged entry points (sup: nullptr for ddn_backproject_filter_ragged; reproj_px as in filter_uniform).
+static int filter_ragged(const SupportParams* sup, float reproj_px, const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
                          const int64_t* layout, const int64_t* layout_host, const float* refined_all, const float* normal,
                          const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
                          uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
   FilterParams p;
   DDN_TRY(fill_filter_params(cfg, refined_all, normal, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, k_nbr, p));
   DDN_TRY(check_support(sup));
+  ReprojParams rpv;
+  const ReprojParams* rp;
+  DDN_TRY(reproj_params(sup, reproj_px, rpv, rp));
   DDN_REQUIRE(layout != nullptr, "null layout");
   DDN_TRY(check_layout(n_views, layout_host));
   DDN_REQUIRE(cfg->stride == layout_host[n_views * DDN_LAYOUT_COLS], "cfg->stride must be the layout's stride");
@@ -926,7 +1026,7 @@ static int filter_ragged(const SupportParams* sup, const ddn_filter_config* cfg,
   p.H = p.W = p.Hs = p.Ws = 0;  // per view, from the layout and the table entries
   p.wbits = p.hbits = 0;
   const int64_t chunks = layout_host[n_views * DDN_LAYOUT_COLS + 5];  // >= 1: every view has a pixel
-  DDN_TRY(launch_filter(cfg, p, sup, dim3((unsigned)chunks), layout, (cudaStream_t)stream));
+  DDN_TRY(launch_filter(cfg, p, sup, rp, dim3((unsigned)chunks), layout, (cudaStream_t)stream));
   return after_launch("backproject_filter_kernel");
 }
 
@@ -962,7 +1062,7 @@ int ddn_backproject_filter(const ddn_filter_config* cfg, int64_t n_views_total, 
                            const float* refined_all, const float* normal, const int32_t* nbr,
                            const float* pair_table, const float* src_table, int32_t vote_threshold,
                            float* xyz, uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
-  return ddn::filter_uniform(nullptr, cfg, n_views_total, src_begin, n_src, height, width, k_nbr, refined_all, normal, nbr,
+  return ddn::filter_uniform(nullptr, 0.f, cfg, n_views_total, src_begin, n_src, height, width, k_nbr, refined_all, normal, nbr,
                              pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, stream);
 }
 
@@ -973,8 +1073,21 @@ int ddn_backproject_filter_support(const ddn_filter_config* cfg, int64_t n_views
                                    float* xyz, uint8_t* votes, uint8_t* support, float* bbox,
                                    const ddn_fuse_session* mark, void* stream) {
   const ddn::SupportParams sup{support, min_support, support_tau};
-  return ddn::filter_uniform(&sup, cfg, n_views_total, src_begin, n_src, height, width, k_nbr, refined_all, normal, nbr,
+  return ddn::filter_uniform(&sup, 0.f, cfg, n_views_total, src_begin, n_src, height, width, k_nbr, refined_all, normal, nbr,
                              pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, stream);
+}
+
+int ddn_backproject_filter_support_reproj(const ddn_filter_config* cfg, int64_t n_views_total, int64_t src_begin,
+                                          int64_t n_src, int64_t height, int64_t width, int64_t k_nbr,
+                                          const float* refined_all, const float* normal, const int32_t* nbr,
+                                          const float* pair_table, const float* src_table, int32_t vote_threshold,
+                                          int32_t min_support, float support_tau, float reproj_px, float* xyz,
+                                          uint8_t* votes, uint8_t* support, float* bbox, const ddn_fuse_session* mark,
+                                          void* stream) {
+  DDN_REQUIRE(reproj_px > 0.f && isfinite(reproj_px), "reproj_px must be positive and finite");
+  const ddn::SupportParams sup{support, min_support, support_tau};
+  return ddn::filter_uniform(&sup, reproj_px, cfg, n_views_total, src_begin, n_src, height, width, k_nbr, refined_all, normal,
+                             nbr, pair_table, src_table, vote_threshold, xyz, votes, bbox, mark, stream);
 }
 
 int ddn_build_pair_tables_ragged(int64_t n_views, int64_t k_nbr, const int64_t* layout, const int64_t* layout_host,
@@ -995,7 +1108,7 @@ int ddn_backproject_filter_ragged(const ddn_filter_config* cfg, int64_t n_views,
                                   const int64_t* layout_host, const float* refined_all, const float* normal,
                                   const float* pair_table, const float* src_table, int32_t vote_threshold, float* xyz,
                                   uint8_t* votes, float* bbox, const ddn_fuse_session* mark, void* stream) {
-  return ddn::filter_ragged(nullptr, cfg, n_views, k_nbr, layout, layout_host, refined_all, normal, pair_table, src_table,
+  return ddn::filter_ragged(nullptr, 0.f, cfg, n_views, k_nbr, layout, layout_host, refined_all, normal, pair_table, src_table,
                             vote_threshold, xyz, votes, bbox, mark, stream);
 }
 
@@ -1006,8 +1119,20 @@ int ddn_backproject_filter_support_ragged(const ddn_filter_config* cfg, int64_t 
                                           uint8_t* votes, uint8_t* support, float* bbox, const ddn_fuse_session* mark,
                                           void* stream) {
   const ddn::SupportParams sup{support, min_support, support_tau};
-  return ddn::filter_ragged(&sup, cfg, n_views, k_nbr, layout, layout_host, refined_all, normal, pair_table, src_table,
+  return ddn::filter_ragged(&sup, 0.f, cfg, n_views, k_nbr, layout, layout_host, refined_all, normal, pair_table, src_table,
                             vote_threshold, xyz, votes, bbox, mark, stream);
+}
+
+int ddn_backproject_filter_support_reproj_ragged(const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
+                                                 const int64_t* layout, const int64_t* layout_host, const float* refined_all,
+                                                 const float* normal, const float* pair_table, const float* src_table,
+                                                 int32_t vote_threshold, int32_t min_support, float support_tau,
+                                                 float reproj_px, float* xyz, uint8_t* votes, uint8_t* support, float* bbox,
+                                                 const ddn_fuse_session* mark, void* stream) {
+  DDN_REQUIRE(reproj_px > 0.f && isfinite(reproj_px), "reproj_px must be positive and finite");
+  const ddn::SupportParams sup{support, min_support, support_tau};
+  return ddn::filter_ragged(&sup, reproj_px, cfg, n_views, k_nbr, layout, layout_host, refined_all, normal, pair_table,
+                            src_table, vote_threshold, xyz, votes, bbox, mark, stream);
 }
 
 }  // extern "C"

@@ -33,10 +33,31 @@ class DensifyConfig:
     # 0: count support (DensifyResult.support) without dropping anything.
     min_support: int | None = None
     support_tau: float = 0.01
+    # With min_support: a neighbour supports a point only when, besides, the round trip source -> neighbour -> source
+    # (MVSNet's forward-backward reprojection) lands within support_reproj_px pixels of the point's pixel.  None: no
+    # such test.
+    support_reproj_px: float | None = None
 
-    def support(self) -> tuple[int, float] | None:
-        """The ``support`` argument of ops.backproject_filter: (min_support, support_tau), or None when off."""
-        return None if self.min_support is None else (int(self.min_support), float(self.support_tau))
+    def __post_init__(self):
+        self._check_reproj()
+
+    def _check_reproj(self):
+        rho = self.support_reproj_px
+        if rho is None:
+            return
+        if self.min_support is None:
+            raise ValueError("support_reproj_px needs min_support")
+        if not (math.isfinite(float(rho)) and float(rho) > 0):
+            raise ValueError(f"support_reproj_px must be positive and finite, got {rho}")
+
+    def support(self) -> tuple[int, float] | tuple[int, float, float] | None:
+        """The ``support`` argument of ops.backproject_filter: (min_support, support_tau), with support_reproj_px
+        appended when set, or None when off."""
+        self._check_reproj()
+        if self.min_support is None:
+            return None
+        base = (int(self.min_support), float(self.support_tau))
+        return base if self.support_reproj_px is None else base + (float(self.support_reproj_px),)
 
     def vote_threshold_for(self, k: int) -> int:
         """The threshold a step with ``k`` neighbours per view votes with (``vote_threshold`` or ceil(k/2), clamped)."""

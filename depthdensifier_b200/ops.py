@@ -225,11 +225,19 @@ def decode_bbox(bbox: torch.Tensor) -> np.ndarray:
     return i.view(np.float32)
 
 
-def _support_args(support) -> tuple[int, float]:
-    m, tau = support
+def _support_args(support) -> tuple[int, float, float | None]:
+    """(min_support, tau, reproj_px or None) from ``support`` = (m, tau) or (m, tau, reproj_px)."""
+    if len(support) not in (2, 3):
+        raise ValueError(f"support = (min_support, tau) or (min_support, tau, reproj_px), got {support}")
+    m, tau = support[:2]
     if not (0 <= int(m) <= 1024) or not (math.isfinite(float(tau)) and float(tau) > 0):
         raise ValueError(f"support = (min_support in [0, 1024], tau > 0 finite), got {support}")
-    return int(m), float(tau)
+    rho = None
+    if len(support) == 3:
+        rho = float(support[2])
+        if not (math.isfinite(rho) and rho > 0):
+            raise ValueError(f"support = (min_support, tau, reproj_px > 0 finite), got {support}")
+    return int(m), float(tau), rho
 
 
 def fusion_threshold(vote_threshold: int, support: bool) -> int:
@@ -250,7 +258,9 @@ def backproject_filter(refined_all, normal, nbr, pair_table, src_table, src_begi
     ``support`` = (min_support, tau): also count the neighbours that see each point within the relative depth error
     tau and keep only points with at least min_support of them (ddn_backproject_filter_support).  Returns
     (xyz, votes, support) then, support [n_src,Hs,Ws] u8 (or ``support_out``); test the votes with
-    ``fusion_threshold(vote_threshold, True)``."""
+    ``fusion_threshold(vote_threshold, True)``.  ``support`` = (min_support, tau, reproj_px): a neighbour supports a
+    point only when, besides, the round trip source -> neighbour -> source lands within reproj_px pixels of the
+    point's pixel (ddn_backproject_filter_support_reproj)."""
     lib = _lib.load()
     dev = _require_cuda_normal(normal, refined_all, nbr, pair_table, src_table, bbox, xyz_out, votes_out)
     V, H, W = refined_all.shape
@@ -265,17 +275,17 @@ def backproject_filter(refined_all, normal, nbr, pair_table, src_table, src_begi
     votes = votes_out if votes_out is not None else torch.empty((n_src, Hs, Ws), dtype=torch.uint8, device=dev)
     cfg = opts.to_c()
     if support is not None:
-        m, tau = _support_args(support)
+        m, tau, rho = _support_args(support)
         sup = support_out if support_out is not None else torch.empty((n_src, Hs, Ws), dtype=torch.uint8, device=dev)
         assert sup.dtype == torch.uint8 and sup.is_contiguous() and tuple(sup.shape) == tuple(votes.shape)
+        head = (C.byref(cfg), V, src_begin, n_src, H, W, K, _p(refined_all), _p(normal), _p(nbr), _p(pair_table),
+                _p(src_table), int(vote_threshold), m, tau)
+        tail = (_p(xyz), _p(votes), _p(sup), _p(bbox), C.byref(mark.c) if mark is not None else None, _stream())
         with torch.cuda.device(dev):
-            _lib.check(
-                lib.ddn_backproject_filter_support(
-                    C.byref(cfg), V, src_begin, n_src, H, W, K, _p(refined_all), _p(normal), _p(nbr), _p(pair_table),
-                    _p(src_table), int(vote_threshold), m, tau, _p(xyz), _p(votes), _p(sup), _p(bbox),
-                    C.byref(mark.c) if mark is not None else None, _stream(),
-                )
-            )
+            if rho is None:
+                _lib.check(lib.ddn_backproject_filter_support(*head, *tail))
+            else:
+                _lib.check(lib.ddn_backproject_filter_support_reproj(*head, rho, *tail))
         return xyz, votes, sup
     with torch.cuda.device(dev):
         _lib.check(
@@ -447,17 +457,17 @@ def backproject_filter_ragged(layout: ViewLayout, refined_all, normal, pair_tabl
     votes = votes_out if votes_out is not None else torch.empty(G, dtype=torch.uint8, device=dev)
     cfg = opts.to_c()
     if support is not None:
-        m, tau = _support_args(support)
+        m, tau, rho = _support_args(support)
         sup = support_out if support_out is not None else torch.empty(G, dtype=torch.uint8, device=dev)
         assert sup.dtype == torch.uint8 and sup.is_contiguous() and tuple(sup.shape) == tuple(votes.shape)
+        head = (C.byref(cfg), V, K, _p(layout.device(dev)), layout.host_ptr(), _p(refined_all), _p(normal),
+                _p(pair_table), _p(src_table), int(vote_threshold), m, tau)
+        tail = (_p(xyz), _p(votes), _p(sup), _p(bbox), C.byref(mark.c) if mark is not None else None, _stream())
         with torch.cuda.device(dev):
-            _lib.check(
-                lib.ddn_backproject_filter_support_ragged(
-                    C.byref(cfg), V, K, _p(layout.device(dev)), layout.host_ptr(), _p(refined_all), _p(normal),
-                    _p(pair_table), _p(src_table), int(vote_threshold), m, tau, _p(xyz), _p(votes), _p(sup), _p(bbox),
-                    C.byref(mark.c) if mark is not None else None, _stream(),
-                )
-            )
+            if rho is None:
+                _lib.check(lib.ddn_backproject_filter_support_ragged(*head, *tail))
+            else:
+                _lib.check(lib.ddn_backproject_filter_support_reproj_ragged(*head, rho, *tail))
         return xyz, votes, sup
     with torch.cuda.device(dev):
         _lib.check(

@@ -87,6 +87,9 @@ class FilteringConfig:
     depth error); None = no such test (reference), 0 = count only."""
     support_tau: float = 0.01
     """new, with min_support: the relative depth error |z - D| <= support_tau * D within which a view supports a point."""
+    support_reproj_px: float | None = None
+    """new, with min_support: a view supports a point only when, besides, the round trip source -> view -> source
+    (forward-backward reprojection) lands within this many pixels of the point's pixel; None = no such test."""
 
 
 @dataclass
@@ -279,11 +282,12 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
                              adaptive_correspondences=rc.adaptive_correspondences, zero_unmasked_passthrough=True)
     filt = ops.FilterOptions(depth_threshold=config.filtering.depth_threshold, sample_mode=config.filtering.sample_mode,
                              stride=max(int(config.processing.downsample_density), 1))
-    ms = config.filtering.min_support
+    ms, rp = config.filtering.min_support, config.filtering.support_reproj_px
     eng = DensifyEngine(DensifyConfig(align=align, filter=filt, vote_threshold=int(config.filtering.vote_threshold),
                                       voxel=config.fusion.voxel_size, dedup_sparse=bool(config.fusion.dedup_sparse),
                                       min_support=None if ms is None else int(ms),
-                                      support_tau=float(config.filtering.support_tau)), device=dev)
+                                      support_tau=float(config.filtering.support_tau),
+                                      support_reproj_px=None if rp is None else float(rp)), device=dev)
     offsets = np.concatenate([[0], np.cumsum([len(p) for p in sparse])]).astype(np.int64)
     to = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(dev)
     maps = ((depths, torch.float32), (normals, torch.float32), (masks, torch.bool), (rgbs, torch.uint8))

@@ -17,12 +17,13 @@ from .synthetic import SceneConfig, make_scene
 
 def multi_gpu_check(dev, rank: int, world: int, n_views: int = 24, width: int = 320, height: int = 240, k: int = 4,
                     voxel: float = 0.02, steps: int = 2, verbose: bool = False, dedup: bool = False, dome_radius: float | None = None,
-                    max_grid_cells: int | None = None, min_support: int | None = None) -> dict:
+                    max_grid_cells: int | None = None, min_support: int | None = None,
+                    support_reproj_px: float | None = None) -> dict:
     """Every rank calls this.  Rank 0 returns {"passed": bool, "path": "peer" | "collective", ...}; the other
     ranks the same dict with their local view of ``path``.  ``dome_radius``: the scene gets a distant background
     (SceneConfig.dome_radius), ``max_grid_cells``: the sessions' bitmap capacity - either can send the step through the
     hashed fusion path (``report["grid"]`` says which path fused).  ``min_support``: DensifyConfig.min_support of both
-    pipelines (the support counts are then compared too)."""
+    pipelines (the support counts are then compared too); ``support_reproj_px``: their DensifyConfig.support_reproj_px."""
     V, W, H = n_views, width, height
     sc = make_scene(SceneConfig(n_views=V, width=W, height=H, n_sparse=1500, seed=4, dome_radius=dome_radius))  # host, identical on all ranks
     nbr = nearest_views_table(sc.cam_from_world.numpy(), k)
@@ -40,7 +41,7 @@ def multi_gpu_check(dev, rank: int, world: int, n_views: int = 24, width: int = 
                 "support": None if res.support is None else res.support.cpu().numpy()}
 
     def config(**kw):
-        cfg = DensifyConfig(voxel=voxel, dedup_sparse=dedup, min_support=min_support, **kw)
+        cfg = DensifyConfig(voxel=voxel, dedup_sparse=dedup, min_support=min_support, support_reproj_px=support_reproj_px, **kw)
         if max_grid_cells is not None:
             cfg.max_grid_cells = max_grid_cells
         return cfg
@@ -57,6 +58,8 @@ def multi_gpu_check(dev, rank: int, world: int, n_views: int = 24, width: int = 
     report = {"passed": True, "path": path, "ranks": world, "views": V, "size": [W, H], "steps": steps, "dedup_sparse": dedup, "different": []}
     if min_support is not None:
         report["min_support"] = min_support
+    if support_reproj_px is not None:
+        report["support_reproj_px"] = support_reproj_px
     if dome_radius is not None or max_grid_cells is not None:
         status = results[-1].session.grid_state().status if results[-1].session is not None else None
         report.update(dome_radius=dome_radius, max_grid_cells=max_grid_cells, grid={0: "dense", 4: "hashed"}.get(status, status))

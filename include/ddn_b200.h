@@ -190,6 +190,29 @@ DDN_API int ddn_backproject_filter_support(const ddn_filter_config* cfg, int64_t
                                    int32_t min_support, float support_tau, float* xyz, uint8_t* votes,
                                    uint8_t* support, float* bbox, const struct ddn_fuse_session* mark, void* stream);
 
+/* ddn_backproject_filter_support with a forward-backward reprojection check (new; parity unpinned: the reference has
+ * no such check).  For the point of source view s at pixel (x, y) with depth d, and neighbour entry t: (u, v, z) is its
+ * projection into t and D the sampled depth, both as for ddn_backproject_filter_support.  Back-project t's pixel at the
+ * CONTINUOUS coordinates (u, v) at depth D, take that point into s: pixel (x', y'), depth z'.  Continuous in both
+ * sampling modes: with bilinear sampling that is MVSNet's check; with nearest, back-projecting the truncated pixel
+ * would add up to sqrt(2) px of lookup error by itself, so the continuous point measures only the depth disagreement
+ * along the epipolar line.  Entry t SUPPORTS the point iff
+ *   the depth test of ddn_backproject_filter_support holds (in bounds, D > 0, |z - D| <= support_tau * D, not the
+ *   source view itself)  and  z' > 0  and  |(x', y') - (x, y)|_2 <= reproj_px.
+ * Closed form, which the kernel evaluates: with e = K_s (R_s c_t + t_s), t's epipole in s (homogeneous), P = d x,
+ * Q = d y and w = (z - D) / z,
+ *   z' = d + w (e_z - d),   (x' - x, y' - y) = w (d e_x - P e_z, d e_y - Q e_z) / (d z'),
+ * so the test is  z' > 0  and  w^2 [(d e_x - P e_z)^2 + (d e_y - Q e_z)^2] <= reproj_px^2 (d z')^2.
+ * reproj_px > 0 and finite.  The support byte, the keep rule and the vote encoding are those of
+ * ddn_backproject_filter_support, with "supports" meaning the combined test. */
+DDN_API int ddn_backproject_filter_support_reproj(const ddn_filter_config* cfg, int64_t n_views_total,
+                                          int64_t src_begin, int64_t n_src, int64_t height, int64_t width,
+                                          int64_t k_nbr, const float* refined_all, const float* normal,
+                                          const int32_t* nbr, const float* pair_table, const float* src_table,
+                                          int32_t vote_threshold, int32_t min_support, float support_tau,
+                                          float reproj_px, float* xyz, uint8_t* votes, uint8_t* support,
+                                          float* bbox, const struct ddn_fuse_session* mark, void* stream);
+
 DDN_API int ddn_bbox_init(float* bbox, void* stream);
 
 /* ------------------------------------------------------------------------------------------
@@ -250,6 +273,15 @@ DDN_API int ddn_backproject_filter_support_ragged(const ddn_filter_config* cfg, 
                                           const float* src_table, int32_t vote_threshold, int32_t min_support,
                                           float support_tau, float* xyz, uint8_t* votes, uint8_t* support,
                                           float* bbox, const struct ddn_fuse_session* mark, void* stream);
+
+/* ddn_backproject_filter_support_ragged with the reprojection check of ddn_backproject_filter_support_reproj. */
+DDN_API int ddn_backproject_filter_support_reproj_ragged(const ddn_filter_config* cfg, int64_t n_views, int64_t k_nbr,
+                                                 const int64_t* layout, const int64_t* layout_host,
+                                                 const float* refined_all, const float* normal,
+                                                 const float* pair_table, const float* src_table,
+                                                 int32_t vote_threshold, int32_t min_support, float support_tau,
+                                                 float reproj_px, float* xyz, uint8_t* votes, uint8_t* support,
+                                                 float* bbox, const struct ddn_fuse_session* mark, void* stream);
 
 /* Neighbouring per-pixel helpers (SURVEY.md 8(f) rank 4).
  * ddn_gradient_mask: compute_depth_normal_gradient_mask, src/depthdensifier/initilizer.py:236-328 - mask_out [H,W]

@@ -3,9 +3,11 @@
 reproduce the 1-rank pipeline bit for bit (depthdensifier_b200/selfcheck.py).  Rank 0 prints one JSON line.
 
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 \
-      scripts/check_multi_gpu.py [--min-support M]
+      scripts/check_multi_gpu.py [--min-support M [--support-reproj-px R]]
 
 --min-support M: run both checks with the multi-view support filter (DensifyConfig.min_support = M) as well.
+--support-reproj-px R: those support checks also with the forward-backward reprojection test
+(DensifyConfig.support_reproj_px = R).
 """
 
 import json
@@ -31,10 +33,13 @@ def main():
     ms = [None]
     if "--min-support" in sys.argv:
         ms.append(int(sys.argv[sys.argv.index("--min-support") + 1]))
+    rho = float(sys.argv[sys.argv.index("--support-reproj-px") + 1]) if "--support-reproj-px" in sys.argv else None
     reports = []
     for m in ms:
-        reports += [multi_gpu_check(dev, rank, world, min_support=m),
-                    multi_gpu_check(dev, rank, world, n_views=29, width=203, height=131, k=3, voxel=0.03, dedup=True, min_support=m)]
+        r = None if m is None else rho
+        reports += [multi_gpu_check(dev, rank, world, min_support=m, support_reproj_px=r),
+                    multi_gpu_check(dev, rank, world, n_views=29, width=203, height=131, k=3, voxel=0.03, dedup=True, min_support=m,
+                                    support_reproj_px=r)]
     if rank == 0:
         print(json.dumps({"multi_gpu_check": reports}))
     dist.barrier()

@@ -5,12 +5,17 @@ voxels), one B200, nearest sampling and bilinear as a second line:
   step   the whole DensifyEngine step, support off / m = 2 / m = 0
   kept   kept points (counts[0]) and voxels of each mode
 
+--arm reproj (writes profiles/r10_support_reproj.json): the forward-backward reprojection form instead,
+
+  k4     K4 with the fused mark: the support form (m = 2, tau = 0.01) against support + reprojection (rho = 1 px)
+  kept   kept points (counts[0]) and voxels of the step at rho in {0.5, 1, 2} and without the reprojection test
+
 Times are medians of N CUDA-event samples, the modes alternating sample by sample in one process.  The step's working set
 (>= 3.9 GB) is far larger than the 126 MB L2.  roofline_frac: algorithmic bytes of back-projection + consistency
 (29 + 4K = 61 B per valid pixel, as bench.py counts them) over the K4 time, against the HBM peak bench.py uses.  The
 card's name and power limit are read in the same call.
 
-  python scripts/gpu/support_bench.py [--samples 15] [--out profiles/r09_support.json]
+  python scripts/gpu/support_bench.py [--samples 15] [--arm support|reproj] [--out PATH]
 """
 
 from __future__ import annotations
@@ -115,18 +120,72 @@ def line(sc, nbr, sample_mode: str, samples: int) -> dict:
     return out
 
 
+def reproj_line(sc, nbr, sample_mode: str, samples: int) -> dict:
+    V, H, W = sc.mono_depth.shape
+    K = nbr.shape[1]
+    fopt = ops.FilterOptions(sample_mode=sample_mode)
+    inputs = (sc.mono_depth, sc.normal, sc.mask, sc.rgb, sc.cam_from_world, sc.intrinsics, sc.sparse_xyz, sc.sparse_offsets, nbr)
+    out = {"sample_mode": sample_mode, "min_support": 2, "kept": {}}
+    ref = None
+    for rho in (None, 0.5, 1.0, 2.0):
+        r = DensifyEngine(DensifyConfig(voxel=VOXEL, filter=fopt, min_support=2, support_tau=TAU, support_reproj_px=rho), "cuda").run(*inputs)
+        out["kept"]["support_only" if rho is None else f"rho_{rho:g}"] = {
+            "support_reproj_px": rho, "valid_pixels": r.num_points(), "kept_points": int(r.counts[0]), "voxels": r.check()}
+        ref = r if rho is None else ref
+    n_valid = out["kept"]["support_only"]["valid_pixels"]
+
+    # K4 with the fused mark on the step's refined maps and grid
+    pair, src = ops.build_pair_tables(sc.cam_from_world, sc.intrinsics, nbr, 0, V, H, W)
+    sess = ops.FuseSession(torch.device("cuda"))
+    grid = ref.host_grid()
+    xyz = torch.empty((V, H, W, 3), dtype=torch.float32, device="cuda")
+    votes = torch.empty((V, H, W), dtype=torch.uint8, device="cuda")
+    sup = torch.empty_like(votes)
+    bbox = ops.new_bbox(torch.device("cuda"))
+    thr = ref.vote_threshold
+
+    def k4(support):
+        return lambda: ops.backproject_filter(ref.refined, sc.normal, nbr, pair, src, 0, thr, fopt, bbox=bbox, xyz_out=xyz,
+                                              votes_out=votes, mark=sess, support=support, support_out=sup)
+
+    k4s = {"support_m2": k4((2, TAU)), "support_m2_reproj_1px": k4((2, TAU, 1.0))}
+    times = {k: [] for k in k4s}
+    for _ in range(3):  # warm-up of every shape
+        for f in k4s.values():
+            sess.begin_grid(grid)
+            f()
+    torch.cuda.synchronize()
+    for _ in range(samples):
+        for k, f in k4s.items():
+            sess.begin_grid(grid)
+            times[k].append(timed(f))
+    peak, src_peak = hbm_peak()
+    bpp = 29 + 4 * K
+    med = {k: float(np.median(v)) for k, v in times.items()}
+    out["k4_with_mark_ms"] = med
+    out["k4_ratio_reproj_over_support"] = med["support_m2_reproj_1px"] / med["support_m2"]
+    out["k4_spread_ms"] = {k: [float(np.min(v)), float(np.max(v))] for k, v in times.items()}
+    out["roofline_frac"] = {k: bpp * n_valid / (ms * 1e-3) / 1e9 / peak for k, ms in med.items()}
+    out["roofline"] = {"algorithmic_bytes_per_pixel": bpp, "peak_gbs": peak, "peak_source": src_peak, "pixels": n_valid}
+    return out
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--samples", type=int, default=15)
-    ap.add_argument("--out", default="profiles/r09_support.json")
+    ap.add_argument("--arm", choices=("support", "reproj"), default="support")
+    ap.add_argument("--out", default=None, help="default: profiles/r09_support.json, or profiles/r10_support_reproj.json")
     args = ap.parse_args()
+    if args.out is None:
+        args.out = "profiles/r09_support.json" if args.arm == "support" else "profiles/r10_support_reproj.json"
     if not torch.cuda.is_available():
         raise SystemExit("support_bench needs a CUDA device")
     V, W, H, K, C, desc = WORKLOADS["cfg2"]
     sc = make_scene(SceneConfig(n_views=V, width=W, height=H, n_sparse=C, seed=0), device="cuda")
     nbr = torch.from_numpy(nearest_views_table(sc.cam_from_world.cpu().numpy(), K).astype(np.int32)).cuda()
+    fn = line if args.arm == "support" else reproj_line
     res = {"card": card(), "workload": desc, "support_tau": TAU, "samples": args.samples,
-           "lines": [line(sc, nbr, m, args.samples) for m in ("nearest", "bilinear")]}
+           "lines": [fn(sc, nbr, m, args.samples) for m in ("nearest", "bilinear")]}
     res["card_after"] = card()
     print(json.dumps(res))
     Path(args.out).parent.mkdir(parents=True, exist_ok=True)
