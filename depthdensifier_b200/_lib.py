@@ -160,7 +160,14 @@ SYMBOLS = {
     "ddn_transform_normals": (C.c_int, [_i64, _vp, C.POINTER(C.c_double), _i32, _vp, _vp]),
     "ddn_project_points": (C.c_int, [_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ddn_unproject_points": (C.c_int, [_i64, _vp, _vp, C.POINTER(C.c_double), _vp, _vp]),
+    "ddn_point_normals": (C.c_int, [_i64, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "ddn_point_normals_ragged": (C.c_int, [_i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ddn_fuse_workspace_bytes": (C.c_int, [C.POINTER(VoxelGrid), _i64, C.POINTER(_i64)]),
+    "ddn_fuse_normals_workspace_bytes": (C.c_int, [C.POINTER(VoxelGrid), _i64, C.POINTER(_i64)]),
+    "ddn_voxel_fuse_normals": (
+        C.c_int,
+        [C.POINTER(VoxelGrid), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
+    ),
     "ddn_voxel_fuse": (
         C.c_int,
         [C.POINTER(VoxelGrid), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
@@ -186,6 +193,10 @@ SYMBOLS = {
         C.c_int,
         [C.POINTER(FuseSession), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
     ),
+    "ddn_fuse_finish_normals": (
+        C.c_int,
+        [C.POINTER(FuseSession), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
+    ),
     "ddn_fuse_finish_partial": (C.c_int, [C.POINTER(FuseSession), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i64, _vp]),
     "ddn_fuse_merge_peers": (
         C.c_int,
@@ -198,6 +209,11 @@ SYMBOLS = {
         C.c_int,
         [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i64,
          _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
+    ),
+    "ddn_fuse_finish_hashed_normals": (
+        C.c_int,
+        [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _i64,
+         _vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
     ),
     "ddn_fuse_finish_hashed_partial": (
         C.c_int,

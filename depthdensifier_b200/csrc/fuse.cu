@@ -25,6 +25,7 @@
 // file - runs without the host looking at any intermediate result.
 // The host-grid entry points fuse grids of more than 2^35 cells with the hashed path (fuse_hash.cu).
 #include <algorithm>
+#include <type_traits>
 
 #include "fuse_hash.cuh"
 
@@ -461,11 +462,20 @@ __device__ __forceinline__ uint32_t slot_of_cell(uint64_t cell, const uint4* __r
 constexpr int kAccTilesPerWarp = DDN_ACC_TPW;
 constexpr int kAccTileW = 16;  // pixel tile of a warp: 16 x 2 (measured at cfg 2: 4 x 8 4.46, 8 x 4 4.35, 16 x 2 4.34, 32 x 1 4.54 ms)
 
-template <int kTW>  // tile width in pixels (tile = kTW x 32/kTW); 0 = no row structure, 32 consecutive points
+// The normals form (Normal = const float*, the plain form has no trailing parameter): every point also adds its
+// quantised normal (normal_fix; normal [n,3] f32 in the order of xyz) - three more 32-bit words in the shuffle walk and
+// three more REDs from the group leader, at accumulator words 5..7 (stride kAccNormalWords).
+template <int kTW, class... Normal>  // tile width in pixels (tile = kTW x 32/kTW); 0 = no row structure, 32 consecutive points
 __global__ void __launch_bounds__(256)
 accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len, const float* __restrict__ xyz,
                          const uint8_t* __restrict__ rgb, const uint8_t* __restrict__ votes, int thr,
-                         const uint4* __restrict__ units, unsigned long long* __restrict__ accum, int stride, long long cap) {
+                         const uint4* __restrict__ units, unsigned long long* __restrict__ accum, int stride, long long cap,
+                         Normal... normal_in) {
+  constexpr bool kNormals = sizeof...(Normal) != 0;
+  const float* __restrict__ normal = normal_arg(normal_in...);
+#if defined(DDN_ACC_REDUX) || defined(DDN_ACC_DEFER)
+  static_assert(!kNormals, "the DDN_ACC_REDUX / DDN_ACC_DEFER experiments have no normals form");
+#endif
   const GridDev g = *gp;
   if (g.n_units == 0) return;
   const float rv = 1.0f / g.voxel;
@@ -494,11 +504,15 @@ accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len,
   }
   // The point of the NEXT tile is loaded (vote, position and colour at once - no dependent round trips)
   // before the current tile is processed, so its latency hides behind the aggregation and the atomics.
-  struct In {
+  struct InBase {
     float x, y, z;
     uint32_t rg, bb;
     bool take;
   };
+  struct InNormal : InBase {
+    float nx, ny, nz;
+  };
+  using In = std::conditional_t<kNormals, InNormal, InBase>;
   auto load_tile = [&](uint32_t t) -> In {
     int64_t i;
     bool in;
@@ -511,13 +525,14 @@ accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len,
       i = (int64_t)t * 32 + lane;
       in = i < n;
     }
-    In r = {0.f, 0.f, 0.f, 0u, 0u, false};
+    In r{};
     if (in) {
       const int v = votes != nullptr ? (int)__ldg(votes + i) : 0;
       r.x = __ldg(xyz + i * 3 + 0), r.y = __ldg(xyz + i * 3 + 1), r.z = __ldg(xyz + i * 3 + 2);
       r.rg = ((uint32_t)__ldg(rgb + i * 3 + 0) << 16) | (uint32_t)__ldg(rgb + i * 3 + 1);
       r.bb = (uint32_t)__ldg(rgb + i * 3 + 2);
       r.take = v < thr || votes == nullptr;
+      if constexpr (kNormals) r.nx = __ldg(normal + i * 3 + 0), r.ny = __ldg(normal + i * 3 + 1), r.nz = __ldg(normal + i * 3 + 2);
     }
     return r;
   };
@@ -565,12 +580,17 @@ accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len,
     const bool leader = valid && (__ffs(peers) - 1) == lane;
     int sx = 0, sy = 0, sz = 0;
     uint32_t srg = 0, sb = 0;
+    int snx = 0, sny = 0, snz = 0;  // kNormals
 #ifndef DDN_ACC_REDUX
     // Three shuffles per step of the walk instead of five: a word per axis holds the offset (|offset| <= 2^19 + 1, far
     // inside 24 signed bits) above one colour byte.  s* sums the offsets (arithmetic shift), t* the whole words modulo
     // 2^32, so a colour sum is t - (s << 8), exact because it is at most 32 * 255 < 2^13.
     const uint32_t wx = ((uint32_t)ox << 8) | (rg >> 16), wy = ((uint32_t)oy << 8) | (rg & 0xffffu), wz = ((uint32_t)oz << 8) | bb;
     uint32_t tx = 0, ty = 0, tz = 0;
+    int qx = 0, qy = 0, qz = 0;
+    if constexpr (kNormals) {
+      if (valid) qx = normal_fix(cur.nx), qy = normal_fix(cur.ny), qz = normal_fix(cur.nz);
+    }
     const int iters = __reduce_max_sync(0xffffffffu, __popc(peers));
     uint32_t rest = peers;
 #pragma unroll 1
@@ -583,6 +603,10 @@ accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len,
       if (has) {
         sx += (int)ax >> 8, sy += (int)ay >> 8, sz += (int)az >> 8;
         tx += ax, ty += ay, tz += az;
+      }
+      if constexpr (kNormals) {
+        const int bx = __shfl_sync(0xffffffffu, qx, src), by = __shfl_sync(0xffffffffu, qy, src), bz = __shfl_sync(0xffffffffu, qz, src);
+        if (has) snx += bx, sny += by, snz += bz;
       }
     }
     srg = ((tx - ((uint32_t)sx << 8)) << 16) | (ty - ((uint32_t)sy << 8));
@@ -606,6 +630,11 @@ accumulate_points_kernel(const GridDev* __restrict__ gp, int64_t n, int row_len,
         atomicAdd(a + 2, (unsigned long long)(long long)sz);
         atomicAdd(a + 3, ((unsigned long long)(srg >> 16) << 32) | (srg & 0xffffu));
         atomicAdd(a + 4, ((unsigned long long)sb << 32) | (unsigned)__popc(peers));
+        if constexpr (kNormals) {
+          atomicAdd(a + 5, (unsigned long long)(long long)snx);
+          atomicAdd(a + 6, (unsigned long long)(long long)sny);
+          atomicAdd(a + 7, (unsigned long long)(long long)snz);
+        }
       }
     }
   }
@@ -645,14 +674,17 @@ accumulate_records_kernel(const GridDev* __restrict__ gp, int64_t n, const unsig
 
 // One thread per voxel.  The colour fields are 32 bits wide: a voxel with 2^24 or more points could
 // have overflowed them, which is reported (counts[0] = -1) instead of returned as a wrong colour.
-__global__ void __launch_bounds__(256)
-finalize_kernel(const GridDev* __restrict__ gp, const unsigned long long* __restrict__ accum, const uint64_t* __restrict__ keys,
-                long long* __restrict__ counts, long long cap, float* __restrict__ out_xyz, uint8_t* __restrict__ out_rgb,
-                int32_t* __restrict__ out_count) {
+// kNormals (finalize_normals_kernel): accumulators of kAccNormalWords words, whose normal sums finalize_normal turns into
+// out_normal.
+template <bool kNormals>
+__device__ __forceinline__ void finalize_body(const GridDev* __restrict__ gp, const unsigned long long* __restrict__ accum,
+                                              const uint64_t* __restrict__ keys, long long* __restrict__ counts, long long cap,
+                                              float* __restrict__ out_xyz, uint8_t* __restrict__ out_rgb, int32_t* __restrict__ out_count,
+                                              float* __restrict__ out_normal) {
   const GridDev g = *gp;
   const long long mv = min(counts[1], cap);
   for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < mv; r += (long long)gridDim.x * blockDim.x) {
-    const unsigned long long* a = accum + (size_t)r * kAccWords;
+    const unsigned long long* a = accum + (size_t)r * (kNormals ? kAccNormalWords : kAccWords);
     const long long sx = (long long)a[0], sy = (long long)a[1], sz = (long long)a[2];
     const unsigned long long rg = a[3], bn = a[4];
     const uint32_t cnt = (uint32_t)bn;
@@ -662,7 +694,22 @@ finalize_kernel(const GridDev* __restrict__ gp, const unsigned long long* __rest
     const uint32_t kx = (uint32_t)(key & 0x1fffff), ky = (uint32_t)((key >> 21) & 0x1fffff), kz = (uint32_t)((key >> 42) & 0x1fffff);
     finalize_voxel(g, voxel_centre(g.ox, kx, g.voxel), voxel_centre(g.oy, ky, g.voxel), voxel_centre(g.oz, kz, g.voxel), sx, sy, sz,
                    rg >> 32, rg & 0xffffffffull, bn >> 32, (long long)cnt, out_xyz + r * 3, out_rgb + r * 3);
+    if constexpr (kNormals) finalize_normal((long long)a[5], (long long)a[6], (long long)a[7], out_normal + r * 3);
   }
+}
+
+__global__ void __launch_bounds__(256)
+finalize_kernel(const GridDev* __restrict__ gp, const unsigned long long* __restrict__ accum, const uint64_t* __restrict__ keys,
+                long long* __restrict__ counts, long long cap, float* __restrict__ out_xyz, uint8_t* __restrict__ out_rgb,
+                int32_t* __restrict__ out_count) {
+  finalize_body<false>(gp, accum, keys, counts, cap, out_xyz, out_rgb, out_count, nullptr);
+}
+
+__global__ void __launch_bounds__(256)
+finalize_normals_kernel(const GridDev* __restrict__ gp, const unsigned long long* __restrict__ accum, const uint64_t* __restrict__ keys,
+                        long long* __restrict__ counts, long long cap, float* __restrict__ out_xyz, uint8_t* __restrict__ out_rgb,
+                        int32_t* __restrict__ out_count, float* __restrict__ out_normal) {
+  finalize_body<true>(gp, accum, keys, counts, cap, out_xyz, out_rgb, out_count, out_normal);
 }
 
 __global__ void canonical_key_kernel(GridDev g, int64_t n, const float* __restrict__ xyz, uint64_t* __restrict__ keys) {
@@ -942,9 +989,10 @@ static int launch_rank(const ddn_fuse_session* s, ScanRange range, uint64_t* key
   return after_launch("unit_prefix_kernel", st);
 }
 
+// normal != nullptr: the normals form (accumulators of kAccNormalWords words)
 static int launch_accumulate_points(const ddn_fuse_session* s, int64_t n, int64_t row_len, const float* xyz, const uint8_t* rgb,
                                     const uint8_t* votes, int thr, unsigned long long* accum, int stride, long long cap,
-                                    cudaStream_t st) {
+                                    cudaStream_t st, const float* normal = nullptr) {
   const GridDev* gp = reinterpret_cast<const GridDev*>(s->grid);
   const uint4* units = reinterpret_cast<const uint4*>(s->units);
   const bool tiled = row_len >= 32 && row_len < (1 << 30);
@@ -952,6 +1000,20 @@ static int launch_accumulate_points(const ddn_fuse_session* s, int64_t n, int64_
   const int th = tw ? 32 / tw : 1, twe = tw ? tw : 32;
   const int64_t n_tiles = tiled ? ((row_len + twe - 1) / twe) * (((n + row_len - 1) / row_len + th - 1) / th) : (n + 31) / 32;
   const unsigned ablocks = (unsigned)((n_tiles + 8 * kAccTilesPerWarp - 1) / (8 * kAccTilesPerWarp));
+  if (normal != nullptr) {
+#if defined(DDN_ACC_REDUX) || defined(DDN_ACC_DEFER)
+    set_error("the DDN_ACC_REDUX / DDN_ACC_DEFER builds have no fused-normals form");
+    return DDN_ERR_UNSUPPORTED;
+#else
+    if (tiled)
+      accumulate_points_kernel<kAccTileW, const float*><<<ablocks, 256, 0, st>>>(gp, n, (int)row_len, xyz, rgb, votes, thr, units, accum,
+                                                                                stride, cap, normal);
+    else
+      accumulate_points_kernel<0, const float*><<<ablocks, 256, 0, st>>>(gp, n, (int)row_len, xyz, rgb, votes, thr, units, accum, stride,
+                                                                        cap, normal);
+    return after_launch("accumulate_points_kernel", st);
+#endif
+  }
   if (tiled)
     accumulate_points_kernel<kAccTileW><<<ablocks, 256, 0, st>>>(gp, n, (int)row_len, xyz, rgb, votes, thr, units, accum, stride, cap);
   else
@@ -960,7 +1022,13 @@ static int launch_accumulate_points(const ddn_fuse_session* s, int64_t n, int64_
 }
 
 static int launch_finalize(const ddn_fuse_session* s, const unsigned long long* accum, const uint64_t* keys, long long cap,
-                           float* out_xyz, uint8_t* out_rgb, int32_t* out_count, cudaStream_t st) {
+                           float* out_xyz, uint8_t* out_rgb, int32_t* out_count, cudaStream_t st, float* out_normal = nullptr) {
+  if (out_normal != nullptr) {
+    finalize_normals_kernel<<<kPersistentCtas, 256, 0, st>>>(reinterpret_cast<const GridDev*>(s->grid), accum, keys,
+                                                             reinterpret_cast<long long*>(s->counts), cap, out_xyz, out_rgb, out_count,
+                                                             out_normal);
+    return after_launch("finalize_normals_kernel", st);
+  }
   finalize_kernel<<<kPersistentCtas, 256, 0, st>>>(reinterpret_cast<const GridDev*>(s->grid), accum, keys,
                                                    reinterpret_cast<long long*>(s->counts), cap, out_xyz, out_rgb, out_count);
   return after_launch("finalize_kernel", st);
@@ -982,7 +1050,8 @@ struct WorkspaceOffsets {
   }
 };
 
-static void dense_layout(const GridDev& g, int64_t n, DenseLayout* L) {  // sized for the non-partial form
+// sized for the non-partial form; words: accumulator words per voxel (kAccWords, or kAccNormalWords for the normals form)
+static void dense_layout(const GridDev& g, int64_t n, DenseLayout* L, int words = kAccWords) {
   L->cells = grid_cells(g);
   L->n_units = (L->cells + kUnitBits - 1) / kUnitBits;
   L->tiles = (L->n_units + kTileUnits - 1) / kTileUnits;
@@ -992,13 +1061,13 @@ static void dense_layout(const GridDev& g, int64_t n, DenseLayout* L) {  // size
   L->grid = o.take(sizeof(GridDev));
   L->units = o.take((size_t)L->n_units * 16);
   L->tile_sums = o.take((size_t)(L->own_tiles + 2) * 4);
-  L->accum = o.take((size_t)max_vox * kAccWords * 8 + 16);
+  L->accum = o.take((size_t)max_vox * words * 8 + 16);
   L->total = o.off + 256;
 }
 
 static int carve_session(const GridDev& g, int64_t n, void* workspace, int64_t workspace_bytes, ddn_fuse_session* s,
-                         int64_t* counts_out, unsigned long long** accum, DenseLayout* L) {
-  dense_layout(g, n, L);
+                         int64_t* counts_out, unsigned long long** accum, DenseLayout* L, int words = kAccWords) {
+  dense_layout(g, n, L, words);
   if ((int64_t)L->total > workspace_bytes) {
     set_error("fuse workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)L->total);
     return DDN_ERR_WORKSPACE_TOO_SMALL;
@@ -1034,12 +1103,13 @@ struct HashedWork {
   int64_t scratch_bytes;
 };
 
-// Bytes of the layout for n > 0 points; with a (256-byte aligned) base also the pointers into it.
-static int hashed_layout(int64_t n, char* base, HashedWork* w, int64_t* total) {
+// Bytes of the layout for n > 0 points; with a (256-byte aligned) base also the pointers into it.  words: accumulator
+// words per point (kAccWords, or kAccNormalWords for the normals form).
+static int hashed_layout(int64_t n, char* base, HashedWork* w, int64_t* total, int words = kAccWords) {
   int64_t cap_slots, table_bytes, slots_bytes, sort_bytes, hist_bytes, merge_bytes;
   DDN_TRY(ddn_hash_fuse_sizes(n, &cap_slots, &table_bytes, &slots_bytes, &sort_bytes, &hist_bytes));
   DDN_TRY(ddn_fuse_merge_hashed_scratch_bytes(1, n, &merge_bytes));
-  const int64_t scratch_bytes = std::max<int64_t>(n * kAccWords * 8 + 16, merge_bytes);
+  const int64_t scratch_bytes = std::max<int64_t>(n * words * 8 + 16, merge_bytes);
   WorkspaceOffsets o;
   const size_t grid = o.take(sizeof(GridDev)), table = o.take(table_bytes), slots = o.take(slots_bytes),
                sort = o.take(sort_bytes), hist = o.take(hist_bytes), state = o.take(DDN_HASH_STATE_BYTES),
@@ -1065,9 +1135,9 @@ static int hashed_layout(int64_t n, char* base, HashedWork* w, int64_t* total) {
 // Checks the workspace before anything is enqueued, then stores the grid with cap_units = 0, i.e. as
 // DDN_GRID_TOO_LARGE (the status on which the hashed path's mode 0 runs), and empties the hash buffers.
 static int carve_hashed(const GridDev& g, int64_t n, void* workspace, int64_t workspace_bytes, int64_t* counts_out, HashedWork* w,
-                        cudaStream_t st) {
+                        cudaStream_t st, int words = kAccWords) {
   int64_t total = 0;
-  DDN_TRY(hashed_layout(n, reinterpret_cast<char*>(align_up((int64_t)(uintptr_t)workspace, 256)), w, &total));
+  DDN_TRY(hashed_layout(n, reinterpret_cast<char*>(align_up((int64_t)(uintptr_t)workspace, 256)), w, &total, words));
   if (total > workspace_bytes) {
     set_error("fuse workspace too small: %lld < %lld", (long long)workspace_bytes, (long long)total);
     return DDN_ERR_WORKSPACE_TOO_SMALL;
@@ -1078,12 +1148,7 @@ static int carve_hashed(const GridDev& g, int64_t n, void* workspace, int64_t wo
   return ddn_hash_fuse_reset(&w->hf, st);
 }
 
-}  // namespace ddn
-
-extern "C" {
-
-int ddn_fuse_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t* bytes_out) {
-  using namespace ddn;
+static int fuse_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t* bytes_out, int words) {
   DDN_REQUIRE(bytes_out != nullptr, "null bytes_out");
   DDN_REQUIRE(n_points >= 0 && n_points < (1ll << 31) - 1024, "n_points");
   const int64_t n = n_points > 0 ? n_points : 1;
@@ -1092,45 +1157,99 @@ int ddn_fuse_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, 
     DDN_TRY(grid_from_host(grid_host, &g));
     if (use_dense(g)) {
       DenseLayout L;
-      dense_layout(g, n, &L);
+      dense_layout(g, n, &L, words);
       *bytes_out = (int64_t)L.total;
       return DDN_OK;
     }
   }
   HashedWork w;
-  return hashed_layout(n, nullptr, &w, bytes_out);
+  return hashed_layout(n, nullptr, &w, bytes_out, words);
 }
 
-int ddn_voxel_fuse(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
-                   const uint8_t* votes, int32_t vote_threshold, uint64_t* out_keys, float* out_xyz,
-                   uint8_t* out_rgb, int32_t* out_count, int64_t* counts_out, void* workspace,
-                   int64_t workspace_bytes, void* stream) {
-  using namespace ddn;
+// ddn_voxel_fuse, and with normal / out_normal its normals form
+static int voxel_fuse(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                      const uint8_t* votes, int32_t vote_threshold, const float* normal, uint64_t* out_keys, float* out_xyz,
+                      uint8_t* out_rgb, int32_t* out_count, float* out_normal, int64_t* counts_out, void* workspace,
+                      int64_t workspace_bytes, cudaStream_t st) {
+  const bool normals = normal != nullptr;
+  const int words = normals ? kAccNormalWords : kAccWords;
   GridDev g;
   DDN_TRY(grid_from_host(grid_host, &g));
   DDN_REQUIRE(n_points >= 0 && n_points < (1ll << 31) - 1024, "n_points");
   DDN_REQUIRE(row_len >= 0, "row_len");
   DDN_REQUIRE(counts_out != nullptr, "null counts_out");
-  cudaStream_t st = (cudaStream_t)stream;
   vote_threshold = std::min(vote_threshold, 255);
   if (n_points == 0) return check_cuda(cudaMemsetAsync(counts_out, 0, 16, st), "memset counts");
   DDN_REQUIRE(xyz && rgb && out_keys && out_xyz && out_rgb && out_count && workspace, "null pointer");
   if (!use_dense(g)) {
     HashedWork w;
-    DDN_TRY(carve_hashed(g, n_points, workspace, workspace_bytes, counts_out, &w, st));
+    DDN_TRY(carve_hashed(g, n_points, workspace, workspace_bytes, counts_out, &w, st, words));
+    if (normals)
+      return ddn_fuse_finish_hashed_normals(&w.s, &w.hf, 0, n_points, row_len, xyz, rgb, votes, vote_threshold, normal, nullptr, 0,
+                                            out_keys, out_xyz, out_rgb, out_count, out_normal, n_points, w.scratch, w.scratch_bytes, st);
     return ddn_fuse_finish_hashed(&w.s, &w.hf, 0, n_points, row_len, xyz, rgb, votes, vote_threshold, nullptr, 0, out_keys, out_xyz,
                                   out_rgb, out_count, n_points, w.scratch, w.scratch_bytes, st);
   }
   ddn_fuse_session s;
   unsigned long long* accum;
   DenseLayout L;
-  DDN_TRY(carve_session(g, n_points, workspace, workspace_bytes, &s, counts_out, &accum, &L));
+  DDN_TRY(carve_session(g, n_points, workspace, workspace_bytes, &s, counts_out, &accum, &L, words));
   DDN_TRY(begin_with_grid(&s, g, st));
   DDN_TRY(launch_mark_points(&s, n_points, xyz, votes, vote_threshold, st));
   const long long cap = (long long)std::min<uint64_t>((uint64_t)n_points, L.cells);
-  DDN_TRY(launch_rank(&s, ScanRange{0, -1}, out_keys, 1, accum, kAccWords, cap, nullptr, st));
-  DDN_TRY(launch_accumulate_points(&s, n_points, row_len, xyz, rgb, votes, vote_threshold, accum, kAccWords, cap, st));
-  return launch_finalize(&s, accum, out_keys, cap, out_xyz, out_rgb, out_count, st);
+  DDN_TRY(launch_rank(&s, ScanRange{0, -1}, out_keys, 1, accum, words, cap, nullptr, st));
+  DDN_TRY(launch_accumulate_points(&s, n_points, row_len, xyz, rgb, votes, vote_threshold, accum, words, cap, st, normal));
+  return launch_finalize(&s, accum, out_keys, cap, out_xyz, out_rgb, out_count, st, out_normal);
+}
+
+// ddn_fuse_finish, and with normal / out_normal its normals form
+static int fuse_finish(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                       const uint8_t* votes, int32_t vote_threshold, const float* normal, uint64_t* out_keys, float* out_xyz,
+                       uint8_t* out_rgb, int32_t* out_count, float* out_normal, int64_t cap_out, void* accum, int64_t accum_bytes,
+                       cudaStream_t st) {
+  const int words = out_normal != nullptr ? kAccNormalWords : kAccWords;
+  DDN_TRY(session_check(s));
+  DDN_REQUIRE(n_points >= 0 && n_points < (1ll << 31) - 1024, "n_points");
+  DDN_REQUIRE(row_len >= 0, "row_len");
+  DDN_REQUIRE(cap_out > 0 && cap_out < (1ll << 31), "cap_out");
+  DDN_REQUIRE(out_keys && out_xyz && out_rgb && out_count && accum, "null pointer");
+  DDN_REQUIRE(accum_bytes >= cap_out * words * 8 + 16 && (uintptr_t)accum % 16 == 0, "accumulator scratch");
+  DDN_REQUIRE(n_points == 0 || (xyz && rgb), "null pointer");
+  vote_threshold = std::min(vote_threshold, 255);
+  unsigned long long* acc = (unsigned long long*)accum;
+  DDN_TRY(launch_rank(s, ScanRange{0, -1}, out_keys, 1, acc, words, cap_out, nullptr, st));
+  if (n_points > 0)
+    DDN_TRY(launch_accumulate_points(s, n_points, row_len, xyz, rgb, votes, vote_threshold, acc, words, cap_out, st, normal));
+  return launch_finalize(s, acc, out_keys, cap_out, out_xyz, out_rgb, out_count, st, out_normal);
+}
+
+}  // namespace ddn
+
+extern "C" {
+
+int ddn_fuse_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t* bytes_out) {
+  return ddn::fuse_workspace_bytes(grid_host, n_points, bytes_out, ddn::kAccWords);
+}
+
+int ddn_fuse_normals_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t* bytes_out) {
+  return ddn::fuse_workspace_bytes(grid_host, n_points, bytes_out, ddn::kAccNormalWords);
+}
+
+int ddn_voxel_fuse(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                   const uint8_t* votes, int32_t vote_threshold, uint64_t* out_keys, float* out_xyz,
+                   uint8_t* out_rgb, int32_t* out_count, int64_t* counts_out, void* workspace,
+                   int64_t workspace_bytes, void* stream) {
+  return ddn::voxel_fuse(grid_host, n_points, row_len, xyz, rgb, votes, vote_threshold, nullptr, out_keys, out_xyz, out_rgb, out_count,
+                         nullptr, counts_out, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int ddn_voxel_fuse_normals(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                           const uint8_t* votes, int32_t vote_threshold, const float* normal, uint64_t* out_keys, float* out_xyz,
+                           uint8_t* out_rgb, int32_t* out_count, float* out_normal, int64_t* counts_out, void* workspace,
+                           int64_t workspace_bytes, void* stream) {
+  DDN_REQUIRE(n_points == 0 || (normal && out_normal), "null pointer");
+  return ddn::voxel_fuse(grid_host, n_points, row_len, xyz, rgb, votes, vote_threshold, normal, out_keys, out_xyz, out_rgb, out_count,
+                         out_normal, counts_out, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int ddn_fuse_tile_info(const ddn_voxel_grid* grid_host, int64_t* n_tiles, int64_t* cells_per_tile) {
@@ -1348,21 +1467,17 @@ int ddn_fuse_unmark_points(const ddn_fuse_session* s, int64_t n_points, const fl
 int ddn_fuse_finish(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
                     const uint8_t* votes, int32_t vote_threshold, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
                     int32_t* out_count, int64_t cap_out, void* accum, int64_t accum_bytes, void* stream) {
-  using namespace ddn;
-  DDN_TRY(session_check(s));
-  DDN_REQUIRE(n_points >= 0 && n_points < (1ll << 31) - 1024, "n_points");
-  DDN_REQUIRE(row_len >= 0, "row_len");
-  DDN_REQUIRE(cap_out > 0 && cap_out < (1ll << 31), "cap_out");
-  DDN_REQUIRE(out_keys && out_xyz && out_rgb && out_count && accum, "null pointer");
-  DDN_REQUIRE(accum_bytes >= cap_out * kAccWords * 8 + 16 && (uintptr_t)accum % 16 == 0, "accumulator scratch");
-  DDN_REQUIRE(n_points == 0 || (xyz && rgb), "null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  vote_threshold = std::min(vote_threshold, 255);
-  unsigned long long* acc = (unsigned long long*)accum;
-  DDN_TRY(launch_rank(s, ScanRange{0, -1}, out_keys, 1, acc, kAccWords, cap_out, nullptr, st));
-  if (n_points > 0)
-    DDN_TRY(launch_accumulate_points(s, n_points, row_len, xyz, rgb, votes, vote_threshold, acc, kAccWords, cap_out, st));
-  return launch_finalize(s, acc, out_keys, cap_out, out_xyz, out_rgb, out_count, st);
+  return ddn::fuse_finish(s, n_points, row_len, xyz, rgb, votes, vote_threshold, nullptr, out_keys, out_xyz, out_rgb, out_count, nullptr,
+                          cap_out, accum, accum_bytes, (cudaStream_t)stream);
+}
+
+int ddn_fuse_finish_normals(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                            const uint8_t* votes, int32_t vote_threshold, const float* normal, uint64_t* out_keys, float* out_xyz,
+                            uint8_t* out_rgb, int32_t* out_count, float* out_normal, int64_t cap_out, void* accum, int64_t accum_bytes,
+                            void* stream) {
+  DDN_REQUIRE(out_normal != nullptr && (n_points == 0 || normal != nullptr), "null pointer");
+  return ddn::fuse_finish(s, n_points, row_len, xyz, rgb, votes, vote_threshold, normal, out_keys, out_xyz, out_rgb, out_count, out_normal,
+                          cap_out, accum, accum_bytes, (cudaStream_t)stream);
 }
 
 int ddn_fuse_finish_partial(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,

@@ -93,6 +93,26 @@ __device__ __forceinline__ void finalize_voxel(const GridDev& g, float cx, float
   orgb[2] = (uint8_t)((2 * sb + cnt) / c2);
 }
 
+// ---- fused normals (the normal forms of every fusion path, include/ddn_b200.h: ddn_fuse_finish_normals) ------------
+// A point adds q = rint(n * 2^20) per component of its unit (or zero) normal to three more 64-bit words of its voxel's
+// accumulator, so the sums are order-independent like the position sums.  |q| <= 2^20, so a warp's 32 points fit a
+// 32-bit partial sum, and a voxel's 2^24 points (the colour-sum limit, counts[0] = -1) stay below 2^44.
+constexpr int kNormalShift = 20;
+constexpr int kAccNormalWords = 8;  // sx, sy, sz, r:g, b:count, then the normal sums nx, ny, nz (u64 each)
+// The optional trailing argument of the point passes' normals forms (their plain instantiations have an empty pack).
+__device__ __forceinline__ const float* normal_arg() { return nullptr; }
+__device__ __forceinline__ const float* normal_arg(const float* p) { return p; }
+__device__ __forceinline__ int normal_fix(float n) { return __float2int_rn(__fmul_rn(n, (float)(1 << kNormalShift))); }
+// Σq / ‖Σq‖ in float64 with every rounding written out, norm = sqrt((x² + y²) + z²), rounded to float32; 0 for Σq = 0.
+__device__ __forceinline__ void finalize_normal(long long nx, long long ny, long long nz, float* __restrict__ onrm) {
+  const double x = (double)nx, y = (double)ny, z = (double)nz;
+  const double len = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z)));
+  const bool any = len > 0.0;
+  onrm[0] = any ? (float)__ddiv_rn(x, len) : 0.f;
+  onrm[1] = any ? (float)__ddiv_rn(y, len) : 0.f;
+  onrm[2] = any ? (float)__ddiv_rn(z, len) : 0.f;
+}
+
 // ---- occupancy units (dense-rank path) --------------------------------------------------------------
 // Occupancy + rank live in ONE array of 16-byte units: words x, y, z = 96 occupancy bits, word w = the
 // exclusive rank prefix of the unit (written by the rank pass).  A slot lookup is a single LDG.128.

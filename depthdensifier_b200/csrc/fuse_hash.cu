@@ -21,6 +21,7 @@
 // the device derives, and nothing is read back.  The results are those of the dense path bit for bit: the same cell
 // of every point, the same integer sums (order-independent), the same finalisation, keys ascending.
 #include <algorithm>
+#include <type_traits>
 
 #include "fuse_hash.cuh"
 
@@ -71,11 +72,16 @@ hash_tomb_kernel(const GridDev* __restrict__ gp, HashDev h, int64_t n, const flo
 
 // accumulate_points_kernel (fuse.cu) with the slot lookup replaced by the table, and the participating points counted
 // into counts[0] (what K4's fused mark counts on the dense path: points that pass the vote and fall inside the grid).
-template <int kTW>  // tile width in pixels (tile = kTW x 32/kTW); 0 = no row structure, 32 consecutive points
+// The normals form (Normal = const float*, the plain form has no trailing parameter): also the quantised normals, as
+// accumulate_points_kernel's normals form, into accumulators of kAccNormalWords words.
+template <int kTW, class... Normal>  // tile width in pixels (tile = kTW x 32/kTW); 0 = no row structure, 32 consecutive points
 __global__ void __launch_bounds__(256)
 hash_insert_kernel(const GridDev* __restrict__ gp, HashDev h, int64_t n, int row_len, const float* __restrict__ xyz,
                    const uint8_t* __restrict__ rgb, const uint8_t* __restrict__ votes, int thr,
-                   unsigned long long* __restrict__ counts, unsigned long long* __restrict__ accum) {
+                   unsigned long long* __restrict__ counts, unsigned long long* __restrict__ accum, Normal... normal_in) {
+  constexpr bool kNormals = sizeof...(Normal) != 0;
+  constexpr int kWords = kNormals ? kAccNormalWords : kHashAccWords;
+  const float* __restrict__ normal = normal_arg(normal_in...);
   if (h.state[kStActive] == 0) return;
   const GridDev g = *gp;
   const float rv = 1.0f / g.voxel;
@@ -94,11 +100,15 @@ hash_insert_kernel(const GridDev* __restrict__ gp, HashDev h, int64_t n, int row
   }
   const int dx = lane % kTWs, dy = lane / kTWs;
   uint32_t ty = 0, tx = 0;
-  struct In {
+  struct InBase {
     float x, y, z;
     uint32_t rg, bb, i;
     bool take;
   };
+  struct InNormal : InBase {
+    float nx, ny, nz;
+  };
+  using In = std::conditional_t<kNormals, InNormal, InBase>;
   auto load_tile = [&](uint32_t t) -> In {
     int64_t i;
     bool in;
@@ -111,13 +121,15 @@ hash_insert_kernel(const GridDev* __restrict__ gp, HashDev h, int64_t n, int row
       i = (int64_t)t * 32 + lane;
       in = i < n;
     }
-    In r = {0.f, 0.f, 0.f, 0u, 0u, (uint32_t)i, false};
+    In r{};
+    r.i = (uint32_t)i;
     if (in) {
       const int v = votes != nullptr ? (int)__ldg(votes + i) : 0;
       r.x = __ldg(xyz + i * 3 + 0), r.y = __ldg(xyz + i * 3 + 1), r.z = __ldg(xyz + i * 3 + 2);
       r.rg = ((uint32_t)__ldg(rgb + i * 3 + 0) << 16) | (uint32_t)__ldg(rgb + i * 3 + 1);
       r.bb = (uint32_t)__ldg(rgb + i * 3 + 2);
       r.take = v < thr || votes == nullptr;
+      if constexpr (kNormals) r.nx = __ldg(normal + i * 3 + 0), r.ny = __ldg(normal + i * 3 + 1), r.nz = __ldg(normal + i * 3 + 2);
     }
     return r;
   };
@@ -156,6 +168,10 @@ hash_insert_kernel(const GridDev* __restrict__ gp, HashDev h, int64_t n, int row
     const bool leader = valid && (__ffs(peers) - 1) == lane;
     int sx = 0, sy = 0, sz = 0;
     uint32_t srg = 0, sb = 0;
+    int qx = 0, qy = 0, qz = 0, snx = 0, sny = 0, snz = 0;  // kNormals
+    if constexpr (kNormals) {
+      if (valid) qx = normal_fix(cur.nx), qy = normal_fix(cur.ny), qz = normal_fix(cur.nz);
+    }
     const int iters = __reduce_max_sync(0xffffffffu, __popc(peers));
     uint32_t rest = peers;
 #pragma unroll 1
@@ -167,16 +183,25 @@ hash_insert_kernel(const GridDev* __restrict__ gp, HashDev h, int64_t n, int row
       const int az = __shfl_sync(0xffffffffu, oz, src);
       const uint32_t arg = __shfl_sync(0xffffffffu, rg, src), ab = __shfl_sync(0xffffffffu, bb, src);
       if (has) sx += ax, sy += ay, sz += az, srg += arg, sb += ab;
+      if constexpr (kNormals) {
+        const int bx = __shfl_sync(0xffffffffu, qx, src), by = __shfl_sync(0xffffffffu, qy, src), bz = __shfl_sync(0xffffffffu, qz, src);
+        if (has) snx += bx, sny += by, snz += bz;
+      }
     }
     if (leader) {
-      const uint32_t idx = hash_voxel_index(h, key, cur.i, accum);
+      const uint32_t idx = hash_voxel_index<kWords, kWords>(h, key, cur.i, accum);
       if (idx != kSkipIndex) {
-        unsigned long long* a = accum + (size_t)idx * kHashAccWords;
+        unsigned long long* a = accum + (size_t)idx * kWords;
         atomicAdd(a + 0, (unsigned long long)(long long)sx);
         atomicAdd(a + 1, (unsigned long long)(long long)sy);
         atomicAdd(a + 2, (unsigned long long)(long long)sz);
         atomicAdd(a + 3, ((unsigned long long)(srg >> 16) << 32) | (srg & 0xffffu));
         atomicAdd(a + 4, ((unsigned long long)sb << 32) | (unsigned)__popc(peers));
+        if constexpr (kNormals) {
+          atomicAdd(a + 5, (unsigned long long)(long long)snx);
+          atomicAdd(a + 6, (unsigned long long)(long long)sny);
+          atomicAdd(a + 7, (unsigned long long)(long long)snz);
+        }
       }
     }
   }
@@ -257,6 +282,14 @@ hash_sort_finalize_kernel(const GridDev* __restrict__ gp, HashDev h, long long* 
   hash_sort_body(gp, h, counts, HashFinalize<kHashAccWords>{counts, cap, out_keys, out_xyz, out_rgb, out_count, accum});
 }
 
+__global__ void __launch_bounds__(kSortThreads, 1)
+hash_sort_finalize_normals_kernel(const GridDev* __restrict__ gp, HashDev h, long long* __restrict__ counts, long long cap,
+                                  uint64_t* __restrict__ out_keys, float* __restrict__ out_xyz, uint8_t* __restrict__ out_rgb,
+                                  int32_t* __restrict__ out_count, const unsigned long long* __restrict__ accum, float* __restrict__ out_normal) {
+  hash_sort_body(gp, h, counts,
+                 HashFinalize<kAccNormalWords, true>{counts, cap, out_keys, out_xyz, out_rgb, out_count, accum, out_normal});
+}
+
 // ---- host side ---------------------------------------------------------------------------------
 struct HashSizes {
   int64_t cap_slots, table_bytes, slots_bytes, sort_bytes, hist_bytes;
@@ -305,7 +338,7 @@ int hash_launch_compact(const GridDev* gp, const HashDev& h, int64_t n, unsigned
 
 int hash_launch_points(GridDev* gp, const HashDev& h, unsigned long long* counts, int mode, int64_t n_points, int64_t row_len,
                        const float* xyz, const uint8_t* rgb, const uint8_t* votes, int thr, const float* dedup_xyz, int64_t n_dedup,
-                       unsigned long long* acc, cudaStream_t st) {
+                       unsigned long long* acc, cudaStream_t st, const float* normal) {
   hash_begin_kernel<<<1, 32, 0, st>>>(gp, h, counts, mode);
   DDN_TRY(after_launch("hash_begin_kernel", st));
   if (n_dedup > 0) {
@@ -318,11 +351,20 @@ int hash_launch_points(GridDev* gp, const HashDev& h, unsigned long long* counts
     const int th = tw ? 32 / tw : 1, twe = tw ? tw : 32;
     const int64_t n_tiles = tiled ? ((row_len + twe - 1) / twe) * (((n_points + row_len - 1) / row_len + th - 1) / th) : (n_points + 31) / 32;
     const unsigned blocks = (unsigned)std::min<int64_t>((n_tiles + 8 * kHashTilesPerWarp - 1) / (8 * kHashTilesPerWarp), kHashCtas);
-    if (tiled)
-      hash_insert_kernel<kHashTileW><<<blocks, 256, 0, st>>>(gp, h, n_points, (int)row_len, xyz, rgb, votes, thr, counts, acc);
-    else
-      hash_insert_kernel<0><<<blocks, 256, 0, st>>>(gp, h, n_points, (int)row_len, xyz, rgb, votes, thr, counts, acc);
-    DDN_TRY(after_launch("hash_insert_kernel", st));
+    if (normal != nullptr) {
+      if (tiled)
+        hash_insert_kernel<kHashTileW, const float*><<<blocks, 256, 0, st>>>(gp, h, n_points, (int)row_len, xyz, rgb, votes, thr, counts, acc,
+                                                                             normal);
+      else
+        hash_insert_kernel<0, const float*><<<blocks, 256, 0, st>>>(gp, h, n_points, (int)row_len, xyz, rgb, votes, thr, counts, acc, normal);
+      DDN_TRY(after_launch("hash_insert_kernel", st));
+    } else {
+      if (tiled)
+        hash_insert_kernel<kHashTileW><<<blocks, 256, 0, st>>>(gp, h, n_points, (int)row_len, xyz, rgb, votes, thr, counts, acc);
+      else
+        hash_insert_kernel<0><<<blocks, 256, 0, st>>>(gp, h, n_points, (int)row_len, xyz, rgb, votes, thr, counts, acc);
+      DDN_TRY(after_launch("hash_insert_kernel", st));
+    }
   }
   return hash_launch_compact(gp, h, n_points, counts, st);
 }
@@ -355,11 +397,17 @@ int ddn_hash_fuse_reset(const struct ddn_hash_fuse* hf, void* stream) {
   return check_cuda(cudaMemsetAsync(hf->state, 0, DDN_HASH_STATE_BYTES, st), "memset hash state");
 }
 
-int ddn_fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_hash_fuse* hf, int32_t mode, int64_t n_points, int64_t row_len,
-                           const float* xyz, const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold, const float* dedup_xyz,
-                           int64_t n_dedup, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t cap_out,
-                           void* accum, int64_t accum_bytes, void* stream) {
-  using namespace ddn;
+}  // extern "C"
+
+namespace ddn {
+
+// ddn_fuse_finish_hashed, and with out_normal its normals form
+static int fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_hash_fuse* hf, int32_t mode, int64_t n_points, int64_t row_len,
+                              const float* xyz, const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold, const float* normal,
+                              const float* dedup_xyz, int64_t n_dedup, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
+                              int32_t* out_count, float* out_normal, int64_t cap_out, void* accum, int64_t accum_bytes, cudaStream_t st) {
+  const bool normals = out_normal != nullptr;
+  const int words = normals ? kAccNormalWords : kHashAccWords;
   DDN_REQUIRE(s != nullptr && s->grid && s->counts, "session: null buffer");
   HashDev h;
   DDN_TRY(hash_dev(hf, &h));
@@ -370,24 +418,53 @@ int ddn_fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_hash_fuse
   DDN_REQUIRE(row_len >= 0, "row_len");
   DDN_REQUIRE(cap_out > 0 && cap_out < (1ll << 31), "cap_out");
   DDN_REQUIRE(out_keys && out_xyz && out_rgb && out_count && accum, "null pointer");
-  DDN_REQUIRE(accum_bytes >= std::max(cap_out, n_points) * kHashAccWords * 8 + 16 && (uintptr_t)accum % 16 == 0,
-              "accumulator scratch (max(cap_out, n_points) * 40 bytes)");
+  DDN_REQUIRE(accum_bytes >= std::max(cap_out, n_points) * words * 8 + 16 && (uintptr_t)accum % 16 == 0,
+              normals ? "accumulator scratch (max(cap_out, n_points) * 64 bytes)" : "accumulator scratch (max(cap_out, n_points) * 40 bytes)");
   DDN_REQUIRE(n_points == 0 || (xyz && rgb), "null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
+  DDN_REQUIRE(!normals || n_points == 0 || normal != nullptr, "null pointer");
   const int thr = std::min(vote_threshold, 255);
   GridDev* gp = reinterpret_cast<GridDev*>(s->grid);
   unsigned long long* counts = reinterpret_cast<unsigned long long*>(s->counts);
   unsigned long long* acc = reinterpret_cast<unsigned long long*>(accum);
   const long long cap = (long long)cap_out;
-  DDN_TRY(hash_launch_points(gp, h, counts, mode, n_points, row_len, xyz, rgb, votes, thr, dedup_xyz, n_dedup, acc, st));
+  DDN_TRY(hash_launch_points(gp, h, counts, mode, n_points, row_len, xyz, rgb, votes, thr, dedup_xyz, n_dedup, acc, st,
+                             normals ? normal : nullptr));
   long long* counts_ll = reinterpret_cast<long long*>(s->counts);
   const unsigned long long* acc_c = acc;
   const GridDev* gpc = gp;
   void* args[] = {(void*)&gpc, (void*)&h, (void*)&counts_ll, (void*)&cap, (void*)&out_keys, (void*)&out_xyz, (void*)&out_rgb,
-                  (void*)&out_count, (void*)&acc_c};
+                  (void*)&out_count, (void*)&acc_c, (void*)&out_normal};
+  if (normals) {
+    DDN_TRY(check_cuda(cudaLaunchCooperativeKernel((const void*)hash_sort_finalize_normals_kernel, dim3(kSortCtas), dim3(kSortThreads), args,
+                                                   0, st),
+                       "hash_sort_finalize_normals_kernel"));
+    return after_launch("hash_sort_finalize_normals_kernel", st);
+  }
   DDN_TRY(check_cuda(cudaLaunchCooperativeKernel((const void*)hash_sort_finalize_kernel, dim3(kSortCtas), dim3(kSortThreads), args, 0, st),
                      "hash_sort_finalize_kernel"));
   return after_launch("hash_sort_finalize_kernel", st);
+}
+
+}  // namespace ddn
+
+extern "C" {
+
+int ddn_fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_hash_fuse* hf, int32_t mode, int64_t n_points, int64_t row_len,
+                           const float* xyz, const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold, const float* dedup_xyz,
+                           int64_t n_dedup, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t cap_out,
+                           void* accum, int64_t accum_bytes, void* stream) {
+  return ddn::fuse_finish_hashed(s, hf, mode, n_points, row_len, xyz, rgb, votes, vote_threshold, nullptr, dedup_xyz, n_dedup, out_keys,
+                                 out_xyz, out_rgb, out_count, nullptr, cap_out, accum, accum_bytes, (cudaStream_t)stream);
+}
+
+int ddn_fuse_finish_hashed_normals(const ddn_fuse_session* s, const struct ddn_hash_fuse* hf, int32_t mode, int64_t n_points,
+                                   int64_t row_len, const float* xyz, const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold,
+                                   const float* normal, const float* dedup_xyz, int64_t n_dedup, uint64_t* out_keys, float* out_xyz,
+                                   uint8_t* out_rgb, int32_t* out_count, float* out_normal, int64_t cap_out, void* accum,
+                                   int64_t accum_bytes, void* stream) {
+  DDN_REQUIRE(out_normal != nullptr, "null pointer");
+  return ddn::fuse_finish_hashed(s, hf, mode, n_points, row_len, xyz, rgb, votes, vote_threshold, normal, dedup_xyz, n_dedup, out_keys,
+                                 out_xyz, out_rgb, out_count, out_normal, cap_out, accum, accum_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

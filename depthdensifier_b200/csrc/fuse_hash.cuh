@@ -66,9 +66,9 @@ __device__ __forceinline__ uint64_t canonical_key(uint32_t kx, uint32_t ky, uint
 }
 
 // Voxel index of `key`: found, or inserted with `self` (the inserting point's index) as its index.  The inserter
-// zeroes the accumulator (kHashAccWords words at accum + self * kStride) before it publishes the index with release
-// semantics; the others acquire it before their REDs.  kSkipIndex for a tombstoned cell.
-template <int kStride = kHashAccWords>
+// zeroes the accumulator (kWords words at accum + self * kStride: kAccNormalWords for the normals form) before it
+// publishes the index with release semantics; the others acquire it before their REDs.  kSkipIndex for a tombstoned cell.
+template <int kStride = kHashAccWords, int kWords = kHashAccWords>
 __device__ __forceinline__ uint32_t hash_voxel_index(const HashDev& h, uint64_t key, uint32_t self, unsigned long long* __restrict__ accum) {
   uint64_t s = hash_slot(h, key);
   const uint64_t mask = (uint64_t)(h.cap_slots - 1);
@@ -81,7 +81,7 @@ __device__ __forceinline__ uint32_t hash_voxel_index(const HashDev& h, uint64_t 
         h.slots[self] = (uint32_t)s;
         unsigned long long* a = accum + (size_t)self * kStride;
 #pragma unroll
-        for (int q = 0; q < kHashAccWords; ++q) a[q] = 0ull;
+        for (int q = 0; q < kWords; ++q) a[q] = 0ull;
         st_release_u32(h.index + s, self);
         return self;
       }
@@ -201,8 +201,9 @@ __device__ __forceinline__ void hash_sort_body(const GridDev* __restrict__ gp, c
 }
 
 // The finalising epilogue (finalize_kernel's arithmetic, the accumulator read through the sorted index): the voxel of
-// sorted element r has its kHashAccWords sums at accum + va[r] * kStride.
-template <int kStride>
+// sorted element r has its kHashAccWords sums at accum + va[r] * kStride.  kNormals: then its normal sums (words 5..7),
+// finalised into out_normal as finalize_normals_kernel does.
+template <int kStride, bool kNormals = false>
 struct HashFinalize {
   long long* counts;
   long long cap;
@@ -211,6 +212,7 @@ struct HashFinalize {
   uint8_t* out_rgb;
   int32_t* out_count;
   const unsigned long long* accum;
+  float* out_normal;  // kNormals only
   __device__ __forceinline__ void operator()(const GridDev& g, long long m, const unsigned long long* ka, const uint32_t* va,
                                              long long gtid, long long gthreads) const {
     const int bx = g.bx, by = g.by;
@@ -228,6 +230,7 @@ struct HashFinalize {
       out_count[r] = (int32_t)cnt;
       finalize_voxel(g, voxel_centre(g.ox, kx, g.voxel), voxel_centre(g.oy, ky, g.voxel), voxel_centre(g.oz, kz, g.voxel), sx, sy, sz,
                      rg >> 32, rg & 0xffffffffull, bn >> 32, (long long)cnt, out_xyz + r * 3, out_rgb + r * 3);
+      if constexpr (kNormals) finalize_normal((long long)a[5], (long long)a[6], (long long)a[7], out_normal + r * 3);
     }
   }
 };
@@ -235,11 +238,11 @@ struct HashFinalize {
 // ---- host side (fuse_hash.cu) --------------------------------------------------------------------
 int hash_dev(const ddn_hash_fuse* hf, HashDev* h);
 // hash_begin (mode as ddn_fuse_finish_hashed), hash_tomb over the dedup points, hash_insert over the points into
-// `accum` (kHashAccWords words per point), hash_compact: the step's voxels as unsorted (compact key, index) pairs,
-// their number in counts[1]
+// `accum` (kHashAccWords words per point; with `normal` [n_points,3] the normals form, kAccNormalWords words), hash_compact:
+// the step's voxels as unsorted (compact key, index) pairs, their number in counts[1]
 int hash_launch_points(GridDev* gp, const HashDev& h, unsigned long long* counts, int mode, int64_t n_points, int64_t row_len,
                        const float* xyz, const uint8_t* rgb, const uint8_t* votes, int thr, const float* dedup_xyz, int64_t n_dedup,
-                       unsigned long long* accum, cudaStream_t st);
+                       unsigned long long* accum, cudaStream_t st, const float* normal = nullptr);
 // hash_compact over the first n entries of the slot list
 int hash_launch_compact(const GridDev* gp, const HashDev& h, int64_t n, unsigned long long* counts, cudaStream_t st);
 

@@ -139,6 +139,9 @@ class ShardedDensifier:
         # `backend` is the module providing the device ops; the product always uses `ops` (CUDA, no CPU
         # fallback).  Tests inject an object with the same functions to exercise the exchange logic on
         # CPU with the gloo backend.
+        if cfg.fuse_normals:
+            raise ValueError("DensifyConfig.fuse_normals: the multi-GPU form of the fused normals is not built; "
+                             "use DensifyEngine on one GPU")
         if backend is None:
             if not torch.cuda.is_available():
                 raise ops.DDNError("ShardedDensifier needs a CUDA device: depthdensifier_b200 has no CPU fallback")

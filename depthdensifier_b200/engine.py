@@ -37,6 +37,10 @@ class DensifyConfig:
     # (MVSNet's forward-backward reprojection) lands within support_reproj_px pixels of the point's pixel.  None: no
     # such test.
     support_reproj_px: float | None = None
+    # Oriented normals (one GPU): the step also computes every grid point's world-frame normal from the normal maps
+    # (DensifyResult.normals, turned toward its camera) and, with fusion, each voxel's fused normal
+    # (DensifyResult.voxel_normal).  Off: the normal maps only feed the grazing gate.
+    fuse_normals: bool = False
 
     def __post_init__(self):
         self._check_reproj()
@@ -98,6 +102,8 @@ class DensifyResult:
     stride: int = 1  # back-projection grid stride: xyz / votes hold every stride-th row and column
     support: torch.Tensor | None = None  # like votes: supporting neighbours, min(count, 254), 255 = no point (None: off)
     min_support: int | None = None  # the step's DensifyConfig.min_support
+    normals: torch.Tensor | None = None  # fuse_normals: like xyz, [n_src,Hs,Ws,3] f32 (flat [G,3] for run_views), unit or 0
+    voxel_normal: torch.Tensor | None = None  # fuse_normals with fusion: [M,3] f32 per voxel, unit or 0
 
     def fusion_threshold(self) -> int:
         """The threshold the vote bytes are tested with (by keep_mask and the fusion passes)."""
@@ -126,6 +132,12 @@ class DensifyResult:
         """xyz [M,3] f32 and rgb [M,3] u8 of the points the vote keeps, view by view in grid order."""
         keep = self.keep_mask()
         return self.xyz[keep], self.grid_rgb()[keep]
+
+    def kept_normals(self) -> torch.Tensor:
+        """normals [M,3] f32 of the points the vote keeps, in the order of kept_points() (needs fuse_normals)."""
+        if self.normals is None:
+            raise ValueError("the step computed no normals: set DensifyConfig.fuse_normals")
+        return self.normals[self.keep_mask()]
 
     def host_grid(self):
         """The voxel grid as a host struct (synchronises; raises when the device could not build one)."""
@@ -246,6 +258,9 @@ class DensifyEngine:
                             layout=layout, rgb=rgb, stride=cfg.filter.stride, support=out[2] if extra else None,
                             min_support=cfg.min_support)
         thr = res.fusion_threshold()
+        if cfg.fuse_normals:
+            res.normals = (ops.point_normals(normal, cam_from_world, intr, votes, cfg.filter.stride) if layout is None
+                           else ops.point_normals_ragged(layout, normal, cam_from_world, intr, votes))
         if fuse:
             points = (xyz.view(-1, 3), res.grid_rgb().view(-1, 3), votes.view(-1))
             dedup = sparse_xyz.float().contiguous() if cfg.dedup_sparse and sparse_xyz.shape[0] > 0 else None
@@ -254,12 +269,17 @@ class DensifyEngine:
             row_len = xyz.shape[2] if layout is None else 0  # 0: the rows differ from view to view
             # Both finishes are enqueued on the same outputs; the device grid decides which one runs (the hashed path
             # takes a grid too large for the session's bitmap, the dense one every other), so nothing is read back.
-            out = ops.fuse_finish(sess, *points, thr, row_len=row_len)[:4]
+            nrm = {} if res.normals is None else {"normal": res.normals.view(-1, 3)}
+            out = ops.fuse_finish(sess, *points, thr, row_len=row_len, **nrm)[:-1]
             hf = self.hash_fuse(points[0].shape[0] + (0 if dedup is None else dedup.shape[0]))
-            k, x, c, n, counts = ops.fuse_finish_hashed(sess, hf, *points, thr, row_len=row_len, dedup_xyz=dedup, out=out)
+            *vox, counts = ops.fuse_finish_hashed(sess, hf, *points, thr, row_len=row_len, dedup_xyz=dedup, out=out, **nrm)
             res.session, res.grid, res.hash = sess, grid, hf
-            res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts.clone()
+            res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count = vox[:4]
+            res.voxel_normal = vox[4] if nrm else None
+            res.counts = counts.clone()
             if sync:
                 mv = res.check()
-                res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count = k[:mv], x[:mv], c[:mv], n[:mv]
+                res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count = (v[:mv] for v in vox[:4])
+                if nrm:
+                    res.voxel_normal = vox[4][:mv]
         return res

@@ -480,6 +480,45 @@ def backproject_filter_ragged(layout: ViewLayout, refined_all, normal, pair_tabl
     return xyz, votes
 
 
+def point_normals(normal, cam_from_world, intr, votes, stride: int, out=None):
+    """Oriented world-frame normals of the back-projection grid (include/ddn_b200.h: ddn_point_normals): normal
+    [V,H,W,3] f32 (device, or pinned host), cam_from_world [V,3,4] f64, intr [V,4] f64 (fx, fy, cx, cy), votes
+    [V,Hs,Ws] u8 of the consistency kernel at ``stride``.  Returns [V,Hs,Ws,3] f32 in the order of its xyz, (0, 0, 0)
+    where a pixel has no point."""
+    lib = _lib.load()
+    dev = _require_cuda_normal(normal, cam_from_world, intr, votes, out)
+    V, H, W = normal.shape[:3]
+    s = int(stride)
+    Hs, Ws = (H + s - 1) // s, (W + s - 1) // s
+    assert normal.dtype == torch.float32 and tuple(normal.shape) == (V, H, W, 3)
+    assert cam_from_world.dtype == torch.float64 and tuple(cam_from_world.shape) == (V, 3, 4)
+    assert intr.dtype == torch.float64 and tuple(intr.shape) == (V, 4)
+    assert votes.dtype == torch.uint8 and tuple(votes.shape) == (V, Hs, Ws)
+    out = out if out is not None else torch.empty((V, Hs, Ws, 3), dtype=torch.float32, device=dev)
+    assert out.dtype == torch.float32 and tuple(out.shape) == (V, Hs, Ws, 3)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ddn_point_normals(V, H, W, s, _p(normal), _p(cam_from_world), _p(intr), _p(votes), _p(out), _stream()))
+    return out
+
+
+def point_normals_ragged(layout: ViewLayout, normal, cam_from_world, intr, votes, out=None):
+    """point_normals for the views of ``layout``: normal flat [P,3] f32 (device, or pinned host), votes [G] u8.
+    Returns [G,3] f32 on the views' strided grids."""
+    lib = _lib.load()
+    dev = _require_cuda_normal(normal, cam_from_world, intr, votes, out)
+    V, P, G = layout.n_views, layout.total_pixels, layout.total_grid
+    assert normal.dtype == torch.float32 and tuple(normal.shape) == (P, 3)
+    assert cam_from_world.dtype == torch.float64 and tuple(cam_from_world.shape) == (V, 3, 4)
+    assert intr.dtype == torch.float64 and tuple(intr.shape) == (V, 4)
+    assert votes.dtype == torch.uint8 and tuple(votes.shape) == (G,)
+    out = out if out is not None else torch.empty((G, 3), dtype=torch.float32, device=dev)
+    assert out.dtype == torch.float32 and tuple(out.shape) == (G, 3)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ddn_point_normals_ragged(V, _p(layout.device(dev)), layout.host_ptr(), _p(normal), _p(cam_from_world), _p(intr),
+                                                _p(votes), _p(out), _stream()))
+    return out
+
+
 def make_grid(bbox_min, bbox_max, voxel: float):
     """Voxel grid from a bounding box: origin = floor(min/voxel)*voxel in float32 (SURVEY.md N4) and the
     number of significant bits per axis."""
@@ -592,8 +631,9 @@ class FuseSession:
             self._merge_scratch = ((world, cap_out), torch.empty(nbytes.value, dtype=torch.uint8, device=self.device))
         return self._merge_scratch[1]
 
-    def accum(self, cap_out: int) -> torch.Tensor:
-        nbytes = cap_out * 40 + 16
+    def accum(self, cap_out: int, words: int = 5) -> torch.Tensor:
+        """Accumulator scratch for ``cap_out`` voxels of ``words`` u64 (5; 8 for the fused-normal forms)."""
+        nbytes = cap_out * words * 8 + 16
         if self._accum is None or self._accum.numel() < nbytes:
             self._accum = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
         return self._accum
@@ -675,19 +715,37 @@ def new_hash_samples(dev) -> torch.Tensor:
     return torch.empty(_lib.HASH_SAMPLES + 1, dtype=torch.int64, device=dev)
 
 
-def new_voxel_outputs(cap_out: int, dev):
-    return (torch.empty(cap_out, dtype=torch.int64, device=dev), torch.empty((cap_out, 3), dtype=torch.float32, device=dev),
-            torch.empty((cap_out, 3), dtype=torch.uint8, device=dev), torch.empty(cap_out, dtype=torch.int32, device=dev))
+def new_voxel_outputs(cap_out: int, dev, normals: bool = False):
+    """keys, xyz, rgb, count (and with ``normals`` the voxel normals [cap_out,3] f32) of ``cap_out`` voxels."""
+    out = (torch.empty(cap_out, dtype=torch.int64, device=dev), torch.empty((cap_out, 3), dtype=torch.float32, device=dev),
+           torch.empty((cap_out, 3), dtype=torch.uint8, device=dev), torch.empty(cap_out, dtype=torch.int32, device=dev))
+    return out + (torch.empty((cap_out, 3), dtype=torch.float32, device=dev),) if normals else out
 
 
-def fuse_finish(sess: FuseSession, xyz, rgb, votes, vote_threshold: int, row_len: int = 0, cap_out: int | None = None, out=None):
+def _check_normal(normal, n: int) -> None:
+    assert normal.dtype == torch.float32 and tuple(normal.shape) == (n, 3) and normal.is_contiguous()
+
+
+def fuse_finish(sess: FuseSession, xyz, rgb, votes, vote_threshold: int, row_len: int = 0, cap_out: int | None = None, out=None,
+                normal=None):
     """Rank + accumulate + finalise of the points marked in ``sess``.  Returns keys, xyz, rgb, count (capacity
-    ``cap_out``, default = the number of points) and the session's device counts [2] = (points, voxels)."""
+    ``cap_out``, default = the number of points) and the session's device counts [2] = (points, voxels).
+
+    ``normal`` [N,3] f32 (point_normals, in the order of xyz): also fuse the normals (ddn_fuse_finish_normals); then
+    returns keys, xyz, rgb, count, normal [cap_out,3] f32 and counts, and ``out`` holds five outputs."""
     lib = _lib.load()
-    dev = _require_cuda(xyz, rgb, votes)
+    dev = _require_cuda(xyz, rgb, votes, normal)
     N = xyz.shape[0]
     assert xyz.dtype == torch.float32 and rgb.dtype == torch.uint8 and tuple(rgb.shape) == (N, 3)
     cap = max(int(cap_out if cap_out is not None else N), 1)
+    if normal is not None:
+        _check_normal(normal, N)
+        k, x, c, n, nrm = out if out is not None else new_voxel_outputs(cap, dev, normals=True)
+        acc = sess.accum(cap, 8)
+        with torch.cuda.device(dev):
+            _lib.check(lib.ddn_fuse_finish_normals(C.byref(sess.c), N, int(row_len), _p(xyz), _p(rgb), _p(votes), int(vote_threshold),
+                                                   _p(normal), _p(k), _p(x), _p(c), _p(n), _p(nrm), cap, _p(acc), acc.numel(), _stream()))
+        return k, x, c, n, nrm, sess.counts
     k, x, c, n = out if out is not None else new_voxel_outputs(cap, dev)
     acc = sess.accum(cap)
     with torch.cuda.device(dev):
@@ -697,20 +755,30 @@ def fuse_finish(sess: FuseSession, xyz, rgb, votes, vote_threshold: int, row_len
 
 
 def fuse_finish_hashed(sess: FuseSession, hf: HashFuse, xyz, rgb, votes, vote_threshold: int, row_len: int = 0,
-                       dedup_xyz=None, mode: int = 0, cap_out: int | None = None, out=None):
+                       dedup_xyz=None, mode: int = 0, cap_out: int | None = None, out=None, normal=None):
     """Hashed fusion of the step's points (include/ddn_b200.h: ddn_fuse_finish_hashed).  ``mode`` 0: only when the
     session's grid is too large for its bitmap (the dense finish returns at once then); 1: on any grid.  ``dedup_xyz``
     [n,3] f32: N5, no voxel in the cells of these points.  Returns keys, xyz, rgb, count and the device counts [2], as
-    fuse_finish; pass the same ``out`` as the dense finish so that one set of outputs holds whichever path ran."""
+    fuse_finish; pass the same ``out`` as the dense finish so that one set of outputs holds whichever path ran.
+    ``normal``: as in fuse_finish (ddn_fuse_finish_hashed_normals)."""
     lib = _lib.load()
-    dev = _require_cuda(xyz, rgb, votes, dedup_xyz)
+    dev = _require_cuda(xyz, rgb, votes, dedup_xyz, normal)
     N = xyz.shape[0]
     assert xyz.dtype == torch.float32 and rgb.dtype == torch.uint8 and tuple(rgb.shape) == (N, 3)
     assert dedup_xyz is None or (dedup_xyz.dtype == torch.float32 and dedup_xyz.dim() == 2 and dedup_xyz.shape[1] == 3)
     cap = max(int(cap_out if cap_out is not None else N), 1)
+    n_dedup = 0 if dedup_xyz is None else dedup_xyz.shape[0]
+    if normal is not None:
+        _check_normal(normal, N)
+        k, x, c, n, nrm = out if out is not None else new_voxel_outputs(cap, dev, normals=True)
+        acc = sess.accum(max(cap, N), 8)
+        with torch.cuda.device(dev):
+            _lib.check(lib.ddn_fuse_finish_hashed_normals(C.byref(sess.c), C.byref(hf.c), int(mode), N, int(row_len), _p(xyz), _p(rgb),
+                                                          _p(votes), int(vote_threshold), _p(normal), _p(dedup_xyz), n_dedup, _p(k), _p(x),
+                                                          _p(c), _p(n), _p(nrm), cap, _p(acc), acc.numel(), _stream()))
+        return k, x, c, n, nrm, sess.counts
     k, x, c, n = out if out is not None else new_voxel_outputs(cap, dev)
     acc = sess.accum(max(cap, N))  # a voxel's accumulator is indexed by the point that created it
-    n_dedup = 0 if dedup_xyz is None else dedup_xyz.shape[0]
     with torch.cuda.device(dev):
         _lib.check(lib.ddn_fuse_finish_hashed(C.byref(sess.c), C.byref(hf.c), int(mode), N, int(row_len), _p(xyz), _p(rgb), _p(votes),
                                               int(vote_threshold), _p(dedup_xyz), n_dedup, _p(k), _p(x), _p(c), _p(n), cap, _p(acc),
@@ -788,24 +856,35 @@ def fuse_merge_peers(sess: FuseSession, rank: int, world: int, peer_records, pee
     return k, x, c, n, sess.counts
 
 
-def voxel_fuse(xyz, rgb, votes, vote_threshold: int, grid: _lib.VoxelGrid, trim: bool = True, row_len: int = 0):
+def voxel_fuse(xyz, rgb, votes, vote_threshold: int, grid: _lib.VoxelGrid, trim: bool = True, row_len: int = 0, normal=None):
     """Stage 4.  xyz [N,3] f32, rgb [N,3] u8, votes [N] u8 or None.  Returns keys, xyz, rgb, count
     (trimmed to the voxel count when ``trim``; that reads the counts back and synchronises) and the
     device counts tensor [2] = (participating points, voxels).  ``row_len``: image width when the points
-    are the pixels of row-major depth maps (locality hint only)."""
+    are the pixels of row-major depth maps (locality hint only).  ``normal`` [N,3] f32: also fuse the normals
+    (ddn_voxel_fuse_normals); then returns keys, xyz, rgb, count, normal [M,3] f32 and counts."""
     lib = _lib.load()
-    dev = _require_cuda(xyz, rgb, votes)
+    dev = _require_cuda(xyz, rgb, votes, normal)
     N = xyz.shape[0]
     assert xyz.dtype == torch.float32 and rgb.dtype == torch.uint8 and tuple(rgb.shape) == (N, 3)
     assert votes is None or (votes.dtype == torch.uint8 and votes.numel() == N)
     nbytes = C.c_int64(0)
-    _lib.check(lib.ddn_fuse_workspace_bytes(C.byref(grid), N, C.byref(nbytes)))
+    sizer = lib.ddn_fuse_workspace_bytes if normal is None else lib.ddn_fuse_normals_workspace_bytes
+    _lib.check(sizer(C.byref(grid), N, C.byref(nbytes)))
     ws = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
     out_keys = torch.empty(N, dtype=torch.int64, device=dev)
     out_xyz = torch.empty((N, 3), dtype=torch.float32, device=dev)
     out_rgb = torch.empty((N, 3), dtype=torch.uint8, device=dev)
     out_cnt = torch.empty(N, dtype=torch.int32, device=dev)
     counts = torch.zeros(2, dtype=torch.int64, device=dev)
+    if normal is not None:
+        _check_normal(normal, N)
+        out_nrm = torch.empty((N, 3), dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(lib.ddn_voxel_fuse_normals(C.byref(grid), N, int(row_len), _p(xyz), _p(rgb), _p(votes), int(vote_threshold),
+                                                  _p(normal), _p(out_keys), _p(out_xyz), _p(out_rgb), _p(out_cnt), _p(out_nrm), _p(counts),
+                                                  _p(ws), nbytes.value, _stream()))
+        mv = checked_voxel_count(counts) if trim else N
+        return out_keys[:mv], out_xyz[:mv], out_rgb[:mv], out_cnt[:mv], out_nrm[:mv], counts
     with torch.cuda.device(dev):
         _lib.check(
             lib.ddn_voxel_fuse(

@@ -32,6 +32,7 @@ import torch
 
 from . import ops
 from .colmap_io import Camera, Image, Reconstruction
+from .ply import write_ply
 from .depth_refiner import RefinerConfig
 from .engine import DensifyConfig, DensifyEngine
 from .neighbours import covisibility_table, nearest_views_table
@@ -49,6 +50,10 @@ class PathsConfig:
     output_model_dir: Path = Path("results/0")
     depth_dir: Path | None = None
     """new: directory of precomputed <image stem>.npz (depth, normal, mask); None -> run MoGe."""
+    output_ply: Path | None = None
+    """new: also write the model's points as a binary PLY with oriented normals (x y z nx ny nz red green blue, the
+    layout of COLMAP's fused.ply and 3DGS's points3D.ply): the sparse points with normal (0, 0, 0), then the dense
+    points with their world-frame normals, turned toward the camera and fused per voxel with fusion.voxel_size."""
 
 
 @dataclass
@@ -212,6 +217,7 @@ class DensifyOutput:
     timings: dict
     candidates: np.ndarray | None = None  # [N,3] f64 every back-projected point (return_candidates=True)
     keep: np.ndarray | None = None  # [N] bool
+    normals: np.ndarray | None = None  # [M,3] f32 normals of the appended points (paths.output_ply)
 
 
 def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, return_candidates: bool = False) -> DensifyOutput:
@@ -283,11 +289,13 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
     filt = ops.FilterOptions(depth_threshold=config.filtering.depth_threshold, sample_mode=config.filtering.sample_mode,
                              stride=max(int(config.processing.downsample_density), 1))
     ms, rp = config.filtering.min_support, config.filtering.support_reproj_px
+    want_normals = config.paths.output_ply is not None
     eng = DensifyEngine(DensifyConfig(align=align, filter=filt, vote_threshold=int(config.filtering.vote_threshold),
                                       voxel=config.fusion.voxel_size, dedup_sparse=bool(config.fusion.dedup_sparse),
                                       min_support=None if ms is None else int(ms),
                                       support_tau=float(config.filtering.support_tau),
-                                      support_reproj_px=None if rp is None else float(rp)), device=dev)
+                                      support_reproj_px=None if rp is None else float(rp), fuse_normals=want_normals),
+                        device=dev)
     offsets = np.concatenate([[0], np.cumsum([len(p) for p in sparse])]).astype(np.int64)
     to = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(dev)
     maps = ((depths, torch.float32), (normals, torch.float32), (masks, torch.bool), (rgbs, torch.uint8))
@@ -298,13 +306,18 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
     res = run(*maps, to(poses_np, torch.float64), to(np.stack(intr), torch.float64), to(np.concatenate(sparse), torch.float64),
               to(offsets, torch.int64), to(nbr, torch.int32))
     n_candidates = res.num_points()
+    nrm_out = None
     if config.fusion.voxel_size is None:
         pts, cols = res.kept_points()
         pts_out, col_out = pts.double().cpu().numpy(), cols.cpu().numpy()
+        if want_normals:
+            nrm_out = res.kept_normals().cpu().numpy()
     else:
         mv = int(res.counts[1].item()) if res.counts is not None else 0
         pts_out = res.voxel_xyz[:mv].double().cpu().numpy() if mv else np.zeros((0, 3))
         col_out = res.voxel_rgb[:mv].cpu().numpy() if mv else np.zeros((0, 3), np.uint8)
+        if want_normals:
+            nrm_out = res.voxel_normal[:mv].cpu().numpy() if mv else np.zeros((0, 3), np.float32)
     torch.cuda.synchronize(dev)
     timings["device_pipeline"] = time.time() - t0
     print(f"-> {n_candidates} candidate points from {V} views, {len(pts_out)} kept"
@@ -316,10 +329,17 @@ def main(config: ScriptConfig, depth_provider: DepthProvider | None = None, retu
     out_dir = Path(config.paths.output_model_dir)
     out_dir.mkdir(parents=True, exist_ok=True)
     rec.write_binary(out_dir)
+    if want_normals:
+        sparse_pts = [rec.points3D[pid] for pid in sorted(rec.points3D)]
+        sp_xyz = np.array([p.xyz for p in sparse_pts], np.float64).reshape(-1, 3)
+        sp_rgb = np.array([p.color for p in sparse_pts], np.uint8).reshape(-1, 3)
+        Path(config.paths.output_ply).parent.mkdir(parents=True, exist_ok=True)
+        write_ply(config.paths.output_ply, np.concatenate([sp_xyz, pts_out]), np.concatenate([np.zeros_like(sp_xyz), nrm_out]),
+                  np.concatenate([sp_rgb, col_out]))
     timings["write"] = time.time() - t0
     timings["total"] = time.time() - t_total
     print(f"Saved model with {rec.num_points3D()} points to {out_dir} (total {timings['total']:.2f}s)")
-    out = DensifyOutput(rec, pts_out, col_out, n_candidates, views, timings)
+    out = DensifyOutput(rec, pts_out, col_out, n_candidates, views, timings, normals=nrm_out)
     if return_candidates:
         valid = res.votes != 255
         out.candidates = res.xyz[valid].double().cpu().numpy()

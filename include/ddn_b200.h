@@ -329,6 +329,33 @@ DDN_API int ddn_pchip_apply(int64_t height, int64_t width, const float* depth, c
                     float* refined, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Oriented normals (new; the reference reads the normal maps only for the grazing gate and drops them).
+ * PER-POINT NORMAL of grid point (x, y) of view v, pixel (x s, y s) for stride s (the integer pixel K4 back-projects):
+ *   n_c = the camera-frame normal of the map at that pixel, as given;  w = R_v^T n_c;  n = w / (|w| + 1e-8)
+ *   (oracle/restatement_masks.py:transform_normals, the formula of normals_in_world);  n is negated when
+ *   n_c . ((x s - cx) / fx, (y s - cy) / fy, 1) > 0, so every normal faces its camera;  a normal with a non-finite
+ *   component, and every grid point without a point (votes == 255), is (0, 0, 0).  Computed in float32 for every
+ *   point, kept or not.
+ * FUSED NORMAL of a voxel (the *_normals forms of the fusion calls): every participating point adds
+ *   q = rint(n * 2^20) per component (round half to even, exact product) to three more 64-bit two's-complement sums,
+ *   so the accumulator is 8 words (64 bytes) per voxel; |sum| <= 2^44 below the 2^24-point limit (counts[0] = -1).
+ *   The voxel's normal is sum / |sum| in float64, |sum| = sqrt((x^2 + y^2) + z^2), rounded to float32; (0, 0, 0) when
+ *   the sum is 0.  The sums are integers, so the dense, hashed and host-grid forms give the same bits.  The input
+ *   normals must have components in [-1, 1] (as ddn_point_normals writes them).
+ * ------------------------------------------------------------------------------------------ */
+/* normal [V,H,W,3] f32 (device or pinned host memory), cam_from_world [V,3,4] f64, intr [V,4] f64 (fx, fy, cx, cy),
+ * votes [V,Hs,Ws] u8 (ddn_backproject_filter's, Hs = ceil(H / stride), Ws = ceil(W / stride)) -> normal_out
+ * [V * Hs * Ws, 3] f32, in the order of xyz. */
+DDN_API int ddn_point_normals(int64_t n_views, int64_t height, int64_t width, int32_t stride, const float* normal,
+                      const double* cam_from_world, const double* intr, const uint8_t* votes, float* normal_out,
+                      void* stream);
+/* The same for the views of a ragged layout: normal flat [total pixels, 3], votes [total grid points],
+ * normal_out [total grid points, 3]; the stride is the layout's. */
+DDN_API int ddn_point_normals_ragged(int64_t n_views, const int64_t* layout, const int64_t* layout_host,
+                             const float* normal, const double* cam_from_world, const double* intr,
+                             const uint8_t* votes, float* normal_out, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Stage 4 - voxel-grid fusion (new capability; the reference only concatenates,
  * scripts/test.py:353-359).  key = kx | ky<<21 | kz<<42 with k = floor((p - origin)/voxel) in
  * IEEE float32.
@@ -357,6 +384,14 @@ DDN_API int ddn_voxel_fuse(const ddn_voxel_grid* grid_host, int64_t n_points, in
                    const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold,
                    uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb, int32_t* out_count,
                    int64_t* counts_out, void* workspace, int64_t workspace_bytes, void* stream);
+/* ddn_voxel_fuse with fused normals: normal [N,3] f32 per point (ddn_point_normals), out_normal [N,3] f32; the
+ * workspace from ddn_fuse_normals_workspace_bytes (64 B per possible voxel on the dense bitmap). */
+DDN_API int ddn_fuse_normals_workspace_bytes(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t* bytes_out);
+DDN_API int ddn_voxel_fuse_normals(const ddn_voxel_grid* grid_host, int64_t n_points, int64_t row_len, const float* xyz,
+                           const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold, const float* normal,
+                           uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb, int32_t* out_count,
+                           float* out_normal, int64_t* counts_out, void* workspace, int64_t workspace_bytes,
+                           void* stream);
 
 /* Multi-GPU form of stage 4.  ddn_voxel_partials fuses the rank's own points into per-voxel PARTIAL
  * records, keys ascending.  A record is DDN_RECORD_WORDS u64:
@@ -453,6 +488,11 @@ DDN_API int ddn_fuse_finish(const ddn_fuse_session* s, int64_t n_points, int64_t
                     const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold, uint64_t* out_keys,
                     float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t cap_out, void* accum,
                     int64_t accum_bytes, void* stream);
+/* ddn_fuse_finish with fused normals: normal [n_points,3] f32, out_normal [cap_out,3] f32; accum: cap_out * 64 bytes. */
+DDN_API int ddn_fuse_finish_normals(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz,
+                            const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold, const float* normal,
+                            uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb, int32_t* out_count,
+                            float* out_normal, int64_t cap_out, void* accum, int64_t accum_bytes, void* stream);
 /* Rank + accumulate into partial RECORDS [cap_records, DDN_RECORD_WORDS] (keys ascending) and, when the session
  * has one, the tile prefix. */
 DDN_API int ddn_fuse_finish_partial(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz,
@@ -516,6 +556,14 @@ DDN_API int ddn_fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_h
                            int32_t vote_threshold, const float* dedup_xyz, int64_t n_dedup, uint64_t* out_keys,
                            float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t cap_out, void* accum,
                            int64_t accum_bytes, void* stream);
+/* ddn_fuse_finish_hashed with fused normals: normal [n_points,3] f32, out_normal [cap_out,3] f32; accum:
+ * max(cap_out, n_points) * 64 bytes.  The normal forms have no multi-GPU counterpart. */
+DDN_API int ddn_fuse_finish_hashed_normals(const ddn_fuse_session* s, const struct ddn_hash_fuse* hash, int32_t mode,
+                                   int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                                   const uint8_t* votes, int32_t vote_threshold, const float* normal,
+                                   const float* dedup_xyz, int64_t n_dedup, uint64_t* out_keys, float* out_xyz,
+                                   uint8_t* out_rgb, int32_t* out_count, float* out_normal, int64_t cap_out,
+                                   void* accum, int64_t accum_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * The HASHED PATH on several GPUs (one process per GPU, peer memory as for ddn_fuse_merge_peers).  A step enqueues
