@@ -93,6 +93,7 @@ MAX_PEERS = 16
 PAIR_TABLE_FLOATS = 24
 LAYOUT_COLS = 8  # DDN_LAYOUT_COLS
 RECORD_WORDS = 6  # DDN_RECORD_WORDS
+RECORD_NORMAL_WORDS = 10  # DDN_RECORD_NORMAL_WORDS: the partial records of the fused-normal forms
 HASH_SAMPLES = 4096  # DDN_HASH_SAMPLES
 
 # every symbol include/ddn_b200.h declares: name -> (restype, argtypes)
@@ -184,6 +185,7 @@ SYMBOLS = {
     "ddn_voxel_keys": (C.c_int, [C.POINTER(VoxelGrid), _i64, _vp, _vp, _vp]),
     "ddn_fuse_session_sizes": (C.c_int, [_i64] + [C.POINTER(_i64)] * 5),
     "ddn_fuse_merge_scratch_bytes": (C.c_int, [_i64, _i32, _i64, C.POINTER(_i64)]),
+    "ddn_fuse_merge_normals_scratch_bytes": (C.c_int, [_i64, _i32, _i64, C.POINTER(_i64)]),
     "ddn_fuse_session_reset": (C.c_int, [C.POINTER(FuseSession), _vp]),
     "ddn_fuse_begin": (C.c_int, [C.POINTER(FuseSession), C.POINTER(_vp), _i32, C.c_float, _vp]),
     "ddn_fuse_begin_grid": (C.c_int, [C.POINTER(FuseSession), C.POINTER(VoxelGrid), _vp]),
@@ -198,10 +200,16 @@ SYMBOLS = {
         [C.POINTER(FuseSession), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
     ),
     "ddn_fuse_finish_partial": (C.c_int, [C.POINTER(FuseSession), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i64, _vp]),
+    "ddn_fuse_finish_partial_normals": (C.c_int, [C.POINTER(FuseSession), _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _i64, _vp]),
     "ddn_fuse_merge_peers": (
         C.c_int,
         [C.POINTER(FuseSession), _i32, _i32, C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _i64, _vp, _i64,
          _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
+    ),
+    "ddn_fuse_merge_peers_normals": (
+        C.c_int,
+        [C.POINTER(FuseSession), _i32, _i32, C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _i64, _vp, _i64,
+         _vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp],
     ),
     "ddn_hash_fuse_sizes": (C.c_int, [_i64] + [C.POINTER(_i64)] * 5),
     "ddn_hash_fuse_reset": (C.c_int, [C.POINTER(HashFuse), _vp]),
@@ -219,11 +227,22 @@ SYMBOLS = {
         C.c_int,
         [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp],
     ),
+    "ddn_fuse_finish_hashed_partial_normals": (
+        C.c_int,
+        [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _i64,
+         _vp],
+    ),
     "ddn_fuse_merge_hashed_scratch_bytes": (C.c_int, [_i32, _i64, C.POINTER(_i64)]),
+    "ddn_fuse_merge_hashed_normals_scratch_bytes": (C.c_int, [_i32, _i64, C.POINTER(_i64)]),
     "ddn_fuse_merge_hashed_peers": (
         C.c_int,
         [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i32, C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _i64, _vp, _vp, _vp, _vp,
          _i64, _vp],
+    ),
+    "ddn_fuse_merge_hashed_peers_normals": (
+        C.c_int,
+        [C.POINTER(FuseSession), C.POINTER(HashFuse), _i32, _i32, C.POINTER(_vp), C.POINTER(_vp), _vp, _vp, _i64, _vp, _vp, _vp, _vp,
+         _vp, _i64, _vp],
     ),
 }
 

@@ -32,9 +32,10 @@
 namespace ddn {
 
 constexpr int kAccWords = 5;  // sx, sy, sz, r:g, b:count (u64 each)
-// Partial-sum RECORD exchanged between ranks: {key, sx, sy, sz, r:g, b:count} = DDN_RECORD_WORDS u64.  In
-// partial mode the accumulators ARE words 1..5 of the output records (stride 6), so there is no
-// finalisation pass and a destination's share of the sorted records is one contiguous slice.
+// Partial-sum RECORD exchanged between ranks: {key, sx, sy, sz, r:g, b:count} = DDN_RECORD_WORDS u64 (Record<kW> in
+// fuse_common.cuh; the fused-normal form adds the three normal sums and a zero word).  In partial mode the
+// accumulators ARE words 1.. of the output records (stride kW), so there is no finalisation pass and a destination's
+// share of the sorted records is one contiguous slice.
 constexpr int kRecWords = DDN_RECORD_WORDS;
 static_assert(kRecWords == kAccWords + 1, "record = key + accumulators");
 constexpr uint64_t kDenseMaxCells = 1ull << 35;  // 5.7 GB of units
@@ -837,10 +838,13 @@ merge_clear_kernel(FuseDev f, const long long* __restrict__ plan) {
 // The shares are walked in rotated rank order, so every rank reads a different peer at any time.
 // Work is proportional to the records, which the cuts balance - the unit-driven occupancy merge this replaces cost
 // the owner of a sparse key range three times what the others paid (profiles/README.md, round 2).
+// merge_pull_mark_normals_kernel is the same loop over the 80-byte records of the fused-normal form (five requests per
+// warp step).  Each form spells the loop out: behind a shared inline body the plain form no longer compiled to the same
+// instructions.
 __global__ void __launch_bounds__(256)
 merge_pull_mark_kernel(FuseDev f, PeerPtrs peer_records, int rank, int R, const long long* __restrict__ plan,
                        ulonglong2* __restrict__ staging, long long cap) {
-  __shared__ ulonglong2 s_rec[8][96];  // per warp: 32 records x 48 bytes
+  __shared__ ulonglong2 s_rec[8][16 * DDN_RECORD_WORDS];  // per warp: 32 records
   const GridDev g = *f.grid;
   if (g.n_units == 0) return;
   const long long total = min(plan[2], cap);
@@ -848,7 +852,27 @@ merge_pull_mark_kernel(FuseDev f, PeerPtrs peer_records, int rank, int R, const 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long n_warps = (long long)gridDim.x * 8;
   for (long long w0 = ((long long)blockIdx.x * 8 + warp) * 32; w0 < total; w0 += n_warps * 32) {
-    const unsigned long long key = pull_share_warp(peer_records, rank, R, plan, staging, w0, total, s_rec[warp], lane);
+    const unsigned long long key = pull_share_warp<DDN_RECORD_WORDS>(peer_records, rank, R, plan, staging, w0, total, s_rec[warp], lane);
+    uint64_t cell = cell_of_key(g, key);
+    if (cell < cell_begin || cell >= cell_end) cell = kNoCell;
+    uint64_t left = __shfl_up_sync(0xffffffffu, cell, 1);
+    if (lane == 0) left = kNoCell;
+    if (cell != kNoCell) set_cell_bit(f.units, f.dirty, cell, left);
+  }
+}
+
+__global__ void __launch_bounds__(256, DDN_PULL_CTAS_PER_SM)  // 32 registers, as the plain form (40 without the bound: 6 CTAs per SM)
+merge_pull_mark_normals_kernel(FuseDev f, PeerPtrs peer_records, int rank, int R, const long long* __restrict__ plan,
+                               ulonglong2* __restrict__ staging, long long cap) {
+  __shared__ ulonglong2 s_rec[8][16 * DDN_RECORD_NORMAL_WORDS];  // per warp: 32 records
+  const GridDev g = *f.grid;
+  if (g.n_units == 0) return;
+  const long long total = min(plan[2], cap);
+  const uint64_t cell_begin = (uint64_t)plan[0] * kOwnUnits * kUnitBits, cell_end = (uint64_t)plan[1] * kOwnUnits * kUnitBits;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const long long n_warps = (long long)gridDim.x * 8;
+  for (long long w0 = ((long long)blockIdx.x * 8 + warp) * 32; w0 < total; w0 += n_warps * 32) {
+    const unsigned long long key = pull_share_warp<DDN_RECORD_NORMAL_WORDS>(peer_records, rank, R, plan, staging, w0, total, s_rec[warp], lane);
     uint64_t cell = cell_of_key(g, key);
     if (cell < cell_begin || cell >= cell_end) cell = kNoCell;
     uint64_t left = __shfl_up_sync(0xffffffffu, cell, 1);
@@ -911,28 +935,42 @@ merge_prefix_kernel(FuseDev f, const long long* __restrict__ plan, const uint32_
   }
 }
 
-// the staged records (local memory now) are looked up in the merged units and added with 64-bit REDs
-__global__ void __launch_bounds__(256)
-merge_accumulate_kernel(FuseDev f, const long long* __restrict__ plan, const ulonglong2* __restrict__ staging, long long cap_records,
-                        unsigned long long* __restrict__ accum, long long cap) {
+// the staged records (local memory now) are looked up in the merged units and added with 64-bit REDs: the kSums words
+// of a record into an accumulator of kSums words (kAccWords; kAccNormalWords for the fused-normal records)
+template <int kW>
+__device__ __forceinline__ void merge_accumulate_body(FuseDev f, const long long* __restrict__ plan, const ulonglong2* __restrict__ staging,
+                                                      long long cap_records, unsigned long long* __restrict__ accum, long long cap) {
+  constexpr int kP = Record<kW>::kPieces, kSums = Record<kW>::kSums;
   const GridDev g = *f.grid;
   if (g.n_units == 0) return;
   const long long total = min(plan[2], cap_records);
   const uint4* units = reinterpret_cast<const uint4*>(f.units);
   const uint64_t cell_begin = (uint64_t)plan[0] * kOwnUnits * kUnitBits, cell_end = (uint64_t)plan[1] * kOwnUnits * kUnitBits;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const ulonglong2 a = __ldg(staging + i * 3), b = __ldg(staging + i * 3 + 1), c = __ldg(staging + i * 3 + 2);
-    const uint64_t cell = cell_of_key(g, a.x);
+    ulonglong2 v[kP];
+#pragma unroll
+    for (int k = 0; k < kP; ++k) v[k] = __ldg(staging + i * kP + k);
+    const uint64_t cell = cell_of_key(g, v[0].x);
     if (cell == kNoCell || cell < cell_begin || cell >= cell_end) continue;
     const uint32_t slot = slot_of_cell(cell, units);
     if ((long long)slot >= cap) continue;
-    unsigned long long* o = accum + (size_t)slot * kAccWords;
-    atomicAdd(o + 0, a.y);
-    atomicAdd(o + 1, b.x);
-    atomicAdd(o + 2, b.y);
-    atomicAdd(o + 3, c.x);
-    atomicAdd(o + 4, c.y);
+    unsigned long long* o = accum + (size_t)slot * kSums;
+#pragma unroll
+    for (int q = 0; q < kSums; ++q) atomicAdd(o + q, record_word(v, q + 1));
   }
+}
+
+__global__ void __launch_bounds__(256)
+merge_accumulate_kernel(FuseDev f, const long long* __restrict__ plan, const ulonglong2* __restrict__ staging, long long cap_records,
+                        unsigned long long* __restrict__ accum, long long cap) {
+  static_assert(Record<DDN_RECORD_WORDS>::kSums == kAccWords, "record = key + accumulators");
+  merge_accumulate_body<DDN_RECORD_WORDS>(f, plan, staging, cap_records, accum, cap);
+}
+
+__global__ void __launch_bounds__(256)
+merge_accumulate_normals_kernel(FuseDev f, const long long* __restrict__ plan, const ulonglong2* __restrict__ staging, long long cap_records,
+                                unsigned long long* __restrict__ accum, long long cap) {
+  merge_accumulate_body<DDN_RECORD_NORMAL_WORDS>(f, plan, staging, cap_records, accum, cap);
 }
 
 // ---- host side ---------------------------------------------------------------------------------
@@ -1223,6 +1261,109 @@ static int fuse_finish(const ddn_fuse_session* s, int64_t n_points, int64_t row_
   return launch_finalize(s, acc, out_keys, cap_out, out_xyz, out_rgb, out_count, st, out_normal);
 }
 
+// ddn_fuse_merge_scratch_bytes for records of rec_words u64: staging [cap_out records], then the gathered tile prefixes
+static int merge_scratch_bytes(int64_t cap_units, int32_t n_ranks, int64_t cap_out, int rec_words, int64_t* bytes_out) {
+  DDN_REQUIRE(bytes_out != nullptr && cap_units > 0 && n_ranks >= 1 && n_ranks <= DDN_MAX_PEERS && cap_out > 0, "arguments");
+  const int64_t stride = cap_units / kOwnUnits + 2;
+  *bytes_out = align_up(cap_out * rec_words * 8, 256) + (int64_t)(n_ranks + 1) * stride * 4 + 256;
+  return DDN_OK;
+}
+
+// ddn_fuse_finish_partial, and with `normals` its normals form: records of DDN_RECORD_NORMAL_WORDS u64, whose zeroed
+// pad word the accumulate pass never touches
+static int fuse_finish_partial(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                               const uint8_t* votes, int32_t vote_threshold, const float* normal, bool normals, uint64_t* records,
+                               int64_t cap_records, cudaStream_t st) {
+  const int w = normals ? DDN_RECORD_NORMAL_WORDS : kRecWords;
+  DDN_TRY(session_check(s));
+  DDN_REQUIRE(n_points >= 0 && n_points < (1ll << 31) - 1024, "n_points");
+  DDN_REQUIRE(row_len >= 0, "row_len");
+  DDN_REQUIRE(cap_records > 0 && cap_records < (1ll << 31), "cap_records");
+  DDN_REQUIRE(records != nullptr && (uintptr_t)records % 16 == 0, "records must be 16-byte aligned");
+  DDN_REQUIRE(n_points == 0 || (xyz && rgb), "null pointer");
+  DDN_REQUIRE(!normals || n_points == 0 || normal != nullptr, "null pointer");
+  vote_threshold = std::min(vote_threshold, 255);
+  unsigned long long* rec = (unsigned long long*)records;
+  DDN_TRY(launch_rank(s, ScanRange{0, -1}, (uint64_t*)rec, w, rec, w, cap_records, s->tile_prefix, st));
+  if (n_points == 0) return DDN_OK;
+  return launch_accumulate_points(s, n_points, row_len, xyz, rgb, votes, vote_threshold, rec + 1, w, cap_records, st,
+                                  normals ? normal : nullptr);
+}
+
+// ddn_fuse_merge_peers, and with `normals` its normals form (records of DDN_RECORD_NORMAL_WORDS u64, accumulators of
+// kAccNormalWords, out_normal)
+static int merge_peers(const ddn_fuse_session* s, int32_t rank, int32_t n_ranks, const void* const* peer_records_host,
+                       const void* const* peer_tile_prefix_host, int64_t* plan, void* scratch, int64_t scratch_bytes, const float* drop_xyz,
+                       int64_t n_drop, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb, int32_t* out_count, float* out_normal,
+                       bool normals, int64_t cap_out, void* accum, int64_t accum_bytes, cudaStream_t st) {
+  const int words = normals ? kAccNormalWords : kAccWords;
+  const int rec_words = normals ? DDN_RECORD_NORMAL_WORDS : kRecWords;
+  DDN_REQUIRE(n_drop >= 0 && n_drop < (1ll << 31) - 1024 && (n_drop == 0 || drop_xyz != nullptr), "drop points");
+  DDN_TRY(session_check(s));
+  DDN_REQUIRE(n_ranks >= 1 && n_ranks <= DDN_MAX_PEERS && rank >= 0 && rank < n_ranks, "rank / n_ranks");
+  DDN_REQUIRE(peer_records_host && peer_tile_prefix_host && plan && scratch, "null pointer");
+  DDN_REQUIRE(cap_out > 0 && cap_out < (1ll << 31), "cap_out");
+  DDN_REQUIRE(out_keys && out_xyz && out_rgb && out_count && accum, "null pointer");
+  DDN_REQUIRE(!normals || out_normal != nullptr, "null pointer");
+  DDN_REQUIRE(accum_bytes >= cap_out * words * 8 + 16 && (uintptr_t)accum % 16 == 0,
+              normals ? "accumulator scratch (cap_out * 64 bytes)" : "accumulator scratch");
+  int64_t need = 0;
+  DDN_TRY(merge_scratch_bytes(s->cap_units, n_ranks, cap_out, rec_words, &need));
+  DDN_REQUIRE(scratch_bytes >= need && (uintptr_t)scratch % 16 == 0,
+              normals ? "merge scratch too small (ddn_fuse_merge_normals_scratch_bytes)" : "merge scratch too small (ddn_fuse_merge_scratch_bytes)");
+  PeerPtrs pr, pp;
+  for (int q = 0; q < DDN_MAX_PEERS; ++q) {
+    pr.p[q] = q < n_ranks ? peer_records_host[q] : nullptr;
+    pp.p[q] = q < n_ranks ? peer_tile_prefix_host[q] : nullptr;
+    if (q < n_ranks) DDN_REQUIRE(pr.p[q] && pp.p[q], "null peer pointer");
+  }
+  if (normals)
+    for (int q = 0; q < n_ranks; ++q) DDN_REQUIRE((uintptr_t)pr.p[q] % 16 == 0, "records must be 16-byte aligned");
+  DDN_REQUIRE(pp.p[rank] == (const void*)s->tile_prefix, "entry `rank` must be the session's own buffers");
+  const GridDev* gp = reinterpret_cast<const GridDev*>(s->grid);
+  const FuseDev f = fuse_dev(s);
+  unsigned long long* counts = reinterpret_cast<unsigned long long*>(s->counts);
+  long long* planll = reinterpret_cast<long long*>(plan);
+  unsigned long long* acc = (unsigned long long*)accum;
+  const long long stride = (long long)(s->cap_units / kOwnUnits + 2);
+  ulonglong2* staging = reinterpret_cast<ulonglong2*>(scratch);                                         // [cap_out] records
+  uint32_t* local = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(scratch) + align_up(cap_out * rec_words * 8, 256));  // [(R + 1) * stride]
+  merge_gather_prefix_kernel<<<kNumSMs * 2, 256, 0, st>>>(gp, pp, n_ranks, local, stride);
+  DDN_TRY(after_launch("merge_gather_prefix_kernel", st));
+  merge_plan_kernel<<<1, 32, 0, st>>>(gp, local, stride, rank, n_ranks, planll);
+  DDN_TRY(after_launch("merge_plan_kernel", st));
+  merge_clear_kernel<<<kPersistentCtas, kOwnUnits, 0, st>>>(f, planll);
+  DDN_TRY(after_launch("merge_clear_kernel", st));
+  // (fewer CTAs per SM, to leave room for another stream's kernels, cost the pull 3-14 % on 2 GPUs: -DDDN_PULL_CTAS_PER_SM)
+  if (normals) {
+    merge_pull_mark_normals_kernel<<<kNumSMs * DDN_PULL_CTAS_PER_SM, 256, 0, st>>>(f, pr, rank, n_ranks, planll, staging, cap_out);
+    DDN_TRY(after_launch("merge_pull_mark_normals_kernel", st));
+  } else {
+    merge_pull_mark_kernel<<<kNumSMs * DDN_PULL_CTAS_PER_SM, 256, 0, st>>>(f, pr, rank, n_ranks, planll, staging, cap_out);
+    DDN_TRY(after_launch("merge_pull_mark_kernel", st));
+  }
+  if (n_drop > 0) {  // N5: the cells of the sparse cloud leave the merged occupancy
+    unmark_points_kernel<<<(unsigned)((n_drop + 255) / 256), 256, 0, st>>>(f, n_drop, drop_xyz, planll);
+    DDN_TRY(after_launch("unmark_points_kernel", st));
+  }
+  merge_count_kernel<<<kPersistentCtas, kOwnUnits, 0, st>>>(f, planll, s->tile_sums);
+  DDN_TRY(after_launch("merge_count_kernel", st));
+  tile_scan_kernel<<<1, 1024, 0, st>>>(gp, ScanRange{0, 0}, planll, s->tile_sums, counts);
+  DDN_TRY(after_launch("tile_scan_kernel", st));
+  zero_accum_kernel<<<kPersistentCtas, 256, 0, st>>>((ulonglong2*)acc, counts, words, cap_out);
+  DDN_TRY(after_launch("zero_accum_kernel", st));
+  merge_prefix_kernel<<<kPersistentCtas, kOwnUnits, 0, st>>>(f, planll, s->tile_sums, out_keys, cap_out);
+  DDN_TRY(after_launch("merge_prefix_kernel", st));
+  if (normals) {
+    merge_accumulate_normals_kernel<<<kPersistentCtas, 256, 0, st>>>(f, planll, staging, cap_out, acc, cap_out);
+    DDN_TRY(after_launch("merge_accumulate_normals_kernel", st));
+  } else {
+    merge_accumulate_kernel<<<kPersistentCtas, 256, 0, st>>>(f, planll, staging, cap_out, acc, cap_out);
+    DDN_TRY(after_launch("merge_accumulate_kernel", st));
+  }
+  return launch_finalize(s, acc, out_keys, cap_out, out_xyz, out_rgb, out_count, st, normals ? out_normal : nullptr);
+}
+
 }  // namespace ddn
 
 extern "C" {
@@ -1402,11 +1543,11 @@ int ddn_fuse_session_sizes(int64_t max_cells, int64_t* cap_units, int64_t* units
 }
 
 int ddn_fuse_merge_scratch_bytes(int64_t cap_units, int32_t n_ranks, int64_t cap_out, int64_t* bytes_out) {
-  using namespace ddn;
-  DDN_REQUIRE(bytes_out != nullptr && cap_units > 0 && n_ranks >= 1 && n_ranks <= DDN_MAX_PEERS && cap_out > 0, "arguments");
-  const int64_t stride = cap_units / kOwnUnits + 2;
-  *bytes_out = align_up(cap_out * kRecWords * 8, 256) + (int64_t)(n_ranks + 1) * stride * 4 + 256;
-  return DDN_OK;
+  return ddn::merge_scratch_bytes(cap_units, n_ranks, cap_out, ddn::kRecWords, bytes_out);
+}
+
+int ddn_fuse_merge_normals_scratch_bytes(int64_t cap_units, int32_t n_ranks, int64_t cap_out, int64_t* bytes_out) {
+  return ddn::merge_scratch_bytes(cap_units, n_ranks, cap_out, DDN_RECORD_NORMAL_WORDS, bytes_out);
 }
 
 int ddn_fuse_session_reset(const ddn_fuse_session* s, void* stream) {
@@ -1482,76 +1623,31 @@ int ddn_fuse_finish_normals(const ddn_fuse_session* s, int64_t n_points, int64_t
 
 int ddn_fuse_finish_partial(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
                             const uint8_t* votes, int32_t vote_threshold, uint64_t* records, int64_t cap_records, void* stream) {
-  using namespace ddn;
-  DDN_TRY(session_check(s));
-  DDN_REQUIRE(n_points >= 0 && n_points < (1ll << 31) - 1024, "n_points");
-  DDN_REQUIRE(row_len >= 0, "row_len");
-  DDN_REQUIRE(cap_records > 0 && cap_records < (1ll << 31), "cap_records");
-  DDN_REQUIRE(records != nullptr && (uintptr_t)records % 16 == 0, "records must be 16-byte aligned");
-  DDN_REQUIRE(n_points == 0 || (xyz && rgb), "null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  vote_threshold = std::min(vote_threshold, 255);
-  unsigned long long* rec = (unsigned long long*)records;
-  DDN_TRY(launch_rank(s, ScanRange{0, -1}, (uint64_t*)rec, kRecWords, rec, kRecWords, cap_records, s->tile_prefix, st));
-  if (n_points == 0) return DDN_OK;
-  return launch_accumulate_points(s, n_points, row_len, xyz, rgb, votes, vote_threshold, rec + 1, kRecWords, cap_records, st);
+  return ddn::fuse_finish_partial(s, n_points, row_len, xyz, rgb, votes, vote_threshold, nullptr, false, records, cap_records,
+                                  (cudaStream_t)stream);
+}
+
+int ddn_fuse_finish_partial_normals(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                                    const uint8_t* votes, int32_t vote_threshold, const float* normal, uint64_t* records,
+                                    int64_t cap_records, void* stream) {
+  return ddn::fuse_finish_partial(s, n_points, row_len, xyz, rgb, votes, vote_threshold, normal, true, records, cap_records,
+                                  (cudaStream_t)stream);
 }
 
 int ddn_fuse_merge_peers(const ddn_fuse_session* s, int32_t rank, int32_t n_ranks, const void* const* peer_records_host,
                          const void* const* peer_tile_prefix_host, int64_t* plan, void* scratch, int64_t scratch_bytes,
                          const float* drop_xyz, int64_t n_drop, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
                          int32_t* out_count, int64_t cap_out, void* accum, int64_t accum_bytes, void* stream) {
-  using namespace ddn;
-  DDN_REQUIRE(n_drop >= 0 && n_drop < (1ll << 31) - 1024 && (n_drop == 0 || drop_xyz != nullptr), "drop points");
-  DDN_TRY(session_check(s));
-  DDN_REQUIRE(n_ranks >= 1 && n_ranks <= DDN_MAX_PEERS && rank >= 0 && rank < n_ranks, "rank / n_ranks");
-  DDN_REQUIRE(peer_records_host && peer_tile_prefix_host && plan && scratch, "null pointer");
-  DDN_REQUIRE(cap_out > 0 && cap_out < (1ll << 31), "cap_out");
-  DDN_REQUIRE(out_keys && out_xyz && out_rgb && out_count && accum, "null pointer");
-  DDN_REQUIRE(accum_bytes >= cap_out * kAccWords * 8 + 16 && (uintptr_t)accum % 16 == 0, "accumulator scratch");
-  int64_t need = 0;
-  DDN_TRY(ddn_fuse_merge_scratch_bytes(s->cap_units, n_ranks, cap_out, &need));
-  DDN_REQUIRE(scratch_bytes >= need && (uintptr_t)scratch % 16 == 0, "merge scratch too small (ddn_fuse_merge_scratch_bytes)");
-  PeerPtrs pr, pp;
-  for (int q = 0; q < DDN_MAX_PEERS; ++q) {
-    pr.p[q] = q < n_ranks ? peer_records_host[q] : nullptr;
-    pp.p[q] = q < n_ranks ? peer_tile_prefix_host[q] : nullptr;
-    if (q < n_ranks) DDN_REQUIRE(pr.p[q] && pp.p[q], "null peer pointer");
-  }
-  DDN_REQUIRE(pp.p[rank] == (const void*)s->tile_prefix, "entry `rank` must be the session's own buffers");
-  cudaStream_t st = (cudaStream_t)stream;
-  const GridDev* gp = reinterpret_cast<const GridDev*>(s->grid);
-  const FuseDev f = fuse_dev(s);
-  unsigned long long* counts = reinterpret_cast<unsigned long long*>(s->counts);
-  long long* planll = reinterpret_cast<long long*>(plan);
-  unsigned long long* acc = (unsigned long long*)accum;
-  const long long stride = (long long)(s->cap_units / kOwnUnits + 2);
-  ulonglong2* staging = reinterpret_cast<ulonglong2*>(scratch);                                         // [cap_out] records
-  uint32_t* local = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(scratch) + align_up(cap_out * kRecWords * 8, 256));  // [(R + 1) * stride]
-  merge_gather_prefix_kernel<<<kNumSMs * 2, 256, 0, st>>>(gp, pp, n_ranks, local, stride);
-  DDN_TRY(after_launch("merge_gather_prefix_kernel", st));
-  merge_plan_kernel<<<1, 32, 0, st>>>(gp, local, stride, rank, n_ranks, planll);
-  DDN_TRY(after_launch("merge_plan_kernel", st));
-  merge_clear_kernel<<<kPersistentCtas, kOwnUnits, 0, st>>>(f, planll);
-  DDN_TRY(after_launch("merge_clear_kernel", st));
-  // (fewer CTAs per SM, to leave room for another stream's kernels, cost the pull 3-14 % on 2 GPUs: -DDDN_PULL_CTAS_PER_SM)
-  merge_pull_mark_kernel<<<kNumSMs * DDN_PULL_CTAS_PER_SM, 256, 0, st>>>(f, pr, rank, n_ranks, planll, staging, cap_out);
-  DDN_TRY(after_launch("merge_pull_mark_kernel", st));
-  if (n_drop > 0) {  // N5: the cells of the sparse cloud leave the merged occupancy
-    unmark_points_kernel<<<(unsigned)((n_drop + 255) / 256), 256, 0, st>>>(f, n_drop, drop_xyz, planll);
-    DDN_TRY(after_launch("unmark_points_kernel", st));
-  }
-  merge_count_kernel<<<kPersistentCtas, kOwnUnits, 0, st>>>(f, planll, s->tile_sums);
-  DDN_TRY(after_launch("merge_count_kernel", st));
-  tile_scan_kernel<<<1, 1024, 0, st>>>(gp, ScanRange{0, 0}, planll, s->tile_sums, counts);
-  DDN_TRY(after_launch("tile_scan_kernel", st));
-  zero_accum_kernel<<<kPersistentCtas, 256, 0, st>>>((ulonglong2*)acc, counts, kAccWords, cap_out);
-  DDN_TRY(after_launch("zero_accum_kernel", st));
-  merge_prefix_kernel<<<kPersistentCtas, kOwnUnits, 0, st>>>(f, planll, s->tile_sums, out_keys, cap_out);
-  DDN_TRY(after_launch("merge_prefix_kernel", st));
-  merge_accumulate_kernel<<<kPersistentCtas, 256, 0, st>>>(f, planll, staging, cap_out, acc, cap_out);
-  DDN_TRY(after_launch("merge_accumulate_kernel", st));
-  return launch_finalize(s, acc, out_keys, cap_out, out_xyz, out_rgb, out_count, st);
+  return ddn::merge_peers(s, rank, n_ranks, peer_records_host, peer_tile_prefix_host, plan, scratch, scratch_bytes, drop_xyz, n_drop,
+                          out_keys, out_xyz, out_rgb, out_count, nullptr, false, cap_out, accum, accum_bytes, (cudaStream_t)stream);
+}
+
+int ddn_fuse_merge_peers_normals(const ddn_fuse_session* s, int32_t rank, int32_t n_ranks, const void* const* peer_records_host,
+                                 const void* const* peer_tile_prefix_host, int64_t* plan, void* scratch, int64_t scratch_bytes,
+                                 const float* drop_xyz, int64_t n_drop, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
+                                 int32_t* out_count, float* out_normal, int64_t cap_out, void* accum, int64_t accum_bytes, void* stream) {
+  return ddn::merge_peers(s, rank, n_ranks, peer_records_host, peer_tile_prefix_host, plan, scratch, scratch_bytes, drop_xyz, n_drop,
+                          out_keys, out_xyz, out_rgb, out_count, out_normal, true, cap_out, accum, accum_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -180,15 +180,28 @@ struct PeerPtrs {
   const void* p[DDN_MAX_PEERS];
 };
 
+// The partial RECORD the ranks exchange (include/ddn_b200.h): kW u64, the key then kSums accumulator words, then zero
+// padding up to a whole number of 16-byte pieces.  kW = DDN_RECORD_WORDS (the five sums) or DDN_RECORD_NORMAL_WORDS
+// (the five sums, the three normal sums and a zero word).  Every kernel that reads or writes records takes kW.
+template <int kW>
+struct Record {
+  static_assert(kW == DDN_RECORD_WORDS || kW == DDN_RECORD_NORMAL_WORDS, "a partial record is 6 or 10 u64");
+  static constexpr int kPieces = kW / 2;                                  // ulonglong2 pieces
+  static constexpr int kSums = kW == DDN_RECORD_WORDS ? 5 : kAccNormalWords;  // words 1 .. kSums
+  static_assert(kW % 2 == 0 && kSums < kW, "record layout");
+};
+
 // One warp's step of the owner-side pull: records w0 .. w0 + 31 of this rank's share, which plan (the layout of
 // merge_plan_kernel, include/ddn_b200.h) lays out as the concatenation of its slices of every rank's sorted records
-// in rotated rank order, are copied from the peers' memory into staging[w0 ...] (DDN_RECORD_WORDS u64 each).  A warp
-// inside one rank's slice (the usual case) moves its 1536 bytes as three fully coalesced 512-byte requests (lane l
-// takes bytes 16 l of each) and re-distributes them through s_rec (this warp's 96 entries of shared memory).
+// in rotated rank order, are copied from the peers' memory into staging[w0 ...] (kW u64 each).  A warp inside one
+// rank's slice (the usual case) moves its 32 * 8 * kW bytes as kW / 2 fully coalesced 512-byte requests (lane l takes
+// bytes 16 l of each) and re-distributes them through s_rec (this warp's 16 * kW entries of shared memory).
 // Returns the key of record w0 + lane, ~0 past the end of the share (total).
+template <int kW>
 __device__ __forceinline__ unsigned long long pull_share_warp(const PeerPtrs& peer_records, int rank, int R, const long long* __restrict__ plan,
                                                               ulonglong2* __restrict__ staging, long long w0, long long total,
                                                               ulonglong2* s_rec, int lane) {
+  constexpr int kP = Record<kW>::kPieces;
   const long long i = w0 + lane;
   const bool in = i < total;
   int kq = 0;
@@ -204,24 +217,33 @@ __device__ __forceinline__ unsigned long long pull_share_warp(const PeerPtrs& pe
   unsigned long long key = ~0ull;
   if (uniform) {
     const long long j0 = __shfl_sync(0xffffffffu, j, 0);
-    const ulonglong2* src = reinterpret_cast<const ulonglong2*>(base + j0 * DDN_RECORD_WORDS);
-    ulonglong2* dst = staging + w0 * 3;
+    const ulonglong2* src = reinterpret_cast<const ulonglong2*>(base + j0 * kW);
+    ulonglong2* dst = staging + w0 * kP;
 #pragma unroll
-    for (int k = 0; k < 3; ++k) {
+    for (int k = 0; k < kP; ++k) {
       const ulonglong2 v = __ldcv(src + k * 32 + lane);
       s_rec[k * 32 + lane] = v;
       dst[k * 32 + lane] = v;
     }
     __syncwarp();
-    key = s_rec[lane * 3].x;
+    key = s_rec[lane * kP].x;
     __syncwarp();
   } else if (in) {
-    const ulonglong2* r = reinterpret_cast<const ulonglong2*>(base + j * DDN_RECORD_WORDS);
-    const ulonglong2 a = __ldcv(r), b = __ldcv(r + 1), c = __ldcv(r + 2);
-    staging[i * 3 + 0] = a, staging[i * 3 + 1] = b, staging[i * 3 + 2] = c;
-    key = a.x;
+    const ulonglong2* r = reinterpret_cast<const ulonglong2*>(base + j * kW);
+    ulonglong2 v[kP];
+#pragma unroll
+    for (int k = 0; k < kP; ++k) v[k] = __ldcv(r + k);
+#pragma unroll
+    for (int k = 0; k < kP; ++k) staging[i * kP + k] = v[k];
+    key = v[0].x;
   }
   return key;
+}
+
+// Word q of a record held as kW / 2 pieces in registers (q a compile-time constant after unrolling).
+template <int kP>
+__device__ __forceinline__ unsigned long long record_word(const ulonglong2 (&v)[kP], int q) {
+  return (q & 1) ? v[q >> 1].y : v[q >> 1].x;
 }
 
 }  // namespace ddn

@@ -139,9 +139,9 @@ class ShardedDensifier:
         # `backend` is the module providing the device ops; the product always uses `ops` (CUDA, no CPU
         # fallback).  Tests inject an object with the same functions to exercise the exchange logic on
         # CPU with the gloo backend.
-        if cfg.fuse_normals:
-            raise ValueError("DensifyConfig.fuse_normals: the multi-GPU form of the fused normals is not built; "
-                             "use DensifyEngine on one GPU")
+        if cfg.fuse_normals and backend is not None:
+            raise ValueError("DensifyConfig.fuse_normals: the multi-GPU form of the fused normals runs on the CUDA device path "
+                             "(peer memory, or one rank), not with an injected backend")
         if backend is None:
             if not torch.cuda.is_available():
                 raise ops.DDNError("ShardedDensifier needs a CUDA device: depthdensifier_b200 has no CPU fallback")
@@ -192,7 +192,8 @@ class ShardedDensifier:
                 # allocate and map both exchange buffers now (collective): a platform without symmetric memory
                 # fails here, on every rank alike, and the collectives take over
                 s_ = cfg.filter.stride
-                self.peer_records_shape = (self._local_max * ((height + s_ - 1) // s_) * ((width + s_ - 1) // s_), 6)
+                width_rec = ops._lib.RECORD_NORMAL_WORDS if cfg.fuse_normals else ops._lib.RECORD_WORDS
+                self.peer_records_shape = (self._local_max * ((height + s_ - 1) // s_) * ((width + s_ - 1) // s_), width_rec)
                 # refined maps and bounding boxes are double-buffered (step parity): a rank may start aligning step i+1
                 # while a peer still pulls its step-i maps, so a step needs no barrier at its start
                 self._parity = 0
@@ -210,6 +211,9 @@ class ShardedDensifier:
                 self.device_path = False
         elif self.device_path and cfg.voxel is not None:
             self._make_session()
+        if cfg.fuse_normals and not self.device_path:
+            raise ValueError("DensifyConfig.fuse_normals: the multi-GPU form of the fused normals needs the peer-memory path "
+                             "(symmetric memory could not be set up); the collective fallback has no fused normals")
 
     def _make_session(self) -> None:
         """Fusion session of this rank; with peers its tile prefix (and the partial records) live in symmetric memory
@@ -235,8 +239,8 @@ class ShardedDensifier:
         # (the hashed merge: its sampled splitters balance the global record count up to hashed_merge_capacity)
         n_max = self._local_max * self.Hs * self.Ws
         self._cap_merge = max(n_max + 24576 * self.world + 1024, ops.hashed_merge_capacity(n_max, self.world))
-        self._merge_out = [ops.new_voxel_outputs(self._cap_merge, self.device), None]  # second set: pipelined host calls
-        self.session.merge_scratch(self.world, self._cap_merge)
+        self._merge_out = [ops.new_voxel_outputs(self._cap_merge, self.device, normals=cfg.fuse_normals), None]  # second set: pipelined host calls
+        self.session.merge_scratch(self.world, self._cap_merge, cfg.fuse_normals)
 
     # -- exchange steps -------------------------------------------------------------------------------
     def _exchange_halo(self, refined_slots: torch.Tensor) -> None:
@@ -362,15 +366,18 @@ class ShardedDensifier:
         xyz, votes, bbox, support = self._halo_and_filter(refined_slots, normal, mark, pair, src, box=box, grid=grid)
         res = ShardResult(refined=refined_slots[: self.n_local], stats=stats, xyz=xyz, votes=votes, vote_threshold=self.thr,
                           bbox=bbox, events=ev, support=support, min_support=cfg.min_support)
+        if cfg.fuse_normals:
+            res.normals = mark("point_normals", lambda: self._point_normals(normal, votes))
         if not fuse:
             return res
         s = cfg.filter.stride
         rgb_s = rgb if s == 1 else rgb[:, ::s, ::s].contiguous()
         if self.device_path:
             drop = self._sparse_for_dedup(sparse_xyz) if cfg.dedup_sparse else None
-            k, x, c, n, counts = mark("voxel_fuse", lambda: self._fuse_device(xyz, rgb_s, votes, mark, drop))
+            k, x, c, n, nrm, counts = mark("voxel_fuse", lambda: self._fuse_device(xyz, rgb_s, votes, mark, drop, normal=res.normals))
             res.session, res.grid, res.hash = self.session, grid, self._hash
             res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = k, x, c, n, counts
+            res.voxel_normal = nrm
             return res
         # collective path: the grid is made on the host from the (all-reduced) box of the kept points
         if grid is None:
@@ -386,6 +393,11 @@ class ShardedDensifier:
             k, x, c, n, counts = mark("voxel_fuse", lambda: self._fuse_sharded(xyz, rgb_s, votes, grid, mark))
         res.grid, res.voxel_keys, res.voxel_xyz, res.voxel_rgb, res.voxel_count, res.counts = grid, k, x, c, n, counts
         return res
+
+    def _point_normals(self, normal, votes):
+        """Oriented world-frame normals of the rank's own grid points, from its own views' normal maps."""
+        n = self.n_local
+        return ops.point_normals(normal, self.poses_slots[:n].contiguous(), self.intr_slots[:n].contiguous(), votes, self.cfg.filter.stride)
 
     def _pair_tables(self):
         return self.ops.build_pair_tables(self.poses_slots, self.intr_slots, self._nbr_full(), 0, self.n_local, self.H, self.W)
@@ -472,7 +484,7 @@ class ShardedDensifier:
 
     def _merge_outputs(self, slot: int):
         if self._merge_out[slot] is None:
-            self._merge_out[slot] = ops.new_voxel_outputs(self._cap_merge, self.device)
+            self._merge_out[slot] = ops.new_voxel_outputs(self._cap_merge, self.device, normals=self.cfg.fuse_normals)
         return self._merge_out[slot]
 
     def _sparse_for_dedup(self, sparse_xyz):
@@ -502,12 +514,14 @@ class ShardedDensifier:
             self._hash = ops.HashFuse(self.device, need)
         return self._hash
 
-    def _fuse_device(self, xyz, rgb, votes, mark=None, drop=None, out_slot: int = 0):
+    def _fuse_device(self, xyz, rgb, votes, mark=None, drop=None, out_slot: int = 0, normal=None):
         """Stage 4 on the device path.  One rank: rank + accumulate + finalise.  R ranks: partial records into
         peer-visible memory, one barrier, then the owner-side merge that reads the peers' units and records over
         NVLink.  Both the dense and the hashed form of each half are enqueued on the same outputs; the device grid
         decides which one runs (the hashed path takes a grid too large for the session's bitmap), so nothing is read
-        back.  Returns persistent output buffers (valid until the next step) and a snapshot of the counts."""
+        back.  ``normal`` (point normals like xyz): the fused-normal forms, whose records carry the three normal sums.
+        Returns persistent output buffers (valid until the next step) - keys, xyz, rgb, count, the voxel normals (None
+        without ``normal``) - and a snapshot of the counts."""
         if mark is None:
             mark = lambda name, fn: fn()
         sess = self.session
@@ -515,31 +529,35 @@ class ShardedDensifier:
         if drop is not None and drop.shape[0] == 0:
             drop = None
         hf = self.hash_fuse(flat[0].shape[0] + (0 if drop is None else drop.shape[0]))
+        nrm = {} if normal is None else {"normal": normal.view(-1, 3)}
+        n_out = 4 if normal is None else 5
         if self.peer is None:
             if drop is not None:
                 sess.unmark_points(drop)
-            out = self.ops.fuse_finish(sess, *flat, self.fthr, row_len=xyz.shape[2])[:4]
-            k, x, c, n, counts = self.ops.fuse_finish_hashed(sess, hf, *flat, self.fthr, row_len=xyz.shape[2], dedup_xyz=drop, out=out)
-            return k, x, c, n, counts.clone()
+            out = self.ops.fuse_finish(sess, *flat, self.fthr, row_len=xyz.shape[2], **nrm)[:n_out]
+            *vox, counts = self.ops.fuse_finish_hashed(sess, hf, *flat, self.fthr, row_len=xyz.shape[2], dedup_xyz=drop, out=out, **nrm)
+            return (*vox[:4], vox[4] if normal is not None else None, counts.clone())
         rec, hdl, _ = self.peer.buffer("records", tuple(self.peer_records_shape), torch.int64)
         samples = self.peer.buffer("hash_samples", (ops._lib.HASH_SAMPLES + 1,), torch.int64)[0]
 
         def partials():
-            self.ops.fuse_finish_partial(sess, *flat, self.fthr, rec, row_len=xyz.shape[2])
+            self.ops.fuse_finish_partial(sess, *flat, self.fthr, rec, row_len=xyz.shape[2], **nrm)
             # N5 on the hashed path: every rank tombstones the cells of all ranks' sparse points, so their points are
             # never sent
-            self.ops.fuse_finish_hashed_partial(sess, hf, *flat, self.fthr, rec, samples, row_len=xyz.shape[2], dedup_xyz=drop)
+            self.ops.fuse_finish_hashed_partial(sess, hf, *flat, self.fthr, rec, samples, row_len=xyz.shape[2], dedup_xyz=drop, **nrm)
+
+        normals = normal is not None
 
         def merge():
             out = self.ops.fuse_merge_peers(sess, self.rank, self.world, self._peer_records, self._peer_prefix, self._plan, self._cap_merge,
-                                            out=self._merge_outputs(out_slot), drop_xyz=drop)[:4]
+                                            out=self._merge_outputs(out_slot), drop_xyz=drop, normals=normals)[:n_out]
             return self.ops.fuse_merge_hashed_peers(sess, hf, self.rank, self.world, self._peer_records, self._peer_samples, self._plan,
-                                                    self._cap_merge, out=out)
+                                                    self._cap_merge, out=out, normals=normals)
 
         mark("fuse_partials", partials)
         hdl.barrier()  # every rank's units, tile prefix, records and samples are complete
-        k, x, c, n, counts = mark("fuse_merge", merge)
-        return k, x, c, n, counts.clone()
+        *vox, counts = mark("fuse_merge", merge)
+        return (*vox[:4], vox[4] if normals else None, counts.clone())
 
     def _nbr_full(self) -> torch.Tensor:
         """Neighbour table padded to n_slots rows (build_pair_tables indexes it by global slot)."""
@@ -666,6 +684,8 @@ class ShardedDensifier:
                    "xyz": torch.empty((cap, 3), dtype=torch.float32).pin_memory(),
                    "rgb": torch.empty((cap, 3), dtype=torch.uint8).pin_memory(),
                    "count": torch.empty(cap, dtype=torch.int32).pin_memory()}
+            if self.cfg.fuse_normals:
+                out["normal"] = torch.empty((cap, 3), dtype=torch.float32).pin_memory()
             st["out"] = out
         return out
 
@@ -731,7 +751,8 @@ class ShardedDensifier:
                                           self._max_sparse, cfg.align, out=refined_slots[c0:c1], **self._box_args(src, box, c0, c1))
             stats.append(s_c)
         with torch.cuda.stream(copy):
-            if normals_in_place and normal.is_pinned():
+            # the fused normals read every valid pixel's normal: the maps are uploaded
+            if normals_in_place and normal.is_pinned() and not cfg.fuse_normals:
                 normal_arg = normal
             else:
                 if st["normal"] is None:
@@ -751,12 +772,13 @@ class ShardedDensifier:
             comp.wait_event(ev_rgb)
             rgb_s = st["rgb"] if s == 1 else st["rgb"][:, ::s, ::s].contiguous()
             drop = self._sparse_for_dedup(st["sparse_xyz"]) if cfg.dedup_sparse else None
+            pn = self._point_normals(normal_arg, votes) if cfg.fuse_normals else None
             # (with peers the merge writes into persistent buffers: each staging set has its own)
-            k, x, c, m, counts = self._fuse_device(xyz, rgb_s, votes, drop=drop, out_slot=hs["next"] ^ 1)
+            k, x, c, m, nrm, counts = self._fuse_device(xyz, rgb_s, votes, drop=drop, out_slot=hs["next"] ^ 1, normal=pn)
             st["small"][:2].copy_(counts, non_blocking=True)
             st["small"][2:10].copy_(self.session.grid.view(torch.int64), non_blocking=True)
             st["small"][10:12].copy_(self._hash.state[:2], non_blocking=True)
-            ticket["fused"] = (k, x, c, m)
+            ticket["fused"] = (k, x, c, m) if nrm is None else (k, x, c, m, nrm)
         elif fuse:
             # collective fallback (host-side grid and plan: it waits for the device on its way)
             bb = self._global_bbox(bbox)
@@ -785,7 +807,7 @@ class ShardedDensifier:
         ticket["done"].synchronize()  # the one wait: the host needs the voxel count to size the download
         if ticket["fused"] is None:
             return out
-        k, x, c, m = ticket["fused"]
+        fused = ticket["fused"]
         small = st["small"]
         n_pts, mv = int(small[0]), int(small[1])
         out["d2h_bytes"] += 16
@@ -805,12 +827,12 @@ class ShardedDensifier:
                 grid.origin[i], grid.bits[i], grid.dims[i] = gs.origin[i], gs.bits[i], gs.dims[i]
         if n_pts < 0:
             raise ops.DDNError("voxel fusion: a voxel collected 2^24 or more points (32-bit colour sums); use a smaller voxel")
-        if mv > k.shape[0]:
-            raise ops.DDNError(f"voxel fusion: {mv} voxels exceed the output capacity {k.shape[0]}")
+        if mv > fused[0].shape[0]:
+            raise ops.DDNError(f"voxel fusion: {mv} voxels exceed the output capacity {fused[0].shape[0]}")
         po = self._pinned_out(st, mv)
         d2h = hs["d2h"]
         with torch.cuda.stream(d2h):
-            for name, t in (("keys", k), ("xyz", x), ("rgb", c), ("count", m)):
+            for name, t in zip(("keys", "xyz", "rgb", "count", "normal"), fused):
                 po[name][:mv].copy_(t[:mv], non_blocking=True)
                 t.record_stream(d2h)
                 out[name] = po[name][:mv]

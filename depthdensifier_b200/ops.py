@@ -623,12 +623,15 @@ class FuseSession:
             g.origin[i], g.bits[i], g.dims[i] = st.origin[i], st.bits[i], st.dims[i]
         return g
 
-    def merge_scratch(self, world: int, cap_out: int) -> torch.Tensor:
-        """Scratch of fuse_merge_peers for ``world`` ranks and ``cap_out`` records (allocated once per session)."""
-        if getattr(self, "_merge_scratch", None) is None or self._merge_scratch[0] != (world, cap_out):
-            nbytes = C.c_int64(0)
-            _lib.check(_lib.load().ddn_fuse_merge_scratch_bytes(self.cap_units, int(world), int(cap_out), C.byref(nbytes)))
-            self._merge_scratch = ((world, cap_out), torch.empty(nbytes.value, dtype=torch.uint8, device=self.device))
+    def merge_scratch(self, world: int, cap_out: int, normals: bool = False) -> torch.Tensor:
+        """Scratch of fuse_merge_peers for ``world`` ranks and ``cap_out`` records (allocated once per session); ``normals``:
+        for the fused-normal records."""
+        key = (world, cap_out, bool(normals))
+        if getattr(self, "_merge_scratch", None) is None or self._merge_scratch[0] != key:
+            lib, nbytes = _lib.load(), C.c_int64(0)
+            sizer = lib.ddn_fuse_merge_normals_scratch_bytes if normals else lib.ddn_fuse_merge_scratch_bytes
+            _lib.check(sizer(self.cap_units, int(world), int(cap_out), C.byref(nbytes)))
+            self._merge_scratch = (key, torch.empty(nbytes.value, dtype=torch.uint8, device=self.device))
         return self._merge_scratch[1]
 
     def accum(self, cap_out: int, words: int = 5) -> torch.Tensor:
@@ -688,13 +691,16 @@ class HashFuse:
         """Raises if the last step overflowed the table (synchronises); with ddn_hash_fuse_sizes' sizing it cannot."""
         check_hash_state(self.state[:2].tolist())
 
-    def merge_scratch(self, world: int, cap_out: int) -> torch.Tensor:
-        """Scratch of fuse_merge_hashed_peers for ``world`` ranks and ``cap_out`` records (allocated once)."""
-        if getattr(self, "_merge_scratch", None) is None or self._merge_scratch[0] != (world, cap_out):
-            nbytes = C.c_int64(0)
-            _lib.check(_lib.load().ddn_fuse_merge_hashed_scratch_bytes(int(world), int(cap_out), C.byref(nbytes)))
+    def merge_scratch(self, world: int, cap_out: int, normals: bool = False) -> torch.Tensor:
+        """Scratch of fuse_merge_hashed_peers for ``world`` ranks and ``cap_out`` records (allocated once); ``normals``: for
+        the fused-normal records."""
+        key = (world, cap_out, bool(normals))
+        if getattr(self, "_merge_scratch", None) is None or self._merge_scratch[0] != key:
+            lib, nbytes = _lib.load(), C.c_int64(0)
+            sizer = lib.ddn_fuse_merge_hashed_normals_scratch_bytes if normals else lib.ddn_fuse_merge_hashed_scratch_bytes
+            _lib.check(sizer(int(world), int(cap_out), C.byref(nbytes)))
             self._merge_scratch = None
-            self._merge_scratch = ((world, cap_out), torch.empty(nbytes.value, dtype=torch.uint8, device=self.device))
+            self._merge_scratch = (key, torch.empty(nbytes.value, dtype=torch.uint8, device=self.device))
         return self._merge_scratch[1]
 
 
@@ -787,19 +793,29 @@ def fuse_finish_hashed(sess: FuseSession, hf: HashFuse, xyz, rgb, votes, vote_th
 
 
 def fuse_finish_hashed_partial(sess: FuseSession, hf: HashFuse, xyz, rgb, votes, vote_threshold: int, records, samples, row_len: int = 0,
-                               dedup_xyz=None, mode: int = 0):
+                               dedup_xyz=None, mode: int = 0, normal=None):
     """Hashed fusion of this rank's points into sorted partial ``records`` [cap, 6] i64 and ``samples``
     [DDN_HASH_SAMPLES + 1] i64 (include/ddn_b200.h: ddn_fuse_finish_hashed_partial); ``mode`` and ``dedup_xyz`` as
-    fuse_finish_hashed.  Returns the session's device counts [2] = (points of this rank, records)."""
+    fuse_finish_hashed.  ``normal`` [N,3] f32 (point_normals): the fused-normal form, ``records`` [cap, 10]
+    (ddn_fuse_finish_hashed_partial_normals).  Returns the session's device counts [2] = (points of this rank, records)."""
     lib = _lib.load()
-    dev = _require_cuda(xyz, rgb, votes, records, samples, dedup_xyz)
+    dev = _require_cuda(xyz, rgb, votes, records, samples, dedup_xyz, normal)
     N = xyz.shape[0]
     assert xyz.dtype == torch.float32 and rgb.dtype == torch.uint8 and tuple(rgb.shape) == (N, 3)
-    assert records.dtype == torch.int64 and records.shape[1] == _lib.RECORD_WORDS and records.is_contiguous()
+    width = _lib.RECORD_WORDS if normal is None else _lib.RECORD_NORMAL_WORDS
+    assert records.dtype == torch.int64 and records.shape[1] == width and records.is_contiguous()
     assert samples.dtype == torch.int64 and samples.numel() >= _lib.HASH_SAMPLES + 1
     assert dedup_xyz is None or (dedup_xyz.dtype == torch.float32 and dedup_xyz.dim() == 2 and dedup_xyz.shape[1] == 3)
-    acc = sess.accum(max(N, 1))
     n_dedup = 0 if dedup_xyz is None else dedup_xyz.shape[0]
+    if normal is not None:
+        _check_normal(normal, N)
+        acc = sess.accum(max(N, 1), 8)
+        with torch.cuda.device(dev):
+            _lib.check(lib.ddn_fuse_finish_hashed_partial_normals(
+                C.byref(sess.c), C.byref(hf.c), int(mode), N, int(row_len), _p(xyz), _p(rgb), _p(votes), int(vote_threshold), _p(normal),
+                _p(dedup_xyz), n_dedup, _p(records), records.shape[0], _p(samples), _p(acc), acc.numel(), _stream()))
+        return sess.counts
+    acc = sess.accum(max(N, 1))
     with torch.cuda.device(dev):
         _lib.check(lib.ddn_fuse_finish_hashed_partial(C.byref(sess.c), C.byref(hf.c), int(mode), N, int(row_len), _p(xyz), _p(rgb), _p(votes),
                                                       int(vote_threshold), _p(dedup_xyz), n_dedup, _p(records), records.shape[0],
@@ -808,16 +824,25 @@ def fuse_finish_hashed_partial(sess: FuseSession, hf: HashFuse, xyz, rgb, votes,
 
 
 def fuse_merge_hashed_peers(sess: FuseSession, hf: HashFuse, rank: int, world: int, peer_records, peer_samples, plan, cap_out: int,
-                            out=None):
+                            out=None, normals: bool = False):
     """Owner-side merge of the hashed partials over peer memory (include/ddn_b200.h: ddn_fuse_merge_hashed_peers); runs
     when this rank's fuse_finish_hashed_partial ran.  ``peer_*``: per rank, the device address of that rank's records /
     samples as mapped into this process.  ``cap_out`` (<= hf.cap_voxels): hashed_merge_capacity of the largest rank.
-    Returns keys, xyz, rgb, count and the device counts, as fuse_merge_peers."""
+    Returns keys, xyz, rgb, count and the device counts, as fuse_merge_peers.  ``normals``: every rank's records are
+    the fused-normal form (ddn_fuse_merge_hashed_peers_normals); then returns keys, xyz, rgb, count, normal and counts,
+    and ``out`` holds five outputs."""
     lib = _lib.load()
     dev = sess.device
-    k, x, c, n = out if out is not None else new_voxel_outputs(cap_out, dev)
-    scratch = hf.merge_scratch(world, cap_out)
+    scratch = hf.merge_scratch(world, cap_out, normals)
     arr = lambda ptrs: (C.c_void_p * world)(*[int(v) for v in ptrs])
+    if normals:
+        k, x, c, n, nrm = out if out is not None else new_voxel_outputs(cap_out, dev, normals=True)
+        with torch.cuda.device(dev):
+            _lib.check(lib.ddn_fuse_merge_hashed_peers_normals(C.byref(sess.c), C.byref(hf.c), int(rank), int(world), arr(peer_records),
+                                                               arr(peer_samples), _p(plan), _p(scratch), scratch.numel(), _p(k), _p(x), _p(c),
+                                                               _p(n), _p(nrm), int(cap_out), _stream()))
+        return k, x, c, n, nrm, sess.counts
+    k, x, c, n = out if out is not None else new_voxel_outputs(cap_out, dev)
     with torch.cuda.device(dev):
         _lib.check(lib.ddn_fuse_merge_hashed_peers(C.byref(sess.c), C.byref(hf.c), int(rank), int(world), arr(peer_records),
                                                    arr(peer_samples), _p(plan), _p(scratch), scratch.numel(), _p(k), _p(x), _p(c), _p(n),
@@ -825,11 +850,19 @@ def fuse_merge_hashed_peers(sess: FuseSession, hf: HashFuse, rank: int, world: i
     return k, x, c, n, sess.counts
 
 
-def fuse_finish_partial(sess: FuseSession, xyz, rgb, votes, vote_threshold: int, records, row_len: int = 0):
-    """Rank + accumulate into partial ``records`` [cap, 6] i64 (and the session's tile prefix)."""
+def fuse_finish_partial(sess: FuseSession, xyz, rgb, votes, vote_threshold: int, records, row_len: int = 0, normal=None):
+    """Rank + accumulate into partial ``records`` [cap, 6] i64 (and the session's tile prefix).  ``normal`` [N,3] f32
+    (point_normals): the fused-normal form, ``records`` [cap, 10] (ddn_fuse_finish_partial_normals)."""
     lib = _lib.load()
-    dev = _require_cuda(xyz, rgb, votes, records)
+    dev = _require_cuda(xyz, rgb, votes, records, normal)
     N = xyz.shape[0]
+    if normal is not None:
+        _check_normal(normal, N)
+        assert records.dtype == torch.int64 and records.shape[1] == _lib.RECORD_NORMAL_WORDS
+        with torch.cuda.device(dev):
+            _lib.check(lib.ddn_fuse_finish_partial_normals(C.byref(sess.c), N, int(row_len), _p(xyz), _p(rgb), _p(votes), int(vote_threshold),
+                                                           _p(normal), _p(records), records.shape[0], _stream()))
+        return sess.counts
     assert records.dtype == torch.int64 and records.shape[1] == _lib.RECORD_WORDS
     with torch.cuda.device(dev):
         _lib.check(lib.ddn_fuse_finish_partial(C.byref(sess.c), N, int(row_len), _p(xyz), _p(rgb), _p(votes), int(vote_threshold),
@@ -838,16 +871,27 @@ def fuse_finish_partial(sess: FuseSession, xyz, rgb, votes, vote_threshold: int,
 
 
 def fuse_merge_peers(sess: FuseSession, rank: int, world: int, peer_records, peer_tile_prefix, plan, cap_out: int, out=None,
-                     drop_xyz=None):
+                     drop_xyz=None, normals: bool = False):
     """Owner-side exchange + merge over peer memory.  ``peer_*``: per rank, the device address of that rank's
     records / tile prefix as mapped into this process.  ``drop_xyz`` [n,3] f32: N5, the sparse points of
-    ALL ranks whose cells are removed from the merged occupancy.  Returns keys, xyz, rgb, count, counts."""
+    ALL ranks whose cells are removed from the merged occupancy.  Returns keys, xyz, rgb, count, counts.
+    ``normals``: every rank's records are the fused-normal form (ddn_fuse_merge_peers_normals); then returns keys, xyz,
+    rgb, count, normal and counts, and ``out`` holds five outputs."""
     lib = _lib.load()
     dev = sess.device
+    scratch = sess.merge_scratch(world, cap_out, normals)
+    arr = lambda ptrs: (C.c_void_p * world)(*[int(v) for v in ptrs])
+    if normals:
+        k, x, c, n, nrm = out if out is not None else new_voxel_outputs(cap_out, dev, normals=True)
+        acc = sess.accum(cap_out, 8)
+        with torch.cuda.device(dev):
+            _lib.check(lib.ddn_fuse_merge_peers_normals(C.byref(sess.c), int(rank), int(world), arr(peer_records), arr(peer_tile_prefix),
+                                                        _p(plan), _p(scratch), scratch.numel(), _p(drop_xyz),
+                                                        0 if drop_xyz is None else drop_xyz.shape[0], _p(k), _p(x), _p(c), _p(n), _p(nrm),
+                                                        int(cap_out), _p(acc), acc.numel(), _stream()))
+        return k, x, c, n, nrm, sess.counts
     k, x, c, n = out if out is not None else new_voxel_outputs(cap_out, dev)
     acc = sess.accum(cap_out)
-    scratch = sess.merge_scratch(world, cap_out)
-    arr = lambda ptrs: (C.c_void_p * world)(*[int(v) for v in ptrs])
     with torch.cuda.device(dev):
         _lib.check(lib.ddn_fuse_merge_peers(C.byref(sess.c), int(rank), int(world), arr(peer_records), arr(peer_tile_prefix),
                                             _p(plan), _p(scratch), scratch.numel(), _p(drop_xyz),

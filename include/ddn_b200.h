@@ -402,6 +402,13 @@ DDN_API int ddn_voxel_fuse_normals(const ddn_voxel_grid* grid_host, int64_t n_po
  * records of equal key (any input order, e.g. the concatenation of the runs received from R ranks)
  * and finalises them.  records: [N, DDN_RECORD_WORDS] u64, 16-byte aligned, sized for the worst case. */
 #define DDN_RECORD_WORDS 6
+/* The partial record of the fused-normal forms (the *_normals entry points of the session merges below) is
+ * DDN_RECORD_NORMAL_WORDS u64 = 80 bytes:
+ *   [0..5] as above   [6..8] sum of rint(n * 2^20) per axis of the points' normals (two's complement, as the
+ *   accumulator words 5..7 of ddn_fuse_finish_normals)   [9] 0
+ * The pad word keeps a record a whole number of 16-byte pieces (the peer pull moves 16-byte pieces; a warp's 32
+ * records are five 512-byte requests) and is always written as 0, so records are deterministic bytes. */
+#define DDN_RECORD_NORMAL_WORDS 10
 /* Ownership is by TILE: a tile is cells_per_tile consecutive cells of the grid in key order, so a range of
  * tiles is a key range.  *n_tiles = 0 means the grid is too large for the dense path (no tiles: partition by
  * sampled splitter keys instead). */
@@ -514,6 +521,23 @@ DDN_API int ddn_fuse_merge_peers(const ddn_fuse_session* s, int32_t rank, int32_
                          const void* const* peer_tile_prefix_host, int64_t* plan, void* scratch, int64_t scratch_bytes,
                          const float* drop_xyz, int64_t n_drop, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
                          int32_t* out_count, int64_t cap_out, void* accum, int64_t accum_bytes, void* stream);
+/* The fused-normal forms of the dense multi-GPU step: ddn_fuse_finish_partial_normals writes records
+ * [cap_records, DDN_RECORD_NORMAL_WORDS] (80 bytes: the five sums, the three normal sums of ddn_fuse_finish_normals, a
+ * zero word), from normal [n_points,3] f32 (ddn_point_normals of the rank's own views; no normal map crosses between
+ * ranks).  ddn_fuse_merge_peers_normals merges such records (every rank's, all of that width) as ddn_fuse_merge_peers
+ * does and finalises the normals as ddn_fuse_finish_normals: out_normal [cap_out,3] f32, accum cap_out * 64 bytes,
+ * scratch from ddn_fuse_merge_normals_scratch_bytes (32 bytes per record more than the plain form).  The sums are
+ * integers, so the rank-ordered concatenation of the outputs, normals included, equals ddn_fuse_finish_normals on one
+ * GPU over all points, bit for bit. */
+DDN_API int ddn_fuse_finish_partial_normals(const ddn_fuse_session* s, int64_t n_points, int64_t row_len, const float* xyz,
+                                    const uint8_t* rgb, const uint8_t* votes, int32_t vote_threshold, const float* normal,
+                                    uint64_t* records, int64_t cap_records, void* stream);
+DDN_API int ddn_fuse_merge_normals_scratch_bytes(int64_t cap_units, int32_t n_ranks, int64_t cap_out, int64_t* bytes_out);
+DDN_API int ddn_fuse_merge_peers_normals(const ddn_fuse_session* s, int32_t rank, int32_t n_ranks,
+                                 const void* const* peer_records_host, const void* const* peer_tile_prefix_host, int64_t* plan,
+                                 void* scratch, int64_t scratch_bytes, const float* drop_xyz, int64_t n_drop, uint64_t* out_keys,
+                                 float* out_xyz, uint8_t* out_rgb, int32_t* out_count, float* out_normal, int64_t cap_out,
+                                 void* accum, int64_t accum_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Stage 4 for grids too large for the session's occupancy bitmap: the HASHED PATH (one GPU).  Memory is sized by
@@ -557,7 +581,8 @@ DDN_API int ddn_fuse_finish_hashed(const ddn_fuse_session* s, const struct ddn_h
                            float* out_xyz, uint8_t* out_rgb, int32_t* out_count, int64_t cap_out, void* accum,
                            int64_t accum_bytes, void* stream);
 /* ddn_fuse_finish_hashed with fused normals: normal [n_points,3] f32, out_normal [cap_out,3] f32; accum:
- * max(cap_out, n_points) * 64 bytes.  The normal forms have no multi-GPU counterpart. */
+ * max(cap_out, n_points) * 64 bytes.  The multi-GPU counterparts are ddn_fuse_finish_hashed_partial_normals and
+ * ddn_fuse_merge_hashed_peers_normals below. */
 DDN_API int ddn_fuse_finish_hashed_normals(const ddn_fuse_session* s, const struct ddn_hash_fuse* hash, int32_t mode,
                                    int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
                                    const uint8_t* votes, int32_t vote_threshold, const float* normal,
@@ -604,6 +629,21 @@ DDN_API int ddn_fuse_merge_hashed_peers(const ddn_fuse_session* s, const struct 
                                 const void* const* peer_records_host, const void* const* peer_samples_host, int64_t* plan,
                                 void* scratch, int64_t scratch_bytes, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
                                 int32_t* out_count, int64_t cap_out, void* stream);
+/* The fused-normal forms of the hashed multi-GPU step: records [cap_records, DDN_RECORD_NORMAL_WORDS] (layout at
+ * DDN_RECORD_NORMAL_WORDS) from normal [n_points,3] f32, accum n_points * 64 bytes; the merge of such records finalises
+ * the normals into out_normal [cap_out,3] f32 as ddn_fuse_finish_hashed_normals, with scratch from
+ * ddn_fuse_merge_hashed_normals_scratch_bytes.  Samples, splitters and plan are those of the plain forms. */
+DDN_API int ddn_fuse_finish_hashed_partial_normals(const ddn_fuse_session* s, const struct ddn_hash_fuse* hash, int32_t mode,
+                                           int64_t n_points, int64_t row_len, const float* xyz, const uint8_t* rgb,
+                                           const uint8_t* votes, int32_t vote_threshold, const float* normal,
+                                           const float* dedup_xyz, int64_t n_dedup, uint64_t* records, int64_t cap_records,
+                                           uint64_t* samples, void* accum, int64_t accum_bytes, void* stream);
+DDN_API int ddn_fuse_merge_hashed_normals_scratch_bytes(int32_t n_ranks, int64_t cap_out, int64_t* bytes_out);
+DDN_API int ddn_fuse_merge_hashed_peers_normals(const ddn_fuse_session* s, const struct ddn_hash_fuse* hash, int32_t rank,
+                                        int32_t n_ranks, const void* const* peer_records_host,
+                                        const void* const* peer_samples_host, int64_t* plan, void* scratch,
+                                        int64_t scratch_bytes, uint64_t* out_keys, float* out_xyz, uint8_t* out_rgb,
+                                        int32_t* out_count, float* out_normal, int64_t cap_out, void* stream);
 
 /* Stand-alone pieces of stage 4 (used by the multi-GPU path and by tests). */
 DDN_API int ddn_voxel_keys(const ddn_voxel_grid* grid_host, int64_t n_points, const float* xyz,
